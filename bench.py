@@ -2,7 +2,7 @@
 """bench.py -- VB-MLP train samples/sec on B200 (BASELINE.json metric).
 
   python bench.py --gpus N --steps K --warmup W [--workload c3|c2|c1] [--scaling weak|strong]
-                  [--batch ROWS_PER_GPU] [--impl reference]
+                  [--batch ROWS_PER_GPU] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one minibatch of main.lua:28-40: S x (sample, forward, loss, backward), the gradient exchange
 when N > 1, and the fused KL + Adam update.  Default workload: BASELINE configs[2], the wide VB-MLP
@@ -24,6 +24,12 @@ Prints ONE JSON line (rank 0):
                         read as strong scaling; at N = 8 that is 1024 rows per GPU, the hard regime);
   dp_parity             (N > 1) a short data-parallel-vs-single-GPU parity check run before timing; the run fails
                         if it is not ok.
+Every timed loop runs exactly K minibatches (extra_workloads: 500 unless --steps is given; their warm-up stays 20).
+--dump-outputs DIR (one GPU; DIR must hold no .npy files yet) writes what the last timed minibatch left the caller as DIR/<name>.npy, float32: see
+dump_outputs().  Inputs, initial parameters and noise are seeded, so two builds run with the same arguments can be
+compared array for array.  Compare with a tolerance: fp32 atomics (bias gradients, the loss sum) make two runs of the
+same build differ in the last bits, and bf16 operands carry that forward -- two C3 runs of 10 + 50 minibatches on one
+B200 (1000 W power limit) differed by <= 7e-4 relative (Frobenius norm) per array, 2.3e-3 on the worst log-probability.
 The oracle is only ever the checker / CPU baseline, never the product."""
 import argparse
 import json
@@ -116,6 +122,11 @@ class ClockSampler:
     def stop(self):
         if self.proc:
             self.proc.terminate()
+            try:
+                self.proc.wait(timeout=10)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
 
     def summary(self, t0, t1):
         sm, mx, reasons, pw = [], 0.0, set(), []
@@ -365,8 +376,34 @@ def gemm_algorithmic_bytes(cls, w, N):
     return None
 
 
-def measure(env, args, w, N, steps, warmup, sampler=None, e2e=True):
-    """Time `steps` minibatches of workload w at N rows per GPU.  Returns the measurement dict."""
+DUMP_MAX_ELEMS = 1 << 18                 # per array; keeps a C3 dump near 10 MB
+
+
+def dump_outputs(net, out_dir):
+    """What a caller of train_step holds after the last minibatch: its [error, accuracy], the LogSoftMax outputs of
+    its forward pass ([S x N x classes]) and every layer's updated parameters, as out_dir/<name>.npy in float32.  An
+    array of more than DUMP_MAX_ELEMS elements is flattened and replaced by the elements at a fixed set of indices
+    (seed 0, sorted): the same sample in every run."""
+    import numpy as np
+    import torch
+    from vbnn_b200 import _lib as VL
+    arrays = {"result": net._res, "logp": torch.stack([net.outputs(s) for s in range(net.opt["S"])])}
+    for k, m in enumerate(net.model):
+        if m.kind == VL.KIND_VB:
+            arrays.update({f"layer{k}_means": m.means, f"layer{k}_lvars": m.lvars, f"layer{k}_bias": m.bias})
+        else:
+            arrays.update({f"layer{k}_weight": m.weight, f"layer{k}_bias": m.bias})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
+def measure(env, args, w, N, steps, warmup, sampler=None, e2e=True, dump_dir=None):
+    """Time `steps` minibatches of workload w at N rows per GPU.  Returns the measurement dict.  With dump_dir, the
+    outputs of the last timed minibatch are written there (dump_outputs) before anything else runs on the net."""
     torch = env.torch
     world, rank, ctx = env.world, env.rank, env.ctx
     net, opt = env.make_net(w, N)
@@ -397,6 +434,8 @@ def measure(env, args, w, N, steps, warmup, sampler=None, e2e=True):
     l0 = net.launch_count()
     ms, t_mark0, t_mark1 = timed_region()
     launches = net.launch_count() - l0
+    if dump_dir:
+        dump_outputs(net, dump_dir)
     out = dict(value=steps * N * world / (ms / 1e3), ms_per_step=ms / steps, gpu_launches=launches,
                marks=(t_mark0, t_mark1), per_gpu_batch=N, global_batch=N * world)
     # ---------------- the same K minibatches again with CUDA events around every GEMM / update launch
@@ -589,8 +628,18 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip extra_workloads / strong_scaling / dp_parity")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed minibatch as DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
+    if args.dump_outputs and (args.impl == "reference" or args.gpus != 1 or os.environ.get("WORLD_SIZE", "1") != "1"):
+        ap.error("--dump-outputs needs --impl vbnn on one GPU")
+    # arrays left by an earlier run (another workload has other layers) would pass for this run's
+    if args.dump_outputs and os.path.isdir(args.dump_outputs) and any(
+            f.endswith(".npy") for f in os.listdir(args.dump_outputs)):
+        ap.error(f"--dump-outputs: {args.dump_outputs} already holds .npy files; give an empty or new directory")
+    # extra_workloads time their own (short) minibatches: 500 unless the command line says otherwise
+    extra_steps = 500 if args.steps is None else args.steps
     if args.steps is None:
         args.steps = 3 if args.impl == "reference" else (200 if args.workload == "c3" else 500)
     if args.warmup is None:
@@ -615,9 +664,11 @@ def main():
             sys.exit(1)
 
     sampler = ClockSampler(env.local_rank) if rank == 0 else None
-    m = measure(env, args, w, N, args.steps, args.warmup, sampler, e2e=not args.no_e2e)
-    if sampler:
-        sampler.stop()
+    try:
+        m = measure(env, args, w, N, args.steps, args.warmup, sampler, e2e=not args.no_e2e, dump_dir=args.dump_outputs)
+    finally:                                        # the nvidia-smi poller would outlive a failed run
+        if sampler:
+            sampler.stop()
 
     # ---------------- strong scaling (N > 1): global batch fixed at the workload's 8192 rows ----------------
     strong = None
@@ -651,15 +702,15 @@ def main():
         extra = {}
         for name in ("c1", "c2"):
             wx = WORKLOADS[name]
-            mx = measure(env, args, wx, wx["N"], 500, 20, None, e2e=not args.no_e2e)
+            mx = measure(env, args, wx, wx["N"], extra_steps, 20, None, e2e=not args.no_e2e)
             d = dict(config=config_dict(wx, 1, wx["N"], "weak"), value=mx["value"], unit="samples/s",
-                     ms_per_step=mx["ms_per_step"], steps=500, warmup=20, gpu_launches=mx["gpu_launches"],
+                     ms_per_step=mx["ms_per_step"], steps=extra_steps, warmup=20, gpu_launches=mx["gpu_launches"],
                      dtype="bf16" if wx["precision"] == "bf16" else "f32",
                      step_tflops=flops_per_sample(wx) * wx["N"] / (mx["ms_per_step"] / 1e3) / 1e12)
             for k in ("e2e", "e2e_u8"):
                 if k in mx:
                     d[k] = mx[k]
-            d.update(roofline_objects(mx, wx, wx["N"], 500, peaks))
+            d.update(roofline_objects(mx, wx, wx["N"], extra_steps, peaks))
             if not args.no_cpu_baseline:
                 cpu_baseline(wx)                                        # warm-up (MKL thread pool, page faults)
                 d["cpu_baseline"] = cpu_baseline(wx)

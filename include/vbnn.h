@@ -132,7 +132,8 @@ int vbnn_ctx_synchronize(vbnn_ctx* ctx);
 /* Per-launch device timing of the tensor-core GEMM: CUDA events on the context's stream around
  * every launch, summed per epilogue class (0 store, 1 fwd, 2 fwd-lrt, 3 dx, 4 dx-lrt, 5 dw,
  * 6 dw-lrt) together with the algorithmic flops; class 7 is the fused KL + Adam update, whose
- * "flops" slot holds its algorithmic HBM bytes (56 B per weight).  Enabling it disables graph replay.  This is
+ * "flops" slot holds its algorithmic HBM bytes (56 B per weight); class 8 is vbnn_mlp_predict's averaging
+ * kernel, whose "flops" slot likewise holds bytes.  Enabling it disables graph replay.  This is
  * what bench.py's roofline object is computed from. */
 int vbnn_ctx_profile(vbnn_ctx* ctx, int enable);
 int vbnn_ctx_profile_read(vbnn_ctx* ctx, int cls, double* total_ms, long long* launches, double* flops);
@@ -256,6 +257,26 @@ int vbnn_mlp_join_streams(vbnn_mlp* mlp);
  * else mean over n_samples sampled forward passes (no wasted backward). */
 int vbnn_mlp_test(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, int N,
                   int n_samples, float* err_host, float* acc_host);
+/* Bayesian model average over n_samples sampled forward passes (no backward, no parameter change): the
+ * predictive distribution p-bar(c|x) = (1/T) sum_t softmax(f_t(x)) and its split of uncertainty.
+ * vbnn_mlp_test keeps the reference's semantics (it averages the error and accuracy SCALARS of the T passes);
+ * this is the average of the probabilities.
+ * n_samples == 0: one MAP pass (clamp_to_map, as quicktest).  Samples use the same noise indices as
+ * vbnn_mlp_test ((1 << 20) + t at the current step), so test and predict at one step see the same weights;
+ * the step counter and every optimiser counter stay as they are.
+ * X_dev [N x I0], N <= max_batch.  targets_dev: nullable 1-based [N]; needed when nll_host or acc_host is given.
+ * logp_dev:  nullable [N x C]  log p-bar(c|x) = logsumexp_t logp_t(c|x) - log T
+ * unc_dev:   nullable [N x 4]  {H[p-bar], mean_t H[p_t], max(H[p-bar] - mean_t H[p_t], 0), argmax_c p-bar (1-based)}
+ *            = total, aleatoric and epistemic (mutual information, "BALD") uncertainty, predicted class
+ * nll_host / acc_host: nullable; mean -log p-bar(target) and % argmax p-bar == target; synchronises only if given.
+ * Targets outside 1..C add 0 to the NLL and never count as correct (as the training loss does).
+ * In VBNN_REPARAM_LOCAL mode the activation noise zeta of a row depends on its row index within the call, so a
+ * row's prediction depends on where it sits in X_dev.  Two calls at the same step give bit-identical outputs.
+ * Afterwards vbnn_mlp_get_outputs(s) and VBNN_BUF_WEIGHT hold sample s of the LAST chunk of S samples, as after
+ * vbnn_mlp_test.  In peer mode the preconditions are those of vbnn_mlp_test.  Profile class 8 ("predict") times
+ * the averaging kernel; its flops slot holds 20 algorithmic bytes per (row, class, sample). */
+int vbnn_mlp_predict(vbnn_mlp* mlp, const float* X_dev, int N, int n_samples, const float* targets_dev,
+                     float* logp_dev, float* unc_dev, float* nll_host, float* acc_host);
 /* last forward's LogSoftMax output [N x C] (self.model.output, visualize.lua:97) */
 int vbnn_mlp_get_outputs(vbnn_mlp* mlp, int sample_idx, float* logp_host);
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */

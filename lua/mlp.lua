@@ -2,7 +2,8 @@
 -- libvbnn.so's net-level entry points: the same duck-typed interface main.lua drives
 --   MLP:buildModel(opt), :resetGradients(), :sample(), :run(inputs, targets), :test(input, target),
 --   :calc_lc(opt), :update(opt)
--- plus :train_minibatch(inputs, targets), the whole closure of main.lua:19-51 as ONE call that keeps the
+-- plus :predict(input, nsamples, target), the Bayesian model average with per-row uncertainty,
+-- and :train_minibatch(inputs, targets), the whole closure of main.lua:19-51 as ONE call that keeps the
 -- minibatch, the sampled weights and the noise on the GPU.
 --
 -- NOT EXECUTED IN THIS REPO (no Lua/Torch7 in the image); vbnn_b200/mlp.py makes the same calls in the
@@ -50,6 +51,24 @@ function MLP:test(input, target)                                      -- mlp.lua
    local samples = self.opt.quicktest and 0 or self.opt.testSamples
    V.check(C.vbnn_mlp_test(self.h, V.ptr(input), V.ptr(target), input:size(1), samples, self.err, self.acc))
    return self.err[0], self.acc[0]
+end
+
+-- Bayesian model average over nsamples sampled forward passes (default: test's count, 0 = one MAP pass under
+-- quicktest).  input / target: CudaTensors, target optional.  Returns logp [N x C] = log p-bar, unc [N x 4] =
+-- {H[p-bar], mean_t H[p_t], mutual information, 1-based argmax} as CudaTensors, then nll and accuracy (nil
+-- without a target).  :test keeps the reference's averaged-scalar semantics; this averages the probabilities.
+function MLP:predict(input, nsamples, target)
+   local n = input:size(1)
+   if nsamples == nil then nsamples = self.opt.quicktest and 0 or self.opt.testSamples end
+   local logp = torch.CudaTensor(n, #self.opt.classes)
+   local unc = torch.CudaTensor(n, 4)
+   if target then
+      V.check(C.vbnn_mlp_predict(self.h, V.ptr(input), n, nsamples, V.ptr(target), V.ptr(logp), V.ptr(unc),
+                                 self.err, self.acc))
+      return logp, unc, self.err[0], self.acc[0]
+   end
+   V.check(C.vbnn_mlp_predict(self.h, V.ptr(input), n, nsamples, nil, V.ptr(logp), V.ptr(unc), nil, nil))
+   return logp, unc
 end
 
 function MLP:calc_lc(opt)                                             -- mlp.lua:109-115

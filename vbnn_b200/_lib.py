@@ -92,6 +92,7 @@ _PROTOS = {
     "vbnn_mlp_submit_host_u8": (C.c_int, [_P, _P, _P, C.c_int, C.c_float, C.c_float]),
     "vbnn_mlp_join_streams": (C.c_int, [_P]),
     "vbnn_mlp_test": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _F, _F]),
+    "vbnn_mlp_predict": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _F, _F]),
     "vbnn_mlp_get_outputs": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_mlp_launch_count": (C.c_int, [_P, C.POINTER(C.c_longlong)]),
     "vbnn_mlp_grad_arena": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_size_t)]),

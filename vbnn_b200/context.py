@@ -47,8 +47,10 @@ class Context:
         L.check(L.lib().vbnn_ctx_profile(self.handle, 1 if enable else 0))
 
     def profile_read(self):
-        """{class: (total_ms, launches, flops)} of the tensor-core GEMM launches since profile(True)."""
-        names = ["store", "fwd", "fwd_lrt", "dx", "dx_lrt", "dw", "dw_lrt", "update"]   # update: "flops" = bytes
+        """{class: (total_ms, launches, flops)} of the tensor-core GEMM launches, the fused update and the predict
+        averaging kernel since profile(True)."""
+        names = ["store", "fwd", "fwd_lrt", "dx", "dx_lrt", "dw", "dw_lrt", "update",
+                 "predict"]                                   # update, predict: "flops" = bytes
         out = {}
         for cls, name in enumerate(names):
             ms, n, fl = C.c_double(), C.c_longlong(), C.c_double()

@@ -516,6 +516,94 @@ __global__ void __launch_bounds__(kThreads) k_loss(LossParams p) {
   }
 }
 
+// ------------------------------------------------------------------ predict -------------
+// acc - exp(lp) * lp: one entropy term.  The per-sample and the averaged entropy both use it, so that a
+// one-sample average, whose log p-bar is bitwise logp, has a mutual information of exactly 0.
+__device__ __forceinline__ float sub_plogp(float acc, float lp) { return acc - expf(lp) * lp; }
+
+// One warp per row, like k_loss.  The warp folds the chunk's samples in order z = 0..zc-1 and every sum has a
+// fixed order (no atomics), so two launches on the same logits give the same bits.
+__global__ void __launch_bounds__(kThreads) k_predict(PredictParams p) {
+  const int warps_per_block = blockDim.x >> 5;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const float log_t = logf((float)p.T);
+  const bool reduce = p.last && p.targets;                              // block-uniform
+  double blk_nll = 0.0, blk_corr = 0.0;                                 // thread 0: the block's rows in order
+  __shared__ float sh_nll[kThreads / 32], sh_corr[kThreads / 32];
+  for (long long r0 = (long long)blockIdx.x * warps_per_block; r0 < p.N;
+       r0 += (long long)gridDim.x * warps_per_block) {
+    const long long n = r0 + w;
+    float my_nll = 0.f, my_corr = 0.f;
+    if (n < p.N) {
+      float* smax = p.st_max + n * p.C;
+      float* ssum = p.st_sum + n * p.C;
+      const int tgt = p.targets ? (int)p.targets[n] - 1 : -1;          // 1-based (data.lua:16)
+      float ent = p.first ? 0.f : p.st_ent[n];
+      float hbar = 0.f, best = -3.0e38f, nll = 0.f;
+      int arg = 0x7fffffff;
+      for (int z = 0; z < p.zc; ++z) {
+        const float* x = p.logits + ((long long)z * p.N + n) * p.ld_logits;
+        // lse formed exactly as k_loss forms it: logp_t is bitwise the LogSoftMax that get_outputs returns
+        float mx = -3.0e38f;
+        for (int c = lane; c < p.C; c += 32) mx = fmaxf(mx, x[c]);
+        mx = warp_max(mx);
+        float se = 0.f;
+        for (int c = lane; c < p.C; c += 32) se += __expf(x[c] - mx);
+        se = warp_sum(se);
+        const float lse = mx + __logf(se);
+        const bool init = p.first && z == 0, fin = p.last && z == p.zc - 1;
+        float h = 0.f;
+        for (int c = lane; c < p.C; c += 32) {
+          const float lp = x[c] - lse;
+          h = sub_plogp(h, lp);
+          float m = lp, s = 1.f;
+          if (!init) {
+            m = smax[c]; s = ssum[c];
+            if (lp > m) { s = s * expf(m - lp) + 1.f; m = lp; }
+            else s += expf(lp - m);
+          }
+          if (!fin) { smax[c] = m; ssum[c] = s; continue; }
+          const float lpb = (m + logf(s)) - log_t;                      // log p-bar(c | x)
+          hbar = sub_plogp(hbar, lpb);
+          if (lpb > best) { best = lpb; arg = c; }
+          if (c == tgt) nll = -lpb;
+          if (p.logp_out) p.logp_out[n * p.C + c] = lpb;
+        }
+        ent += warp_sum(h);
+      }
+      if (p.last) {
+        hbar = warp_sum(hbar);
+        nll = warp_sum(nll);                                            // one lane holds the target's term
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {                              // lowest index on ties, as k_loss
+          float ob = __shfl_xor_sync(0xffffffffu, best, o);
+          int oa = __shfl_xor_sync(0xffffffffu, arg, o);
+          if (ob > best || (ob == best && oa < arg)) { best = ob; arg = oa; }
+        }
+        const float e = ent / (float)p.T;
+        if (lane == 0 && p.unc_out) {
+          float* u = p.unc_out + n * 4;
+          u[0] = hbar; u[1] = e; u[2] = fmaxf(hbar - e, 0.f); u[3] = (float)(arg + 1);
+        }
+        if (lane == 0 && reduce) {
+          my_nll = (tgt >= 0 && tgt < p.C) ? nll : 0.f;
+          my_corr = arg == tgt ? 1.f : 0.f;
+        }
+      } else if (lane == 0) {
+        p.st_ent[n] = ent;
+      }
+    }
+    if (reduce) {
+      if (lane == 0) { sh_nll[w] = my_nll; sh_corr[w] = my_corr; }
+      __syncthreads();
+      if (threadIdx.x == 0)
+        for (int k = 0; k < warps_per_block; ++k) { blk_nll += sh_nll[k]; blk_corr += sh_corr[k]; }
+      __syncthreads();
+    }
+  }
+  if (reduce && threadIdx.x == 0) { p.partials[2 * blockIdx.x] = blk_nll; p.partials[2 * blockIdx.x + 1] = blk_corr; }
+}
+
 __global__ void k_finalize_result(const float* acc, int Z, int N, float* out2) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     float e = 0.f, a = 0.f;
@@ -829,6 +917,16 @@ int launch_loss(const LossParams& p, cudaStream_t st) {
   if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
   k_loss<<<(int)blocks, kThreads, 0, st>>>(p);
   VB_CUDA(cudaGetLastError());
+  return VBNN_OK;
+}
+
+int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st) {
+  const int wpb = kThreads / 32;
+  long long blocks = ((long long)p.N + wpb - 1) / wpb;
+  if (blocks > kMaxPartials) blocks = kMaxPartials;
+  k_predict<<<(int)blocks, kThreads, 0, st>>>(p);
+  VB_CUDA(cudaGetLastError());
+  if (grid_out) *grid_out = (int)blocks;
   return VBNN_OK;
 }
 

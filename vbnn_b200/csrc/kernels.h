@@ -106,6 +106,26 @@ struct LossParams {
 };
 int launch_loss(const LossParams& p, cudaStream_t st);
 
+// Bayesian model average over sampled forward passes (vbnn_mlp_predict), one chunk of zc samples per launch.
+// Per (row, class) the state is an online log-sum-exp over samples of logp_t = x_t - lse_t: a running max and
+// the sum of exp(logp_t - max), so log p-bar = max + log(sum) - log T stays finite wherever every logp_t is.
+// Per row it also keeps the sum over samples of the entropies H[p_t].  The first chunk initialises the state,
+// the last one finalises it into the outputs instead of storing it.
+struct PredictParams {
+  const float* logits; int ld_logits;   // [zc*N x ld]
+  int N, C, zc;
+  int first, last;                      // this chunk starts / ends the average
+  int T;                                // samples averaged in all (last chunk)
+  float *st_max, *st_sum;               // [N x C] log-sum-exp state
+  float* st_ent;                        // [N] sum_t H[p_t]
+  float* logp_out;                      // nullable [N x C] log p-bar (last chunk)
+  float* unc_out;                       // nullable [N x 4] {H[p-bar], mean_t H[p_t], mutual information, argmax + 1}
+  const float* targets;                 // nullable [N] 1-based floats (last chunk)
+  double* partials;                     // [grid x 2] per-block {sum nll, #correct} when targets is set
+};
+// returns the grid in *grid_out (the number of partial pairs written)
+int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st);
+
 // gradBias += column sums of G over all rows (nn.Linear:accGradParameters addmv)
 int launch_colsum(const void* G, int is_bf16, long long rows, int cols, int ld, float scale,
                   float* gb, cudaStream_t st);

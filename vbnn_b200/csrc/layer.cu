@@ -309,7 +309,7 @@ int tc_gemm(vbnn_ctx* c, int mode, const TcGemmArgs& g, const EpiParams& p, int 
   vbnn_ctx::ProfRec r;
   VB_TRY(get_event(&r.a));
   VB_TRY(get_event(&r.b));
-  r.cls = prof_cls >= 0 ? prof_cls : mode;
+  r.cls = (prof_cls >= 0 ? prof_cls : mode) & 7;        // GEMM classes 0-7; class 8 is predict (mlp.cu)
   r.flops = 2.0 * g.M * (double)g.N * g.K * g.batch * (epi_is_dual(mode) ? 2.0 : 1.0);
   VB_CUDA(cudaEventRecord(r.a, c->stream));
   int rc = gemm_tc_launch(mode, g, p, c->stream, &c->launches);
@@ -345,7 +345,7 @@ int prof_collect(vbnn_ctx* c) {
   for (auto& r : c->prof_recs) {
     float ms = 0.f;
     VB_CUDA(cudaEventElapsedTime(&ms, r.a, r.b));
-    c->prof_ms[r.cls & 7] += ms; c->prof_flops[r.cls & 7] += r.flops; c->prof_n[r.cls & 7] += 1;
+    c->prof_ms[r.cls] += ms; c->prof_flops[r.cls] += r.flops; c->prof_n[r.cls] += 1;
     c->prof_pool.push_back(r.a); c->prof_pool.push_back(r.b);
   }
   c->prof_recs.clear();
@@ -450,12 +450,12 @@ extern "C" int vbnn_ctx_profile(vbnn_ctx* c, int enable) {
   VB_CHECK(c, VBNN_E_INVALID, "null ctx");
   VB_TRY(prof_collect(c));
   c->profiling = enable != 0;
-  if (enable) for (int i = 0; i < 8; ++i) { c->prof_ms[i] = 0; c->prof_flops[i] = 0; c->prof_n[i] = 0; }
+  if (enable) for (int i = 0; i < vbnn_ctx::kProfClasses; ++i) { c->prof_ms[i] = 0; c->prof_flops[i] = 0; c->prof_n[i] = 0; }
   if (enable) for (int i = 0; i < 16; ++i) { c->phase_ms[i] = 0; c->phase_n[i] = 0; }
   return VBNN_OK;
 }
 extern "C" int vbnn_ctx_profile_read(vbnn_ctx* c, int cls, double* total_ms, long long* launches, double* flops) {
-  VB_CHECK(c && cls >= 0 && cls < 8, VBNN_E_INVALID, "vbnn_ctx_profile_read: bad argument");
+  VB_CHECK(c && cls >= 0 && cls < vbnn_ctx::kProfClasses, VBNN_E_INVALID, "vbnn_ctx_profile_read: bad argument");
   VB_TRY(prof_collect(c));
   if (total_ms) *total_ms = c->prof_ms[cls];
   if (launches) *launches = c->prof_n[cls];

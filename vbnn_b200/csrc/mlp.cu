@@ -502,6 +502,54 @@ int step_enqueue(vbnn_mlp* m, int N) {
   return VBNN_OK;
 }
 
+// The evaluation forward of vbnn_mlp_test and vbnn_mlp_predict (mlp.lua:86-107): stage the input, wait for the
+// peers' parameters, then one MAP pass (n_samples == 0, quicktest) or n_samples sampled passes in chunks of Z whose
+// noise indices (1 << 20) + t never reuse a training sample.  consume(zc, first, last) runs after each chunk.
+template <typename Consume>
+int eval_forward(vbnn_mlp* m, const float* X, const float* T, int N, int n_samples, const char* who,
+                 Consume&& consume) {
+  VB_TRY(stage_input(m, X, T, N));
+  if (m->peer && m->peer->active) {
+    VB_CHECK(n_samples > 0 || !m->peer->stale, VBNN_E_STATE,
+             "%s(quicktest) in peer mode: call vbnn_mlp_sync_replicas on every rank first", who);
+    VB_TRY(peer_wait_params(m, -1, false));
+  }
+  const int Lc = nlayers(m);
+  if (n_samples == 0) {
+    VB_TRY(clamp_all(m));                                                    // mlp.lua:88-90 (quicktest)
+    for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, 1, 0, true));
+    VB_TRY(consume(1, true, true));
+    for (vbnn_layer* L : m->layers) L->map_mode = false;
+    return VBNN_OK;
+  }
+  const int base = 1 << 20;                                                  // test noise never reuses train samples
+  for (int s0 = 0; s0 < n_samples; s0 += m->Z) {                             // mlp.lua:94-100
+    const int zc = n_samples - s0 < m->Z ? n_samples - s0 : m->Z;
+    VB_TRY(sample_all(m, base + s0, zc));
+    for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, zc, base + s0, false));
+    VB_TRY(consume(zc, s0 == 0, s0 + zc == n_samples));
+  }
+  return VBNN_OK;
+}
+
+// launch() under a pair of CUDA events while profiling, accounted to class cls with `work` in its flops slot
+template <typename Launch>
+int prof_launch(vbnn_ctx* c, int cls, double work, Launch&& launch) {
+  if (!c->profiling) return launch();
+  vbnn_ctx::ProfRec r;
+  for (cudaEvent_t* e : {&r.a, &r.b}) {
+    if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); }
+    else VB_CUDA(cudaEventCreate(e));
+  }
+  r.cls = cls; r.flops = work;
+  VB_CUDA(cudaEventRecord(r.a, c->stream));
+  VB_TRY(launch());
+  VB_CUDA(cudaEventRecord(r.b, c->stream));
+  c->prof_recs.push_back(r);
+  if (c->prof_recs.size() + c->marks.size() >= 4096) VB_TRY(prof_collect(c));
+  return VBNN_OK;
+}
+
 }  // namespace
 
 // ============================================================ create / destroy =============
@@ -622,6 +670,10 @@ extern "C" int vbnn_mlp_destroy(vbnn_mlp* m) {
   if (m->dw_partials) cudaFree(m->dw_partials);
   if (m->logits) cudaFree(m->logits);
   if (m->logp) cudaFree(m->logp);
+  if (m->pred_max) cudaFree(m->pred_max);
+  if (m->pred_sum) cudaFree(m->pred_sum);
+  if (m->pred_ent) cudaFree(m->pred_ent);
+  if (m->pred_partials) cudaFree(m->pred_partials);
   if (m->targets) cudaFree(m->targets);
   if (m->result_acc) cudaFree(m->result_acc);
   if (m->result) cudaFree(m->result);
@@ -843,37 +895,68 @@ extern "C" int vbnn_mlp_test(vbnn_mlp* m, const float* X, const float* T, int N,
   VB_CHECK(N > 0 && N <= m->max_batch && n_samples >= 0, VBNN_E_INVALID, "vbnn_mlp_test: bad N/n_samples");
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
-  VB_TRY(stage_input(m, X, T, N));
   VB_CUDA(cudaMemsetAsync(m->result_acc, 0, (size_t)2 * m->Z * 4, st));
-  if (m->peer && m->peer->active) {
-    VB_CHECK(n_samples > 0 || !m->peer->stale, VBNN_E_STATE,
-             "vbnn_mlp_test(quicktest) in peer mode: call vbnn_mlp_sync_replicas on every rank first");
-    VB_TRY(peer_wait_params(m, -1, false));
-  }
-  const int Lc = nlayers(m);
-  int total = 0;
-  if (n_samples == 0) {
-    VB_TRY(clamp_all(m));                                                    // mlp.lua:88-90 (quicktest)
-    for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, 1, 0, true));
-    VB_TRY(loss_all(m, N, 1, false, nullptr, m->result_acc));
-    for (vbnn_layer* L : m->layers) L->map_mode = false;
-    total = 1;
-  } else {
-    const int base = 1 << 20;                                                // test noise never reuses train samples
-    for (int s0 = 0; s0 < n_samples; s0 += m->Z) {                           // mlp.lua:94-100
-      const int zc = n_samples - s0 < m->Z ? n_samples - s0 : m->Z;
-      VB_TRY(sample_all(m, base + s0, zc));
-      for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, zc, base + s0, false));
-      VB_TRY(loss_all(m, N, zc, false, nullptr, m->result_acc));
-    }
-    total = n_samples;
-  }
+  VB_TRY(eval_forward(m, X, T, N, n_samples, "vbnn_mlp_test",
+                      [&](int zc, bool, bool) { return loss_all(m, N, zc, false, nullptr, m->result_acc); }));
+  const int total = n_samples == 0 ? 1 : n_samples;
   VB_CUDA(cudaMemcpyAsync(c->h_scalars, m->result_acc, (size_t)2 * m->Z * 4, cudaMemcpyDeviceToHost, st));
   VB_CUDA(cudaStreamSynchronize(st));
   double e = 0, a = 0;
   for (int z = 0; z < m->Z; ++z) { e += c->h_scalars[2 * z]; a += c->h_scalars[2 * z + 1]; }
   if (err_host) *err_host = (float)(e / ((double)total * N));               // mlp.lua:101
   if (acc_host) *acc_host = (float)(a / ((double)total * N) * 100.0);
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_samples, const float* targets,
+                                float* logp_dev, float* unc_dev, float* nll_host, float* acc_host) {
+  VB_CHECK(m && X, VBNN_E_INVALID, "vbnn_mlp_predict: null argument");
+  VB_CHECK(N > 0 && N <= m->max_batch && n_samples >= 0, VBNN_E_INVALID,
+           "vbnn_mlp_predict: N=%d (max_batch %d), n_samples=%d", N, m->max_batch, n_samples);
+  VB_CHECK(targets || !(nll_host || acc_host), VBNN_E_INVALID, "vbnn_mlp_predict: nll / accuracy need targets");
+  vbnn_ctx* c = m->ctx;
+  cudaStream_t st = c->stream;
+  VB_CUDA(cudaSetDevice(c->device));
+  const int C = m->sizes.back();
+  if (!m->pred_partials) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    VB_CUDA(cudaStreamIsCapturing(st, &cs));
+    VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE,
+             "vbnn_mlp_predict: the first call allocates its state and cannot be captured");
+    for (float** q : {&m->pred_max, &m->pred_sum, &m->pred_ent})
+      if (*q) { cudaFree(*q); *q = nullptr; }
+    VB_TRY(dalloc(&m->pred_max, (size_t)m->max_batch * C * 4));
+    VB_TRY(dalloc(&m->pred_sum, (size_t)m->max_batch * C * 4));
+    VB_TRY(dalloc(&m->pred_ent, (size_t)m->max_batch * 4));
+    VB_TRY(dalloc(&m->pred_partials, (size_t)kMaxPartials * 2 * sizeof(double)));
+  }
+  const bool reduce = nll_host || acc_host;
+  int grid = 0;
+  auto consume = [&](int zc, bool first, bool last) -> int {
+    PredictParams p;
+    memset(&p, 0, sizeof(p));
+    p.logits = m->logits; p.ld_logits = m->ld_logits;
+    p.N = N; p.C = C; p.zc = zc; p.first = first; p.last = last;
+    p.T = n_samples == 0 ? 1 : n_samples;
+    p.st_max = m->pred_max; p.st_sum = m->pred_sum; p.st_ent = m->pred_ent;
+    if (last) {
+      p.logp_out = logp_dev; p.unc_out = unc_dev;
+      p.targets = reduce ? targets : nullptr; p.partials = m->pred_partials;
+    }
+    // profile class 8; its "flops" slot holds the algorithmic bytes: 4 B of logits + 16 B of state read and
+    // write per (row, class, sample)
+    return prof_launch(c, 8, 20.0 * zc * (double)N * C, [&] { return launch_predict(p, &grid, st); });
+  };
+  VB_TRY(eval_forward(m, X, nullptr, N, n_samples, "vbnn_mlp_predict", consume));
+  if (reduce) {
+    VB_CUDA(cudaMemcpyAsync(c->h_partials, m->pred_partials, (size_t)grid * 2 * sizeof(double), cudaMemcpyDeviceToHost,
+                            st));
+    VB_CUDA(cudaStreamSynchronize(st));
+    double nll = 0, corr = 0;
+    for (int b = 0; b < grid; ++b) { nll += c->h_partials[2 * b]; corr += c->h_partials[2 * b + 1]; }   // fixed order
+    if (nll_host) *nll_host = (float)(nll / N);
+    if (acc_host) *acc_host = (float)(corr / N * 100.0);
+  }
   return VBNN_OK;
 }
 

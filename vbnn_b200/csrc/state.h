@@ -19,12 +19,13 @@ struct vbnn_ctx {
   float* h_scalars = nullptr;        // pinned scratch for scalar read-backs
   int next_layer_id = 0;
   long long launches = 0;
-  // per-launch device timing of the tensor-core GEMM (bench.py roofline)
+  // per-launch device timing of the tensor-core GEMM (bench.py roofline), the fused update (7) and predict (8)
+  static constexpr int kProfClasses = 9;
   bool profiling = false;
   struct ProfRec { cudaEvent_t a, b; int cls; double flops; };
   std::vector<ProfRec> prof_recs;
   std::vector<cudaEvent_t> prof_pool;
-  double prof_ms[8] = {0}; double prof_flops[8] = {0}; long long prof_n[8] = {0};
+  double prof_ms[kProfClasses] = {0}; double prof_flops[kProfClasses] = {0}; long long prof_n[kProfClasses] = {0};
   // phase marks of one minibatch (same switch): time from the previous mark to mark `id`
   struct Mark { cudaEvent_t e; int id; };
   std::vector<Mark> marks;
@@ -120,6 +121,10 @@ struct vbnn_mlp {
   float* dw_partials = nullptr;             // fp32 [Z x O x I] of the plain output layer: per-sample dW products (Z > 1)
   float* logits = nullptr; int ld_logits = 0;
   float* logp = nullptr;
+  // vbnn_mlp_predict state, allocated by the first call: log-sum-exp max / sum [max_batch x C], entropy sum
+  // [max_batch], per-block {nll, correct} partials [kMaxPartials x 2]
+  float *pred_max = nullptr, *pred_sum = nullptr, *pred_ent = nullptr;
+  double* pred_partials = nullptr;
   float* targets = nullptr;          // staged targets [N]
   float* xstage[2] = {nullptr, nullptr};   // fp32 H2D staging for the host-buffer API
   float* tstage[2] = {nullptr, nullptr};

@@ -5,11 +5,23 @@ main.lua-style loop drives it unchanged -- plus the fused per-minibatch entry po
 from __future__ import annotations
 
 import ctypes as C
+from typing import NamedTuple, Optional
 
 from . import _lib as L
 from .config import opts_struct
 from .context import Context, as_dev_f32, default_context
 from .vblinear import Linear, VBLinear
+
+
+class Prediction(NamedTuple):
+    """MLP.predict's result: device tensors over the N input rows, and the two scalars when targets were given."""
+    logp: "torch.Tensor"                  # [N x C] log p-bar(c | x)
+    entropy: "torch.Tensor"               # [N] H[p-bar]: total uncertainty
+    expected_entropy: "torch.Tensor"      # [N] mean_t H[p_t]: aleatoric
+    mutual_info: "torch.Tensor"           # [N] H[p-bar] - mean_t H[p_t] (clamped at 0): epistemic, "BALD"
+    label: "torch.Tensor"                 # [N] int64, 1-based argmax of p-bar
+    nll: Optional[float]                  # mean -log p-bar(target)
+    accuracy: Optional[float]             # % argmax p-bar == target
 
 
 class MLP:
@@ -98,6 +110,37 @@ class MLP:
         L.check(L.lib().vbnn_mlp_test(self.handle, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
                                       x.shape[0], ns, C.byref(err), C.byref(acc)))
         return err.value, acc.value
+
+    def predict(self, inputs, n_samples=None, targets=None):
+        """Bayesian model average over n_samples sampled forward passes (vbnn_mlp_predict); test() keeps the
+        reference's averaged error / accuracy scalars, this averages the probabilities.  n_samples defaults to
+        what test() uses: 0 (one MAP pass) under quicktest, else testSamples.  Returns a Prediction of device
+        tensors -- logp [N x C] = log p-bar, entropy H[p-bar], expected_entropy mean_t H[p_t], mutual_info (their
+        difference, clamped at 0), label (1-based argmax of p-bar) -- plus nll / accuracy floats, None without
+        targets.  Parameters, optimiser state and the step counter are left as they are."""
+        import torch
+        x = as_dev_f32(inputs, self.ctx.device)
+        x = x.reshape(x.shape[0], -1)
+        if x.shape[1] != self.sizes[0]:
+            raise L.VbnnError(L.E_INVALID, f"inputs must be [N x {self.sizes[0]}]")
+        if n_samples is None:
+            n_samples = 0 if self.opt.get("quicktest") else int(self.opt["testSamples"])
+        n = x.shape[0]
+        t = None
+        if targets is not None:
+            t = as_dev_f32(targets, self.ctx.device).reshape(-1)
+            if t.shape[0] != n:
+                raise L.VbnnError(L.E_INVALID, "predict needs one target per input row")
+        logp = torch.empty(n, self.sizes[-1], dtype=torch.float32, device=x.device)
+        unc = torch.empty(n, 4, dtype=torch.float32, device=x.device)
+        nll, acc = C.c_float(), C.c_float()
+        want = t is not None
+        L.check(L.lib().vbnn_mlp_predict(self.handle, C.c_void_p(x.data_ptr()), n, int(n_samples),
+                                         C.c_void_p(t.data_ptr()) if want else None, C.c_void_p(logp.data_ptr()),
+                                         C.c_void_p(unc.data_ptr()), C.byref(nll) if want else None,
+                                         C.byref(acc) if want else None))
+        return Prediction(logp, unc[:, 0], unc[:, 1], unc[:, 2], unc[:, 3].long(),
+                          nll.value if want else None, acc.value if want else None)
 
     def calc_lc(self, opt=None):                                        # mlp.lua:109-115
         v = C.c_float()

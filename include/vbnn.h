@@ -234,6 +234,26 @@ int vbnn_mlp_calc_lc(vbnn_mlp* mlp, float* lc_host);                       /* ml
  * = {mean error, mean accuracy %} as main.lua:38-39. */
 int vbnn_mlp_step(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, int N,
                   float* result_dev);
+/* vbnn_mlp_step that also returns the gradient with respect to its input, so that the net can train as the head of
+ * a feature extractor (convnet.lua:23-33, whose model:backward sends the head's gradInput into the conv stack once
+ * per MC sample: mlp.lua:76-84 driven by main.lua:32-37).
+ * The function does exactly what vbnn_mlp_step does: it runs the same kernels on the same data and leaves the same
+ * parameters, Adam state, gradients, result and step counter, bit for bit.  It also OVERWRITES dX_dev, a dense
+ * fp32 [N x I0] device buffer that must be non-NULL, with
+ *     dX = sum_{s < S} d l_s / dX
+ * where l_s is the size-averaged ClassNLL of MC sample s over the GLOBAL batch (gradient scale 1 / (N * nranks), as
+ * for the parameter gradients).  The derivative is taken through this minibatch's sampled weights (weight mode) or
+ * its zeta (local reparameterisation, pathwise: G mu + 2 X .* (H sigma^2)), with the parameters BEFORE this
+ * minibatch's update.  This is what Torch7 accumulates into the extractor over main.lua:32-37, so feats:backward(dX)
+ * afterwards gives the extractor the reference's gradients; like the parameter gradients (quirk Q3) nothing is
+ * divided by S.
+ * Data parallel: each rank receives the rows it stepped, and the result is the derivative of the GLOBAL mean loss.
+ * A torch DDP extractor, which averages its gradients over ranks, must therefore scale dX by nranks (or sum its
+ * gradients instead of averaging them).
+ * The minibatch is replayed as its own CUDA graph, keyed on (N, dX_dev): reusing one buffer captures once, and
+ * vbnn_mlp_step's graph is never re-captured because of this call (nor the other way round). */
+int vbnn_mlp_step_grad_input(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, int N,
+                             float* result_dev, float* dX_dev);
 /* same with HOST buffers: H2D of inputs + D2H of {error, accuracy} inside the call
  * (replaces inputs:cuda()/targets:cuda() main.lua:23-24 and the scalar reads mlp.lua:80-82). */
 int vbnn_mlp_step_host(vbnn_mlp* mlp, const float* X_host, const float* targets_host, int N,

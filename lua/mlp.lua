@@ -4,7 +4,8 @@
 --   :calc_lc(opt), :update(opt)
 -- plus :predict(input, nsamples, target), the Bayesian model average with per-row uncertainty,
 -- and :train_minibatch(inputs, targets), the whole closure of main.lua:19-51 as ONE call that keeps the
--- minibatch, the sampled weights and the noise on the GPU.
+-- minibatch, the sampled weights and the noise on the GPU, and :train_minibatch_grad(inputs, targets, gradInput),
+-- the same on device tensors that also returns the gradient for a feature extractor below the net.
 --
 -- NOT EXECUTED IN THIS REPO (no Lua/Torch7 in the image); vbnn_b200/mlp.py makes the same calls in the
 -- same order and is what tests/ and bench.py drive.
@@ -22,8 +23,10 @@ function MLP:buildModel(opt)                                          -- referen
    sizes[#sizes + 1] = #opt.classes
    local csizes = ffi.new('int[?]', #sizes, sizes)
    local out = ffi.new('vbnn_mlp*[1]')
-   -- hidden layers: VBLinear + ReLU; output: plain nn.Linear + LogSoftMax (mlp.lua:29-30)
-   V.check(C.vbnn_mlp_create(V.context(opt.seed, true), csizes, #sizes, 0, opt.batchSize, V.opts(opt), out))
+   -- hidden layers: VBLinear + ReLU; output: plain nn.Linear + LogSoftMax (mlp.lua:29-30), or a VBLinear with
+   -- opt.vb_output (the convnet.lua:30 head)
+   V.check(C.vbnn_mlp_create(V.context(opt.seed, true), csizes, #sizes, opt.vb_output and 1 or 0, opt.batchSize,
+                             V.opts(opt), out))
    net.h = ffi.gc(out[0], C.vbnn_mlp_destroy)
    V.check(C.vbnn_mlp_init_params(net.h, opt.param_seed or 4, opt.msr_init and 1 or 0))     -- mlp.lua:47-55
    net.s = 0
@@ -87,6 +90,20 @@ function MLP:train_minibatch(inputs, targets)
    V.check(C.vbnn_mlp_submit_host(self.h, inputs:data(), targets:data(), inputs:size(1)))
    V.check(C.vbnn_mlp_collect(self.h, self.err, self.acc))
    return self.err[0], self.acc[0]
+end
+
+-- The same minibatch when the net is the head of a feature extractor (convnet.lua:23-33, with opt.vb_output for its
+-- VBLinear output layer): inputs / targets / gradInput are CudaTensors, and gradInput [N x input_size] is OVERWRITTEN
+-- with the sum over the S samples of d loss_s / d inputs (the parameters before this minibatch's update), which is
+-- what model:backward sends into the extractor over main.lua:32-37:  feats:backward(x, gradInput).
+function MLP:train_minibatch_grad(inputs, targets, gradInput)
+   local n = inputs:size(1)
+   assert(gradInput:isContiguous() and gradInput:size(1) == n and gradInput:size(2) == self.opt.input_size,
+          'gradInput must be a contiguous CudaTensor [N x input_size]')
+   self.res = self.res or torch.CudaTensor(2)
+   V.check(C.vbnn_mlp_step_grad_input(self.h, V.ptr(inputs), V.ptr(targets), n, V.ptr(self.res), V.ptr(gradInput)))
+   local r = self.res:float()
+   return r[1], r[2]
 end
 
 return MLP

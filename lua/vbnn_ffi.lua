@@ -46,6 +46,7 @@ int vbnn_mlp_run(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N,
 int vbnn_mlp_update(vbnn_mlp*);
 int vbnn_mlp_calc_lc(vbnn_mlp*, float* lc_host);
 int vbnn_mlp_step(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev);
+int vbnn_mlp_step_grad_input(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev, float* dX_dev);
 int vbnn_mlp_submit_host(vbnn_mlp*, const float* X_host, const float* targets_host, int N);
 int vbnn_mlp_collect(vbnn_mlp*, float* err_host, float* acc_host);
 int vbnn_mlp_test(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, int n_samples, float* err_host, float* acc_host);

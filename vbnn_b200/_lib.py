@@ -86,6 +86,7 @@ _PROTOS = {
     "vbnn_mlp_update": (C.c_int, [_P]),
     "vbnn_mlp_calc_lc": (C.c_int, [_P, _F]),
     "vbnn_mlp_step": (C.c_int, [_P, _P, _P, C.c_int, _P]),
+    "vbnn_mlp_step_grad_input": (C.c_int, [_P, _P, _P, C.c_int, _P, _P]),
     "vbnn_mlp_step_host": (C.c_int, [_P, _P, _P, C.c_int, _F, _F]),
     "vbnn_mlp_submit_host": (C.c_int, [_P, _P, _P, C.c_int]),
     "vbnn_mlp_collect": (C.c_int, [_P, _F, _F]),

@@ -14,6 +14,9 @@ struct SimtGemmArgs {
   const float* A2; long long sA2m, sA2k, zsA2;
   const float* B2; long long sB2n, sB2k, zsB2;
   int M, N, K;
+  // > 1: sum the products of samples z = 0 .. zsum-1 into ONE output (z = 0 of the epilogue), register
+  // accumulation in a fixed order; launch with batch = 1
+  int zsum;
 };
 int gemm_simt_launch(int mode, const SimtGemmArgs& g, const EpiParams& p, int batch,
                      cudaStream_t st, long long* launches);
@@ -32,6 +35,9 @@ struct TcOperand {
 struct TcGemmArgs {
   TcOperand A1, B1, A2, B2;
   int M, N, K, batch;
+  // 1: sample-summing form (not for the z-accumulating dW modes): D = sum_z A_z B_z as ONE contraction over
+  // K = batch x K (the accumulate bit stays set across z in TMEM), one work unit and one epilogue (z = 0) per tile
+  int zsum;
 };
 int gemm_tc_launch(int mode, const TcGemmArgs& g, const EpiParams& p, cudaStream_t st,
                    long long* launches);

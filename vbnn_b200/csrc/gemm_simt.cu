@@ -59,42 +59,46 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(SimtGemmArgs g, EpiParam
   const int z = blockIdx.z / ksplit, ks = blockIdx.z - z * ksplit;
   const int m0 = blockIdx.y * TM, n0 = blockIdx.x * TN;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  const float* A1 = g.A1 + z * g.zsA1;
-  const float* B1 = g.B1 + z * g.zsB1;
-  const float* A2 = DUAL ? g.A2 + z * g.zsA2 : nullptr;
-  const float* B2 = DUAL ? g.B2 + z * g.zsB2 : nullptr;
   const int kchunk = ksplit > 1 ? round_up_dev(ceil_div_dev(g.K, ksplit), TK) : g.K;
   const int k_begin = ks * kchunk, k_end = min(g.K, k_begin + kchunk);
 
   float acc1[4][4] = {}, acc2[4][4] = {};
-  for (int k0 = k_begin; k0 < k_end; k0 += TK) {
-    load_tile(sm.a[0], A1, g.sA1m, g.sA1k, m0, k0, g.M, k_end);
-    load_tile(sm.b[0], B1, g.sB1n, g.sB1k, n0, k0, g.N, k_end);
-    if (DUAL) {
-      load_tile(sm.a[DUAL ? 1 : 0], A2, g.sA2m, g.sA2k, m0, k0, g.M, k_end);
-      load_tile(sm.b[DUAL ? 1 : 0], B2, g.sB2n, g.sB2k, n0, k0, g.N, k_end);
-    }
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < TK; ++k) {
-      float4 av = *reinterpret_cast<const float4*>(&sm.a[0][k][ty * 4]);
-      float4 bv = *reinterpret_cast<const float4*>(&sm.b[0][k][tx * 4]);
-      float a[4] = {av.x, av.y, av.z, av.w}, b[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc1[i][j] = fmaf(a[i], b[j], acc1[i][j]);
+  // sample-summing form (g.zsum > 1, z = 0): the samples' products accumulate in registers, sample by sample
+  const int nz = g.zsum > 1 ? g.zsum : 1;
+  for (int zz = z; zz < z + nz; ++zz) {
+    const float* A1 = g.A1 + zz * g.zsA1;
+    const float* B1 = g.B1 + zz * g.zsB1;
+    const float* A2 = DUAL ? g.A2 + zz * g.zsA2 : nullptr;
+    const float* B2 = DUAL ? g.B2 + zz * g.zsB2 : nullptr;
+    for (int k0 = k_begin; k0 < k_end; k0 += TK) {
+      load_tile(sm.a[0], A1, g.sA1m, g.sA1k, m0, k0, g.M, k_end);
+      load_tile(sm.b[0], B1, g.sB1n, g.sB1k, n0, k0, g.N, k_end);
       if (DUAL) {
-        float4 av2 = *reinterpret_cast<const float4*>(&sm.a[DUAL ? 1 : 0][k][ty * 4]);
-        float4 bv2 = *reinterpret_cast<const float4*>(&sm.b[DUAL ? 1 : 0][k][tx * 4]);
-        float a2[4] = {av2.x, av2.y, av2.z, av2.w}, b2[4] = {bv2.x, bv2.y, bv2.z, bv2.w};
+        load_tile(sm.a[DUAL ? 1 : 0], A2, g.sA2m, g.sA2k, m0, k0, g.M, k_end);
+        load_tile(sm.b[DUAL ? 1 : 0], B2, g.sB2n, g.sB2k, n0, k0, g.N, k_end);
+      }
+      __syncthreads();
+#pragma unroll
+      for (int k = 0; k < TK; ++k) {
+        float4 av = *reinterpret_cast<const float4*>(&sm.a[0][k][ty * 4]);
+        float4 bv = *reinterpret_cast<const float4*>(&sm.b[0][k][tx * 4]);
+        float a[4] = {av.x, av.y, av.z, av.w}, b[4] = {bv.x, bv.y, bv.z, bv.w};
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
-          for (int j = 0; j < 4; ++j) acc2[i][j] = fmaf(a2[i], b2[j], acc2[i][j]);
+          for (int j = 0; j < 4; ++j) acc1[i][j] = fmaf(a[i], b[j], acc1[i][j]);
+        if (DUAL) {
+          float4 av2 = *reinterpret_cast<const float4*>(&sm.a[DUAL ? 1 : 0][k][ty * 4]);
+          float4 bv2 = *reinterpret_cast<const float4*>(&sm.b[DUAL ? 1 : 0][k][tx * 4]);
+          float a2[4] = {av2.x, av2.y, av2.z, av2.w}, b2[4] = {bv2.x, bv2.y, bv2.z, bv2.w};
+#pragma unroll
+          for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc2[i][j] = fmaf(a2[i], b2[j], acc2[i][j]);
+        }
       }
+      __syncthreads();
     }
-    __syncthreads();
   }
   if (ksplit > 1) {
     constexpr int NACC = DUAL ? 2 : 1;
@@ -215,6 +219,8 @@ static int launch_mode(const SimtGemmArgs& g, const EpiParams& p, int batch, cud
 
 int gemm_simt_launch(int mode, const SimtGemmArgs& g, const EpiParams& p, int batch,
                      cudaStream_t st, long long* launches) {
+  VB_CHECK(g.zsum <= 1 || (batch == 1 && !epi_z_accumulates(mode)), VBNN_E_INVALID,
+           "gemm_simt: the sample-summing form runs with batch 1 and no dW mode");
   if (launches) {
     const bool zacc = epi_z_accumulates(mode);
     *launches += (long long)(zacc ? batch : 1) * (choose_ksplit(g, zacc ? 1 : batch) > 1 ? 2 : 1);   // + the K-split finish kernel

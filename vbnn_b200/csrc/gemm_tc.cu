@@ -288,6 +288,7 @@ struct TcShape {
   int clc;                  // dynamic scheduling: one cluster per work unit, resident clusters steal pending ones
   int zA1, zB1, zA2, zB2;   // 0: the operand is shared by every batch index z (stride 0), 1: batched
   int hintA, hintB;         // L2 eviction priority of the A / B operand tiles: 0 normal, 1 evict-last, 2 evict-first
+  int zsum;                 // sample-summing form: one work unit per tile walks every z into one TMEM accumulator
 };
 
 // Tile rasterisation: bands of `gm` m-tiles, inside a band n-major.  The ~#SM/CG tiles in flight
@@ -396,7 +397,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
 
   const int tiles = sh.mt * sh.nt;
-  const int num_work = ZACC ? tiles : tiles * sh.batch;
+  // one work unit per tile when the unit walks every z (ZACC, zsum): w < tiles, so z = w / tiles = 0 below
+  const int num_work = (ZACC || sh.zsum) ? tiles : tiles * sh.batch;
   const int group = blockIdx.x / CG, num_groups = gridDim.x / CG;
   const bool dyn = sh.clc != 0;
   // next work unit of a role: static round-robin, or the response of the CLC query issued by the
@@ -431,7 +433,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
           if (++is == 2) { is = 0; ip ^= 1; }
         }
         const int tile = ZACC ? w : w % tiles;
-        const int zb = ZACC ? 0 : w / tiles, zn = ZACC ? sh.batch : 1;
+        const int zb = ZACC ? 0 : w / tiles, zn = (ZACC || sh.zsum) ? sh.batch : 1;
         int mi, ni;
         decode_tile(sh, tile, mi, ni);
         const int m0 = mi * (BM * CG) + rank * BM;
@@ -462,10 +464,16 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
       int as = 0; uint32_t aphase = 0;
       int cs = 0; uint32_t cp = 0;
       for (int w = group; w >= 0 && w < num_work; w = next_work(w, cs, cp, false)) {
-        const int zn = ZACC ? sh.batch : 1;
+        const int zn = (ZACC || sh.zsum) ? sh.batch : 1;
         for (int zi = 0; zi < zn; ++zi) {
-          mbar_wait(tempty_bar(as), aphase ^ 1);
-          tc_fence_after();
+          // ZACC: one accumulator (and epilogue pass) per z; zsum: the samples are K-concatenated into one
+          // accumulator, claimed before z = 0 and handed to the epilogue after the last z
+          const bool first_z = zi == 0 || !sh.zsum, last_z = zi + 1 == zn || !sh.zsum;
+          const int kz = sh.zsum ? zi : 0;
+          if (first_z) {
+            mbar_wait(tempty_bar(as), aphase ^ 1);
+            tc_fence_after();
+          }
           const uint32_t d1 = tmem_base + as * C::ACC_COLS;
           for (int kb = 0; kb < sh.num_kb; ++kb) {
             mbar_wait(full_bar(stage), phase);
@@ -474,7 +482,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
             const uint32_t sb = sa + C::NACC * C::A_BYTES;
 #pragma unroll
             for (int k = 0; k < BK / UK; ++k) {
-              const uint32_t acc = (kb | k) != 0 ? 1u : 0u;
+              const uint32_t acc = (kz | kb | k) != 0 ? 1u : 0u;
               umma_bf16<CG>(d1, make_sdesc<AK>(sa + k * kslice_bytes<AK>()),
                             make_sdesc<BKM>(sb + k * kslice_bytes<BKM>()), idesc, acc);
               if (DUAL)
@@ -484,8 +492,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
             tc_commit<CG>(empty_bar(stage));     // smem slot free (in every CTA) once these MMAs retire
             if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
           }
-          tc_commit<CG>(tfull_bar(as));          // accumulator ready for the epilogue warps
-          if (++as == AS) { as = 0; aphase ^= 1; }
+          if (last_z) {
+            tc_commit<CG>(tfull_bar(as));        // accumulator ready for the epilogue warps
+            if (++as == AS) { as = 0; aphase ^= 1; }
+          }
         }
       }
     }
@@ -810,6 +820,7 @@ int launch_cfg(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
   sh.M = g.M; sh.N = g.N; sh.K = g.K; sh.batch = g.batch;
   sh.mt = ceil_div(g.M, BM * CG); sh.nt = ceil_div(g.N, BN); sh.num_kb = ceil_div(g.K, BK);
   sh.zA1 = g.A1.zs != 0; sh.zB1 = g.B1.zs != 0; sh.zA2 = g.A2.zs != 0; sh.zB2 = g.B2.zs != 0;
+  sh.zsum = g.zsum && g.batch > 1;
   {
     const Knobs& k = knobs();
     sh.gm = k.tc_gm > 0 ? k.tc_gm : 8;
@@ -847,7 +858,7 @@ int launch_cfg(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
     attr_set = true;
   }
   const int tiles = sh.mt * sh.nt;
-  const int num_work = epi_z_accumulates(MODE) ? tiles : tiles * g.batch;
+  const int num_work = (epi_z_accumulates(MODE) || sh.zsum) ? tiles : tiles * g.batch;
   static int sms = 0;
   if (!sms) {
     int dev = 0;
@@ -886,7 +897,7 @@ TcChoice choose_cfg(const TcGemmArgs& g) {
     if (k.tc_tacc && !epi_is_dual(MODE)) return TcChoice{128, k.tc_tacc == 2 && g.M >= 256 ? 2 : 1};
     if (k.tc_dw64) return TcChoice{64, 1};
   }
-  const long long zmul = epi_z_accumulates(MODE) ? 1 : g.batch;
+  const long long zmul = (epi_z_accumulates(MODE) || g.zsum) ? 1 : g.batch;
   auto cost = [&](int bn, int cg, double speed) {
     const long long work = (long long)ceil_div(g.M, BM * cg) * ceil_div(g.N, bn) * zmul;
     const long long slots = kNumSMs / cg;
@@ -923,6 +934,7 @@ int gemm_tc_launch(int mode, const TcGemmArgs& g, const EpiParams& p, cudaStream
                    long long* launches) {
   VB_CHECK(g.M > 0 && g.N > 0 && g.K > 0 && g.batch > 0, VBNN_E_INVALID,
            "gemm_tc: empty problem %d x %d x %d (batch %d)", g.M, g.N, g.K, g.batch);
+  VB_CHECK(!g.zsum || !epi_z_accumulates(mode), VBNN_E_INVALID, "gemm_tc: the dW modes already sum over z");
   if (launches) *launches += 1;
   const bool ak = g.A1.kmajor != 0, bk = g.B1.kmajor != 0;
   switch (mode) {

@@ -255,6 +255,55 @@ int backward_data_layer(vbnn_mlp* m, int j, int N, int Zrun) {
       }
       VB_TRY(gemm_simt_launch(mode, g, p, Zrun, st, &m->ctx->launches));
     }
+  } else if (m->dX) {
+    // vbnn_mlp_step_grad_input: the first layer's gradInput summed over the Z samples, dX = sum_z dl_z/dX, written
+    // straight into the caller's [N x I0] buffer by ONE GEMM whose contraction runs over the samples too (K-concat:
+    // no atomics, no partials).  Nothing below the input: no ReLU mask.  The staged input act[0] is shared by every
+    // sample (zs_x = 0), so the LRT join is exact on the sums: sum_z (G_z mu + 2 X .* H_z s2) = (sum_z G_z) mu +
+    // 2 X .* ((sum_z H_z) s2).
+    EpiParams p;
+    memset(&p, 0, sizeof(p));
+    p.M = N; p.N = L->I;
+    p.out_f32 = m->dX; p.ld_f32 = L->I;
+    if (lrt) { p.xprev = m->act[0]; p.ld_x = ldi; p.zs_x = 0; }
+    const int mode = lrt ? EPI_DX_LRT : EPI_DX;
+    if (m->bf16) {
+      TcGemmArgs g;
+      memset(&g, 0, sizeof(g));
+      g.M = N; g.N = L->I; g.K = L->O; g.batch = Zrun; g.zsum = 1;
+      g.A1 = {(const bf16*)m->G[0], ldo, 1, zs_out};
+      g.B1 = {lrt ? L->mu_bf16 : L->w_bf16, L->ldI, 0, w_batched ? (long long)L->O * L->ldI : 0};
+      if (lrt && lrt_split(m, 2)) {
+        TcGemmArgs g1 = g;                  // sum_z H_z s2 into aux (z = 0 slice), then sum_z G_z mu joined with it
+        g1.A1 = {(const bf16*)m->H[0], ldo, 1, zs_out};
+        g1.B1 = {L->s2_bf16, L->ldI, 0, 0};
+        EpiParams p0;
+        memset(&p0, 0, sizeof(p0));
+        p0.M = N; p0.N = L->I;
+        p0.out_f32 = m->aux; p0.ld_f32 = m->ld_aux;
+        VB_TRY(tc_gemm(m->ctx, EPI_STORE, g1, p0, EPI_DX_LRT));
+        p.aux = m->aux; p.ld_aux = m->ld_aux;
+        VB_TRY(tc_gemm(m->ctx, EPI_DX_LRT2, g, p, EPI_DX_LRT));
+      } else {
+        if (lrt) {
+          g.A2 = {(const bf16*)m->H[0], ldo, 1, zs_out};
+          g.B2 = {L->s2_bf16, L->ldI, 0, 0};
+        }
+        VB_TRY(tc_gemm(m->ctx, mode, g, p));
+      }
+    } else {
+      SimtGemmArgs g;
+      memset(&g, 0, sizeof(g));
+      g.M = N; g.N = L->I; g.K = L->O; g.zsum = Zrun;
+      g.A1 = (const float*)m->G[0]; g.sA1m = ldo; g.sA1k = 1; g.zsA1 = zs_out;
+      g.B1 = lrt ? L->means : L->weight; g.sB1k = L->I; g.sB1n = 1;
+      g.zsB1 = w_batched ? (long long)L->O * L->I : 0;
+      if (lrt) {
+        g.A2 = (const float*)m->H[0]; g.sA2m = ldo; g.sA2k = 1; g.zsA2 = zs_out;
+        g.B2 = L->s2_f32; g.sB2k = L->I; g.sB2n = 1; g.zsB2 = 0;
+      }
+      VB_TRY(gemm_simt_launch(mode, g, p, 1, st, &m->ctx->launches));
+    }
   }
   return VBNN_OK;
 }
@@ -358,8 +407,8 @@ int backward_weight_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, int 
   return VBNN_OK;
 }
 
-// model:backward for layer j (mlp.lua:79): updateGradInput (skipped for the first layer, whose
-// gradInput nobody reads) + accGradParameters.
+// model:backward for layer j (mlp.lua:79): updateGradInput (for the first layer only when the caller asked for
+// the input gradient, vbnn_mlp_step_grad_input) + accGradParameters.
 int backward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, int accumulate) {
   VB_TRY(backward_data_layer(m, j, N, Zrun));
   return backward_weight_layer(m, j, N, Zrun, sample0, accumulate, false);
@@ -386,7 +435,10 @@ int run_samples(vbnn_mlp* m, int N, int Zrun, int sample0, int accumulate, bool 
     // minibatch's forward needs -- then finishes its exchange (reduce-scatter in the dW epilogue, owner update,
     // operand all-gather on the side stream) while the dW GEMMs of the layers above still run, and the tail
     // after the last dW belongs to the output layer, which the next forward reads last.
-    for (int j = Lc - 1; j >= 1; --j) { VB_TRY(backward_data_layer(m, j, N, Zrun)); VB_TRY(prof_mark(c, 5)); }
+    // The input gradient (m->dX, layer 0's backward-data) belongs to this chain and must stay before
+    // backward_weight_layer(0): once layer 0 raises grad_ready, its owners may update it and all-gather the new
+    // operands into this rank's mu_bf16 / s2_bf16 / w_bf16, which that GEMM reads.
+    for (int j = Lc - 1; j >= (m->dX ? 0 : 1); --j) { VB_TRY(backward_data_layer(m, j, N, Zrun)); VB_TRY(prof_mark(c, 5)); }
     for (int j = 0; j < Lc; ++j) {
       VB_TRY(backward_weight_layer(m, j, N, Zrun, sample0, accumulate, true));
       VB_TRY(prof_mark(c, 5));
@@ -473,16 +525,18 @@ int step_body(vbnn_mlp* m, int N) {
 int step_enqueue(vbnn_mlp* m, int N) {
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
+  // m->dX set: vbnn_mlp_step_grad_input, whose graph bakes the caller's buffer into its first-layer dX GEMM
+  vbnn_mlp::StepGraph& sg = m->dX ? m->graph_dx : m->graph;
   const bool graphable = m->use_graph && c->capturable && c->nranks == 1 && !c->profiling;
-  if (!graphable || m->eager_steps < 1) {
-    m->eager_steps++;
+  if (!graphable || sg.eager_steps < 1) {
+    sg.eager_steps++;
     return step_body(m, N);
   }
-  if (m->graph && m->graph_N != N) {
-    cudaGraphExecDestroy(m->graph);
-    m->graph = nullptr;
+  if (sg.exec && (sg.N != N || sg.dX != m->dX)) {
+    cudaGraphExecDestroy(sg.exec);
+    sg.exec = nullptr;
   }
-  if (!m->graph) {
+  if (!sg.exec) {
     const long long before = c->launches;
     VB_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
     int r = step_body(m, N);
@@ -490,15 +544,16 @@ int step_enqueue(vbnn_mlp* m, int N) {
     cudaError_t e = cudaStreamEndCapture(st, &gr);
     if (r != VBNN_OK) { if (gr) cudaGraphDestroy(gr); return r; }
     if (e != cudaSuccess) { set_error("cudaStreamEndCapture: %s", cudaGetErrorString(e)); return VBNN_E_CUDA; }
-    e = cudaGraphInstantiate(&m->graph, gr, 0);
+    e = cudaGraphInstantiate(&sg.exec, gr, 0);
     cudaGraphDestroy(gr);
-    if (e != cudaSuccess) { set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e)); m->graph = nullptr; return VBNN_E_CUDA; }
-    m->graph_N = N;
-    m->graph_launches = c->launches - before;
+    if (e != cudaSuccess) { set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e)); sg.exec = nullptr; return VBNN_E_CUDA; }
+    sg.N = N;
+    sg.dX = m->dX;
+    sg.launches = c->launches - before;
     c->launches = before;
   }
-  VB_CUDA(cudaGraphLaunch(m->graph, st));
-  c->launches += m->graph_launches;
+  VB_CUDA(cudaGraphLaunch(sg.exec, st));
+  c->launches += sg.launches;
   return VBNN_OK;
 }
 
@@ -656,7 +711,8 @@ extern "C" int vbnn_mlp_destroy(vbnn_mlp* m) {
   cudaSetDevice(m->ctx->device);
   cudaStreamSynchronize(m->ctx->stream);
   cudaStreamSynchronize(m->ctx->copy_stream);
-  if (m->graph) cudaGraphExecDestroy(m->graph);
+  if (m->graph.exec) cudaGraphExecDestroy(m->graph.exec);
+  if (m->graph_dx.exec) cudaGraphExecDestroy(m->graph_dx.exec);
   peer_destroy(m);
   for (cudaEvent_t e : m->ev_bwd) cudaEventDestroy(e);
   for (cudaEvent_t e : m->ev_red) cudaEventDestroy(e);
@@ -793,6 +849,22 @@ extern "C" int vbnn_mlp_step(vbnn_mlp* m, const float* X, const float* T, int N,
   VB_CUDA(cudaSetDevice(m->ctx->device));
   VB_TRY(stage_input(m, X, T, N));
   VB_TRY(step_enqueue(m, N));
+  if (result_dev)
+    VB_CUDA(cudaMemcpyAsync(result_dev, m->result, 8, cudaMemcpyDeviceToDevice, m->ctx->stream));
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_step_grad_input(vbnn_mlp* m, const float* X, const float* T, int N, float* result_dev,
+                                        float* dX) {
+  VB_CHECK(m && X && T && dX, VBNN_E_INVALID, "vbnn_mlp_step_grad_input: null argument");
+  VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_step_grad_input: N=%d exceeds max_batch=%d", N,
+           m->max_batch);
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  VB_TRY(stage_input(m, X, T, N));
+  m->dX = dX;                             // read by backward_data_layer(0) and step_enqueue while the step is enqueued
+  const int r = step_enqueue(m, N);
+  m->dX = nullptr;
+  VB_TRY(r);
   if (result_dev)
     VB_CUDA(cudaMemcpyAsync(result_dev, m->result, 8, cudaMemcpyDeviceToDevice, m->ctx->stream));
   return VBNN_OK;

@@ -135,9 +135,15 @@ struct vbnn_mlp {
   std::vector<size_t> grad_off, grad_len;       // per-layer slice {gW, gS, gb} of the arena
   std::vector<cudaEvent_t> ev_bwd, ev_red;      // dW of layer j done / its allreduce done
   int** t_list_dev = nullptr; int n_t = 0;
-  // CUDA graph of one step, keyed by N
-  cudaGraphExec_t graph = nullptr; int graph_N = -1; int eager_steps = 0; bool use_graph = true;
-  long long graph_launches = 0;
+  // CUDA graphs of one step: vbnn_mlp_step's keyed by N, vbnn_mlp_step_grad_input's by (N, dX); neither call
+  // destroys or re-captures the other's
+  struct StepGraph {
+    cudaGraphExec_t exec = nullptr; int N = -1; float* dX = nullptr; int eager_steps = 0; long long launches = 0;
+  };
+  StepGraph graph, graph_dx;
+  bool use_graph = true;
+  // vbnn_mlp_step_grad_input's output [N x I0] fp32, set only while that call enqueues its step
+  float* dX = nullptr;
   // host-buffer pipeline
   struct Slot { cudaEvent_t copied, consumed, done; float* h_result; bool busy; int N; };
   Slot slots[2];

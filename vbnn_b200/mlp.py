@@ -164,15 +164,33 @@ class MLP:
         L.check(L.lib().vbnn_mlp_update(self.handle))
 
     # ---- fused minibatch: main.lua:28-40 in one call ----
-    def train_step(self, inputs, targets, sync=True):
+    def train_step(self, inputs, targets, sync=True, grad_input=None):
         """inputs/targets already on the device.  Returns (error, accuracy) averaged over the S
-        samples as main.lua:38-39 (or None when sync=False)."""
+        samples as main.lua:38-39 (or None when sync=False).
+
+        grad_input: optional preallocated contiguous float32 CUDA tensor [N, input_size] on the context's device.
+        The step is then vbnn_mlp_step_grad_input: the same minibatch, bit for bit, and grad_input is overwritten
+        with sum_s d loss_s / d inputs through this minibatch's samples and the parameters before its update --
+        what a feature extractor below the net receives in the reference (feats.backward(grad_input)).  Data
+        parallel: the derivative of the global mean loss (a DDP extractor, which averages, must scale by nranks).
+        Reuse one tensor: the step's CUDA graph is keyed on its address."""
         import torch
         x, t = self._io(inputs, targets)
         if not hasattr(self, "_res"):
             self._res = torch.zeros(2, dtype=torch.float32, device=x.device)
-        L.check(L.lib().vbnn_mlp_step(self.handle, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
-                                      x.shape[0], C.c_void_p(self._res.data_ptr())))
+        if grad_input is None:
+            L.check(L.lib().vbnn_mlp_step(self.handle, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
+                                          x.shape[0], C.c_void_p(self._res.data_ptr())))
+        else:
+            g = grad_input
+            if (not isinstance(g, torch.Tensor) or g.dtype != torch.float32 or not g.is_cuda
+                    or g.device != x.device or tuple(g.shape) != (x.shape[0], self.sizes[0])
+                    or not g.is_contiguous()):
+                raise L.VbnnError(L.E_INVALID, f"grad_input must be a contiguous float32 tensor [{x.shape[0]}, "
+                                               f"{self.sizes[0]}] on {x.device}")
+            L.check(L.lib().vbnn_mlp_step_grad_input(self.handle, C.c_void_p(x.data_ptr()), C.c_void_p(t.data_ptr()),
+                                                     x.shape[0], C.c_void_p(self._res.data_ptr()),
+                                                     C.c_void_p(g.data_ptr())))
         if not sync:
             return None
         r = self._res.cpu()

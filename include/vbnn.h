@@ -254,6 +254,43 @@ int vbnn_mlp_step(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, i
  * vbnn_mlp_step's graph is never re-captured because of this call (nor the other way round). */
 int vbnn_mlp_step_grad_input(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, int N,
                              float* result_dev, float* dX_dev);
+/* The fused minibatch under ANY loss, in two halves around the caller's criterion (mlp.lua:30-32 builds the criterion
+ * as a separate, swappable object: nn.MSECriterion, a soft-label or a user criterion instead of ClassNLL).
+ *
+ * vbnn_mlp_forward_train: the first half of vbnn_mlp_step without its loss.  Stages X_dev [N x I0], samples, and
+ * runs the forward of the S samples at the current step (the noise indices of vbnn_mlp_step), writing the output
+ * layer's pre-LogSoftMax outputs Y_s into logits_dev, a dense fp32 [S x N x C] device buffer (sample slowest,
+ * 16-byte aligned).  Opens a step on the net.
+ *
+ * vbnn_mlp_backward_update: the second half.  grad_dev is a dense fp32 [S x N x C] device buffer holding dL/dY_s,
+ * where L = sum_s l_s.  Runs the backward, [the data-parallel exchange], the KL + Adam update and the step-counter
+ * bump exactly as vbnn_mlp_step does after its loss.  dX_dev (nullable) is overwritten with dL/dX [N x I0] as in
+ * vbnn_mlp_step_grad_input.  Closes the step, also when it fails.
+ *
+ * Gradient convention: vbnn_mlp_step is the special case grad_dev[s] = d l_s / dY_s with l_s the mean over the
+ * GLOBAL batch of ClassNLL(LogSoftMax(Y_s)).  The S samples are summed as in vbnn_mlp_step: gradWeight is divided by
+ * S in the VB update, gradBias and the plain nn.Linear output layer are not (quirk Q3); nothing is rescaled.  In
+ * data-parallel runs each rank passes its rows of the gradient of the global loss, so a mean divides by
+ * N * nranks, as vbnn_mlp_step does.
+ *
+ * Ordering: both calls enqueue on the context's stream and neither synchronises.  The caller's loss must run on that
+ * stream or be ordered against it with events (the Python Context makes its stream torch's current stream).
+ *
+ * Open step: while it is open every vbnn_mlp_* entry point that enqueues work returns VBNN_E_STATE, a second
+ * vbnn_mlp_forward_train included; only vbnn_mlp_backward_update and vbnn_mlp_reset_gradients are accepted.
+ * vbnn_mlp_forward_train is refused while the host pipeline (vbnn_mlp_submit_host*) has minibatches not collected.
+ * vbnn_mlp_reset_gradients abandons an open step: no update, and the step counter does not move.  In peer mode it
+ * refuses (the forward half has already advanced the peers' flag protocol): pass zeros to vbnn_mlp_backward_update
+ * instead, which drops this minibatch's likelihood term and still applies the KL update.
+ * vbnn_mlp_get_outputs returns VBNN_E_STATE after vbnn_mlp_forward_train until the next step, test or predict: this
+ * minibatch's outputs are in the caller's buffer.
+ *
+ * Each half is replayed as its own CUDA graph where vbnn_mlp_step would be: the forward keyed on (N, logits_dev),
+ * the backward on (N, grad_dev, dX_dev), with and without dX_dev in graphs of their own (each runs eagerly once
+ * before it is captured, and alternating the two never re-captures).  Neither re-captures the graphs of vbnn_mlp_step or
+ * vbnn_mlp_step_grad_input.  NULL X_dev / logits_dev / grad_dev and N outside 1..max_batch: VBNN_E_INVALID. */
+int vbnn_mlp_forward_train(vbnn_mlp* mlp, const float* X_dev, int N, float* logits_dev);
+int vbnn_mlp_backward_update(vbnn_mlp* mlp, const float* grad_dev, float* dX_dev);
 /* same with HOST buffers: H2D of inputs + D2H of {error, accuracy} inside the call
  * (replaces inputs:cuda()/targets:cuda() main.lua:23-24 and the scalar reads mlp.lua:80-82). */
 int vbnn_mlp_step_host(vbnn_mlp* mlp, const float* X_host, const float* targets_host, int N,
@@ -301,6 +338,10 @@ int vbnn_mlp_predict(vbnn_mlp* mlp, const float* X_dev, int N, int n_samples, co
 int vbnn_mlp_get_outputs(vbnn_mlp* mlp, int sample_idx, float* logp_host);
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */
 int vbnn_mlp_launch_count(vbnn_mlp* mlp, long long* count);
+/* CUDA graphs this handle has captured since creation, over all its step graphs (vbnn_mlp_step,
+ * vbnn_mlp_step_grad_input and the two halves of the split step): a caller that keeps its buffers and N fixed sees it
+ * stop growing after the second call of each entry point */
+int vbnn_mlp_graph_captures(vbnn_mlp* mlp, long long* count);
 /* flat gradient arena {gW, gS, gb per layer}: what the data-parallel allreduce sums */
 int vbnn_mlp_grad_arena(vbnn_mlp* mlp, float** ptr_dev, size_t* count);
 

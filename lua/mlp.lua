@@ -5,7 +5,8 @@
 -- plus :predict(input, nsamples, target), the Bayesian model average with per-row uncertainty,
 -- and :train_minibatch(inputs, targets), the whole closure of main.lua:19-51 as ONE call that keeps the
 -- minibatch, the sampled weights and the noise on the GPU, and :train_minibatch_grad(inputs, targets, gradInput),
--- the same on device tensors that also returns the gradient for a feature extractor below the net.
+-- the same on device tensors that also returns the gradient for a feature extractor below the net, and
+-- :forward_train(inputs) / :backward_update(gradLogits, gradInput), the same minibatch split around ANY criterion.
 --
 -- NOT EXECUTED IN THIS REPO (no Lua/Torch7 in the image); vbnn_b200/mlp.py makes the same calls in the
 -- same order and is what tests/ and bench.py drive.
@@ -104,6 +105,44 @@ function MLP:train_minibatch_grad(inputs, targets, gradInput)
    V.check(C.vbnn_mlp_step_grad_input(self.h, V.ptr(inputs), V.ptr(targets), n, V.ptr(self.res), V.ptr(gradInput)))
    local r = self.res:float()
    return r[1], r[2]
+end
+
+-- The fused minibatch under any nn criterion, in place of the ClassNLL of mlp.lua:78-79:
+--   local Y = net:forward_train(inputs)                           -- S x N x C pre-LogSoftMax outputs
+--   local err = 0
+--   local dY = Y.new():resizeAs(Y)
+--   for s = 1, S do err = err + crit:forward(Y[s], t); dY[s]:copy(crit:backward(Y[s], t)) end
+--   net:backward_update(dY)                                      -- backward, KL + Adam update, step counter
+-- gradLogits is the gradient of the SUM over the S samples of the per-sample loss (mlp.lua:79 accumulates the S
+-- backward passes the same way); a size-averaged criterion divides by N as ClassNLL does.  inputs / gradLogits /
+-- gradInput are CudaTensors on the library's stream; Y is reused from call to call (the graph is keyed on it), so copy
+-- it to keep it.  gradInput (optional, [N x input_size]) is overwritten as in :train_minibatch_grad.
+function MLP:forward_train(inputs)
+   local n = inputs:size(1)
+   assert(inputs:isContiguous() and inputs:size(2) == self.opt.input_size,
+          'inputs must be a contiguous CudaTensor [N x input_size]')
+   self.logits = self.logits or {}
+   local Y = self.logits[n]
+   if not Y then
+      Y = torch.CudaTensor(self.opt.S, n, #self.opt.classes)
+      self.logits[n] = Y
+   end
+   V.check(C.vbnn_mlp_forward_train(self.h, V.ptr(inputs), n, V.ptr(Y)))
+   self.open_n = n
+   return Y
+end
+
+function MLP:backward_update(gradLogits, gradInput)
+   local n = self.open_n
+   assert(n, 'backward_update: call forward_train first')
+   assert(gradLogits:isContiguous() and gradLogits:nElement() == self.opt.S * n * #self.opt.classes,
+          'gradLogits must be a contiguous CudaTensor [S x N x C]')
+   if gradInput then
+      assert(gradInput:isContiguous() and gradInput:size(1) == n and gradInput:size(2) == self.opt.input_size,
+             'gradInput must be a contiguous CudaTensor [N x input_size]')
+   end
+   self.open_n = nil
+   V.check(C.vbnn_mlp_backward_update(self.h, V.ptr(gradLogits), gradInput and V.ptr(gradInput) or nil))
 end
 
 return MLP

@@ -47,6 +47,8 @@ int vbnn_mlp_update(vbnn_mlp*);
 int vbnn_mlp_calc_lc(vbnn_mlp*, float* lc_host);
 int vbnn_mlp_step(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev);
 int vbnn_mlp_step_grad_input(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev, float* dX_dev);
+int vbnn_mlp_forward_train(vbnn_mlp*, const float* X_dev, int N, float* logits_dev);
+int vbnn_mlp_backward_update(vbnn_mlp*, const float* grad_dev, float* dX_dev);
 int vbnn_mlp_submit_host(vbnn_mlp*, const float* X_host, const float* targets_host, int N);
 int vbnn_mlp_collect(vbnn_mlp*, float* err_host, float* acc_host);
 int vbnn_mlp_test(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, int n_samples, float* err_host, float* acc_host);

@@ -87,6 +87,8 @@ _PROTOS = {
     "vbnn_mlp_calc_lc": (C.c_int, [_P, _F]),
     "vbnn_mlp_step": (C.c_int, [_P, _P, _P, C.c_int, _P]),
     "vbnn_mlp_step_grad_input": (C.c_int, [_P, _P, _P, C.c_int, _P, _P]),
+    "vbnn_mlp_forward_train": (C.c_int, [_P, _P, C.c_int, _P]),
+    "vbnn_mlp_backward_update": (C.c_int, [_P, _P, _P]),
     "vbnn_mlp_step_host": (C.c_int, [_P, _P, _P, C.c_int, _F, _F]),
     "vbnn_mlp_submit_host": (C.c_int, [_P, _P, _P, C.c_int]),
     "vbnn_mlp_collect": (C.c_int, [_P, _F, _F]),
@@ -96,6 +98,7 @@ _PROTOS = {
     "vbnn_mlp_predict": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _F, _F]),
     "vbnn_mlp_get_outputs": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_mlp_launch_count": (C.c_int, [_P, C.POINTER(C.c_longlong)]),
+    "vbnn_mlp_graph_captures": (C.c_int, [_P, C.POINTER(C.c_longlong)]),
     "vbnn_mlp_grad_arena": (C.c_int, [_P, C.POINTER(_P), C.POINTER(C.c_size_t)]),
     "vbnn_comm_unique_id": (C.c_int, [_P]),
     "vbnn_comm_init": (C.c_int, [_P, _P, C.c_int, C.c_int]),

@@ -755,6 +755,43 @@ __global__ void __launch_bounds__(kThreads) k_mul_act(const TA* a, int lda, cons
   }
 }
 
+// The caller's dL/dY (vbnn_mlp_backward_update) into the output layer's gradient operand: G = T(grad) over the
+// padded width (the padding columns zeroed exactly as k_loss leaves them) and, for an LRT output layer, H = T(G .* R)
+// as k_mul_act forms it from the stored G.  One thread per 4 columns: ld_g is a multiple of 8, so G / R / H quads are
+// aligned for one vector access each; the caller's rows of C floats carry no alignment and are read per element.
+template <typename T>
+struct alignas(4 * sizeof(T)) Quad { T v[4]; };
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) k_grad_logits(const float* __restrict__ grad, long long rows, int C,
+                                                          T* __restrict__ g, int ld_g, const T* __restrict__ r,
+                                                          T* __restrict__ h) {
+  const int qpr = ld_g >> 2;
+  const long long n = rows * qpr;
+  const bool narrow = n <= 0xFFFFFFFFll;                            // 32-bit index division where it fits
+  for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < n; q += (long long)gridDim.x * blockDim.x) {
+    const long long row = narrow ? (long long)((uint32_t)q / (uint32_t)qpr) : q / qpr;
+    const int c0 = (int)(q - row * qpr) * 4;
+    const float* src = grad + row * C;
+    Quad<T> gq;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) gq.v[e] = from_f32<T>(c0 + e < C ? src[c0 + e] : 0.f);
+    const long long off = row * ld_g + c0;
+    *reinterpret_cast<Quad<T>*>(g + off) = gq;
+    if (r && c0 < C) {
+      const Quad<T> rq = *reinterpret_cast<const Quad<T>*>(r + off);
+      Quad<T> hq;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) hq.v[e] = from_f32<T>(to_f32(gq.v[e]) * to_f32(rq.v[e]));
+      if (c0 + 4 <= C) {
+        *reinterpret_cast<Quad<T>*>(h + off) = hq;
+      } else {
+        for (int e = 0; c0 + e < C; ++e) h[off + e] = hq.v[e];      // H's padding is left as k_mul_act leaves it
+      }
+    }
+  }
+}
+
 __global__ void __launch_bounds__(kThreads) k_fill(float* dst, long long n, float v) {
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
        e += (long long)gridDim.x * blockDim.x)
@@ -927,6 +964,17 @@ int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st) {
   k_predict<<<(int)blocks, kThreads, 0, st>>>(p);
   VB_CUDA(cudaGetLastError());
   if (grid_out) *grid_out = (int)blocks;
+  return VBNN_OK;
+}
+
+int launch_grad_logits(const float* grad, long long rows, int C, void* g, int ld_g, const void* r, void* h, int is_bf16,
+                       cudaStream_t st) {
+  const int grid = grid_for(rows * (ld_g / 4));
+  if (is_bf16)
+    k_grad_logits<bf16><<<grid, kThreads, 0, st>>>(grad, rows, C, (bf16*)g, ld_g, (const bf16*)r, (bf16*)h);
+  else
+    k_grad_logits<float><<<grid, kThreads, 0, st>>>(grad, rows, C, (float*)g, ld_g, (const float*)r, (float*)h);
+  VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }
 

@@ -105,6 +105,11 @@ struct LossParams {
   int z_slot0;
 };
 int launch_loss(const LossParams& p, cudaStream_t st);
+// A caller-supplied dLoss/dlogits (vbnn_mlp_backward_update), dense fp32 [rows x C], into the output layer's
+// gradient operand g [rows x ld_g] (bf16 or fp32, padding columns zeroed as launch_loss leaves them) and, when r is
+// set (LRT output layer), h = g .* r [rows x ld_g] in the same pass (launch_mul_act's H).
+int launch_grad_logits(const float* grad, long long rows, int C, void* g, int ld_g, const void* r, void* h, int is_bf16,
+                       cudaStream_t st);
 
 // Bayesian model average over sampled forward passes (vbnn_mlp_predict), one chunk of zc samples per launch.
 // Per (row, class) the state is an online log-sum-exp over samples of logp_t = x_t - lse_t: a running max and

@@ -54,6 +54,7 @@ int stage_input(vbnn_mlp* m, const float* X, const float* T, int N) {
   }
   if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * 4, cudaMemcpyDeviceToDevice, st));
   m->last_N = N;
+  m->outputs_external = false;
   return VBNN_OK;
 }
 
@@ -70,6 +71,7 @@ int stage_input_u8(vbnn_mlp* m, const uint8_t* X, const float* T, int N, float m
   m->ctx->launches++;
   if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * 4, cudaMemcpyDeviceToDevice, st));
   m->last_N = N;
+  m->outputs_external = false;
   return VBNN_OK;
 }
 
@@ -118,8 +120,13 @@ int forward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, bool map_mod
   p.bias = L->bias;
   p.relu = last ? 0 : 1;
   p.ld_act = ldo; p.zs_act = (long long)N * ldo;
-  if (last) { p.out_f32 = m->logits; p.ld_f32 = m->ld_logits; p.zs_f32 = (long long)N * m->ld_logits; }
-  else { p.out_act = m->act[j + 1]; }
+  if (last && m->ext_logits) {            // vbnn_mlp_forward_train: straight into the caller's dense [Z x N x C]
+    p.out_f32 = m->ext_logits; p.ld_f32 = L->O; p.zs_f32 = (long long)N * L->O;
+  } else if (last) {
+    p.out_f32 = m->logits; p.ld_f32 = m->ld_logits; p.zs_f32 = (long long)N * m->ld_logits;
+  } else {
+    p.out_act = m->act[j + 1];
+  }
   int mode = EPI_FWD;
   if (lrt) {
     mode = EPI_FWD_LRT;
@@ -414,8 +421,8 @@ int backward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, int accumul
   return backward_weight_layer(m, j, N, Zrun, sample0, accumulate, false);
 }
 
-int run_samples(vbnn_mlp* m, int N, int Zrun, int sample0, int accumulate, bool backward, bool reduce_overlap = false,
-                bool peer = false) {
+// model:forward of Zrun samples (mlp.lua:77) up to the output layer's pre-LogSoftMax outputs
+int forward_samples(vbnn_mlp* m, int N, int Zrun, int sample0, bool peer = false) {
   const int Lc = nlayers(m);
   vbnn_ctx* c = m->ctx;
   for (int j = 0; j < Lc; ++j) {
@@ -426,9 +433,14 @@ int run_samples(vbnn_mlp* m, int N, int Zrun, int sample0, int accumulate, bool 
     VB_TRY(forward_layer(m, j, N, Zrun, sample0, false));
     VB_TRY(prof_mark(c, 3));
   }
-  VB_TRY(loss_all(m, N, Zrun, backward, nullptr, m->result_acc));
-  VB_TRY(prof_mark(c, 4));
-  if (!backward) return VBNN_OK;
+  return VBNN_OK;
+}
+
+// model:backward of Zrun samples (mlp.lua:79) from the output layer's gradient G[L-1] (and H[L-1])
+int backward_samples(vbnn_mlp* m, int N, int Zrun, int sample0, int accumulate, bool reduce_overlap = false,
+                     bool peer = false) {
+  const int Lc = nlayers(m);
+  vbnn_ctx* c = m->ctx;
   if (peer) {
     // Peer mode runs the backward-data chain first and the parameter-gradient GEMMs afterwards in FORWARD order
     // (same GEMMs, same operands: G_j / H_j stay in their per-layer buffers).  Layer 0 -- the first one the next
@@ -483,13 +495,13 @@ int update_all(vbnn_mlp* m, bool wait_reduce = false) {
   return VBNN_OK;
 }
 
-// everything of one minibatch after input staging: main.lua:28-40
-int step_body(vbnn_mlp* m, int N) {
+// The first half of one minibatch after input staging (main.lua:28-34 up to the criterion): the gradBias reset, the
+// peer waits, mlp:sample() and the forward of the S samples.
+int step_forward(vbnn_mlp* m, int N) {
   cudaStream_t st = m->ctx->stream;
-  VB_TRY(prof_mark(m->ctx, 0));
-  VB_CUDA(cudaMemsetAsync(m->result_acc, 0, (size_t)2 * m->Z * 4, st));
   for (vbnn_layer* L : m->layers) VB_CUDA(cudaMemsetAsync(L->gb, 0, (size_t)L->O * 4, st));   // main.lua:28
-  if (m->peer && m->peer->active) {
+  const bool peer = m->peer && m->peer->active;
+  if (peer) {
     // data parallel over NVLink peer memory (peer.cu): no collective call anywhere in the step
     VB_TRY(peer_check(m));
     m->peer_waited_all = !m->lrt;
@@ -497,49 +509,84 @@ int step_body(vbnn_mlp* m, int N) {
       VB_TRY(peer_wait_params(m, -1, true));
       VB_TRY(prof_mark(m->ctx, 1));
     }
-    VB_TRY(sample_all(m, 0, m->Z));
-    VB_TRY(prof_mark(m->ctx, 2));
-    VB_TRY(run_samples(m, N, m->Z, 0, 0, true, false, true));
-    VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st));
+  } else {
+    VB_TRY(prof_mark(m->ctx, 1));
+  }
+  VB_TRY(sample_all(m, 0, m->Z));                                                              // :33
+  VB_TRY(prof_mark(m->ctx, 2));
+  return forward_samples(m, N, m->Z, 0, peer);                                                 // :34
+}
+
+// The second half, from the output layer's gradient on: backward, [exchange], update, [the fused loss's result] and
+// the step-counter bump.
+int step_backward(vbnn_mlp* m, int N, bool finalize) {
+  cudaStream_t st = m->ctx->stream;
+  if (m->peer && m->peer->active) {
+    VB_TRY(backward_samples(m, N, m->Z, 0, 0, false, true));
+    if (finalize) { VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st)); m->ctx->launches++; }
     VB_TRY(launch_bump(m->ctx->d_step, m->t_list_dev, 0, st));    // the layers' t counters advance on the side stream
-    m->ctx->launches += 2;
+    m->ctx->launches++;
     VB_TRY(prof_mark(m->ctx, 7));
     return VBNN_OK;
   }
-  VB_TRY(prof_mark(m->ctx, 1));
-  VB_TRY(sample_all(m, 0, m->Z));                                                              // :33
-  VB_TRY(prof_mark(m->ctx, 2));
   const bool dp = m->ctx->nranks > 1;
   const bool overlap = dp && knobs().dp_overlap && m->ctx->comm_stream != nullptr;
-  VB_TRY(run_samples(m, N, m->Z, 0, /*accumulate=*/0, true, overlap));                         // :34
+  VB_TRY(backward_samples(m, N, m->Z, 0, /*accumulate=*/0, overlap));                          // :34
   if (dp && !overlap) VB_TRY(comm_allreduce_internal(m->ctx, m->grad_arena, m->grad_count, st));
   VB_TRY(update_all(m, overlap));                                                              // :40
   VB_TRY(prof_mark(m->ctx, 6));
-  VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st));                       // :38-39
+  if (finalize) {                                                                              // :38-39
+    VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st));
+    m->ctx->launches++;
+  }
   VB_TRY(launch_bump(m->ctx->d_step, m->t_list_dev, m->n_t, st));
-  m->ctx->launches += 2;
+  m->ctx->launches++;
   VB_TRY(prof_mark(m->ctx, 7));
   return VBNN_OK;
 }
 
-int step_enqueue(vbnn_mlp* m, int N) {
+// everything of one minibatch after input staging: main.lua:28-40
+int step_body(vbnn_mlp* m, int N) {
+  VB_TRY(prof_mark(m->ctx, 0));
+  VB_CUDA(cudaMemsetAsync(m->result_acc, 0, (size_t)2 * m->Z * 4, m->ctx->stream));
+  VB_TRY(step_forward(m, N));
+  VB_TRY(loss_all(m, N, m->Z, true, nullptr, m->result_acc));
+  VB_TRY(prof_mark(m->ctx, 4));
+  return step_backward(m, N, true);
+}
+
+// vbnn_mlp_backward_update's half: the caller's dL/dY becomes the output layer's gradient operand, then the rest of
+// the step.  Phase mark 0 first, so that the caller's loss since the forward half is not timed as this step's.
+int split_backward_body(vbnn_mlp* m, int N, const float* grad) {
+  const int Lc = nlayers(m);
+  vbnn_layer* Lo = m->layers[Lc - 1];
+  VB_TRY(prof_mark(m->ctx, 0));
+  VB_TRY(launch_grad_logits(grad, (long long)m->Z * N, Lo->O, m->G[Lc - 1], m->ld[Lc],
+                            layer_lrt(Lo) ? m->R[Lc - 1] : nullptr, m->H[Lc - 1], m->bf16, m->ctx->stream));
+  m->ctx->launches++;
+  VB_TRY(prof_mark(m->ctx, 4));
+  return step_backward(m, N, false);
+}
+
+// body() enqueued eagerly, or captured once into sg and replayed while (N, key) stays the same: one GPU, a
+// capturable stream, profiling off, and never on the first call (which warms up and allocates lazily)
+template <typename Body>
+int graph_enqueue(vbnn_mlp* m, vbnn_mlp::StepGraph& sg, int N, const void* key0, const void* key1, Body&& body) {
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
-  // m->dX set: vbnn_mlp_step_grad_input, whose graph bakes the caller's buffer into its first-layer dX GEMM
-  vbnn_mlp::StepGraph& sg = m->dX ? m->graph_dx : m->graph;
   const bool graphable = m->use_graph && c->capturable && c->nranks == 1 && !c->profiling;
   if (!graphable || sg.eager_steps < 1) {
     sg.eager_steps++;
-    return step_body(m, N);
+    return body();
   }
-  if (sg.exec && (sg.N != N || sg.dX != m->dX)) {
+  if (sg.exec && (sg.N != N || sg.key[0] != key0 || sg.key[1] != key1)) {
     cudaGraphExecDestroy(sg.exec);
     sg.exec = nullptr;
   }
   if (!sg.exec) {
     const long long before = c->launches;
     VB_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    int r = step_body(m, N);
+    int r = body();
     cudaGraph_t gr = nullptr;
     cudaError_t e = cudaStreamEndCapture(st, &gr);
     if (r != VBNN_OK) { if (gr) cudaGraphDestroy(gr); return r; }
@@ -548,12 +595,27 @@ int step_enqueue(vbnn_mlp* m, int N) {
     cudaGraphDestroy(gr);
     if (e != cudaSuccess) { set_error("cudaGraphInstantiate: %s", cudaGetErrorString(e)); sg.exec = nullptr; return VBNN_E_CUDA; }
     sg.N = N;
-    sg.dX = m->dX;
+    sg.key[0] = key0; sg.key[1] = key1;
     sg.launches = c->launches - before;
     c->launches = before;
+    m->graph_captures++;
   }
   VB_CUDA(cudaGraphLaunch(sg.exec, st));
   c->launches += sg.launches;
+  return VBNN_OK;
+}
+
+int step_enqueue(vbnn_mlp* m, int N) {
+  // m->dX set: vbnn_mlp_step_grad_input, whose graph bakes the caller's buffer into its first-layer dX GEMM
+  return graph_enqueue(m, m->graphs[m->dX ? vbnn_mlp::kGraphStepDx : vbnn_mlp::kGraphStep], N, m->dX, nullptr,
+                       [&] { return step_body(m, N); });
+}
+
+// While a split step is open, only vbnn_mlp_backward_update and vbnn_mlp_reset_gradients may enqueue work.
+int refuse_open_step(const vbnn_mlp* m, const char* who) {
+  VB_CHECK(!m->step_open, VBNN_E_STATE,
+           "%s: a vbnn_mlp_forward_train step is open: close it with vbnn_mlp_backward_update (or abandon it with "
+           "vbnn_mlp_reset_gradients)", who);
   return VBNN_OK;
 }
 
@@ -711,8 +773,8 @@ extern "C" int vbnn_mlp_destroy(vbnn_mlp* m) {
   cudaSetDevice(m->ctx->device);
   cudaStreamSynchronize(m->ctx->stream);
   cudaStreamSynchronize(m->ctx->copy_stream);
-  if (m->graph.exec) cudaGraphExecDestroy(m->graph.exec);
-  if (m->graph_dx.exec) cudaGraphExecDestroy(m->graph_dx.exec);
+  for (vbnn_mlp::StepGraph& sg : m->graphs)
+    if (sg.exec) cudaGraphExecDestroy(sg.exec);
   peer_destroy(m);
   for (cudaEvent_t e : m->ev_bwd) cudaEventDestroy(e);
   for (cudaEvent_t e : m->ev_red) cudaEventDestroy(e);
@@ -758,6 +820,7 @@ extern "C" int vbnn_mlp_layer(vbnn_mlp* m, int k, vbnn_layer** out) {
 
 extern "C" int vbnn_mlp_init_params(vbnn_mlp* m, uint64_t seed, int he_means) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_init_params"));
   cudaStream_t st = m->ctx->stream;
   for (vbnn_layer* L : m->layers) {
     const long long W = (long long)L->O * L->I;
@@ -784,6 +847,14 @@ extern "C" int vbnn_mlp_init_params(vbnn_mlp* m, uint64_t seed, int he_means) {
 // ============================================================ step pieces ==================
 extern "C" int vbnn_mlp_reset_gradients(vbnn_mlp* m) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
+  if (m->step_open) {
+    // abandon the split step: no update, the step counter stays.  In peer mode the forward half has already
+    // advanced the peers' flag protocol, so the step must be closed by vbnn_mlp_backward_update.
+    VB_CHECK(!(m->peer && m->peer->active), VBNN_E_STATE,
+             "vbnn_mlp_reset_gradients: an open step cannot be abandoned in peer mode; pass a zero gradient to "
+             "vbnn_mlp_backward_update instead");
+    m->step_open = false;
+  }
   cudaStream_t st = m->ctx->stream;
   VB_CUDA(cudaMemsetAsync(m->grad_arena, 0, m->grad_count * 4, st));     // mlp.lua:63-66
   VB_CUDA(cudaMemsetAsync(m->result_acc, 0, (size_t)2 * m->Z * 4, st));
@@ -792,6 +863,7 @@ extern "C" int vbnn_mlp_reset_gradients(vbnn_mlp* m) {
 
 extern "C" int vbnn_mlp_sample(vbnn_mlp* m, int sample_idx) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_sample"));
   for (vbnn_layer* L : m->layers) L->cur_sample = sample_idx;
   return sample_all(m, sample_idx, 1);
 }
@@ -800,6 +872,7 @@ extern "C" int vbnn_mlp_run(vbnn_mlp* m, const float* X, const float* T, int N, 
                             float* err_host, float* acc_host) {
   VB_CHECK(m && X && T, VBNN_E_INVALID, "vbnn_mlp_run: null argument");
   VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_run: N=%d exceeds max_batch=%d", N, m->max_batch);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_run"));
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
   VB_TRY(stage_input(m, X, T, N));
@@ -820,6 +893,7 @@ extern "C" int vbnn_mlp_run(vbnn_mlp* m, const float* X, const float* T, int N, 
 
 extern "C" int vbnn_mlp_update(vbnn_mlp* m) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_update"));
   VB_CHECK(!(m->peer && m->peer->active), VBNN_E_UNSUPPORTED,
            "peer mode drives the whole minibatch through vbnn_mlp_step / vbnn_mlp_submit_host");
   if (m->ctx->nranks > 1)
@@ -832,6 +906,7 @@ extern "C" int vbnn_mlp_update(vbnn_mlp* m) {
 
 extern "C" int vbnn_mlp_calc_lc(vbnn_mlp* m, float* lc_host) {
   VB_CHECK(m && lc_host, VBNN_E_INVALID, "null argument");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_calc_lc"));
   double lc = 0;
   for (vbnn_layer* L : m->layers) {
     if (L->kind != VBNN_KIND_VB) continue;
@@ -846,6 +921,7 @@ extern "C" int vbnn_mlp_calc_lc(vbnn_mlp* m, float* lc_host) {
 extern "C" int vbnn_mlp_step(vbnn_mlp* m, const float* X, const float* T, int N, float* result_dev) {
   VB_CHECK(m && X && T, VBNN_E_INVALID, "vbnn_mlp_step: null argument");
   VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_step: N=%d exceeds max_batch=%d", N, m->max_batch);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_step"));
   VB_CUDA(cudaSetDevice(m->ctx->device));
   VB_TRY(stage_input(m, X, T, N));
   VB_TRY(step_enqueue(m, N));
@@ -859,6 +935,7 @@ extern "C" int vbnn_mlp_step_grad_input(vbnn_mlp* m, const float* X, const float
   VB_CHECK(m && X && T && dX, VBNN_E_INVALID, "vbnn_mlp_step_grad_input: null argument");
   VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_step_grad_input: N=%d exceeds max_batch=%d", N,
            m->max_batch);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_step_grad_input"));
   VB_CUDA(cudaSetDevice(m->ctx->device));
   VB_TRY(stage_input(m, X, T, N));
   m->dX = dX;                             // read by backward_data_layer(0) and step_enqueue while the step is enqueued
@@ -868,6 +945,46 @@ extern "C" int vbnn_mlp_step_grad_input(vbnn_mlp* m, const float* X, const float
   if (result_dev)
     VB_CUDA(cudaMemcpyAsync(result_dev, m->result, 8, cudaMemcpyDeviceToDevice, m->ctx->stream));
   return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_forward_train(vbnn_mlp* m, const float* X, int N, float* logits_dev) {
+  VB_CHECK(m && X && logits_dev, VBNN_E_INVALID, "vbnn_mlp_forward_train: null argument");
+  VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_forward_train: N=%d outside 1..max_batch=%d", N,
+           m->max_batch);
+  VB_CHECK((reinterpret_cast<uintptr_t>(logits_dev) & 15) == 0, VBNN_E_INVALID,
+           "vbnn_mlp_forward_train: logits_dev must be 16-byte aligned");
+  VB_CHECK(!m->step_open, VBNN_E_STATE, "vbnn_mlp_forward_train: a step is already open: call "
+           "vbnn_mlp_backward_update (or vbnn_mlp_reset_gradients) first");
+  VB_CHECK(m->inflight == 0, VBNN_E_STATE, "vbnn_mlp_forward_train: %d host-pipeline minibatch(es) not collected",
+           m->inflight);
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  VB_TRY(stage_input(m, X, nullptr, N));
+  m->ext_logits = logits_dev;             // read by forward_layer(L-1) and the graph key while the half is enqueued
+  const int r = graph_enqueue(m, m->graphs[vbnn_mlp::kGraphFwd], N, logits_dev, nullptr, [&] {
+    VB_TRY(prof_mark(m->ctx, 0));
+    return step_forward(m, N);
+  });
+  m->ext_logits = nullptr;
+  VB_TRY(r);
+  m->step_open = true;
+  m->open_N = N;
+  m->outputs_external = true;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_backward_update(vbnn_mlp* m, const float* grad_dev, float* dX_dev) {
+  VB_CHECK(m && grad_dev, VBNN_E_INVALID, "vbnn_mlp_backward_update: null argument");
+  VB_CHECK(m->step_open, VBNN_E_STATE, "vbnn_mlp_backward_update: no open step: call vbnn_mlp_forward_train first");
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  const int N = m->open_N;
+  m->step_open = false;                   // closed whatever the outcome: an error leaves the net to be re-initialised
+  m->dX = dX_dev;                         // read by backward_data_layer(0) and the graph key while the half is enqueued
+  // with and without dX in graphs of their own, so that each form runs eagerly once before it is captured (as
+  // vbnn_mlp_step / vbnn_mlp_step_grad_input do) and alternating the two never re-captures
+  vbnn_mlp::StepGraph& sg = m->graphs[dX_dev ? vbnn_mlp::kGraphBwdDx : vbnn_mlp::kGraphBwd];
+  const int r = graph_enqueue(m, sg, N, grad_dev, dX_dev, [&] { return split_backward_body(m, N, grad_dev); });
+  m->dX = nullptr;
+  return r;
 }
 
 static int ensure_pipeline(vbnn_mlp* m) {
@@ -889,6 +1006,7 @@ static int submit_host_any(vbnn_mlp* m, const float* X_host, const uint8_t* X8_h
                            float mean, float inv_std) {
   VB_CHECK(m && (X_host || X8_host) && T_host, VBNN_E_INVALID, "vbnn_mlp_submit_host: null argument");
   VB_CHECK(N > 0 && N <= m->max_batch, VBNN_E_INVALID, "vbnn_mlp_submit_host: N=%d exceeds max_batch=%d", N, m->max_batch);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_submit_host"));
   VB_CUDA(cudaSetDevice(m->ctx->device));
   VB_TRY(ensure_pipeline(m));
   VB_CHECK(m->inflight < 2, VBNN_E_STATE, "vbnn_mlp_submit_host: two minibatches in flight, collect first");
@@ -965,6 +1083,7 @@ extern "C" int vbnn_mlp_test(vbnn_mlp* m, const float* X, const float* T, int N,
                              float* err_host, float* acc_host) {
   VB_CHECK(m && X && T, VBNN_E_INVALID, "vbnn_mlp_test: null argument");
   VB_CHECK(N > 0 && N <= m->max_batch && n_samples >= 0, VBNN_E_INVALID, "vbnn_mlp_test: bad N/n_samples");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_test"));
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
   VB_CUDA(cudaMemsetAsync(m->result_acc, 0, (size_t)2 * m->Z * 4, st));
@@ -986,6 +1105,7 @@ extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_sample
   VB_CHECK(N > 0 && N <= m->max_batch && n_samples >= 0, VBNN_E_INVALID,
            "vbnn_mlp_predict: N=%d (max_batch %d), n_samples=%d", N, m->max_batch, n_samples);
   VB_CHECK(targets || !(nll_host || acc_host), VBNN_E_INVALID, "vbnn_mlp_predict: nll / accuracy need targets");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_predict"));
   vbnn_ctx* c = m->ctx;
   cudaStream_t st = c->stream;
   VB_CUDA(cudaSetDevice(c->device));
@@ -1035,6 +1155,9 @@ extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_sample
 extern "C" int vbnn_mlp_get_outputs(vbnn_mlp* m, int sample_idx, float* logp_host) {
   VB_CHECK(m && logp_host, VBNN_E_INVALID, "null argument");
   VB_CHECK(m->last_N > 0 && sample_idx >= 0 && sample_idx < m->Z, VBNN_E_STATE, "vbnn_mlp_get_outputs: no forward yet");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_get_outputs"));
+  VB_CHECK(!m->outputs_external, VBNN_E_STATE,
+           "vbnn_mlp_get_outputs: the last forward was vbnn_mlp_forward_train, whose outputs are in the caller's buffer");
   vbnn_ctx* c = m->ctx;
   const int N = m->last_N, C = m->sizes.back();
   if (!m->logp) VB_TRY(dalloc(&m->logp, (size_t)m->max_batch * C * 4));
@@ -1054,6 +1177,12 @@ extern "C" int vbnn_mlp_get_outputs(vbnn_mlp* m, int sample_idx, float* logp_hos
 extern "C" int vbnn_mlp_launch_count(vbnn_mlp* m, long long* count) {
   VB_CHECK(m && count, VBNN_E_INVALID, "null argument");
   *count = m->ctx->launches;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_graph_captures(vbnn_mlp* m, long long* count) {
+  VB_CHECK(m && count, VBNN_E_INVALID, "null argument");
+  *count = m->graph_captures;
   return VBNN_OK;
 }
 

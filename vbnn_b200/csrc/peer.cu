@@ -557,6 +557,7 @@ extern "C" int vbnn_mlp_peer_export(vbnn_mlp* m, void* blob, size_t capacity, si
 
 extern "C" int vbnn_mlp_peer_import(vbnn_mlp* m, const void* blobs, size_t blob_len) {
   VB_CHECK(m && blobs, VBNN_E_INVALID, "vbnn_mlp_peer_import: null argument");
+  VB_CHECK(!m->step_open, VBNN_E_STATE, "vbnn_mlp_peer_import: a vbnn_mlp_forward_train step is open");
   vbnn_peer* P = m->peer;
   VB_CHECK(P && P->exported && !P->active, VBNN_E_STATE, "vbnn_mlp_peer_import: call vbnn_mlp_peer_export first");
   vbnn_ctx* c = m->ctx;
@@ -643,6 +644,7 @@ extern "C" int vbnn_mlp_peer_import(vbnn_mlp* m, const void* blobs, size_t blob_
 // the whole layer (utils.lua:73-80, main.lua:181).
 extern "C" int vbnn_mlp_sync_replicas(vbnn_mlp* m) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
+  VB_CHECK(!m->step_open, VBNN_E_STATE, "vbnn_mlp_sync_replicas: a vbnn_mlp_forward_train step is open");
   vbnn_peer* P = m->peer;
   if (!P || !P->active) return VBNN_OK;
   vbnn_ctx* c = m->ctx;

@@ -135,15 +135,26 @@ struct vbnn_mlp {
   std::vector<size_t> grad_off, grad_len;       // per-layer slice {gW, gS, gb} of the arena
   std::vector<cudaEvent_t> ev_bwd, ev_red;      // dW of layer j done / its allreduce done
   int** t_list_dev = nullptr; int n_t = 0;
-  // CUDA graphs of one step: vbnn_mlp_step's keyed by N, vbnn_mlp_step_grad_input's by (N, dX); neither call
-  // destroys or re-captures the other's
+  // CUDA graphs of one step: vbnn_mlp_step's keyed by N, vbnn_mlp_step_grad_input's by (N, dX), the forward half of
+  // the split step by (N, logits), its backward half by (N, grad) without and (N, grad, dX) with an input gradient;
+  // no call destroys or re-captures another's.  Each graph runs its body eagerly once before it captures.
   struct StepGraph {
-    cudaGraphExec_t exec = nullptr; int N = -1; float* dX = nullptr; int eager_steps = 0; long long launches = 0;
+    cudaGraphExec_t exec = nullptr; int N = -1; const void* key[2] = {nullptr, nullptr}; int eager_steps = 0;
+    long long launches = 0;
   };
-  StepGraph graph, graph_dx;
+  enum { kGraphStep, kGraphStepDx, kGraphFwd, kGraphBwd, kGraphBwdDx, kNumGraphs };
+  StepGraph graphs[kNumGraphs];
+  long long graph_captures = 0;      // captures made by all of them (vbnn_mlp_graph_captures)
   bool use_graph = true;
-  // vbnn_mlp_step_grad_input's output [N x I0] fp32, set only while that call enqueues its step
+  // vbnn_mlp_step_grad_input's / vbnn_mlp_backward_update's output [N x I0] fp32, set only while that call enqueues
   float* dX = nullptr;
+  // vbnn_mlp_forward_train's output [Z x N x C] fp32, set only while that call enqueues its forward half
+  float* ext_logits = nullptr;
+  // split step (vbnn_mlp_forward_train .. vbnn_mlp_backward_update): open, its N, and whether the last forward's
+  // outputs went to the caller's buffer instead of `logits` (vbnn_mlp_get_outputs has nothing to return)
+  bool step_open = false;
+  int open_N = 0;
+  bool outputs_external = false;
   // host-buffer pipeline
   struct Slot { cudaEvent_t copied, consumed, done; float* h_result; bool busy; int N; };
   Slot slots[2];

@@ -83,6 +83,7 @@ class MLP:
     def resetGradients(self):
         L.check(L.lib().vbnn_mlp_reset_gradients(self.handle))
         self._s = 0
+        self._open_n = None                                             # an open forward_train step is abandoned
 
     def sample(self, sample_idx=None):
         if sample_idx is not None:
@@ -195,6 +196,75 @@ class MLP:
             return None
         r = self._res.cpu()
         return float(r[0]), float(r[1])
+
+    # ---- the fused minibatch split around the caller's loss (vbnn_mlp_forward_train / vbnn_mlp_backward_update) ----
+    def forward_train(self, inputs):
+        """First half of train_step without its loss: sample and run the forward of the S samples at the current step.
+        Returns the output layer's pre-LogSoftMax outputs Y, a float32 device tensor [S, N, C].  The tensor belongs to
+        the binding and is overwritten by the next forward_train of the same N (the forward's CUDA graph is keyed on
+        it): clone it to keep it.  Opens a step that backward_update closes (resetGradients abandons it)."""
+        import torch
+        x = as_dev_f32(inputs, self.ctx.device)
+        x = x.reshape(x.shape[0], -1)
+        if x.shape[1] != self.sizes[0]:
+            raise L.VbnnError(L.E_INVALID, f"inputs must be [N x {self.sizes[0]}]")
+        n = x.shape[0]
+        if not hasattr(self, "_logits"):
+            self._logits = {}
+        y = self._logits.get(n)
+        if y is None:
+            y = torch.empty(int(self.opt["S"]), n, self.sizes[-1], dtype=torch.float32, device=x.device)
+            self._logits[n] = y
+        L.check(L.lib().vbnn_mlp_forward_train(self.handle, C.c_void_p(x.data_ptr()), n, C.c_void_p(y.data_ptr())))
+        self._open_n = n
+        return y
+
+    def backward_update(self, grad, grad_input=None):
+        """Second half: grad = dL/dY, a contiguous float32 device tensor [S, N, C] where L is the SUM over the S samples
+        of the per-sample loss (train_step is the case of the batch-mean ClassNLL of LogSoftMax(Y_s) per sample).
+        Runs the backward, [exchange], KL + Adam update and step-counter bump of train_step; grad_input, as in
+        train_step, is overwritten with dL/d inputs.  Asynchronous."""
+        import torch
+        n = getattr(self, "_open_n", None)
+        if n is None:
+            raise L.VbnnError(L.E_STATE, "backward_update: no open step (call forward_train first)")
+        dev = torch.device(f"cuda:{self.ctx.device}")
+        shape = (int(self.opt["S"]), n, self.sizes[-1])
+        if (not isinstance(grad, torch.Tensor) or grad.dtype != torch.float32 or not grad.is_cuda or grad.device != dev
+                or tuple(grad.shape) != shape or not grad.is_contiguous()):
+            raise L.VbnnError(L.E_INVALID, f"grad must be a contiguous float32 tensor {list(shape)} on {dev}")
+        g = grad_input
+        if g is not None and (not isinstance(g, torch.Tensor) or g.dtype != torch.float32 or not g.is_cuda
+                              or g.device != dev or tuple(g.shape) != (n, self.sizes[0]) or not g.is_contiguous()):
+            raise L.VbnnError(L.E_INVALID, f"grad_input must be a contiguous float32 tensor [{n}, {self.sizes[0]}] "
+                                           f"on {dev}")
+        self._open_n = None
+        L.check(L.lib().vbnn_mlp_backward_update(self.handle, C.c_void_p(grad.data_ptr()),
+                                                 C.c_void_p(g.data_ptr()) if g is not None else None))
+
+    def train_step_loss(self, inputs, loss_fn, grad_input=None):
+        """One minibatch under any torch loss: forward_train, loss = loss_fn(Y) on a detached leaf Y [S, N, C] that
+        requires grad, torch.autograd.grad, backward_update.  loss_fn must return the SUM over the S samples of the
+        per-sample loss to match train_step (for ClassNLL: sum_s nll_loss(log_softmax(Y[s]), t), each a batch mean).
+        Returns the loss as a device tensor without synchronising.  If loss_fn or the argument checks raise, the step
+        is abandoned (resetGradients; in peer mode it is closed with a zero gradient, which keeps the peers in step)."""
+        import torch
+        y = self.forward_train(inputs)
+        try:
+            leaf = y.detach().requires_grad_(True)
+            with torch.enable_grad():
+                loss = loss_fn(leaf)
+                (g,) = torch.autograd.grad(loss, leaf)
+            self.backward_update(g.contiguous(), grad_input)
+        except BaseException:
+            if self._open_n is not None:
+                if self.peer_active:
+                    self.backward_update(torch.zeros_like(y))
+                else:
+                    self._open_n = None
+                    self.resetGradients()
+            raise
+        return loss.detach()
 
     def train_step_host(self, inputs_host, targets_host):
         """HOST buffers in, host scalars out: H2D and D2H inside the call (main.lua:23-24)."""
@@ -317,6 +387,12 @@ class MLP:
     def launch_count(self):
         v = C.c_longlong()
         L.check(L.lib().vbnn_mlp_launch_count(self.handle, C.byref(v)))
+        return v.value
+
+    def graph_captures(self):
+        """CUDA graphs this net has captured (vbnn_mlp_graph_captures)."""
+        v = C.c_longlong()
+        L.check(L.lib().vbnn_mlp_graph_captures(self.handle, C.byref(v)))
         return v.value
 
     def grad_arena(self):

@@ -50,6 +50,10 @@ enum vbnn_reparam {
   VBNN_REPARAM_WEIGHT = 0, /* W = mu + sigma*eps per MC sample -- the reference (VBLinear.lua:59)  */
   VBNN_REPARAM_LOCAL = 1   /* local reparameterisation: Y = X mu^T + sqrt(X^2 s2^T)*zeta (new)    */
 };
+/* Local reparameterisation keeps R = zeta / (2 sqrt(V)), V = X^2 s2^T, for the backward.  Where V == 0 (an all-zero
+ * input row: zero-padded minibatch rows, or a hidden row whose units are all dead after ReLU) R := 0, so the variance
+ * term adds nothing to gradInput or gradSum for that row; the row's output is X mu^T + b.  Any V > 0, subnormal ones
+ * included, gets the finite zeta / (2 sqrt(V)). */
 
 enum vbnn_precision {
   VBNN_PREC_FP32 = 0,      /* fp32 operands, fp32 accumulate, CUDA-core GEMM (exact-parity mode)   */
@@ -231,7 +235,10 @@ int vbnn_mlp_calc_lc(vbnn_mlp* mlp, float* lc_host);                       /* ml
 
 /* One whole minibatch of main.lua:28-40 (reset, S x (sample, run), [allreduce], update) as one
  * enqueued sequence (CUDA graph when the shape repeats).  result_dev: nullable device float[2]
- * = {mean error, mean accuracy %} as main.lua:38-39. */
+ * = {mean error, mean accuracy %} as main.lua:38-39.
+ * Targets: a target outside 1..C (0 or C+1, e.g. a padding row) adds 0 to the error, is never counted correct and
+ * gives its row the gradient softmax(Y) * scale with no -1 term; the mean still divides by N.  The predicted class is
+ * the lowest index among tied maximal logits, as in vbnn_mlp_predict. */
 int vbnn_mlp_step(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, int N,
                   float* result_dev);
 /* vbnn_mlp_step that also returns the gradient with respect to its input, so that the net can train as the head of

@@ -261,7 +261,9 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
       const float mleg = gw[j] * inv_S;                                 // :92
       const float mlcg = mu[j] * inv_BV;                                // :91
       const float vleg = p.lrt ? gs[j] * inv_S * var : gs[j] * (0.5f * inv_S) * sd;   // :97 / A12
-      const float vlcg = (inv_vh - 1.f / var) * inv_2B * var;           // :96-97
+      // :96-97, (1/var_hat - 1/var) * var / (2B) without the division: var = __expf(lv) is 0 for lv < ln(FLT_MIN),
+      // where the reference's form is inf * 0 = NaN and this one is the finite limit -1/(2B)
+      const float vlcg = (var * inv_vh - 1.f) * inv_2B;
       const float gmu = mleg + mlcg;                                    // :132
       const float gvar = vleg + vlcg;                                   // :134
       // optim.adam on means (:135-138)
@@ -372,7 +374,7 @@ __global__ void __launch_bounds__(kThreads) k_grads(const float* mu, const float
       const float b = lrt ? gS[e] / S * var : gS[e] / (2.f * S) * sd;   // :97 (in place)
       gS[e] = b;
       if (vleg) vleg[e] = b;
-      if (vlcg) vlcg[e] = (1.f / var_hat - 1.f / var) / (2.f * B) * var;  // :96-97
+      if (vlcg) vlcg[e] = (var * (1.f / var_hat) - 1.f) / (2.f * B);   // :96-97, finite at var = 0 (k_update)
     }
   }
 }

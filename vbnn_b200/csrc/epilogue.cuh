@@ -155,6 +155,15 @@ __device__ __forceinline__ void load_bias4(const float* bias, int col, int nvali
   }
 }
 
+// 1/sqrt(V) of the local-reparameterisation forward, from which sqrt(V) = V * rs and R = zeta * rs / 2 follow.
+// V >= FLT_MIN: one MUFU.RSQ.  0 < V < FLT_MIN (a row whose inputs are all below ~1e-19): the .ftz of that
+// instruction would flush V to 0 and return +inf, turning Y and R into +-inf; V * 2^64 is exact and normal, and
+// rsqrt(V * 2^64) * 2^32 = rsqrt(V).  V = 0 (an all-zero input row): 0, so that R = 0 (include/vbnn.h).
+__device__ __forceinline__ float lrt_rsqrt(float v) {
+  if (v >= 1.17549435e-38f) return rsqrt_fast(v);
+  return v > 0.f ? rsqrt_fast(v * 18446744073709551616.f) * 4294967296.f : 0.f;
+}
+
 // Process one quad.  a1/a2: accumulator values (a2 only for dual modes).
 template <int MODE, typename AT>
 __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream& ps0, int z, int row, int col,
@@ -210,7 +219,7 @@ __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream&
     for (int j = 0; j < 4; ++j) {
       // sqrt(V) and zeta / (2 sqrt(V)) from one MUFU.RSQ (V = 0 only for an all-zero input row)
       const float v = a2[j];
-      const float rs = v > 0.f ? rsqrt_fast(v) : 0.f;
+      const float rs = lrt_rsqrt(v);
       const float sq = v * rs;
       y[j] = a1[j] + b[j] + sq * zt[j];
       r[j] = 0.5f * zt[j] * rs;

@@ -201,7 +201,7 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const float v = v2[4 * j + e];
-        const float rs = v > 0.f ? rsqrt_fast(v) : 0.f;
+        const float rs = lrt_rsqrt(v);
         const float y = v1[4 * j + e] + b[e] + (v * rs) * zt[e];
         yf[4 * j + e] = y;
         ya[e] = p.relu ? fmaxf(y, 0.f) : y;

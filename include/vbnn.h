@@ -78,7 +78,18 @@ enum vbnn_buf {
   VBNN_BUF_EPS = 11,       /* self.e (last epsilon)  VBLinear.lua:37,55        */
   VBNN_BUF_STDV = 12,      /* self.stdv cached by compute_prior  VBLinear.lua:79 */
   VBNN_BUF_MU_SQE = 13,    /* self.mu_sqe cached by compute_prior VBLinear.lua:82 */
-  VBNN_BUF__COUNT = 14
+  VBNN_BUF_PRIOR_MEANS = 14, /* prior means mu0 [O x I]        (VBNN_PRIOR_PER_WEIGHT only) */
+  VBNN_BUF_PRIOR_LVARS = 15, /* prior log-variances l0 [O x I] (VBNN_PRIOR_PER_WEIGHT only) */
+  VBNN_BUF__COUNT = 16
+};
+
+/* The prior N(mu_hat, var_hat) of the KL ("complexity") terms of a VB layer (vbnn_layer_set_prior). */
+enum vbnn_prior {
+  VBNN_PRIOR_EMPIRICAL = 0,  /* Graves' empirical Bayes, the reference: mu_hat = 0 (VBLinear.lua:81),
+                                var_hat = mean(sigma^2 + mu^2) re-estimated at every update (:86)         */
+  VBNN_PRIOR_FIXED = 1,      /* scalars mu_hat = mu0, var_hat = var0 > 0                                  */
+  VBNN_PRIOR_PER_WEIGHT = 2  /* per-weight arrays mu_hat = mu0[o,i], var_hat = exp(l0[o,i]): the buffers
+                                VBNN_BUF_PRIOR_MEANS / _LVARS, same parameterisation as means / lvars     */
 };
 
 /* config.lua restated; vbnn_opts_default() fills the reference's shipped values. */
@@ -136,7 +147,7 @@ int vbnn_ctx_synchronize(vbnn_ctx* ctx);
 /* Per-launch device timing of the tensor-core GEMM: CUDA events on the context's stream around
  * every launch, summed per epilogue class (0 store, 1 fwd, 2 fwd-lrt, 3 dx, 4 dx-lrt, 5 dw,
  * 6 dw-lrt) together with the algorithmic flops; class 7 is the fused KL + Adam update, whose
- * "flops" slot holds its algorithmic HBM bytes (56 B per weight); class 8 is vbnn_mlp_predict's averaging
+ * "flops" slot holds its algorithmic HBM bytes (56 B per weight, 64 under VBNN_PRIOR_PER_WEIGHT); class 8 is vbnn_mlp_predict's averaging
  * kernel, whose "flops" slot likewise holds bytes.  Enabling it disables graph replay.  This is
  * what bench.py's roofline object is computed from. */
 int vbnn_ctx_profile(vbnn_ctx* ctx, int enable);
@@ -175,7 +186,8 @@ int vbnn_layer_acc_grad(vbnn_layer* layer, const float* X_dev, const float* G_de
 /* VBLinear:resetAcc() VBLinear.lua:120-122 plus gradParameters:zero() (mlp.lua:63) */
 int vbnn_layer_reset_acc(vbnn_layer* layer);
 
-/* VBLinear:compute_prior()  VBLinear.lua:77-88 -> mu_hat, var_hat (host scalars, synchronises) */
+/* VBLinear:compute_prior()  VBLinear.lua:77-88 -> mu_hat, var_hat (host scalars, synchronises); under a
+ * non-empirical prior see vbnn_layer_set_prior */
 int vbnn_layer_compute_prior(vbnn_layer* layer, float* mu_hat, float* var_hat);
 /* VBLinear:compute_mugrads / compute_vargrads  VBLinear.lua:90-98.  Each out pointer is a
  * nullable [O x I] device buffer: mleg/vleg likelihood terms, mlcg/vlcg complexity terms.
@@ -187,6 +199,41 @@ int vbnn_layer_grads(vbnn_layer* layer, float* mleg_dev, float* mlcg_dev, float*
 int vbnn_layer_update(vbnn_layer* layer, vbnn_stats* stats);
 /* VBLinear:calc_lc(opt)  VBLinear.lua:99-103.  lc_dev: nullable [O x I]; sum_host: nullable. */
 int vbnn_layer_calc_lc(vbnn_layer* layer, float* lc_dev, float* sum_host);
+
+/* Choose the prior of the KL terms (enum vbnn_prior; a new layer is VBNN_PRIOR_EMPIRICAL).  Per weight, divided by
+ * B, the KL gradient w.r.t. mu is (mu - mu_hat) / var_hat (VBLinear.lua:91), the one w.r.t. log sigma^2 is
+ * (sigma^2 / var_hat - 1) / 2 (:96-97), and calc_lc is 1/2 log var_hat - 1/2 log sigma^2 + ((mu - mu_hat)^2 +
+ * sigma^2 - var_hat) / (2 var_hat) (:100-101); only where mu_hat and var_hat come from changes.
+ *   - It changes the KL terms of every update path -- vbnn_layer_update, vbnn_mlp_update, vbnn_mlp_step,
+ *     vbnn_mlp_step_grad_input, vbnn_mlp_backward_update, vbnn_mlp_submit_host* -- and of vbnn_layer_grads,
+ *     vbnn_layer_calc_lc and vbnn_mlp_calc_lc.  The likelihood terms, the loss and the noise are unchanged.
+ *   - mu0 / var0 are read for VBNN_PRIOR_FIXED only.
+ *   - VBNN_PRIOR_PER_WEIGHT initialises the prior arrays with a copy of the layer's current means and lvars (the
+ *     continual-learning step: the posterior becomes the next prior).  At that moment both KL gradients are exactly
+ *     0 for any finite log-variance, and so is calc_lc from the log-variances.  Afterwards the arrays are ordinary
+ *     buffers (vbnn_layer_get / _set / _device_ptr with VBNN_BUF_PRIOR_MEANS / _LVARS, which return VBNN_E_STATE
+ *     under any other kind); an edit takes effect at the next update.  They are allocated by the first PER_WEIGHT
+ *     call and kept until vbnn_layer_destroy, so a pointer from vbnn_layer_device_ptr stays valid across kind
+ *     changes.  In peer mode each rank keeps its own copy: edit it on every rank.
+ *   - FIXED and PER_WEIGHT compute the KL terms from log var_hat (FIXED: log var0) without a division: they are
+ *     finite wherever the exact value is representable in fp32 (for log var_hat >= -177), and the mean term is
+ *     exactly 0 where mu == mu_hat.
+ *   - vbnn_layer_compute_prior returns (mu0, var0) for FIXED and NaN for PER_WEIGHT, where there is no scalar
+ *     prior; the var_hat diagnostic of vbnn_stats follows the same rule.  With strict_reference the mu_sqe cache
+ *     keeps its reference meaning (mu - mu_hat)^2, with the prior mean.
+ *   - Every update keeps writing the partial sums of the empirical var_hat, so switching back to
+ *     VBNN_PRIOR_EMPIRICAL needs no extra pass and gives the reference's prior again.
+ *   - Stream-ordered on the context's stream: a PER_WEIGHT snapshot sees the posterior left by everything enqueued
+ *     before it, host-pipeline minibatches still in flight included.
+ *   - A layer of a vbnn_mlp: each of the net's step graphs re-captures once at its next use after this call.
+ *     Editing the PER_WEIGHT arrays needs no re-capture.
+ * VBNN_E_INVALID: a plain nn.Linear layer, an unknown kind, or FIXED with a non-finite mu0 or a var0 that is not
+ * finite and > 0.  VBNN_E_STATE: the layer's net has an open split step (vbnn_mlp_forward_train); or, in peer mode
+ * with PER_WEIGHT, rows owned by other ranks are stale -- run the vbnn_mlp_sync_replicas protocol first so that
+ * every rank snapshots the same posterior. */
+int vbnn_layer_set_prior(vbnn_layer* layer, int kind, float mu0, float var0);
+/* the current kind; mu0 / var0 (nullable) receive FIXED's scalars, NaN under the other kinds */
+int vbnn_layer_get_prior(const vbnn_layer* layer, int* kind, float* mu0, float* var0);
 
 /* parameters() / field access (mlp.lua:37,48-49; main.lua:123; checkpointing utils.lua:73-80) */
 int vbnn_layer_get(vbnn_layer* layer, int which, float* dst_host);

@@ -136,6 +136,14 @@ function VBLinear:calc_lc(opt)                                       -- :99-103
    return lc
 end
 
+-- The prior of the KL terms (vbnn_layer_set_prior): 'empirical' (the reference's, the default), 'fixed'
+-- N(mean, var) or 'per_weight' (this layer's current posterior becomes its prior)
+local PRIOR = { empirical = 0, fixed = 1, per_weight = 2 }
+function VBLinear:set_prior(kind, mean, var)
+   assert(PRIOR[kind], "set_prior: kind must be 'empirical', 'fixed' or 'per_weight'")
+   V.check(C.vbnn_layer_set_prior(self.h, PRIOR[kind], mean or 0, var or 0))
+end
+
 function VBLinear:clamp_to_map()                                     -- :105-107
    self:bind()
    V.check(C.vbnn_layer_clamp_to_map(self.h))

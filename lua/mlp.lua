@@ -32,7 +32,24 @@ function MLP:buildModel(opt)                                          -- referen
    V.check(C.vbnn_mlp_init_params(net.h, opt.param_seed or 4, opt.msr_init and 1 or 0))     -- mlp.lua:47-55
    net.s = 0
    net.err, net.acc = ffi.new('float[1]'), ffi.new('float[1]')
+   assert(opt.prior == nil or opt.prior == 'empirical' or opt.prior == 'fixed',
+          "opt.prior must be 'empirical' or 'fixed'")
+   if opt.prior == 'fixed' then net:set_prior('fixed', opt.prior_mean, opt.prior_var) end
    return net
+end
+
+-- VBLinear:set_prior on every VB layer of the net (the hidden layers and a vb_output layer)
+local PRIOR = { empirical = 0, fixed = 1, per_weight = 2 }
+function MLP:set_prior(kind, mean, var)
+   assert(PRIOR[kind], "set_prior: kind must be 'empirical', 'fixed' or 'per_weight'")
+   local n = C.vbnn_mlp_num_layers(self.h)
+   local layer = ffi.new('vbnn_layer*[1]')
+   for k = 0, n - 1 do
+      if k < n - 1 or self.opt.vb_output then
+         V.check(C.vbnn_mlp_layer(self.h, k, layer))
+         V.check(C.vbnn_layer_set_prior(layer[0], PRIOR[kind], mean or 0, var or 0))
+      end
+   end
 end
 
 function MLP:resetGradients()                                         -- mlp.lua:62-67

@@ -32,12 +32,15 @@ int vbnn_layer_compute_prior(vbnn_layer*, float* mu_hat, float* var_hat);
 int vbnn_layer_grads(vbnn_layer*, float* mleg, float* mlcg, float* vleg, float* vlcg);
 int vbnn_layer_update(vbnn_layer*, vbnn_stats*);
 int vbnn_layer_calc_lc(vbnn_layer*, float* lc_dev, float* sum_host);
+int vbnn_layer_set_prior(vbnn_layer*, int kind, float mu0, float var0);
+int vbnn_layer_get_prior(const vbnn_layer*, int* kind, float* mu0, float* var0);
 int vbnn_layer_device_ptr(vbnn_layer*, int which, float** ptr_dev, size_t* count);
 int vbnn_layer_bind(vbnn_layer*, int which, float* ptr_dev);
 /* net level (lua/mlp.lua): the mlp.lua object and the main.lua:19-51 closure */
 typedef struct vbnn_mlp vbnn_mlp;
 int vbnn_mlp_create(vbnn_ctx*, const int* sizes, int n_sizes, int vb_output, int max_batch, const vbnn_opts*, vbnn_mlp** out);
 int vbnn_mlp_destroy(vbnn_mlp*);
+int vbnn_mlp_num_layers(const vbnn_mlp*);
 int vbnn_mlp_layer(vbnn_mlp*, int k, vbnn_layer** out);
 int vbnn_mlp_init_params(vbnn_mlp*, uint64_t seed, int he_means);
 int vbnn_mlp_reset_gradients(vbnn_mlp*);

@@ -16,7 +16,9 @@ PREC_FP32, PREC_BF16 = 0, 1
 KIND_VB, KIND_LINEAR = 0, 1
 (BUF_MEANS, BUF_LVARS, BUF_BIAS, BUF_WEIGHT, BUF_GRAD_WEIGHT, BUF_GRAD_SUM, BUF_GRAD_BIAS,
  BUF_ADAM_M_MU, BUF_ADAM_V_MU, BUF_ADAM_M_VAR, BUF_ADAM_V_VAR, BUF_EPS, BUF_STDV,
- BUF_MU_SQE) = range(14)
+ BUF_MU_SQE, BUF_PRIOR_MEANS, BUF_PRIOR_LVARS) = range(16)
+PRIOR_EMPIRICAL, PRIOR_FIXED, PRIOR_PER_WEIGHT = 0, 1, 2
+PRIOR_KINDS = {"empirical": PRIOR_EMPIRICAL, "fixed": PRIOR_FIXED, "per_weight": PRIOR_PER_WEIGHT}
 
 
 class VbnnOpts(C.Structure):
@@ -67,6 +69,8 @@ _PROTOS = {
     "vbnn_layer_grads": (C.c_int, [_P, _P, _P, _P, _P]),
     "vbnn_layer_update": (C.c_int, [_P, C.POINTER(VbnnStats)]),
     "vbnn_layer_calc_lc": (C.c_int, [_P, _P, _F]),
+    "vbnn_layer_set_prior": (C.c_int, [_P, C.c_int, C.c_float, C.c_float]),
+    "vbnn_layer_get_prior": (C.c_int, [_P, C.POINTER(C.c_int), _F, _F]),
     "vbnn_layer_get": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_layer_set": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_layer_device_ptr": (C.c_int, [_P, C.c_int, C.POINTER(_P), C.POINTER(C.c_size_t)]),

@@ -146,19 +146,26 @@ __global__ void __launch_bounds__(kThreads) k_prior_partials(const float* __rest
 __global__ void __launch_bounds__(kThreads) k_prior_finalize(const double* partials, int np,
                                                              long long W, float* var_hat,
                                                              const float* mu, const float* lvar,
-                                                             float* stdv, float* mu_sqe) {
+                                                             float* stdv, float* mu_sqe, PriorArgs pr) {
   __shared__ double sh[32];
   if (blockIdx.x == 0) {
-    double a = 0.0;
-    for (int i = threadIdx.x; i < np; i += blockDim.x) a += partials[i];
-    double r = block_sum(a, sh);
-    if (threadIdx.x == 0) *var_hat = (float)(r / (double)W);          // VBLinear.lua:86
+    if (pr.kind == VBNN_PRIOR_EMPIRICAL) {
+      double a = 0.0;
+      for (int i = threadIdx.x; i < np; i += blockDim.x) a += partials[i];
+      double r = block_sum(a, sh);
+      if (threadIdx.x == 0) *var_hat = (float)(r / (double)W);        // VBLinear.lua:86
+    } else if (threadIdx.x == 0) {
+      *var_hat = pr.kind == VBNN_PRIOR_FIXED ? pr.var0 : __int_as_float(0x7fc00000);
+    }
   }
   if (stdv || mu_sqe) {
     for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < W;
          e += (long long)gridDim.x * blockDim.x) {
       if (stdv) stdv[e] = __expf(0.5f * lvar[e]);                       // VBLinear.lua:78-79
-      if (mu_sqe) mu_sqe[e] = mu[e] * mu[e];                            // VBLinear.lua:82
+      if (mu_sqe) {                                                     // VBLinear.lua:82
+        const float d = mu[e] - (pr.mu ? pr.mu[e] : pr.mu0);
+        mu_sqe[e] = d * d;
+      }
     }
   }
 }
@@ -169,22 +176,45 @@ __global__ void __launch_bounds__(kThreads) k_prior_finalize(const double* parti
 //   -> one pass: 32 B read + 24 B written per weight (+ caches / operand copies).
 struct AdamCoef { float step_mu, step_var; };
 
-template <bool VEC, bool STATS, int TPB>
+// The KL terms of a prior given by mu_hat and l0 = log var_hat (FIXED and PER_WEIGHT; k_update, k_grads), without a
+// division.  The mean term (mu - mu_hat) / (B var_hat) applies exp(-l0) as two factors exp(-l0 / 2) after the 1/B scale,
+// so it stays finite for l0 >= -177 wherever the exact value is representable; it is exactly 0 where mu == mu_hat for
+// any l0 (no 0 * inf).  The log-variance term (var / var_hat - 1) / (2B) is exp(lvar - l0): exactly 0 where
+// lvar == l0, finite whatever the two are when their difference is.
+__device__ __forceinline__ float kl_mu(float d, float l0, float inv_B) {
+  const float e = __expf(-0.5f * l0);
+  return d == 0.f ? 0.f : d * inv_B * e * e;
+}
+__device__ __forceinline__ float kl_lvar(float lv, float l0, float inv_2B) { return (__expf(lv - l0) - 1.f) * inv_2B; }
+
+// PK (enum vbnn_prior) selects where the prior N(mu_hat, var_hat) of the KL terms comes from:
+//   EMPIRICAL   the reduction of the partials below (VBLinear.lua:81-86), the reference's arithmetic;
+//   FIXED       p.prior.mu0 and l0 = p.prior.lvar0 = log var0, no reduction;
+//   PER_WEIGHT  mu_hat, l0 read next to mu / lvar (+8 B per weight).
+// FIXED and PER_WEIGHT share kl_mu / kl_lvar.
+template <bool VEC, bool STATS, int TPB, int PK>
 __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams p) {
   __shared__ double sh[32];
   __shared__ float s_var_hat;
   __shared__ AdamCoef s_coef;
   const int t_now = *p.t_dev;
   {
-    const double* part = p.partials + (p.partials_pingpong ? (size_t)(t_now & 1) * kMaxPartials : 0);
-    double a = 0.0;
-    for (int i = threadIdx.x; i < p.n_partials; i += blockDim.x) a += part[i];
-    double r = block_sum(a, sh);
+    double r = 0.0;
+    if (PK == VBNN_PRIOR_EMPIRICAL) {
+      const double* part = p.partials + (p.partials_pingpong ? (size_t)(t_now & 1) * kMaxPartials : 0);
+      double a = 0.0;
+      for (int i = threadIdx.x; i < p.n_partials; i += blockDim.x) a += part[i];
+      r = block_sum(a, sh);
+    }
     if (threadIdx.x == 0) {
-      const long long W = p.W_total > 0 ? p.W_total : (long long)p.O * p.I;
-      float vh = (float)(r / (double)W);
-      s_var_hat = vh;
-      if (blockIdx.x == 0) *p.var_hat_dev = vh;
+      if (PK == VBNN_PRIOR_EMPIRICAL) {
+        const long long W = p.W_total > 0 ? p.W_total : (long long)p.O * p.I;
+        float vh = (float)(r / (double)W);
+        s_var_hat = vh;
+        if (blockIdx.x == 0) *p.var_hat_dev = vh;
+      } else {
+        s_var_hat = 1.f;                                                // unused: kl_mu / kl_lvar
+      }
       const int t = t_now + 1;                                          // state.t = state.t + 1
       double bc1 = 1.0 - pow((double)p.beta1, (double)t);
       double bc2 = 1.0 - pow((double)p.beta2, (double)t);
@@ -250,22 +280,56 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
         for (int j = 0; j < 4; ++j) { gw[j] += a[j]; gs[j] += b[j]; }
       }
     }
-    load(p.m_mu, mm); load(p.v_mu, vm); load(p.m_var, mv); load(p.v_var, vv);
     float sd_old[4], musq[4], s2_new[4];
+    // FIXED / PER_WEIGHT: the KL terms are formed first (without STATS: added to the data terms in gw / gs).  The
+    // co-resident variant (80 registers) also stores the caches and only then loads the Adam state, so that the prior
+    // quads are dead by then; the others load the Adam state up front, as EMPIRICAL does, and keep every load in
+    // flight at once.  EMPIRICAL keeps the parent's statements: they compile to the same instructions.
+    constexpr bool kl_first = TPB == 128 && PK != VBNN_PRIOR_EMPIRICAL;
+    if constexpr (!kl_first) { load(p.m_mu, mm); load(p.v_mu, vm); load(p.m_var, mv); load(p.v_var, vv); }
+    float klm[4], klv[4], kvar[4];
+    if constexpr (PK != VBNN_PRIOR_EMPIRICAL) {
+      float pm[4], pl[4];
+      if constexpr (PK == VBNN_PRIOR_PER_WEIGHT) { load(p.prior.mu, pm); load(p.prior.lvar, pl); }
+      else {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { pm[j] = p.prior.mu0; pl[j] = p.prior.lvar0; }
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float var = __expf(lv[j]);                                // :78
+        kvar[j] = var;
+        sd_old[j] = sqrtf(var);                                         // :79
+        const float dmu0 = mu[j] - pm[j];                               // mu - mu_hat, :81-82
+        musq[j] = dmu0 * dmu0;
+        klm[j] = kl_mu(dmu0, pl[j], 2.f * inv_2B);                      // :91; 2 * inv_2B == 1/B in fp32
+        klv[j] = kl_lvar(lv[j], pl[j], inv_2B);                         // :96-97
+        if (!STATS) {
+          gw[j] = gw[j] * inv_S + klm[j];
+          gs[j] = (p.lrt ? gs[j] * inv_S * var : gs[j] * (0.5f * inv_S) * sd_old[j]) + klv[j];
+        }
+      }
+      if constexpr (kl_first) {
+        if (p.stdv) store(p.stdv, sd_old);
+        if (p.mu_sqe) store(p.mu_sqe, musq);
+      }
+    }
+    if constexpr (kl_first) { load(p.m_mu, mm); load(p.v_mu, vm); load(p.m_var, mv); load(p.v_var, vv); }
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      const float var = __expf(lv[j]);                                  // :78
-      const float sd = sqrtf(var);                                      // :79
+      const float var = PK == VBNN_PRIOR_EMPIRICAL ? __expf(lv[j]) : kvar[j];   // :78
+      const float sd = PK == VBNN_PRIOR_EMPIRICAL ? sqrtf(var) : sd_old[j];      // :79
       sd_old[j] = sd;
-      musq[j] = mu[j] * mu[j];                                          // :82
+      if (PK == VBNN_PRIOR_EMPIRICAL) musq[j] = mu[j] * mu[j];          // :82
       const float mleg = gw[j] * inv_S;                                 // :92
-      const float mlcg = mu[j] * inv_BV;                                // :91
+      const float mlcg = PK == VBNN_PRIOR_EMPIRICAL ? mu[j] * inv_BV : klm[j];   // :91
       const float vleg = p.lrt ? gs[j] * inv_S * var : gs[j] * (0.5f * inv_S) * sd;   // :97 / A12
       // :96-97, (1/var_hat - 1/var) * var / (2B) without the division: var = __expf(lv) is 0 for lv < ln(FLT_MIN),
       // where the reference's form is inf * 0 = NaN and this one is the finite limit -1/(2B)
-      const float vlcg = (var * inv_vh - 1.f) * inv_2B;
-      const float gmu = mleg + mlcg;                                    // :132
-      const float gvar = vleg + vlcg;                                   // :134
+      const float vlcg = PK == VBNN_PRIOR_EMPIRICAL ? (var * inv_vh - 1.f) * inv_2B : klv[j];
+      const bool folded = PK != VBNN_PRIOR_EMPIRICAL && !STATS;
+      const float gmu = folded ? gw[j] : mleg + mlcg;                   // :132
+      const float gvar = folded ? gs[j] : vleg + vlcg;                  // :134
       // optim.adam on means (:135-138)
       mm[j] = b1 * mm[j] + omb1 * gmu;
       vm[j] = b2 * vm[j] + omb2 * gmu * gmu;
@@ -290,8 +354,8 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
     }
     store(p.mu, mu); store(p.lvar, lv);
     store(p.m_mu, mm); store(p.v_mu, vm); store(p.m_var, mv); store(p.v_var, vv);
-    if (p.stdv) store(p.stdv, sd_old);
-    if (p.mu_sqe) store(p.mu_sqe, musq);
+    if (!kl_first && p.stdv) store(p.stdv, sd_old);
+    if (!kl_first && p.mu_sqe) store(p.mu_sqe, musq);
     if (p.s2_f32) store(p.s2_f32, s2_new);
     if (p.mu_bf16) {
       bf16* d1 = p.mu_bf16 + (long long)o * p.ld_bf16 + i0;
@@ -357,24 +421,30 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
 // ------------------------------------------------------------------ grads (API parity) ---
 __global__ void __launch_bounds__(kThreads) k_grads(const float* mu, const float* lvar, float* gW,
                                                     float* gS, long long n, const float* var_hat_dev,
-                                                    float B, float S, int lrt, float* mleg,
+                                                    PriorArgs pr, float B, float S, int lrt, float* mleg,
                                                     float* mlcg, float* vleg, float* vlcg) {
-  const float var_hat = *var_hat_dev;
+  const float var_hat = *var_hat_dev;                                   // EMPIRICAL
+  const bool args = pr.kind != VBNN_PRIOR_EMPIRICAL;                    // mu_hat, l0 from pr: as k_update
   const bool do_mu = mleg || mlcg, do_var = vleg || vlcg;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
        e += (long long)gridDim.x * blockDim.x) {
     const float var = __expf(lvar[e]), sd = sqrtf(var);
+    const float l0 = pr.lvar ? pr.lvar[e] : pr.lvar0;
     if (do_mu) {
       const float a = gW[e] / S;                                        // :92 (in place)
       gW[e] = a;
       if (mleg) mleg[e] = a;
-      if (mlcg) mlcg[e] = mu[e] / (B * var_hat);                        // :91
+      if (mlcg) {                                                       // :91
+        const float d = mu[e] - (pr.mu ? pr.mu[e] : pr.mu0);
+        mlcg[e] = args ? kl_mu(d, l0, 1.f / B) : d / (B * var_hat);
+      }
     }
     if (do_var) {
       const float b = lrt ? gS[e] / S * var : gS[e] / (2.f * S) * sd;   // :97 (in place)
       gS[e] = b;
       if (vleg) vleg[e] = b;
-      if (vlcg) vlcg[e] = (var * (1.f / var_hat) - 1.f) / (2.f * B);   // :96-97, finite at var = 0 (k_update)
+      if (vlcg)                                                         // :96-97, finite at var = 0 (k_update)
+        vlcg[e] = args ? kl_lvar(lvar[e], l0, 1.f / (2.f * B)) : (var * (1.f / var_hat) - 1.f) / (2.f * B);
     }
   }
 }
@@ -382,21 +452,35 @@ __global__ void __launch_bounds__(kThreads) k_grads(const float* mu, const float
 // ------------------------------------------------------------------ calc_lc -------------
 __global__ void __launch_bounds__(kThreads) k_calc_lc(const float* var_src, int var_kind,
                                                       const float* mu_src, int mu_is_sq, long long n,
-                                                      const float* var_hat_dev, float B, float* lc_out,
-                                                      double* partials) {
+                                                      const float* var_hat_dev, PriorArgs pr, float B,
+                                                      float* lc_out, double* partials) {
   __shared__ double sh[32];
-  const float var_hat = *var_hat_dev;
+  const float var_hat = *var_hat_dev;                                   // EMPIRICAL
   const float log_sd_hat = 0.5f * logf(var_hat);
+  const bool args = pr.kind != VBNN_PRIOR_EMPIRICAL;                    // mu_hat, l0 from pr
   double acc = 0.0;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
        e += (long long)gridDim.x * blockDim.x) {
-    float var, log_sd;
+    float var, log_sd, sd = 0.f;
     if (var_kind == 0) { log_sd = 0.5f * var_src[e]; var = expf(var_src[e]); }
-    else { float sd = var_src[e]; var = sd * sd; log_sd = logf(sd); }
+    else { sd = var_src[e]; var = sd * sd; log_sd = logf(sd); }
     float m = mu_src[e];
-    float musq = mu_is_sq ? m : m * m;
-    float first = -log_sd + log_sd_hat;                                 // :100
-    float second = (musq + (var - var_hat)) / (2.f * var_hat);          // :101
+    float musq = m;
+    if (!mu_is_sq) { const float d = m - (pr.mu ? pr.mu[e] : pr.mu0); musq = d * d; }
+    float first, second;
+    if (args) {
+      // (l0 - log var) / 2 + ((mu - mu_hat)^2 e^-l0 + var e^-l0 - 1) / 2 with e^-l0 as two factors e^(-l0/2), as kl_mu:
+      // finite at any representable l0 down to -177, and exactly 0 at a snapshot from the log-variances
+      // (exp(lvar - l0) = 1, mu == mu_hat)
+      const float l0 = pr.lvar ? pr.lvar[e] : pr.lvar0;
+      const float eh = expf(-0.5f * l0);
+      const float ratio = var_kind == 0 ? expf(var_src[e] - l0) : (sd * eh) * (sd * eh);
+      first = 0.5f * l0 - log_sd;                                       // :100
+      second = 0.5f * ((musq == 0.f ? 0.f : musq * eh * eh) + (ratio - 1.f));   // :101
+    } else {
+      first = -log_sd + log_sd_hat;                                     // :100
+      second = (musq + (var - var_hat)) / (2.f * var_hat);              // :101
+    }
     float lc = (first + second) * (1.f / B);                            // :102
     if (lc_out) lc_out[e] = lc;
     acc += (double)lc;
@@ -889,44 +973,54 @@ int launch_prior_partials_pp(const float* mu, const float* lvar, long long n, do
 }
 
 int launch_prior_finalize(const double* partials, int n_partials, long long W, float* var_hat_dev,
-                          const float* mu, const float* lvar, float* stdv, float* mu_sqe,
+                          const float* mu, const float* lvar, float* stdv, float* mu_sqe, const PriorArgs& pr,
                           cudaStream_t st) {
   int grid = (stdv || mu_sqe) ? grid_for(W) : 1;
   k_prior_finalize<<<grid, kThreads, 0, st>>>(partials, n_partials, W, var_hat_dev, mu, lvar, stdv,
-                                              mu_sqe);
+                                              mu_sqe, pr);
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }
 
-int launch_update(const UpdateParams& p, int* grid_out, cudaStream_t st) {
-  const int grid = p.grid_override > 0 ? p.grid_override : update_grid(p.O, p.I);
+template <int PK>
+static void launch_update_kind(const UpdateParams& p, int grid, cudaStream_t st) {
   const bool vec = (p.I & 3) == 0;
   const bool stats = p.stat_partials != nullptr;
-  if (p.coresident && vec && !stats) k_update<true, false, 128><<<grid, 128, 0, st>>>(p);
-  else if (vec && stats) k_update<true, true, kThreads><<<grid, kThreads, 0, st>>>(p);
-  else if (vec) k_update<true, false, kThreads><<<grid, kThreads, 0, st>>>(p);
-  else if (stats) k_update<false, true, kThreads><<<grid, kThreads, 0, st>>>(p);
-  else k_update<false, false, kThreads><<<grid, kThreads, 0, st>>>(p);
+  if (p.coresident && vec && !stats) k_update<true, false, 128, PK><<<grid, 128, 0, st>>>(p);
+  else if (vec && stats) k_update<true, true, kThreads, PK><<<grid, kThreads, 0, st>>>(p);
+  else if (vec) k_update<true, false, kThreads, PK><<<grid, kThreads, 0, st>>>(p);
+  else if (stats) k_update<false, true, kThreads, PK><<<grid, kThreads, 0, st>>>(p);
+  else k_update<false, false, kThreads, PK><<<grid, kThreads, 0, st>>>(p);
+}
+
+int launch_update(const UpdateParams& p, int* grid_out, cudaStream_t st) {
+  const int grid = p.grid_override > 0 ? p.grid_override : update_grid(p.O, p.I);
+  switch (p.prior.kind) {
+    case VBNN_PRIOR_EMPIRICAL: launch_update_kind<VBNN_PRIOR_EMPIRICAL>(p, grid, st); break;
+    case VBNN_PRIOR_FIXED: launch_update_kind<VBNN_PRIOR_FIXED>(p, grid, st); break;
+    case VBNN_PRIOR_PER_WEIGHT: launch_update_kind<VBNN_PRIOR_PER_WEIGHT>(p, grid, st); break;
+    default: set_error("launch_update: unknown prior kind %d", p.prior.kind); return VBNN_E_INVALID;
+  }
   VB_CUDA(cudaGetLastError());
   if (grid_out) *grid_out = grid;
   return VBNN_OK;
 }
 
 int launch_grads(const float* mu, const float* lvar, float* gW, float* gS, long long n,
-                 const float* var_hat_dev, float B, float S, int lrt, float* mleg, float* mlcg,
+                 const float* var_hat_dev, const PriorArgs& pr, float B, float S, int lrt, float* mleg, float* mlcg,
                  float* vleg, float* vlcg, cudaStream_t st) {
-  k_grads<<<grid_for(n), kThreads, 0, st>>>(mu, lvar, gW, gS, n, var_hat_dev, B, S, lrt, mleg, mlcg,
+  k_grads<<<grid_for(n), kThreads, 0, st>>>(mu, lvar, gW, gS, n, var_hat_dev, pr, B, S, lrt, mleg, mlcg,
                                             vleg, vlcg);
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }
 
 int launch_calc_lc(const float* var_src, int var_kind, const float* mu_src, int mu_is_sq, long long n,
-                   const float* var_hat_dev, float B, float* lc_out, double* partials,
+                   const float* var_hat_dev, const PriorArgs& pr, float B, float* lc_out, double* partials,
                    int* n_partials_out, cudaStream_t st) {
   int grid = grid_for(n, 4);
   if (grid > kMaxPartials) grid = kMaxPartials;
-  k_calc_lc<<<grid, kThreads, 0, st>>>(var_src, var_kind, mu_src, mu_is_sq, n, var_hat_dev, B, lc_out,
+  k_calc_lc<<<grid, kThreads, 0, st>>>(var_src, var_kind, mu_src, mu_is_sq, n, var_hat_dev, pr, B, lc_out,
                                        partials);
   VB_CUDA(cudaGetLastError());
   *n_partials_out = grid;

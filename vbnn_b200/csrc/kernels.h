@@ -32,9 +32,17 @@ int launch_prior_partials(const float* mu, const float* lvar, long long n, doubl
 int launch_prior_partials_pp(const float* mu, const float* lvar, long long n, double* partials2,
                              const int* t_dev, int grid, cudaStream_t st);
 int update_grid(int O, int I);
-// finalise var_hat = sum / W into a device scalar (+ optional caches stdv, mu_sqe)
+// The prior N(mu_hat, var_hat) of the KL terms (include/vbnn.h, enum vbnn_prior): Graves' empirical
+// (mu_hat = 0, var_hat = mean(sigma^2 + mu^2)), fixed scalars, or per-weight arrays [O x I].
+struct PriorArgs {
+  int kind;                             // enum vbnn_prior
+  float mu0, var0, lvar0;               // VBNN_PRIOR_FIXED (lvar0 = log var0)
+  const float *mu, *lvar;               // VBNN_PRIOR_PER_WEIGHT: prior means, prior log-variances
+};
+// finalise var_hat into a device scalar (+ optional caches stdv, mu_sqe = (mu - mu_hat)^2): EMPIRICAL reduces
+// the partials (sum / W), FIXED stores var0, PER_WEIGHT stores NaN (there is no scalar prior)
 int launch_prior_finalize(const double* partials, int n_partials, long long W, float* var_hat_dev,
-                          const float* mu, const float* lvar, float* stdv, float* mu_sqe,
+                          const float* mu, const float* lvar, float* stdv, float* mu_sqe, const PriorArgs& pr,
                           cudaStream_t st);
 
 // VBLinear:update (VBLinear.lua:124-166) minus the bias SGD: KL + likelihood gradients and both
@@ -73,17 +81,22 @@ struct UpdateParams {
   // that fit beside a resident tcgen05 GEMM CTA, so a shard's update starts while the persistent GEMMs
   // of the layers below own every SM ----
   int coresident;
+  // ---- prior of the KL terms: EMPIRICAL reads var_hat from `partials`; FIXED uses prior.mu0 / prior.lvar0 and
+  // skips that reduction; PER_WEIGHT reads prior.mu / prior.lvar (pre-offset to the shard like mu / lvar) ----
+  PriorArgs prior;
 };
 int launch_update(const UpdateParams& p, int* grid_out, cudaStream_t st);
 
-// compute_mugrads / compute_vargrads (VBLinear.lua:90-98) as standalone tensors (API parity).
+// compute_mugrads / compute_vargrads (VBLinear.lua:90-98) as standalone tensors (API parity).  EMPIRICAL reads var_hat
+// from var_hat_dev (mu_hat = 0); FIXED and PER_WEIGHT take mu_hat and log var_hat from pr, as k_update.
 int launch_grads(const float* mu, const float* lvar, float* gW, float* gS, long long n,
-                 const float* var_hat_dev, float B, float S, int lrt, float* mleg, float* mlcg,
+                 const float* var_hat_dev, const PriorArgs& pr, float B, float S, int lrt, float* mleg, float* mlcg,
                  float* vleg, float* vlcg, cudaStream_t st);
 
-// VBLinear:calc_lc (VBLinear.lua:99-103)
+// VBLinear:calc_lc (VBLinear.lua:99-103); mu_is_sq: mu_src is the mu_sqe cache (mu - mu_hat)^2.  Prior as in
+// launch_grads.
 int launch_calc_lc(const float* var_src, int var_kind /*0 lvar, 1 stdv*/, const float* mu_src,
-                   int mu_is_sq, long long n, const float* var_hat_dev, float B, float* lc_out,
+                   int mu_is_sq, long long n, const float* var_hat_dev, const PriorArgs& pr, float B, float* lc_out,
                    double* partials, int* n_partials_out, cudaStream_t st);
 
 // x -= lr * g  (optim.sgd, VBLinear.lua:125-128, mlp.lua:120-123) + optional bf16 operand copy

@@ -74,14 +74,24 @@ int layer_refresh_copies(vbnn_layer* L) {
   return VBNN_OK;
 }
 
+PriorArgs layer_prior(const vbnn_layer* L, size_t row_off) {
+  PriorArgs pr;
+  memset(&pr, 0, sizeof(pr));
+  pr.kind = L->prior_kind;
+  if (L->prior_kind == VBNN_PRIOR_FIXED) { pr.mu0 = L->prior_mu0; pr.var0 = L->prior_var0; pr.lvar0 = logf(L->prior_var0); }
+  if (L->prior_kind == VBNN_PRIOR_PER_WEIGHT) { pr.mu = L->prior_means + row_off; pr.lvar = L->prior_lvars + row_off; }
+  return pr;
+}
+
 int layer_compute_prior_internal(vbnn_layer* L) {
   vbnn_ctx* c = L->ctx;
   int np = 0;
   const long long W = (long long)L->O * L->I;
-  VB_TRY(launch_prior_partials(L->means, L->lvars, W, c->d_partials, &np, c->stream));
+  const bool empirical = L->prior_kind == VBNN_PRIOR_EMPIRICAL;
+  if (empirical) VB_TRY(launch_prior_partials(L->means, L->lvars, W, c->d_partials, &np, c->stream));
   VB_TRY(launch_prior_finalize(c->d_partials, np, W, L->var_hat_dev, L->means, L->lvars, L->stdv,
-                               L->mu_sqe, c->stream));
-  c->launches += 2;
+                               L->mu_sqe, layer_prior(L, 0), c->stream));
+  c->launches += empirical ? 2 : 1;
   L->prior_valid = true;
   return VBNN_OK;
 }
@@ -243,13 +253,15 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
   u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
   u.lrt = is_lrt(L);
+  u.prior = layer_prior(L, 0);
   double* stat_dev = stats ? c->d_partials + kMaxPartials : nullptr;
   u.stat_partials = stat_dev;
   int grid = 0;
   cudaEvent_t pa = nullptr, pb = nullptr;
   const bool timed = c->profiling;
   if (timed) {
-    // bench.py's HBM roofline: class 7 = fused update, "flops" slot = algorithmic bytes (56 B / weight)
+    // bench.py's HBM roofline: class 7 = fused update, "flops" slot = algorithmic bytes (56 B / weight, + the
+    // 8 B of the prior's mean and log-variance under PER_WEIGHT)
     for (cudaEvent_t* e : {&pa, &pb}) {
       if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); }
       else VB_CUDA(cudaEventCreate(e));
@@ -259,7 +271,7 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   VB_TRY(launch_update(u, &grid, st));                                                   // :131-143
   if (timed) {
     VB_CUDA(cudaEventRecord(pb, st));
-    c->prof_recs.push_back({pa, pb, 7, 56.0 * (double)W});
+    c->prof_recs.push_back({pa, pb, 7, (L->prior_kind == VBNN_PRIOR_PER_WEIGHT ? 64.0 : 56.0) * (double)W});
   }
   c->launches += 2;
   L->prior_valid = true;
@@ -506,6 +518,7 @@ extern "C" int vbnn_layer_destroy(vbnn_layer* L) {
   DEV_FREE(L->w_bf16); DEV_FREE(L->mu_bf16); DEV_FREE(L->s2_bf16); DEV_FREE(L->eps16);
   DEV_FREE(L->xs); DEV_FREE(L->xs2); DEV_FREE(L->gs_); DEV_FREE(L->hs); DEV_FREE(L->R);
   DEV_FREE(L->zeta_keep);
+  DEV_FREE(L->prior_means); DEV_FREE(L->prior_lvars);
   delete L;
   return VBNN_OK;
 }
@@ -712,16 +725,17 @@ extern "C" int vbnn_layer_compute_prior(vbnn_layer* L, float* mu_hat, float* var
   cudaStream_t st = L->ctx->stream;
   VB_CUDA(cudaMemcpyAsync(L->ctx->h_scalars, L->var_hat_dev, 4, cudaMemcpyDeviceToHost, st));
   VB_CUDA(cudaStreamSynchronize(st));
-  if (mu_hat) *mu_hat = 0.f;                                           // VBLinear.lua:81
-  if (var_hat) *var_hat = L->ctx->h_scalars[0];
+  if (mu_hat) *mu_hat = L->prior_kind == VBNN_PRIOR_EMPIRICAL ? 0.f             // VBLinear.lua:81
+                      : L->prior_kind == VBNN_PRIOR_FIXED ? L->prior_mu0 : nanf("");
+  if (var_hat) *var_hat = L->ctx->h_scalars[0];                        // FIXED: var0, PER_WEIGHT: NaN
   return VBNN_OK;
 }
 
 extern "C" int vbnn_layer_grads(vbnn_layer* L, float* mleg, float* mlcg, float* vleg, float* vlcg) {
   VB_CHECK(L && L->kind == VBNN_KIND_VB, VBNN_E_INVALID, "vbnn_layer_grads: not a VB layer");
   VB_CHECK(L->prior_valid, VBNN_E_STATE, "vbnn_layer_grads before compute_prior");
-  VB_TRY(launch_grads(L->means, L->lvars, L->gW, L->gS, (long long)L->O * L->I, L->var_hat_dev, L->opts.B,
-                      (float)L->opts.S, is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
+  VB_TRY(launch_grads(L->means, L->lvars, L->gW, L->gS, (long long)L->O * L->I, L->var_hat_dev, layer_prior(L, 0),
+                      L->opts.B, (float)L->opts.S, is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
   L->ctx->launches++;
   return VBNN_OK;
 }
@@ -740,10 +754,12 @@ extern "C" int vbnn_layer_calc_lc(vbnn_layer* L, float* lc_dev, float* sum_host)
   int np = 0;
   if (L->opts.strict_reference && L->stdv && L->mu_sqe) {
     // quirk Q6: tensors cached by the last compute_prior (VBLinear.lua:100-101 read self.vars etc.)
-    VB_TRY(launch_calc_lc(L->stdv, 1, L->mu_sqe, 1, W, L->var_hat_dev, L->opts.B, lc_dev, c->d_partials, &np, st));
+    VB_TRY(launch_calc_lc(L->stdv, 1, L->mu_sqe, 1, W, L->var_hat_dev, layer_prior(L, 0), L->opts.B, lc_dev,
+                          c->d_partials, &np, st));
   } else {
     VB_TRY(layer_compute_prior_internal(L));
-    VB_TRY(launch_calc_lc(L->lvars, 0, L->means, 0, W, L->var_hat_dev, L->opts.B, lc_dev, c->d_partials, &np, st));
+    VB_TRY(launch_calc_lc(L->lvars, 0, L->means, 0, W, L->var_hat_dev, layer_prior(L, 0), L->opts.B, lc_dev,
+                          c->d_partials, &np, st));
   }
   c->launches++;
   if (sum_host) {
@@ -753,6 +769,61 @@ extern "C" int vbnn_layer_calc_lc(vbnn_layer* L, float* lc_dev, float* sum_host)
     for (int i = 0; i < np; ++i) s += c->h_partials[i];
     *sum_host = (float)s;
   }
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_layer_set_prior(vbnn_layer* L, int kind, float mu0, float var0) {
+  VB_CHECK(L && L->kind == VBNN_KIND_VB, VBNN_E_INVALID, "vbnn_layer_set_prior: not a VB layer");
+  VB_CHECK(kind == VBNN_PRIOR_EMPIRICAL || kind == VBNN_PRIOR_FIXED || kind == VBNN_PRIOR_PER_WEIGHT, VBNN_E_INVALID,
+           "vbnn_layer_set_prior: unknown kind %d", kind);
+  VB_CHECK(kind != VBNN_PRIOR_FIXED || (isfinite(mu0) && isfinite(var0) && var0 > 0.f), VBNN_E_INVALID,
+           "vbnn_layer_set_prior: FIXED needs a finite mu0 and a finite var0 > 0 (got %g, %g)", mu0, var0);
+  VB_CHECK(!(L->owner && L->owner->step_open), VBNN_E_STATE,
+           "vbnn_layer_set_prior: the net has an open vbnn_mlp_forward_train step");
+  VB_CHECK(!(kind == VBNN_PRIOR_PER_WEIGHT && L->shard_stale && *L->shard_stale), VBNN_E_STATE,
+           "vbnn_layer_set_prior(PER_WEIGHT) in peer mode: rows owned by other ranks are out of date; call "
+           "vbnn_mlp_sync_replicas on every rank first");
+  vbnn_ctx* c = L->ctx;
+  cudaStream_t st = c->stream;
+  const size_t W = (size_t)L->O * L->I;
+  const int old = L->prior_kind;
+  if (kind == VBNN_PRIOR_PER_WEIGHT) {
+    if (!L->prior_means) {
+      VB_TRY(dev_alloc(&L->prior_means, W));
+      int r = dev_alloc(&L->prior_lvars, W);
+      if (r != VBNN_OK) { DEV_FREE(L->prior_means); return r; }
+    }
+    // the snapshot: this posterior becomes the prior (variational continual learning)
+    VB_CUDA(cudaMemcpyAsync(L->prior_means, L->means, W * 4, cudaMemcpyDeviceToDevice, st));
+    VB_CUDA(cudaMemcpyAsync(L->prior_lvars, L->lvars, W * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  // the arrays, once allocated, stay until vbnn_layer_destroy: pointers handed out by vbnn_layer_device_ptr stay valid
+  // across kind changes (VBNN_BUF_PRIOR_* are refused while the kind is not PER_WEIGHT)
+  L->prior_kind = kind;
+  L->prior_mu0 = kind == VBNN_PRIOR_FIXED ? mu0 : 0.f;
+  L->prior_var0 = kind == VBNN_PRIOR_FIXED ? var0 : 0.f;
+  if (kind == VBNN_PRIOR_FIXED || kind == VBNN_PRIOR_PER_WEIGHT) {
+    // the scalar vbnn_layer_grads / calc_lc / compute_prior / vbnn_stats read: var0, or NaN (no scalar prior)
+    VB_TRY(launch_fill(L->var_hat_dev, 1, kind == VBNN_PRIOR_FIXED ? var0 : nanf(""), st));
+    c->launches++;
+  } else if (old != VBNN_PRIOR_EMPIRICAL) {
+    // back to the reference's prior: var_hat of the current parameters, the strict_reference caches untouched
+    int np = 0;
+    VB_TRY(launch_prior_partials(L->means, L->lvars, (long long)W, c->d_partials, &np, st));
+    VB_TRY(launch_prior_finalize(c->d_partials, np, (long long)W, L->var_hat_dev, L->means, L->lvars, nullptr,
+                                 nullptr, layer_prior(L, 0), st));
+    c->launches += 2;
+  }
+  if (L->owner) mlp_drop_graphs(L->owner);   // the update kernels of the step graphs bake the prior in
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_layer_get_prior(const vbnn_layer* L, int* kind, float* mu0, float* var0) {
+  VB_CHECK(L && L->kind == VBNN_KIND_VB, VBNN_E_INVALID, "vbnn_layer_get_prior: not a VB layer");
+  const bool fixed = L->prior_kind == VBNN_PRIOR_FIXED;
+  if (kind) *kind = L->prior_kind;
+  if (mu0) *mu0 = fixed ? L->prior_mu0 : nanf("");
+  if (var0) *var0 = fixed ? L->prior_var0 : nanf("");
   return VBNN_OK;
 }
 
@@ -774,6 +845,12 @@ static int buf_lookup(vbnn_layer* L, int which, float** p, size_t* n) {
     case VBNN_BUF_EPS: *p = L->eps; break;
     case VBNN_BUF_STDV: *p = L->stdv; break;
     case VBNN_BUF_MU_SQE: *p = L->mu_sqe; break;
+    case VBNN_BUF_PRIOR_MEANS:
+    case VBNN_BUF_PRIOR_LVARS:
+      VB_CHECK(L->prior_kind == VBNN_PRIOR_PER_WEIGHT, VBNN_E_STATE,
+               "buffer %d: the layer's prior is not VBNN_PRIOR_PER_WEIGHT (vbnn_layer_set_prior)", which);
+      *p = which == VBNN_BUF_PRIOR_MEANS ? L->prior_means : L->prior_lvars;
+      break;
     default:
       set_error("unknown buffer id %d", which);
       return VBNN_E_INVALID;

@@ -669,6 +669,12 @@ int prof_launch(vbnn_ctx* c, int cls, double work, Launch&& launch) {
 
 }  // namespace
 
+// a prior change (vbnn_layer_set_prior): the update kernels the graphs captured bake the old prior in
+void vbnn::mlp_drop_graphs(vbnn_mlp* m) {
+  for (vbnn_mlp::StepGraph& sg : m->graphs)
+    if (sg.exec) { cudaGraphExecDestroy(sg.exec); sg.exec = nullptr; }
+}
+
 // ============================================================ create / destroy =============
 extern "C" int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int vb_output, int max_batch,
                                const vbnn_opts* opts, vbnn_mlp** out) {
@@ -711,7 +717,7 @@ extern "C" int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int
     r = layer_create_internal(ctx, sizes[j], sizes[j + 1], vb ? VBNN_KIND_VB : VBNN_KIND_LINEAR, opts,
                               (vb && !m->lrt) ? m->Z : 1, m->grad_arena + off_gW[j],
                               vb ? m->grad_arena + off_gS[j] : nullptr, m->grad_arena + off_gb[j], j, &L);
-    if (r == VBNN_OK) { L->owned_by_mlp = true; m->layers.push_back(L); }
+    if (r == VBNN_OK) { L->owned_by_mlp = true; L->owner = m; m->layers.push_back(L); }
   }
   // ---- activations ----
   const size_t e = esz(m);

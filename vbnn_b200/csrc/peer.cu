@@ -406,6 +406,7 @@ int peer_after_dw(vbnn_mlp* m, int j) {
     u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
     u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
     u.lrt = layer_lrt(L);
+    u.prior = layer_prior(L, roff);
     // knob peer_fused_push: the update kernel stores the refreshed operands to every rank itself instead of
     // 2 x (G-1) copy-engine copies.  It paid when layer 0's update was the tail of the minibatch (idle SMs); with
     // the dW GEMMs issued in forward order every update runs under GEMMs, where SM-free copy engines win.

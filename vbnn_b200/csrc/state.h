@@ -69,6 +69,11 @@ struct vbnn_layer {
   bool map_mode = false;
   bool prior_valid = false;
   const bool* shard_stale = nullptr;  // peer mode: fp32 state of the rows other ranks own is out of date
+  vbnn_mlp* owner = nullptr;         // the net whose step graphs bake this layer's prior in (mlp-owned layers)
+  // prior of the KL terms (vbnn_layer_set_prior): kind, FIXED scalars, PER_WEIGHT arrays [O x I]
+  int prior_kind = VBNN_PRIOR_EMPIRICAL;
+  float prior_mu0 = 0.f, prior_var0 = 0.f;
+  float *prior_means = nullptr, *prior_lvars = nullptr;
 };
 
 // ---- peer mode (peer.cu): the data-parallel gradient exchange over NVLink peer memory -------
@@ -171,6 +176,8 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t);
 int layer_refresh_copies(vbnn_layer* L);
 int layer_compute_prior_internal(vbnn_layer* L);
 int layer_refresh_prior_partials(vbnn_layer* L);
+PriorArgs layer_prior(const vbnn_layer* L, size_t row_off);   // row_off: first element of a peer-mode row shard
+void mlp_drop_graphs(vbnn_mlp* m);                            // each step graph re-captures at its next use
 PhiloxStream layer_stream(const vbnn_layer* L, uint32_t kind, int sample);
 int comm_allreduce_internal(vbnn_ctx* ctx, float* buf, size_t count, cudaStream_t st);
 // peer mode (peer.cu)

@@ -54,7 +54,18 @@ class MLP:
             if vb:
                 self.vb_indices.append(k)
         self._s = 0
+        prior = opt.get("prior", "empirical")
+        if prior not in ("empirical", "fixed"):
+            raise L.VbnnError(L.E_INVALID, f"opt.prior must be 'empirical' or 'fixed', got {prior!r}")
+        if prior == "fixed":
+            self.set_prior("fixed", opt.get("prior_mean", 0.0), opt.get("prior_var"))
         return self
+
+    def set_prior(self, kind, mean=0.0, var=None):
+        """VBLinear.set_prior on every VB layer (the hidden layers and a vb_output layer); "per_weight" makes each
+        layer's current posterior its prior.  Each step graph of the net re-captures once at its next use."""
+        for k in self.vb_indices:
+            self.model[k].set_prior(kind, mean, var)
 
     def init_params(self, seed=4, he_means=False):
         """means per VBLinear.lua:22-29 (or He-scaled, SURVEY 8d), Linear weights N(0, 2/fan_in)
@@ -340,6 +351,13 @@ class MLP:
                 if self.opt.get("strict_reference", True):
                     sd[f"{k}.stdv"] = m.get(L.BUF_STDV)
                     sd[f"{k}.mu_sqe"] = m.get(L.BUF_MU_SQE)
+                kind, mean, var = m.prior
+                sd[f"{k}.prior"] = L.PRIOR_KINDS[kind]
+                if kind == "fixed":
+                    sd[f"{k}.prior_mean"], sd[f"{k}.prior_var"] = mean, var
+                if kind == "per_weight":
+                    sd[f"{k}.prior_means"] = m.get(L.BUF_PRIOR_MEANS)
+                    sd[f"{k}.prior_lvars"] = m.get(L.BUF_PRIOR_LVARS)
             else:
                 sd[f"{k}.weight"] = m.get(L.BUF_WEIGHT)
                 sd[f"{k}.bias"] = m.get(L.BUF_BIAS)
@@ -352,8 +370,17 @@ class MLP:
         codes = dict(means=L.BUF_MEANS, lvars=L.BUF_LVARS, bias=L.BUF_BIAS, m_mu=L.BUF_ADAM_M_MU, v_mu=L.BUF_ADAM_V_MU,
                      m_var=L.BUF_ADAM_M_VAR, v_var=L.BUF_ADAM_V_VAR, weight=L.BUF_WEIGHT, stdv=L.BUF_STDV,
                      mu_sqe=L.BUF_MU_SQE)
+        kinds = {c: n for n, c in L.PRIOR_KINDS.items()}
         for k, m in enumerate(self.model):
             L.check(L.lib().vbnn_layer_set_t(m.handle, int(sd[f"{k}.t"])))
+            if m.kind == L.KIND_VB:
+                # before the parameters: a per_weight prior snapshots them, then takes its own arrays below.  A
+                # checkpoint without prior keys (older files) is the empirical prior.
+                kind = kinds[int(sd.get(f"{k}.prior", L.PRIOR_EMPIRICAL))]
+                m.set_prior(kind, float(sd.get(f"{k}.prior_mean", 0.0)), sd.get(f"{k}.prior_var"))
+                if kind == "per_weight":
+                    m.set(L.BUF_PRIOR_MEANS, sd[f"{k}.prior_means"])
+                    m.set(L.BUF_PRIOR_LVARS, sd[f"{k}.prior_lvars"])
             for n, b in codes.items():
                 if f"{k}.{n}" in sd:
                     m.set(b, sd[f"{k}.{n}"])

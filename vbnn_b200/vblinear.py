@@ -62,6 +62,8 @@ class VBLinear:
     gradBias = property(lambda s: s._view(L.BUF_GRAD_BIAS))
     stdv = property(lambda s: s._view(L.BUF_STDV))
     mu_sqe = property(lambda s: s._view(L.BUF_MU_SQE))
+    prior_means = property(lambda s: s._view(L.BUF_PRIOR_MEANS))      # "per_weight" prior only
+    prior_lvars = property(lambda s: s._view(L.BUF_PRIOR_LVARS))
 
     @property
     def weight(self):
@@ -171,6 +173,26 @@ class VBLinear:
     def resetAcc(self, opt=None):                                       # VBLinear.lua:120-122
         L.check(L.lib().vbnn_layer_reset_acc(self.handle))
         self._sample_idx = 0
+
+    # ---- the prior of the KL terms (vbnn_layer_set_prior) ----
+    def set_prior(self, kind, mean=0.0, var=None):
+        """kind "empirical" (the reference's N(0, mean(sigma^2 + mu^2)), the default), "fixed" (N(mean, var),
+        var > 0) or "per_weight": the prior becomes a copy of the current posterior, N(means, exp(lvars)), kept in
+        prior_means / prior_lvars, which may be edited afterwards.  mean / var are read for "fixed" only."""
+        if kind not in L.PRIOR_KINDS:
+            raise L.VbnnError(L.E_INVALID, f"set_prior: kind must be one of {sorted(L.PRIOR_KINDS)}, got {kind!r}")
+        if kind == "fixed" and var is None:
+            raise L.VbnnError(L.E_INVALID, "set_prior('fixed') needs var")
+        L.check(L.lib().vbnn_layer_set_prior(self.handle, L.PRIOR_KINDS[kind], C.c_float(mean),
+                                             C.c_float(var if var is not None else 0.0)))
+
+    @property
+    def prior(self):
+        """(kind, mean, var): the fixed prior's scalars, None for "empirical" and "per_weight"."""
+        k, m, v = C.c_int(), C.c_float(), C.c_float()
+        L.check(L.lib().vbnn_layer_get_prior(self.handle, C.byref(k), C.byref(m), C.byref(v)))
+        name = {c: n for n, c in L.PRIOR_KINDS.items()}[k.value]
+        return (name, m.value, v.value) if k.value == L.PRIOR_FIXED else (name, None, None)
 
     # ---- VBLinear.lua:77-103 ----
     def compute_prior(self):

@@ -148,7 +148,10 @@ int vbnn_ctx_synchronize(vbnn_ctx* ctx);
  * every launch, summed per epilogue class (0 store, 1 fwd, 2 fwd-lrt, 3 dx, 4 dx-lrt, 5 dw,
  * 6 dw-lrt) together with the algorithmic flops; class 7 is the fused KL + Adam update, whose
  * "flops" slot holds its algorithmic HBM bytes (56 B per weight, 64 under VBNN_PRIOR_PER_WEIGHT); class 8 is vbnn_mlp_predict's averaging
- * kernel, whose "flops" slot likewise holds bytes.  Enabling it disables graph replay.  This is
+ * kernel and vbnn_mlp_predict_outputs' moments kernel, whose "flops" slot likewise holds bytes (20 B per (row,
+ * class, sample) for predict; for predict_outputs, per (row, sample), 28 B per mean column and 12 B per
+ * log-variance column: zc * N * 28 * C under RAW, zc * N * 40 * K under GAUSSIAN, per chunk of zc samples).
+ * Enabling it disables graph replay.  This is
  * what bench.py's roofline object is computed from. */
 int vbnn_ctx_profile(vbnn_ctx* ctx, int enable);
 int vbnn_ctx_profile_read(vbnn_ctx* ctx, int cls, double* total_ms, long long* launches, double* flops);
@@ -388,6 +391,47 @@ int vbnn_mlp_test(vbnn_mlp* mlp, const float* X_dev, const float* targets_dev, i
  * the averaging kernel; its flops slot holds 20 algorithmic bytes per (row, class, sample). */
 int vbnn_mlp_predict(vbnn_mlp* mlp, const float* X_dev, int N, int n_samples, const float* targets_dev,
                      float* logp_dev, float* unc_dev, float* nll_host, float* acc_host);
+/* How vbnn_mlp_predict_outputs reads the net's C raw outputs f_t(x) (no LogSoftMax anywhere). */
+enum vbnn_output_model {
+  VBNN_OUTPUT_RAW = 0,      /* K = C outputs m_t = f_t(x) themselves                                        */
+  VBNN_OUTPUT_GAUSSIAN = 1  /* C = 2K: columns [0,K) are means m_t, [K,2K) log-variances s_t of a
+                               heteroscedastic Gaussian likelihood (torch: gaussian_nll_loss(Y[..., :K],
+                               y, Y[..., K:].exp()))                                                     */
+};
+/* Model average of the RAW outputs over n_samples sampled forward passes, for regression heads: the predictive
+ * mean and the split of its variance into epistemic (weight posterior) and aleatoric (heteroscedastic head) parts.
+ * Sampling is that of vbnn_mlp_predict: the same noise indices ((1 << 20) + t at the current step), the same chunks of
+ * S samples, no backward, no parameter, optimiser-state or step-counter change, the same LRT caveat (a row's zeta
+ * depends on its row index within the call) and the same peer-mode preconditions.  n_samples == 0: one MAP pass
+ * (clamp_to_map), and T = 1 below.  Otherwise T = n_samples.
+ * X_dev [N x I0], 1 <= N <= max_batch.  K = C (RAW) or C / 2 (GAUSSIAN; an odd C is VBNN_E_INVALID).
+ * Every output is nullable:
+ *   samples_dev   [T x N x C] dense fp32, sample slowest, 16-byte aligned: every sampled raw output, stored there by
+ *                 the output layer's epilogue (no extra copy)
+ *   mean_dev      [N x K] (1/T) sum_t m_t
+ *   epistemic_dev [N x K] (1/T) sum_t (m_t - mean)^2: the population variance over samples, exactly 0 at T = 1 and for
+ *                 MAP.  Formed from sums of deviations from the first sample, so it does not cancel when |mean| is
+ *                 large against the spread.
+ *   aleatoric_dev [N x K] (1/T) sum_t exp(s_t), GAUSSIAN only; +inf where exp(s) overflows fp32 (s > ~88.7).
+ *                 The predictive variance of the mixture is epistemic + aleatoric.
+ * targets_dev: dense fp32 [N x K] regression targets y (not 1-based labels); needed when nll_host or rmse_host is given.
+ *   rmse_host  sqrt(mean over N*K of (y - mean)^2)
+ *   nll_host   GAUSSIAN only: -(1/N) sum_n log p-bar(y_n | x_n), log p-bar = logsumexp_t sum_k log N(y_nk; m_tnk,
+ *              e^{s_tnk}) - log T: the full density (with 1/2 log 2 pi per output) of the joint per-row mixture, not a
+ *              product of per-column mixtures.  log N = -1/2 (log 2 pi + s + (y - m)^2 e^{-s}) is formed in the log
+ *              domain with the product taken as 0 where y == m, so nll is finite wherever its value is, s = +-100
+ *              included.
+ * Either scalar synchronises only if asked for; both are sums of per-block partials added on the host in a fixed
+ * order (no atomics): two calls at the same step give bit-identical results, and the result does not depend on S.
+ * VBNN_E_INVALID: NULL net or X_dev, N outside 1..max_batch, n_samples < 0, an unknown output_model, aleatoric_dev or
+ * nll_host under RAW, nll_host or rmse_host without targets_dev, an unaligned samples_dev.  VBNN_E_STATE while a
+ * vbnn_mlp_forward_train step is open.  The first call allocates the kernel's state and cannot be captured.
+ * Afterwards vbnn_mlp_get_outputs(s) returns sample s of the last chunk, as after vbnn_mlp_predict, unless
+ * samples_dev was given: then it returns VBNN_E_STATE until the next step, test or predict (the outputs are in the
+ * caller's buffer, as after vbnn_mlp_forward_train).  Profile class 8 ("predict") times the moments kernel. */
+int vbnn_mlp_predict_outputs(vbnn_mlp* mlp, const float* X_dev, int N, int n_samples, int output_model,
+                             const float* targets_dev, float* samples_dev, float* mean_dev,
+                             float* epistemic_dev, float* aleatoric_dev, float* nll_host, float* rmse_host);
 /* last forward's LogSoftMax output [N x C] (self.model.output, visualize.lua:97) */
 int vbnn_mlp_get_outputs(vbnn_mlp* mlp, int sample_idx, float* logp_host);
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */

@@ -3,6 +3,7 @@
 --   MLP:buildModel(opt), :resetGradients(), :sample(), :run(inputs, targets), :test(input, target),
 --   :calc_lc(opt), :update(opt)
 -- plus :predict(input, nsamples, target), the Bayesian model average with per-row uncertainty,
+-- :predict_outputs(input, nsamples, model, target), the same over the raw outputs of a regression head,
 -- and :train_minibatch(inputs, targets), the whole closure of main.lua:19-51 as ONE call that keeps the
 -- minibatch, the sampled weights and the noise on the GPU, and :train_minibatch_grad(inputs, targets, gradInput),
 -- the same on device tensors that also returns the gradient for a feature extractor below the net, and
@@ -90,6 +91,24 @@ function MLP:predict(input, nsamples, target)
    end
    V.check(C.vbnn_mlp_predict(self.h, V.ptr(input), n, nsamples, nil, V.ptr(logp), V.ptr(unc), nil, nil))
    return logp, unc
+end
+
+-- Model average of the RAW outputs for a regression head (vbnn_mlp_predict_outputs): model 'raw' (K = C outputs) or
+-- 'gaussian' (C = 2K: means, then log-variances).  Returns mean and epistemic variance [n x K], the aleatoric variance
+-- under 'gaussian' (else nil), and with a target [n x K] the mixture NLL ('gaussian', else nil) and the RMSE.
+function MLP:predict_outputs(input, nsamples, model, target)
+   local n = input:size(1)
+   if nsamples == nil then nsamples = self.opt.quicktest and 0 or self.opt.testSamples end
+   local gaussian = model == 'gaussian'
+   local k = gaussian and #self.opt.classes / 2 or #self.opt.classes
+   local mean, epi = torch.CudaTensor(n, k), torch.CudaTensor(n, k)
+   local ale = gaussian and torch.CudaTensor(n, k) or nil
+   local nll = (gaussian and target) and ffi.new('float[1]') or nil
+   local rmse = target and ffi.new('float[1]') or nil
+   V.check(C.vbnn_mlp_predict_outputs(self.h, V.ptr(input), n, nsamples, gaussian and 1 or 0,
+                                      target and V.ptr(target) or nil, nil, V.ptr(mean), V.ptr(epi),
+                                      ale and V.ptr(ale) or nil, nll, rmse))
+   return mean, epi, ale, nll and nll[0] or nil, rmse and rmse[0] or nil
 end
 
 function MLP:calc_lc(opt)                                             -- mlp.lua:109-115

@@ -7,8 +7,8 @@ from . import _lib
 from ._lib import VbnnError, knob, lib
 from .config import default_opt, opts_struct
 from .context import Context, default_context
-from .mlp import MLP, Prediction
+from .mlp import MLP, OutputPrediction, Prediction
 from .vblinear import Linear, VBLinear
 
 __all__ = ["VbnnError", "lib", "knob", "default_opt", "opts_struct", "Context", "default_context", "MLP",
-           "Prediction", "VBLinear", "Linear"]
+           "OutputPrediction", "Prediction", "VBLinear", "Linear"]

@@ -19,6 +19,8 @@ KIND_VB, KIND_LINEAR = 0, 1
  BUF_MU_SQE, BUF_PRIOR_MEANS, BUF_PRIOR_LVARS) = range(16)
 PRIOR_EMPIRICAL, PRIOR_FIXED, PRIOR_PER_WEIGHT = 0, 1, 2
 PRIOR_KINDS = {"empirical": PRIOR_EMPIRICAL, "fixed": PRIOR_FIXED, "per_weight": PRIOR_PER_WEIGHT}
+OUTPUT_RAW, OUTPUT_GAUSSIAN = 0, 1
+OUTPUT_MODELS = {"raw": OUTPUT_RAW, "gaussian": OUTPUT_GAUSSIAN}
 
 
 class VbnnOpts(C.Structure):
@@ -100,6 +102,7 @@ _PROTOS = {
     "vbnn_mlp_join_streams": (C.c_int, [_P]),
     "vbnn_mlp_test": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _F, _F]),
     "vbnn_mlp_predict": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _P, _P, _F, _F]),
+    "vbnn_mlp_predict_outputs": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _F, _F]),
     "vbnn_mlp_get_outputs": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_mlp_launch_count": (C.c_int, [_P, C.POINTER(C.c_longlong)]),
     "vbnn_mlp_graph_captures": (C.c_int, [_P, C.POINTER(C.c_longlong)]),

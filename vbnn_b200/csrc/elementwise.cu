@@ -690,6 +690,101 @@ __global__ void __launch_bounds__(kThreads) k_predict(PredictParams p) {
   if (reduce && threadIdx.x == 0) { p.partials[2 * blockIdx.x] = blk_nll; p.partials[2 * blockIdx.x + 1] = blk_corr; }
 }
 
+// Moments of the raw outputs over sampled forward passes (vbnn_mlp_predict_outputs).  One warp per row as in
+// k_predict; lane l owns the output columns l, l + 32, ...  Per (row, mean column) the state is the first sample's
+// value f0 and the sums of d = m_t - f0 and d^2: f0 is within the spread of the samples, so the variance formed from
+// those sums does not cancel when |mean| >> spread (m_t - f0 is exact by Sterbenz wherever m_t and f0 are within a
+// factor 2).  GAUSSIAN keeps sum_t exp(s_t) in the log-variance column's first state slot and, with targets, a
+// per-row online log-sum-exp (running max, scaled sum) of l_t = sum_k log N(y_k; m_tk, e^{s_tk}).  Samples are
+// folded in order and every sum has a fixed order, so the result depends neither on the chunking nor on the launch.
+__global__ void __launch_bounds__(kThreads) k_predict_moments(MomentsParams p) {
+  const int warps_per_block = blockDim.x >> 5;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int C = p.gaussian ? 2 * p.K : p.K;
+  const float inv_t = 1.f / (float)p.T;
+  const float half_log_2pi = 0.91893853320467274f;
+  const bool reduce = p.last && p.partials;                             // block-uniform
+  double blk_nll = 0.0, blk_se = 0.0;                                   // thread 0: the block's rows in order
+  __shared__ float sh_nll[kThreads / 32], sh_se[kThreads / 32];
+  for (long long r0 = (long long)blockIdx.x * warps_per_block; r0 < p.N;
+       r0 += (long long)gridDim.x * warps_per_block) {
+    const long long n = r0 + w;
+    float my_nll = 0.f, my_se = 0.f;
+    if (n < p.N) {
+      float* s0 = p.st_f0 + n * C;
+      float* s1 = p.st_sum + n * C;
+      float* s2 = p.st_sq + n * C;
+      const float* y = p.targets ? p.targets + n * p.K : nullptr;
+      float lmax = 0.f, lsum = 0.f;
+      if (p.lse && !p.first) { lmax = p.st_lmax[n]; lsum = p.st_lsum[n]; }
+      float se = 0.f;
+      for (int z = 0; z < p.zc; ++z) {
+        const float* x = p.out + ((long long)z * p.N + n) * p.ld_out;
+        const bool init = p.first && z == 0, fin = p.last && z == p.zc - 1;
+        float ll = 0.f;                                                 // this lane's part of l_t
+        for (int k = lane; k < p.K; k += 32) {
+          const float m = x[k];
+          float f0 = m, a = 0.f, b = 0.f;
+          if (!init) {
+            f0 = s0[k];
+            const float d = m - f0;
+            a = s1[k] + d;
+            b = fmaf(d, d, s2[k]);
+          }
+          float sv = 0.f, ev = 0.f;
+          if (p.gaussian) {
+            sv = x[p.K + k];
+            ev = expf(sv);
+            if (!init) ev += s1[p.K + k];
+            if (p.lse) {
+              // log N formed in the log domain: (y - m)^2 e^{-s} as (d e^{-s/2})^2, 0 where y == m
+              const float dy = y[k] - m;
+              const float q = dy == 0.f ? 0.f : dy * expf(-0.5f * sv);
+              ll -= half_log_2pi + 0.5f * (sv + q * q);
+            }
+          }
+          if (!fin) {
+            s0[k] = f0; s1[k] = a; s2[k] = b;
+            if (p.gaussian) s1[p.K + k] = ev;
+            continue;
+          }
+          const float mean = f0 + a * inv_t;
+          if (p.mean_out) p.mean_out[n * p.K + k] = mean;
+          if (p.epi_out) p.epi_out[n * p.K + k] = fmaxf((b - a * (a * inv_t)) * inv_t, 0.f);
+          if (p.ale_out) p.ale_out[n * p.K + k] = ev * inv_t;
+          if (reduce) { const float e = y[k] - mean; se = fmaf(e, e, se); }
+        }
+        if (p.lse) {
+          ll = warp_sum(ll);
+          // l_t = -inf (a density that underflows, (y - m)^2 e^{-s} beyond fp32) adds 0, not exp(-inf + inf) = NaN
+          if (init) { lmax = ll; lsum = 1.f; }
+          else if (ll > lmax) { lsum = lsum * expf(lmax - ll) + 1.f; lmax = ll; }
+          else if (ll > -INFINITY) lsum += expf(ll - lmax);
+        }
+      }
+      if (p.last) {
+        if (reduce) {
+          se = warp_sum(se);
+          if (lane == 0) {
+            my_se = se;
+            my_nll = p.lse ? -((lmax + logf(lsum)) - logf((float)p.T)) : 0.f;
+          }
+        }
+      } else if (p.lse && lane == 0) {
+        p.st_lmax[n] = lmax; p.st_lsum[n] = lsum;
+      }
+    }
+    if (reduce) {
+      if (lane == 0) { sh_nll[w] = my_nll; sh_se[w] = my_se; }
+      __syncthreads();
+      if (threadIdx.x == 0)
+        for (int k = 0; k < warps_per_block; ++k) { blk_nll += sh_nll[k]; blk_se += sh_se[k]; }
+      __syncthreads();
+    }
+  }
+  if (reduce && threadIdx.x == 0) { p.partials[2 * blockIdx.x] = blk_nll; p.partials[2 * blockIdx.x + 1] = blk_se; }
+}
+
 __global__ void k_finalize_result(const float* acc, int Z, int N, float* out2) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     float e = 0.f, a = 0.f;
@@ -1058,6 +1153,16 @@ int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st) {
   long long blocks = ((long long)p.N + wpb - 1) / wpb;
   if (blocks > kMaxPartials) blocks = kMaxPartials;
   k_predict<<<(int)blocks, kThreads, 0, st>>>(p);
+  VB_CUDA(cudaGetLastError());
+  if (grid_out) *grid_out = (int)blocks;
+  return VBNN_OK;
+}
+
+int launch_predict_moments(const MomentsParams& p, int* grid_out, cudaStream_t st) {
+  const int wpb = kThreads / 32;
+  long long blocks = ((long long)p.N + wpb - 1) / wpb;
+  if (blocks > kMaxPartials) blocks = kMaxPartials;
+  k_predict_moments<<<(int)blocks, kThreads, 0, st>>>(p);
   VB_CUDA(cudaGetLastError());
   if (grid_out) *grid_out = (int)blocks;
   return VBNN_OK;

@@ -144,6 +144,26 @@ struct PredictParams {
 // returns the grid in *grid_out (the number of partial pairs written)
 int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st);
 
+// Moments of the raw outputs over sampled forward passes (vbnn_mlp_predict_outputs), one chunk of zc samples per
+// launch.  K output columns (RAW: C = K; GAUSSIAN: C = 2K, columns [0, K) means m, [K, 2K) log-variances s).  Per
+// (row, mean column) the state is the first sample's value f0, sum_t (m_t - f0) and sum_t (m_t - f0)^2; per (row,
+// log-variance column) sum_t exp(s_t) in st_sum; per row (lse) an online log-sum-exp of sum_k log N(y_k; m_tk, e^s_tk).
+// The first chunk initialises the state, the last one writes the outputs instead of storing it.
+struct MomentsParams {
+  const float* out; int ld_out;         // [zc*N x ld] raw outputs of this chunk
+  int N, K, gaussian, zc;
+  int first, last;                      // this chunk starts / ends the average
+  int T;                                // samples averaged in all
+  float *st_f0, *st_sum, *st_sq;        // [N x C]
+  float *st_lmax, *st_lsum;             // [N] (lse)
+  int lse;                              // GAUSSIAN with targets on every chunk: keep the per-row mixture likelihood
+  float *mean_out, *epi_out, *ale_out;  // nullable [N x K] (last chunk)
+  const float* targets;                 // nullable dense [N x K]
+  double* partials;                     // nullable [grid x 2] per-block {sum_n -log p-bar, sum (y - mean)^2} (last chunk)
+};
+// returns the grid in *grid_out (the number of partial pairs written)
+int launch_predict_moments(const MomentsParams& p, int* grid_out, cudaStream_t st);
+
 // gradBias += column sums of G over all rows (nn.Linear:accGradParameters addmv)
 int launch_colsum(const void* G, int is_bf16, long long rows, int cols, int ld, float scale,
                   float* gb, cudaStream_t st);

@@ -622,9 +622,11 @@ int refuse_open_step(const vbnn_mlp* m, const char* who) {
 // The evaluation forward of vbnn_mlp_test and vbnn_mlp_predict (mlp.lua:86-107): stage the input, wait for the
 // peers' parameters, then one MAP pass (n_samples == 0, quicktest) or n_samples sampled passes in chunks of Z whose
 // noise indices (1 << 20) + t never reuse a training sample.  consume(zc, first, last) runs after each chunk.
+// samples (vbnn_mlp_predict_outputs): the output layer's epilogue stores sample t into the caller's dense
+// [T x N x C] buffer at t * N * C instead of `logits`; the caller resets m->ext_logits afterwards, error or not.
 template <typename Consume>
 int eval_forward(vbnn_mlp* m, const float* X, const float* T, int N, int n_samples, const char* who,
-                 Consume&& consume) {
+                 Consume&& consume, float* samples = nullptr) {
   VB_TRY(stage_input(m, X, T, N));
   if (m->peer && m->peer->active) {
     VB_CHECK(n_samples > 0 || !m->peer->stale, VBNN_E_STATE,
@@ -632,7 +634,9 @@ int eval_forward(vbnn_mlp* m, const float* X, const float* T, int N, int n_sampl
     VB_TRY(peer_wait_params(m, -1, false));
   }
   const int Lc = nlayers(m);
+  const long long C = m->sizes.back();
   if (n_samples == 0) {
+    if (samples) m->ext_logits = samples;
     VB_TRY(clamp_all(m));                                                    // mlp.lua:88-90 (quicktest)
     for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, 1, 0, true));
     VB_TRY(consume(1, true, true));
@@ -642,6 +646,7 @@ int eval_forward(vbnn_mlp* m, const float* X, const float* T, int N, int n_sampl
   const int base = 1 << 20;                                                  // test noise never reuses train samples
   for (int s0 = 0; s0 < n_samples; s0 += m->Z) {                             // mlp.lua:94-100
     const int zc = n_samples - s0 < m->Z ? n_samples - s0 : m->Z;
+    if (samples) m->ext_logits = samples + (long long)s0 * N * C;
     VB_TRY(sample_all(m, base + s0, zc));
     for (int j = 0; j < Lc; ++j) VB_TRY(forward_layer(m, j, N, zc, base + s0, false));
     VB_TRY(consume(zc, s0 == 0, s0 + zc == n_samples));
@@ -665,6 +670,21 @@ int prof_launch(vbnn_ctx* c, int cls, double work, Launch&& launch) {
   c->prof_recs.push_back(r);
   if (c->prof_recs.size() + c->marks.size() >= 4096) VB_TRY(prof_collect(c));
   return VBNN_OK;
+}
+
+// the first call of an evaluation entry point allocates its state: not while the stream is being captured
+int refuse_capture(cudaStream_t st, const char* who) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  VB_CUDA(cudaStreamIsCapturing(st, &cs));
+  VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE, "%s: the first call allocates its state and cannot be captured",
+           who);
+  return VBNN_OK;
+}
+
+// per-block {sum, sum} partials of vbnn_mlp_predict and vbnn_mlp_predict_outputs [kMaxPartials x 2]
+int ensure_pred_partials(vbnn_mlp* m) {
+  if (m->pred_partials) return VBNN_OK;
+  return dalloc(&m->pred_partials, (size_t)kMaxPartials * 2 * sizeof(double));
 }
 
 }  // namespace
@@ -798,6 +818,7 @@ extern "C" int vbnn_mlp_destroy(vbnn_mlp* m) {
   if (m->pred_sum) cudaFree(m->pred_sum);
   if (m->pred_ent) cudaFree(m->pred_ent);
   if (m->pred_partials) cudaFree(m->pred_partials);
+  if (m->mom_state) cudaFree(m->mom_state);
   if (m->targets) cudaFree(m->targets);
   if (m->result_acc) cudaFree(m->result_acc);
   if (m->result) cudaFree(m->result);
@@ -1116,17 +1137,14 @@ extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_sample
   cudaStream_t st = c->stream;
   VB_CUDA(cudaSetDevice(c->device));
   const int C = m->sizes.back();
-  if (!m->pred_partials) {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    VB_CUDA(cudaStreamIsCapturing(st, &cs));
-    VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE,
-             "vbnn_mlp_predict: the first call allocates its state and cannot be captured");
-    for (float** q : {&m->pred_max, &m->pred_sum, &m->pred_ent})
+  if (!m->pred_ent) {                     // allocated last: set only once all of predict's state is
+    VB_TRY(refuse_capture(st, "vbnn_mlp_predict"));
+    VB_TRY(ensure_pred_partials(m));
+    for (float** q : {&m->pred_max, &m->pred_sum})
       if (*q) { cudaFree(*q); *q = nullptr; }
     VB_TRY(dalloc(&m->pred_max, (size_t)m->max_batch * C * 4));
     VB_TRY(dalloc(&m->pred_sum, (size_t)m->max_batch * C * 4));
     VB_TRY(dalloc(&m->pred_ent, (size_t)m->max_batch * 4));
-    VB_TRY(dalloc(&m->pred_partials, (size_t)kMaxPartials * 2 * sizeof(double)));
   }
   const bool reduce = nll_host || acc_host;
   int grid = 0;
@@ -1154,6 +1172,75 @@ extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_sample
     for (int b = 0; b < grid; ++b) { nll += c->h_partials[2 * b]; corr += c->h_partials[2 * b + 1]; }   // fixed order
     if (nll_host) *nll_host = (float)(nll / N);
     if (acc_host) *acc_host = (float)(corr / N * 100.0);
+  }
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_predict_outputs(vbnn_mlp* m, const float* X, int N, int n_samples, int output_model,
+                                        const float* targets, float* samples_dev, float* mean_dev, float* epi_dev,
+                                        float* ale_dev, float* nll_host, float* rmse_host) {
+  VB_CHECK(m && X, VBNN_E_INVALID, "vbnn_mlp_predict_outputs: null argument");
+  VB_CHECK(N > 0 && N <= m->max_batch && n_samples >= 0, VBNN_E_INVALID,
+           "vbnn_mlp_predict_outputs: N=%d (max_batch %d), n_samples=%d", N, m->max_batch, n_samples);
+  VB_CHECK(output_model == VBNN_OUTPUT_RAW || output_model == VBNN_OUTPUT_GAUSSIAN, VBNN_E_INVALID,
+           "vbnn_mlp_predict_outputs: unknown output model %d", output_model);
+  const int C = m->sizes.back();
+  const bool gaussian = output_model == VBNN_OUTPUT_GAUSSIAN;
+  VB_CHECK(!gaussian || C % 2 == 0, VBNN_E_INVALID,
+           "vbnn_mlp_predict_outputs: VBNN_OUTPUT_GAUSSIAN needs an even number of outputs, the net has %d", C);
+  VB_CHECK(gaussian || !(ale_dev || nll_host), VBNN_E_INVALID,
+           "vbnn_mlp_predict_outputs: aleatoric variance and nll need VBNN_OUTPUT_GAUSSIAN");
+  VB_CHECK(targets || !(nll_host || rmse_host), VBNN_E_INVALID, "vbnn_mlp_predict_outputs: nll / rmse need targets");
+  VB_CHECK((reinterpret_cast<uintptr_t>(samples_dev) & 15) == 0, VBNN_E_INVALID,
+           "vbnn_mlp_predict_outputs: samples_dev must be 16-byte aligned");
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_predict_outputs"));
+  vbnn_ctx* c = m->ctx;
+  cudaStream_t st = c->stream;
+  VB_CUDA(cudaSetDevice(c->device));
+  if (!m->mom_state) {
+    VB_TRY(refuse_capture(st, "vbnn_mlp_predict_outputs"));
+    VB_TRY(ensure_pred_partials(m));
+    VB_TRY(dalloc(&m->mom_state, (size_t)m->max_batch * (3 * (size_t)C + 2) * 4));
+  }
+  const int K = gaussian ? C / 2 : C;
+  const size_t NC = (size_t)N * C;
+  const bool reduce = nll_host || rmse_host;
+  const bool lse = gaussian && nll_host;
+  int grid = 0, done = 0;
+  auto consume = [&](int zc, bool first, bool last) -> int {
+    MomentsParams p;
+    memset(&p, 0, sizeof(p));
+    if (samples_dev) { p.out = samples_dev + (size_t)done * NC; p.ld_out = C; }
+    else { p.out = m->logits; p.ld_out = m->ld_logits; }
+    done += zc;
+    p.N = N; p.K = K; p.gaussian = gaussian; p.zc = zc; p.first = first; p.last = last;
+    p.T = n_samples == 0 ? 1 : n_samples;
+    p.st_f0 = m->mom_state; p.st_sum = p.st_f0 + NC; p.st_sq = p.st_sum + NC;
+    p.st_lmax = p.st_sq + NC; p.st_lsum = p.st_lmax + N;
+    p.lse = lse;
+    p.targets = lse || (last && rmse_host) ? targets : nullptr;
+    if (last) {
+      p.mean_out = mean_dev; p.epi_out = epi_dev; p.ale_out = ale_dev;
+      p.partials = reduce ? m->pred_partials : nullptr;
+    }
+    // profile class 8; its "flops" slot holds the algorithmic bytes, counted as if every sample read and wrote the
+    // state: per (row, sample) 28 B per mean column (4 B output, 12 B state read, 12 B written) and, under GAUSSIAN,
+    // 12 B per log-variance column (4 B output, 4 B state read, 4 B written)
+    const double bytes = (double)zc * N * (gaussian ? 40.0 * K : 28.0 * C);
+    return prof_launch(c, 8, bytes, [&] { return launch_predict_moments(p, &grid, st); });
+  };
+  const int r = eval_forward(m, X, nullptr, N, n_samples, "vbnn_mlp_predict_outputs", consume, samples_dev);
+  m->ext_logits = nullptr;
+  if (samples_dev) m->outputs_external = true;      // get_outputs: the outputs are in the caller's buffer
+  VB_TRY(r);
+  if (reduce) {
+    VB_CUDA(cudaMemcpyAsync(c->h_partials, m->pred_partials, (size_t)grid * 2 * sizeof(double), cudaMemcpyDeviceToHost,
+                            st));
+    VB_CUDA(cudaStreamSynchronize(st));
+    double nll = 0, se = 0;
+    for (int b = 0; b < grid; ++b) { nll += c->h_partials[2 * b]; se += c->h_partials[2 * b + 1]; }   // fixed order
+    if (nll_host) *nll_host = (float)(nll / N);
+    if (rmse_host) *rmse_host = (float)sqrt(se / ((double)N * K));
   }
   return VBNN_OK;
 }

@@ -129,7 +129,10 @@ struct vbnn_mlp {
   // vbnn_mlp_predict state, allocated by the first call: log-sum-exp max / sum [max_batch x C], entropy sum
   // [max_batch], per-block {nll, correct} partials [kMaxPartials x 2]
   float *pred_max = nullptr, *pred_sum = nullptr, *pred_ent = nullptr;
-  double* pred_partials = nullptr;
+  double* pred_partials = nullptr;   // shared with vbnn_mlp_predict_outputs
+  // vbnn_mlp_predict_outputs state, allocated by its first call: {f0, sum d, sum d^2} [3 x max_batch x C], then the
+  // per-row log-sum-exp max / sum [2 x max_batch]
+  float* mom_state = nullptr;
   float* targets = nullptr;          // staged targets [N]
   float* xstage[2] = {nullptr, nullptr};   // fp32 H2D staging for the host-buffer API
   float* tstage[2] = {nullptr, nullptr};

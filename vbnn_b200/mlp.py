@@ -24,6 +24,16 @@ class Prediction(NamedTuple):
     accuracy: Optional[float]             # % argmax p-bar == target
 
 
+class OutputPrediction(NamedTuple):
+    """MLP.predict_outputs's result over the N input rows (K = C raw, C / 2 gaussian); None where not asked for."""
+    mean: "torch.Tensor"                  # [N x K] mean_t m_t
+    epistemic: "torch.Tensor"             # [N x K] mean_t (m_t - mean)^2: variance over the weight posterior
+    aleatoric: Optional["torch.Tensor"]   # [N x K] mean_t exp(s_t) (gaussian): the head's noise variance
+    samples: Optional["torch.Tensor"]     # [T x N x C] every sampled raw output (return_samples)
+    nll: Optional[float]                  # mean -log p-bar(y | x) of the per-row Gaussian mixture (gaussian, targets)
+    rmse: Optional[float]                 # sqrt(mean (y - mean)^2) (targets)
+
+
 class MLP:
     def __init__(self, opt=None, ctx: Context = None, max_batch=None):
         self.handle = None
@@ -153,6 +163,46 @@ class MLP:
                                          C.byref(acc) if want else None))
         return Prediction(logp, unc[:, 0], unc[:, 1], unc[:, 2], unc[:, 3].long(),
                           nll.value if want else None, acc.value if want else None)
+
+    def predict_outputs(self, inputs, n_samples=None, model="raw", targets=None, return_samples=False):
+        """Model average of the raw outputs for regression heads (vbnn_mlp_predict_outputs): the sampled forward
+        passes of predict(), read without LogSoftMax.  model "raw": the C outputs are the prediction (K = C);
+        "gaussian": C = 2K, columns [0, K) are means and [K, 2K) log-variances of a heteroscedastic Gaussian, as
+        trained under gaussian_nll_loss(Y[..., :K], y, Y[..., K:].exp()).  n_samples defaults as in predict().
+        targets: [N x K] regression targets, which add rmse and, under "gaussian", the mixture's mean NLL.  Returns an
+        OutputPrediction; the predictive variance is epistemic + aleatoric.  Parameters, optimiser state and the step
+        counter are left as they are."""
+        import torch
+        if model not in L.OUTPUT_MODELS:
+            raise L.VbnnError(L.E_INVALID, f"model must be 'raw' or 'gaussian', got {model!r}")
+        gaussian = model == "gaussian"
+        x = as_dev_f32(inputs, self.ctx.device)
+        x = x.reshape(x.shape[0], -1)
+        if x.shape[1] != self.sizes[0]:
+            raise L.VbnnError(L.E_INVALID, f"inputs must be [N x {self.sizes[0]}]")
+        if n_samples is None:
+            n_samples = 0 if self.opt.get("quicktest") else int(self.opt["testSamples"])
+        n, c = x.shape[0], self.sizes[-1]
+        k = c // 2 if gaussian else c
+        t = None
+        if targets is not None:
+            t = as_dev_f32(targets, self.ctx.device).reshape(n, -1)
+            if t.shape[1] != k:
+                raise L.VbnnError(L.E_INVALID, f"targets must be [N x {k}]")
+        dev = x.device
+        mean = torch.empty(n, k, dtype=torch.float32, device=dev)
+        epi = torch.empty(n, k, dtype=torch.float32, device=dev)
+        ale = torch.empty(n, k, dtype=torch.float32, device=dev) if gaussian else None
+        smp = torch.empty(max(int(n_samples), 1), n, c, dtype=torch.float32, device=dev) if return_samples else None
+        nll, rmse = C.c_float(), C.c_float()
+        want_nll = t is not None and gaussian
+        ptr = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
+        L.check(L.lib().vbnn_mlp_predict_outputs(self.handle, ptr(x), n, int(n_samples), L.OUTPUT_MODELS[model], ptr(t),
+                                                 ptr(smp), ptr(mean), ptr(epi), ptr(ale),
+                                                 C.byref(nll) if want_nll else None,
+                                                 C.byref(rmse) if t is not None else None))
+        return OutputPrediction(mean, epi, ale, smp, nll.value if want_nll else None,
+                                rmse.value if t is not None else None)
 
     def calc_lc(self, opt=None):                                        # mlp.lua:109-115
         v = C.c_float()

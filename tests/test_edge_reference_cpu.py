@@ -187,3 +187,127 @@ def test_minibatch_matches_split_reference():
                 assert torch.allclose(out[f"gW{k}"][0], l.gradWeight, rtol=1e-12, atol=1e-15)
             for key, (v, e) in out.items():
                 assert torch.isfinite(v).all() and torch.isfinite(e).all(), key
+
+
+# ---------------------------------------------------------------- the exactness rule
+def _ternary(rng, shape, density=0.5):
+    return torch.from_numpy(rng.choice([-1.0, 1.0], size=shape) * (rng.rand(*shape) < density))
+
+
+def test_exact_operands_any_order():
+    """Ternary operands at K = 8192: an fp32 sum in each of three orders equals fp64 exactly and the exactness rule
+    gives the bound 0; one off-grid operand element restores the old bound on its row; under the zero bound a dropped
+    64-wide k-block or a row written one row off is flagged."""
+    rng = np.random.RandomState(9)
+    M, N, K = 12, 10, 8192
+    A, B = _ternary(rng, (M, K)), _ternary(rng, (N, K))
+    ref = A @ B.t()
+    bound = E.contraction_bound(A, B)
+    assert float(bound.abs().max()) == 0.0
+    for order in ("matmul", "reverse", "blocks"):
+        got = _fp32_sum(A, B, order)
+        assert torch.equal(got, ref), order
+        assert E.violations(got.numpy(), ref, bound) == [], order
+    A2 = A.clone()
+    A2[3, 100] = 0.5 + 2.0 ** -9                                    # a bf16 value off the integer grid
+    b2 = E.contraction_bound(A2, B)
+    assert float(b2[3].min()) > 0 and float(b2[[i for i in range(M) if i != 3]].abs().max()) == 0.0
+    old = E.C_ACC * ((A2[3].abs() > 0).double() @ (B.abs() > 0).double().t()) * E.U32 * (A2[3].abs() @ B.abs().t())
+    assert torch.allclose(b2[3], old + ((A2[3].abs() > 0).double() @ (B.abs() > 0).double().t()) * E.ETA, rtol=1e-15)
+    e = torch.zeros_like(A); e[5, 7] = 1e-3                          # an operand error does the same
+    assert float(E.contraction_bound(A, B, e, None)[5].min()) > 0
+    part = A[7, 64:128] @ B[:, 64:128].t()
+    j = int(part.abs().argmax())
+    assert float(part[j]) != 0
+    got = _fp32_sum(A, B, "blocks").clone()
+    got[7, j] -= float(part[j])
+    assert [x[0] for x in E.violations(got.numpy(), ref, bound)] == [(7, j)]
+    got = _fp32_sum(A, B, "matmul").clone()
+    got[4] = got[5].clone()
+    v = E.violations(got.numpy(), ref, bound)
+    assert len(v) >= 1 and all(x[0][0] == 4 for x in v if x[0] != "...")
+    # past 2^24 the rule does not apply: a sum of 2^25 ones
+    big = torch.ones(1, 2 ** 25, dtype=torch.float64)
+    assert float(E.contraction_bound(big, big)) > 0
+
+
+def _exact_oracle(sizes, N, S, reparam, vb_output, seed):
+    """An oracle net with integer means / weights and biases and sigma flushed to 0, and its minibatch inputs."""
+    opt = O.default_opt(input_size=sizes[0], hidden=list(sizes[1:-1]), classes=[str(i) for i in range(sizes[-1])],
+                        S=S, B=10.0, mu_init=1, var_init=0.01, reparam=reparam, vb_output=vb_output,
+                        strict_reference=False)
+    ref = O.MLPOracle(opt, torch.float64, seed=3, operand_round=O.round_bf16)
+    rng = np.random.RandomState(seed)
+    params = []
+    for l in ref.vb + [ref.out]:
+        W = _ternary(rng, (l.weight.shape[0], l.weight.shape[1]), 0.3)
+        b = torch.from_numpy(rng.randint(-2, 3, l.bias.shape[0]).astype(np.float64))
+        if isinstance(l, O.VBLinearOracle):
+            l.means.copy_(W); l.lvars.fill_(-300.0); l.compute_prior()
+        else:
+            l.weight.copy_(W)
+        l.bias.copy_(b)
+        params.append((W, b))
+    x = _ternary(rng, (N, sizes[0]))
+    G = _ternary(rng, (S, N, sizes[-1]), 0.25)
+    lrt = reparam == "local"
+    noise = [[torch.from_numpy(rng.randn(*((N, l.O) if lrt else (l.O, l.I)))) for l in ref.vb_all] for _ in range(S)]
+    return ref, opt, params, x, G, noise
+
+
+def test_exact_minibatch_is_the_edge_reference():
+    """On exact operands with sigma flushed to 0, tests/edge_reference.py's minibatch gives bound 0 on logits, dX,
+    gW, gB (and gS under local reparameterisation), and exact_minibatch -- the plain fp64 chain the multi-wave GPU
+    tests use at full size -- reproduces its values bit for bit; weight-mode gradSum agrees with it in value and
+    bound."""
+    sizes, N, S = [40, 24, 20, 6], 64, 2
+    for reparam in ("weight", "local"):
+        for vb_output in (False, True):
+            ref, opt, params, x, G, noise = _exact_oracle(sizes, N, S, reparam, vb_output, seed=12)
+            lrt = reparam == "local"
+            want = E.mlp_minibatch(ref, x, G, noise, lrt, bf=True, strict=False, opt=opt)
+            vb = [True] * (len(sizes) - 2) + [vb_output]
+            eps = None if lrt else [[noise[s][k] if vb[k] else None for k in range(len(vb))] for s in range(S)]
+            got = E.exact_minibatch(x, params, G, lrt, vb, eps)
+            assert max(got["worst"].values()) < E.EXACT
+            for key, (v, e) in want.items():
+                gv, ge = got[key]
+                assert torch.equal(gv, v), (reparam, vb_output, key)
+                if key.startswith("gS") and not lrt:
+                    assert float(e.max()) > 0
+                    assert torch.allclose(ge, e, rtol=1e-12, atol=0), (reparam, vb_output, key)
+                else:
+                    assert float(e.abs().max()) == 0.0, (reparam, vb_output, key, float(e.max()))
+                    assert float(ge.abs().max()) == 0.0
+
+
+def test_exact_minibatch_refuses_past_2_24():
+    """exact_minibatch asserts the 2^24 condition instead of trusting an estimate."""
+    X = torch.ones(4, 8, dtype=torch.float64)
+    W = torch.full((3, 8), 2.0 ** 22, dtype=torch.float64)
+    G = torch.ones(1, 4, 3, dtype=torch.float64)
+    with np.testing.assert_raises(AssertionError):
+        E.exact_minibatch(X, [(W, torch.zeros(3, dtype=torch.float64))], G, True, [False])
+
+
+def test_exactness_across_samples_counts_terms():
+    """The cross-sample rule tests the magnitudes of the terms the device may sum in one fp32 accumulator, not of the
+    per-sample results: terms 2^23 .. 2^16 in sample 1 (sum 16711680) and +65536, +1, -65536 in sample 2 (sum 1) have
+    results summing below 2^24, yet one fp32 accumulator over all terms loses the 1."""
+    lyr = O.LinearOracle(1, 1, torch.float64)
+    lyr.weight.fill_(1.0); lyr.bias.zero_()
+    ps = E.LayerPass(lyr, bf=False)
+    lyr.gradWeight.zero_(); lyr.gradBias.zero_()
+    for xs in ([2.0 ** k for k in range(23, 15, -1)], [65536.0, 1.0, -65536.0]):
+        x = torch.tensor(xs, dtype=torch.float64)[:, None]
+        g = torch.ones_like(x)
+        ps.forward(x, torch.zeros_like(x))
+        ps.backward(g, torch.zeros_like(g))
+    ew, _, eb = ps.grad_bounds()
+    want = float(lyr.gradWeight[0, 0])
+    assert want == 16711681.0
+    fused = np.float32(0)
+    for v in [2.0 ** k for k in range(23, 15, -1)] + [65536.0, 1.0, -65536.0]:
+        fused = np.float32(fused + np.float32(v))
+    assert float(fused) != want and abs(float(fused) - want) <= float(ew[0, 0])
+    assert float(eb[0]) == 0.0                                       # 11 ones: exact

@@ -3,7 +3,10 @@
 // Every knob has a measured-best default; the environment variable VBNN_<NAME> (read once per
 // process) or vbnn_debug_knob("<name>", value) (include/vbnn.h, self-test hooks; what the parity
 // tests use to force a tile shape or a GEMM form in-process) overrides it.  None of them changes
-// results beyond fp32 summation order.
+// results beyond fp32 summation order, except dw_eps16, which also rounds epsilon to fp16 in the
+// weight-mode gradSum (<= 2^-11 relative per product).  On operands where every fp32 partial sum is
+// exact, every GEMM knob gives bit-identical logits, dX, gradWeight and gradBias
+// (tests/test_gpu_multiwave.py).
 #pragma once
 
 namespace vbnn {

@@ -15,6 +15,18 @@
 
 namespace vbnn {
 
+// The kernel's view of GemmArgs: element (m,k) of A at A[m*sAm + k*sAk], (k,n) of B at B[k*sBk + n*sBn].
+struct SimtGemmArgs {
+  const float* A1; long long sA1m, sA1k, zsA1;
+  const float* B1; long long sB1n, sB1k, zsB1;
+  const float* A2; long long sA2m, sA2k, zsA2;
+  const float* B2; long long sB2n, sB2k, zsB2;
+  int M, N, K;
+  // > 1: sum the products of samples z = 0 .. zsum-1 into ONE output (z = 0 of the epilogue), register
+  // accumulation in a fixed order; launch with batch = 1
+  int zsum;
+};
+
 constexpr int TM = 64, TN = 64, TK = 16;
 __device__ __forceinline__ int ceil_div_dev(int a, int b) { return (a + b - 1) / b; }
 __device__ __forceinline__ int round_up_dev(int a, int b) { return (a + b - 1) / b * b; }
@@ -217,8 +229,26 @@ static int launch_mode(const SimtGemmArgs& g, const EpiParams& p, int batch, cud
   return launch_one<MODE>(g, p, batch, st);
 }
 
-int gemm_simt_launch(int mode, const SimtGemmArgs& g, const EpiParams& p, int batch,
-                     cudaStream_t st, long long* launches) {
+// A (m,k) / B (k,n) of a GemmOperand as a stride pair
+static void simt_operand(const GemmOperand& o, const float** ptr, long long* s_mn, long long* s_k, long long* zs) {
+  *ptr = static_cast<const float*>(o.ptr);
+  *s_mn = o.kmajor ? o.ld : 1;
+  *s_k = o.kmajor ? 1 : o.ld;
+  *zs = o.zs;
+}
+
+int gemm_simt_launch(int mode, const GemmArgs& a, const EpiParams& p, cudaStream_t st, long long* launches) {
+  SimtGemmArgs g = {};
+  simt_operand(a.A1, &g.A1, &g.sA1m, &g.sA1k, &g.zsA1);
+  simt_operand(a.B1, &g.B1, &g.sB1n, &g.sB1k, &g.zsB1);
+  if (epi_is_dual(mode)) {
+    simt_operand(a.A2, &g.A2, &g.sA2m, &g.sA2k, &g.zsA2);
+    simt_operand(a.B2, &g.B2, &g.sB2n, &g.sB2k, &g.zsB2);
+  }
+  g.M = a.M; g.N = a.N; g.K = a.K;
+  // the sample-summing form runs the samples inside one CTA: zsum = batch, launched with batch 1
+  g.zsum = a.zsum ? a.batch : 0;
+  const int batch = a.zsum ? 1 : a.batch;
   VB_CHECK(g.zsum <= 1 || (batch == 1 && !epi_z_accumulates(mode)), VBNN_E_INVALID,
            "gemm_simt: the sample-summing form runs with batch 1 and no dW mode");
   if (launches) {

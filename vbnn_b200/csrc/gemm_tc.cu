@@ -778,7 +778,7 @@ PFN_encodeTiled get_encode() {
 }
 
 // rows_mn: MN extent, K: contraction extent, box_mn: tile rows for a K-major operand
-int make_tmap(CUtensorMap* tm, const TcOperand& op, int rows_mn, int K, int batch, int box_mn) {
+int make_tmap(CUtensorMap* tm, const GemmOperand& op, int rows_mn, int K, int batch, int box_mn) {
   PFN_encodeTiled enc = get_encode();
   VB_CHECK(enc != nullptr, VBNN_E_CUDA, "cuTensorMapEncodeTiled unavailable (no CUDA driver?)");
   VB_CHECK(op.ptr != nullptr, VBNN_E_INVALID, "gemm_tc: null operand");
@@ -799,7 +799,7 @@ int make_tmap(CUtensorMap* tm, const TcOperand& op, int rows_mn, int K, int batc
   box[2] = 1;
   strides[0] = (cuuint64_t)op.ld * 2;
   strides[1] = batched ? (cuuint64_t)op.zs * 2 : strides[0] * dims[1];
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<bf16*>(op.ptr), dims, strides,
+  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(op.ptr), dims, strides,
                    box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VB_CHECK(r == CUDA_SUCCESS, VBNN_E_CUDA,
@@ -810,11 +810,9 @@ int make_tmap(CUtensorMap* tm, const TcOperand& op, int rows_mn, int K, int batc
 }
 
 struct TcChoice { int bn, cg; };   // bn == 64: multi-sample dW with register accumulation
-int g_block_n_override = 0;
-int g_cg_override = 0;
 
 template <int MODE, int BN, int CG, bool AK, bool BKM>
-int launch_cfg(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
+int launch_cfg(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
   using C = TcCfg<MODE, BN, CG>;
   TcShape sh;
   sh.M = g.M; sh.N = g.N; sh.K = g.K; sh.batch = g.batch;
@@ -888,9 +886,9 @@ int launch_cfg(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
 // problem has enough 256 x 256 tiles to fill the 74 pairs; small problems quantise better on
 // 128 x 128 single-CTA tiles.  cost = waves x (tile MACs / relative per-MAC speed).
 template <int MODE>
-TcChoice choose_cfg(const TcGemmArgs& g) {
+TcChoice choose_cfg(const GemmArgs& g) {
   const Knobs& k = knobs();
-  TcChoice c{g_block_n_override ? g_block_n_override : k.tc_bn, g_cg_override ? g_cg_override : k.tc_cg};
+  TcChoice c{k.tc_bn, k.tc_cg};
   if ((c.bn == 128 || c.bn == 256) && (c.cg == 1 || c.cg == 2) && !(c.bn == 128 && c.cg == 2 && !epi_is_dual(MODE))) return c;
   if (epi_z_accumulates(MODE) && g.batch > 1) {
     // TMEM-resident accumulators: 128 x 128 tiles (1), or 256 x 128 CTA-pair tiles (2) when M allows
@@ -909,7 +907,7 @@ TcChoice choose_cfg(const TcGemmArgs& g) {
 }
 
 template <int MODE, bool AK, bool BKM>
-int launch_any(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
+int launch_any(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
   const TcChoice c = choose_cfg<MODE>(g);
   if constexpr (epi_z_accumulates(MODE)) {
     if (c.bn == 64) return launch_cfg<MODE, 64, 1, AK, BKM>(g, p, st);
@@ -928,10 +926,7 @@ int launch_any(const TcGemmArgs& g, const EpiParams& p, cudaStream_t st) {
 
 }  // namespace
 
-void gemm_tc_set_debug(int block_n_override) { g_block_n_override = block_n_override; }
-
-int gemm_tc_launch(int mode, const TcGemmArgs& g, const EpiParams& p, cudaStream_t st,
-                   long long* launches) {
+int gemm_tc_launch(int mode, const GemmArgs& g, const EpiParams& p, cudaStream_t st, long long* launches) {
   VB_CHECK(g.M > 0 && g.N > 0 && g.K > 0 && g.batch > 0, VBNN_E_INVALID,
            "gemm_tc: empty problem %d x %d x %d (batch %d)", g.M, g.N, g.K, g.batch);
   VB_CHECK(!g.zsum || !epi_z_accumulates(mode), VBNN_E_INVALID, "gemm_tc: the dW modes already sum over z");

@@ -21,17 +21,6 @@ void set_error(const char* fmt, ...) {
 }
 
 template <typename T>
-static int dev_alloc(T** p, size_t count) {
-  *p = nullptr;
-  if (count == 0) return VBNN_OK;
-  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-  if (e != cudaSuccess) {
-    set_error("cudaMalloc(%zu bytes) failed: %s", count * sizeof(T), cudaGetErrorString(e));
-    return e == cudaErrorMemoryAllocation ? VBNN_E_NOMEM : VBNN_E_CUDA;
-  }
-  return VBNN_OK;
-}
-template <typename T>
 static int dev_zalloc(T** p, size_t count, cudaStream_t st) {
   VB_TRY(dev_alloc(p, count));
   if (count) VB_CUDA(cudaMemsetAsync(*p, 0, count * sizeof(T), st));
@@ -50,14 +39,11 @@ PhiloxStream layer_stream(const vbnn_layer* L, uint32_t kind, int sample) {
 }
 
 static inline bool is_bf16(const vbnn_layer* L) { return L->opts.precision == VBNN_PREC_BF16; }
-static inline bool is_lrt(const vbnn_layer* L) {
-  return L->kind == VBNN_KIND_VB && L->opts.reparam == VBNN_REPARAM_LOCAL;
-}
 static inline size_t esz(const vbnn_layer* L) { return is_bf16(L) ? 2 : 4; }
 // peer mode: mu / log sigma^2 of rows owned by other ranks are only kept current when the forward pass
 // needs them in fp32 (weight sampling); otherwise whole-layer reads need vbnn_mlp_sync_replicas first
 static int check_params_fresh(const vbnn_layer* L, const char* what) {
-  VB_CHECK(!(L->shard_stale && *L->shard_stale && is_lrt(L)), VBNN_E_STATE,
+  VB_CHECK(!(L->shard_stale && *L->shard_stale && layer_is_lrt(L)), VBNN_E_STATE,
            "%s in peer mode: rows owned by other ranks are out of date; call vbnn_mlp_sync_replicas on every rank first", what);
   return VBNN_OK;
 }
@@ -124,7 +110,7 @@ int layer_create_internal(vbnn_ctx* ctx, int I, int O, int kind, const vbnn_opts
   L->n_part = update_grid(O, I);
   cudaStream_t st = ctx->stream;
   const size_t W = (size_t)O * I;
-  const bool vb = kind == VBNN_KIND_VB, b16 = is_bf16(L), lrt = is_lrt(L);
+  const bool vb = kind == VBNN_KIND_VB, b16 = is_bf16(L), lrt = layer_is_lrt(L);
   int r = VBNN_OK;
 #define A_(expr) do { if (r == VBNN_OK) r = (expr); } while (0)
   A_(dev_zalloc(&L->bias, O, st));
@@ -184,7 +170,7 @@ static int ensure_scratch(vbnn_layer* L, int N) {
   char* p;
   VB_TRY(dev_alloc(&p, (size_t)N * L->ldI * e)); L->xs = p;
   VB_TRY(dev_alloc(&p, (size_t)N * L->ldO * e)); L->gs_ = p;
-  if (is_lrt(L)) {
+  if (layer_is_lrt(L)) {
     VB_TRY(dev_alloc(&p, (size_t)N * L->ldI * e)); L->xs2 = p;
     VB_TRY(dev_alloc(&p, (size_t)N * L->ldO * e)); L->hs = p;
     VB_TRY(dev_alloc(&p, (size_t)N * L->ldO * e)); L->R = p;
@@ -197,13 +183,22 @@ static int ensure_scratch(vbnn_layer* L, int N) {
 static int stage_x(vbnn_layer* L, const float* X, int N) {
   cudaStream_t st = L->ctx->stream;
   if (is_bf16(L)) {
-    VB_TRY(launch_cast(X, L->I, N, L->I, (bf16*)L->xs, is_lrt(L) ? (bf16*)L->xs2 : nullptr, L->ldI, st));
+    VB_TRY(launch_cast(X, L->I, N, L->I, (bf16*)L->xs, layer_is_lrt(L) ? (bf16*)L->xs2 : nullptr, L->ldI, st));
     L->ctx->launches++;
-  } else if (is_lrt(L)) {
+  } else if (layer_is_lrt(L)) {
     VB_TRY(launch_square(X, (float*)L->xs2, (long long)N * L->I, st));   // dense [N x I]
     L->ctx->launches++;
   }
   return VBNN_OK;
+}
+
+// The caller's X [N x I] and G [N x O] as GEMM operands: the bf16 copies stage_x / stage_g made, or the dense fp32
+// buffers themselves
+static GemmOperand x_operand(const vbnn_layer* L, const float* X, int kmajor) {
+  return is_bf16(L) ? GemmOperand{L->xs, L->ldI, kmajor, 0} : GemmOperand{X, L->I, kmajor, 0};
+}
+static GemmOperand g_operand(const vbnn_layer* L, const float* G, int kmajor) {
+  return is_bf16(L) ? GemmOperand{L->gs_, L->ldO, kmajor, 0} : GemmOperand{G, L->O, kmajor, 0};
 }
 
 static void fill_noise(vbnn_layer* L, EpiParams& p, uint32_t kind, const float* injected) {
@@ -252,27 +247,15 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   u.B = L->opts.B; u.S = (float)L->opts.S;
   u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
   u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
-  u.lrt = is_lrt(L);
+  u.lrt = layer_is_lrt(L);
   u.prior = layer_prior(L, 0);
   double* stat_dev = stats ? c->d_partials + kMaxPartials : nullptr;
   u.stat_partials = stat_dev;
   int grid = 0;
-  cudaEvent_t pa = nullptr, pb = nullptr;
-  const bool timed = c->profiling;
-  if (timed) {
-    // bench.py's HBM roofline: class 7 = fused update, "flops" slot = algorithmic bytes (56 B / weight, + the
-    // 8 B of the prior's mean and log-variance under PER_WEIGHT)
-    for (cudaEvent_t* e : {&pa, &pb}) {
-      if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); }
-      else VB_CUDA(cudaEventCreate(e));
-    }
-    VB_CUDA(cudaEventRecord(pa, st));
-  }
-  VB_TRY(launch_update(u, &grid, st));                                                   // :131-143
-  if (timed) {
-    VB_CUDA(cudaEventRecord(pb, st));
-    c->prof_recs.push_back({pa, pb, 7, (L->prior_kind == VBNN_PRIOR_PER_WEIGHT ? 64.0 : 56.0) * (double)W});
-  }
+  // bench.py's HBM roofline: class 7 = fused update, "flops" slot = algorithmic bytes (56 B / weight, + the 8 B of
+  // the prior's mean and log-variance under PER_WEIGHT)
+  const double bytes = (L->prior_kind == VBNN_PRIOR_PER_WEIGHT ? 64.0 : 56.0) * (double)W;
+  VB_TRY(prof_launch(c, 7, bytes, [&] { return launch_update(u, &grid, st); }));         // :131-143
   c->launches += 2;
   L->prior_valid = true;
   // single counter bump: the layer owns t_dev.  The kernel left the new sums in half
@@ -311,24 +294,19 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   return VBNN_OK;
 }
 
-int tc_gemm(vbnn_ctx* c, int mode, const TcGemmArgs& g, const EpiParams& p, int prof_cls) {
-  if (!c->profiling) return gemm_tc_launch(mode, g, p, c->stream, &c->launches);
-  auto get_event = [&](cudaEvent_t* e) -> int {
-    if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); return VBNN_OK; }
-    VB_CUDA(cudaEventCreate(e));
-    return VBNN_OK;
-  };
-  vbnn_ctx::ProfRec r;
-  VB_TRY(get_event(&r.a));
-  VB_TRY(get_event(&r.b));
-  r.cls = (prof_cls >= 0 ? prof_cls : mode) & 7;        // GEMM classes 0-7; class 8 is predict (mlp.cu)
-  r.flops = 2.0 * g.M * (double)g.N * g.K * g.batch * (epi_is_dual(mode) ? 2.0 : 1.0);
-  VB_CUDA(cudaEventRecord(r.a, c->stream));
-  int rc = gemm_tc_launch(mode, g, p, c->stream, &c->launches);
-  VB_CUDA(cudaEventRecord(r.b, c->stream));
-  c->prof_recs.push_back(r);
-  if (c->prof_recs.size() + c->marks.size() >= 4096) VB_TRY(prof_collect(c));
-  return rc;
+void weight_operands(GemmArgs& g, const vbnn_layer* L, int kmajor, bool batched, bool lrt) {
+  const bool b16 = is_bf16(L), mu = layer_is_lrt(L);
+  const int ld = b16 ? L->ldI : L->I;
+  const void* w = b16 ? (mu ? (const void*)L->mu_bf16 : L->w_bf16) : (mu ? L->means : L->weight);
+  g.B1 = {w, ld, kmajor, batched ? (long long)L->O * ld : 0};
+  if (lrt) g.B2 = {b16 ? (const void*)L->s2_bf16 : L->s2_f32, ld, kmajor, 0};
+}
+
+int gemm(vbnn_ctx* c, bool bf16, int mode, const GemmArgs& g, const EpiParams& p, int prof_cls) {
+  if (!bf16) return gemm_simt_launch(mode, g, p, c->stream, &c->launches);
+  const int cls = (prof_cls >= 0 ? prof_cls : mode) & 7;        // GEMM classes 0-7; class 8 is predict (mlp.cu)
+  const double flops = 2.0 * g.M * (double)g.N * g.K * g.batch * (epi_is_dual(mode) ? 2.0 : 1.0);
+  return prof_launch(c, cls, flops, [&] { return gemm_tc_launch(mode, g, p, c->stream, &c->launches); });
 }
 
 int prof_mark(vbnn_ctx* c, int id) {
@@ -536,7 +514,7 @@ extern "C" int vbnn_layer_sample(vbnn_layer* L, int sample_idx, const float* eps
   L->map_mode = false;
   L->eps_injected = eps_dev != nullptr;
   L->eps16_valid = false;
-  if (is_lrt(L)) return VBNN_OK;     // local reparameterisation draws its noise in forward()
+  if (layer_is_lrt(L)) return VBNN_OK;     // local reparameterisation draws its noise in forward()
   cudaStream_t st = L->ctx->stream;
   const size_t W = (size_t)L->O * L->I;
   if (eps_dev && !L->eps) VB_TRY(dev_alloc(&L->eps, W));
@@ -562,7 +540,7 @@ extern "C" int vbnn_layer_clamp_to_map(vbnn_layer* L) {
   VB_TRY(check_params_fresh(L, "vbnn_layer_clamp_to_map"));
   cudaStream_t st = L->ctx->stream;
   L->map_mode = true;
-  if (is_lrt(L)) {
+  if (layer_is_lrt(L)) {
     if (L->mu_bf16) VB_TRY(layer_refresh_copies(L));
     return VBNN_OK;
   }
@@ -577,8 +555,7 @@ extern "C" int vbnn_layer_forward(vbnn_layer* L, const float* X, int N, float* Y
   VB_CHECK(L && X && Y && N > 0, VBNN_E_INVALID, "vbnn_layer_forward: bad argument");
   VB_TRY(ensure_scratch(L, N));
   VB_TRY(stage_x(L, X, N));
-  cudaStream_t st = L->ctx->stream;
-  const bool lrt = is_lrt(L) && !L->map_mode;
+  const bool lrt = layer_is_lrt(L) && !L->map_mode;
   EpiParams p;
   memset(&p, 0, sizeof(p));
   p.M = N; p.N = L->O;
@@ -593,32 +570,19 @@ extern "C" int vbnn_layer_forward(vbnn_layer* L, const float* X, int N, float* Y
     VB_CHECK((unsigned long long)N * (unsigned long long)((L->O + 3) / 4) <= 0xFFFFFFFFull, VBNN_E_UNSUPPORTED,
              "Philox zeta counter would wrap: %d rows x %d outputs", N, L->O);
   }
-  if (is_bf16(L)) {
-    TcGemmArgs g;
-    memset(&g, 0, sizeof(g));
-    g.M = N; g.N = L->O; g.K = L->I; g.batch = 1;
-    g.A1 = {(const bf16*)L->xs, L->ldI, 1, 0};
-    const bf16* w = L->kind == VBNN_KIND_LINEAR ? L->w_bf16 : (is_lrt(L) ? L->mu_bf16 : L->w_bf16);
-    g.B1 = {w, L->ldI, 1, 0};
-    if (lrt) { g.A2 = {(const bf16*)L->xs2, L->ldI, 1, 0}; g.B2 = {L->s2_bf16, L->ldI, 1, 0}; }
-    return tc_gemm(L->ctx, mode, g, p);
-  }
-  SimtGemmArgs g;
+  GemmArgs g;
   memset(&g, 0, sizeof(g));
-  g.M = N; g.N = L->O; g.K = L->I;
-  g.A1 = X; g.sA1m = L->I; g.sA1k = 1;
-  g.B1 = (is_lrt(L) ? L->means : L->weight); g.sB1n = L->I; g.sB1k = 1;
-  if (lrt) {
-    g.A2 = (const float*)L->xs2; g.sA2m = L->I; g.sA2k = 1;
-    g.B2 = L->s2_f32; g.sB2n = L->I; g.sB2k = 1;
-  }
-  return gemm_simt_launch(mode, g, p, 1, st, &L->ctx->launches);
+  g.M = N; g.N = L->O; g.K = L->I; g.batch = 1;
+  g.A1 = x_operand(L, X, 1);
+  if (lrt) g.A2 = {L->xs2, g.A1.ld, 1, 0};
+  weight_operands(g, L, 1, false, lrt);
+  return gemm(L->ctx, is_bf16(L), mode, g, p);
 }
 
 // H = G .* R for the local-reparameterisation backward; also stages G in operand form
 static int stage_g(vbnn_layer* L, const float* G, int N) {
   cudaStream_t st = L->ctx->stream;
-  const bool lrt = is_lrt(L) && !L->map_mode;
+  const bool lrt = layer_is_lrt(L) && !L->map_mode;
   if (is_bf16(L)) {
     VB_TRY(launch_cast(G, L->O, N, L->O, (bf16*)L->gs_, nullptr, L->ldO, st));
     L->ctx->launches++;
@@ -633,8 +597,7 @@ static int stage_g(vbnn_layer* L, const float* G, int N) {
 extern "C" int vbnn_layer_backward_data(vbnn_layer* L, const float* X, const float* G, int N, float* dX) {
   VB_CHECK(L && X && G && dX && N > 0, VBNN_E_INVALID, "vbnn_layer_backward_data: bad argument");
   VB_CHECK(N <= L->cap_N, VBNN_E_STATE, "vbnn_layer_backward_data before forward (N=%d)", N);
-  cudaStream_t st = L->ctx->stream;
-  const bool lrt = is_lrt(L) && !L->map_mode;
+  const bool lrt = layer_is_lrt(L) && !L->map_mode;
   VB_TRY(stage_g(L, G, N));
   EpiParams p;
   memset(&p, 0, sizeof(p));
@@ -643,35 +606,24 @@ extern "C" int vbnn_layer_backward_data(vbnn_layer* L, const float* X, const flo
   p.ld_act = L->ldI;
   p.mask = 0;
   const int mode = lrt ? EPI_DX_LRT : EPI_DX;
-  if (is_bf16(L)) {
-    if (lrt) { p.xprev = L->xs; p.ld_x = L->ldI; }
-    TcGemmArgs g;
-    memset(&g, 0, sizeof(g));
-    g.M = N; g.N = L->I; g.K = L->O; g.batch = 1;
-    g.A1 = {(const bf16*)L->gs_, L->ldO, 1, 0};
-    const bf16* w = L->kind == VBNN_KIND_LINEAR ? L->w_bf16 : (is_lrt(L) ? L->mu_bf16 : L->w_bf16);
-    g.B1 = {w, L->ldI, 0, 0};
-    if (lrt) { g.A2 = {(const bf16*)L->hs, L->ldO, 1, 0}; g.B2 = {L->s2_bf16, L->ldI, 0, 0}; }
-    return tc_gemm(L->ctx, mode, g, p);
-  }
-  if (lrt) { p.xprev = X; p.ld_x = L->I; }
-  SimtGemmArgs g;
+  GemmArgs g;
   memset(&g, 0, sizeof(g));
-  g.M = N; g.N = L->I; g.K = L->O;
-  g.A1 = G; g.sA1m = L->O; g.sA1k = 1;
-  g.B1 = is_lrt(L) ? L->means : L->weight; g.sB1k = L->I; g.sB1n = 1;
+  g.M = N; g.N = L->I; g.K = L->O; g.batch = 1;
+  g.A1 = g_operand(L, G, 1);
   if (lrt) {
-    g.A2 = (const float*)L->hs; g.sA2m = L->ldO; g.sA2k = 1;
-    g.B2 = L->s2_f32; g.sB2k = L->I; g.sB2n = 1;
+    const GemmOperand x = x_operand(L, X, 1);
+    p.xprev = x.ptr; p.ld_x = x.ld;
+    g.A2 = {L->hs, L->ldO, 1, 0};
   }
-  return gemm_simt_launch(mode, g, p, 1, st, &L->ctx->launches);
+  weight_operands(g, L, 0, false, lrt);
+  return gemm(L->ctx, is_bf16(L), mode, g, p);
 }
 
 extern "C" int vbnn_layer_acc_grad(vbnn_layer* L, const float* X, const float* G, int N, float scale) {
   VB_CHECK(L && X && G && N > 0, VBNN_E_INVALID, "vbnn_layer_acc_grad: bad argument");
   VB_TRY(ensure_scratch(L, N));
   cudaStream_t st = L->ctx->stream;
-  const bool lrt = is_lrt(L) && !L->map_mode;
+  const bool lrt = layer_is_lrt(L) && !L->map_mode;
   // operands may not have been staged by forward/backward_data of this call sequence
   VB_TRY(stage_x(L, X, N));
   VB_TRY(stage_g(L, G, N));
@@ -683,26 +635,13 @@ extern "C" int vbnn_layer_acc_grad(vbnn_layer* L, const float* X, const float* G
   fill_noise(L, p, kStreamEps, L->eps_injected ? L->eps : nullptr);
   if (L->map_mode) { p.gS = nullptr; }
   const int mode = lrt ? EPI_DW_LRT : EPI_DW;
-  if (is_bf16(L)) {
-    TcGemmArgs g;
-    memset(&g, 0, sizeof(g));
-    g.M = L->O; g.N = L->I; g.K = N; g.batch = 1;
-    g.A1 = {(const bf16*)L->gs_, L->ldO, 0, 0};
-    g.B1 = {(const bf16*)L->xs, L->ldI, 0, 0};
-    if (lrt) { g.A2 = {(const bf16*)L->hs, L->ldO, 0, 0}; g.B2 = {(const bf16*)L->xs2, L->ldI, 0, 0}; }
-    VB_TRY(tc_gemm(L->ctx, mode, g, p));
-  } else {
-    SimtGemmArgs g;
-    memset(&g, 0, sizeof(g));
-    g.M = L->O; g.N = L->I; g.K = N;
-    g.A1 = G; g.sA1m = 1; g.sA1k = L->O;
-    g.B1 = X; g.sB1k = L->I; g.sB1n = 1;
-    if (lrt) {
-      g.A2 = (const float*)L->hs; g.sA2m = 1; g.sA2k = L->ldO;
-      g.B2 = (const float*)L->xs2; g.sB2k = L->I; g.sB2n = 1;
-    }
-    VB_TRY(gemm_simt_launch(mode, g, p, 1, st, &L->ctx->launches));
-  }
+  GemmArgs g;
+  memset(&g, 0, sizeof(g));
+  g.M = L->O; g.N = L->I; g.K = N; g.batch = 1;
+  g.A1 = g_operand(L, G, 0);
+  g.B1 = x_operand(L, X, 0);
+  if (lrt) { g.A2 = {L->hs, L->ldO, 0, 0}; g.B2 = {L->xs2, g.B1.ld, 0, 0}; }
+  VB_TRY(gemm(L->ctx, is_bf16(L), mode, g, p));
   VB_TRY(launch_colsum(G, 0, N, L->O, L->O, scale, L->gb, st));       // gradBias += scale * G^T 1
   L->ctx->launches++;
   return VBNN_OK;
@@ -735,7 +674,7 @@ extern "C" int vbnn_layer_grads(vbnn_layer* L, float* mleg, float* mlcg, float* 
   VB_CHECK(L && L->kind == VBNN_KIND_VB, VBNN_E_INVALID, "vbnn_layer_grads: not a VB layer");
   VB_CHECK(L->prior_valid, VBNN_E_STATE, "vbnn_layer_grads before compute_prior");
   VB_TRY(launch_grads(L->means, L->lvars, L->gW, L->gS, (long long)L->O * L->I, L->var_hat_dev, layer_prior(L, 0),
-                      L->opts.B, (float)L->opts.S, is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
+                      L->opts.B, (float)L->opts.S, layer_is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
   L->ctx->launches++;
   return VBNN_OK;
 }
@@ -996,7 +935,7 @@ extern "C" int vbnn_layer_draw_noise(vbnn_layer* L, uint32_t step, int sample_id
                                      float* out_dev) {
   VB_CHECK(L && out_dev, VBNN_E_INVALID, "null argument");
   PhiloxStream ps;
-  if (is_lrt(L)) {
+  if (layer_is_lrt(L)) {
     ps = layer_stream(L, kStreamZeta, sample_idx);
     ps.step = step;
     VB_TRY(launch_philox_matrix(out_dev, rows, L->O, row0, ps, L->ctx->stream));
@@ -1024,13 +963,13 @@ extern "C" int vbnn_gemm_bf16(vbnn_ctx* ctx, const uint16_t* A, int lda, int a_k
                               int ldb, int b_kmajor, float* D, int ldd, int M, int N, int K, int batch,
                               long long strideA, long long strideB, long long strideD) {
   VB_CHECK(ctx && A && B && D, VBNN_E_INVALID, "vbnn_gemm_bf16: null argument");
-  TcGemmArgs g;
+  GemmArgs g;
   memset(&g, 0, sizeof(g));
   g.M = M; g.N = N; g.K = K; g.batch = batch < 1 ? 1 : batch;
-  g.A1 = {(const bf16*)A, lda, a_kmajor, strideA};
-  g.B1 = {(const bf16*)B, ldb, b_kmajor, strideB};
+  g.A1 = {A, lda, a_kmajor, strideA};
+  g.B1 = {B, ldb, b_kmajor, strideB};
   EpiParams p;
   memset(&p, 0, sizeof(p));
   p.M = M; p.N = N; p.out_f32 = D; p.ld_f32 = ldd; p.zs_f32 = strideD;
-  return tc_gemm(ctx, EPI_STORE, g, p);
+  return gemm(ctx, true, EPI_STORE, g, p);
 }

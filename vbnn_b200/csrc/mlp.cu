@@ -11,22 +11,7 @@ using namespace vbnn;
 
 namespace {
 
-template <typename T>
-int dalloc(T** p, size_t bytes) {
-  *p = nullptr;
-  if (!bytes) return VBNN_OK;
-  cudaError_t e = cudaMalloc((void**)p, bytes);
-  if (e != cudaSuccess) {
-    set_error("cudaMalloc(%zu bytes) failed: %s", bytes, cudaGetErrorString(e));
-    return e == cudaErrorMemoryAllocation ? VBNN_E_NOMEM : VBNN_E_CUDA;
-  }
-  return VBNN_OK;
-}
-
 inline size_t esz(const vbnn_mlp* m) { return m->bf16 ? 2 : 4; }
-inline bool layer_lrt(const vbnn_layer* L) {
-  return L->kind == VBNN_KIND_VB && L->opts.reparam == VBNN_REPARAM_LOCAL;
-}
 inline int nlayers(const vbnn_mlp* m) { return (int)m->layers.size(); }
 // LRT forward / backward-data as two single-accumulator GEMMs (default) or one dual-accumulator GEMM
 // (VBNN_LRT_SPLIT bit 0: forward, bit 1: backward-data).  Measured on C3 under the 1000 W cap: the split
@@ -78,7 +63,7 @@ int stage_input_u8(vbnn_mlp* m, const uint8_t* X, const float* T, int N, float m
 // mlp:sample() for Zrun samples at once (mlp.lua:69-74 x main.lua:32-33)
 int sample_all(vbnn_mlp* m, int sample0, int Zrun) {
   for (vbnn_layer* L : m->layers) {
-    if (L->kind != VBNN_KIND_VB || layer_lrt(L)) continue;
+    if (L->kind != VBNN_KIND_VB || layer_is_lrt(L)) continue;
     SampleParams p;
     memset(&p, 0, sizeof(p));
     p.mu = L->means;
@@ -105,15 +90,35 @@ int clamp_all(vbnn_mlp* m) {
   return VBNN_OK;
 }
 
+// The split form of the dual LRT GEMM g (mode EPI_FWD_LRT or EPI_DX_LRT, bf16 only): one product alone into aux as a
+// plain fp32 store, then the other with the LRT2 epilogue joining it -- forward: X mu^T first, then the variance
+// X^2 s2^T; backward-data: H s2 first, then G mu with the 2 X .* T join.  Each GEMM has a single TMEM accumulator,
+// double-buffered, so the epilogue of tile i runs under the MMAs of tile i+1 (the dual kernel fills all 512 TMEM
+// columns and cannot).  Both launches are profiled under `mode`.
+int gemm_lrt_split(vbnn_mlp* m, int mode, const GemmArgs& g, EpiParams p) {
+  const bool fwd = mode == EPI_FWD_LRT;
+  GemmArgs first = g, second = g;
+  first.A2 = first.B2 = second.A2 = second.B2 = GemmOperand{};
+  if (fwd) { second.A1 = g.A2; second.B1 = g.B2; }
+  else { first.A1 = g.A2; first.B1 = g.B2; }
+  const long long zs_aux = g.zsum ? 0 : (long long)p.M * m->ld_aux;       // summing form: the z = 0 slice only
+  EpiParams p0;
+  memset(&p0, 0, sizeof(p0));
+  p0.M = p.M; p0.N = p.N;
+  p0.out_f32 = m->aux; p0.ld_f32 = m->ld_aux; p0.zs_f32 = zs_aux;
+  VB_TRY(gemm(m->ctx, m->bf16, EPI_STORE, first, p0, mode));
+  p.aux = m->aux; p.ld_aux = m->ld_aux; p.zs_aux = zs_aux;
+  return gemm(m->ctx, m->bf16, fwd ? EPI_FWD_LRT2 : EPI_DX_LRT2, second, p, mode);
+}
+
 // One layer forward for Zrun batched samples.
 int forward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, bool map_mode) {
   vbnn_layer* L = m->layers[j];
   const bool last = j == nlayers(m) - 1;
-  const bool lrt = layer_lrt(L) && !map_mode;
+  const bool lrt = layer_is_lrt(L) && !map_mode;
   const int ldi = m->ld[j], ldo = m->ld[j + 1];
   const long long zs_in = j == 0 ? 0 : (long long)N * ldi;
-  const bool w_batched = L->kind == VBNN_KIND_VB && !layer_lrt(L) && !map_mode;
-  cudaStream_t st = m->ctx->stream;
+  const bool w_batched = L->kind == VBNN_KIND_VB && !layer_is_lrt(L) && !map_mode;
   EpiParams p;
   memset(&p, 0, sizeof(p));
   p.M = N; p.N = L->O;
@@ -139,44 +144,14 @@ int forward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, bool map_mod
     VB_CHECK((unsigned long long)m->ctx->nranks * (unsigned long long)N * (unsigned long long)((L->O + 3) / 4) <= 0xFFFFFFFFull,
              VBNN_E_UNSUPPORTED, "Philox zeta counter would wrap: %d ranks x %d rows x %d outputs", m->ctx->nranks, N, L->O);
   }
-  if (m->bf16) {
-    TcGemmArgs g;
-    memset(&g, 0, sizeof(g));
-    g.M = N; g.N = L->O; g.K = L->I; g.batch = Zrun;
-    g.A1 = {(const bf16*)m->act[j], ldi, 1, zs_in};
-    const bf16* w = layer_lrt(L) ? L->mu_bf16 : L->w_bf16;
-    g.B1 = {w, L->ldI, 1, w_batched ? (long long)L->O * L->ldI : 0};
-    if (lrt && lrt_split(m, 1)) {
-      // Split LRT forward: mean product first (plain fp32 store), then the variance GEMM whose single
-      // TMEM accumulator is double-buffered, so the Philox / rsqrt / three-tensor epilogue of tile i runs
-      // under the MMAs of tile i+1 (the dual-accumulator kernel fills all 512 TMEM columns and cannot).
-      EpiParams p0;
-      memset(&p0, 0, sizeof(p0));
-      p0.M = N; p0.N = L->O;
-      p0.out_f32 = m->aux; p0.ld_f32 = m->ld_aux; p0.zs_f32 = (long long)N * m->ld_aux;
-      VB_TRY(tc_gemm(m->ctx, EPI_STORE, g, p0, EPI_FWD_LRT));
-      g.A1 = {(const bf16*)m->act2[j], ldi, 1, zs_in};
-      g.B1 = {L->s2_bf16, L->ldI, 1, 0};
-      p.aux = m->aux; p.ld_aux = m->ld_aux; p.zs_aux = (long long)N * m->ld_aux;
-      return tc_gemm(m->ctx, EPI_FWD_LRT2, g, p, EPI_FWD_LRT);
-    }
-    if (lrt) {
-      g.A2 = {(const bf16*)m->act2[j], ldi, 1, zs_in};
-      g.B2 = {L->s2_bf16, L->ldI, 1, 0};
-    }
-    return tc_gemm(m->ctx, mode, g, p);
-  }
-  SimtGemmArgs g;
+  GemmArgs g;
   memset(&g, 0, sizeof(g));
-  g.M = N; g.N = L->O; g.K = L->I;
-  g.A1 = (const float*)m->act[j]; g.sA1m = ldi; g.sA1k = 1; g.zsA1 = zs_in;
-  g.B1 = layer_lrt(L) ? L->means : L->weight; g.sB1n = L->I; g.sB1k = 1;
-  g.zsB1 = w_batched ? (long long)L->O * L->I : 0;
-  if (lrt) {
-    g.A2 = (const float*)m->act2[j]; g.sA2m = ldi; g.sA2k = 1; g.zsA2 = zs_in;
-    g.B2 = L->s2_f32; g.sB2n = L->I; g.sB2k = 1; g.zsB2 = 0;
-  }
-  return gemm_simt_launch(mode, g, p, Zrun, st, &m->ctx->launches);
+  g.M = N; g.N = L->O; g.K = L->I; g.batch = Zrun;
+  g.A1 = {m->act[j], ldi, 1, zs_in};
+  if (lrt) g.A2 = {m->act2[j], ldi, 1, zs_in};
+  weight_operands(g, L, 1, w_batched, lrt);
+  if (lrt && lrt_split(m, 1)) return gemm_lrt_split(m, mode, g, p);
+  return gemm(m->ctx, m->bf16, mode, g, p);
 }
 
 int loss_all(vbnn_mlp* m, int N, int Zrun, bool backward, float* logp_out, float* result) {
@@ -197,7 +172,7 @@ int loss_all(vbnn_mlp* m, int N, int Zrun, bool backward, float* logp_out, float
   lp.z_slot0 = 0;
   VB_TRY(launch_loss(lp, m->ctx->stream));
   m->ctx->launches++;
-  if (backward && layer_lrt(Lo)) {
+  if (backward && layer_is_lrt(Lo)) {
     VB_TRY(launch_mul_act(m->G[Lc - 1], m->ld[Lc], m->bf16, m->R[Lc - 1], m->ld[Lc], m->H[Lc - 1], m->ld[Lc],
                           (long long)Zrun * N, Lo->O, m->bf16, m->ctx->stream));
     m->ctx->launches++;
@@ -207,118 +182,44 @@ int loss_all(vbnn_mlp* m, int N, int Zrun, bool backward, float* logp_out, float
 
 // updateGradInput of layer j (its gradInput is layer j-1's gradOutput, ReLU backward fused)
 int backward_data_layer(vbnn_mlp* m, int j, int N, int Zrun) {
+  if (j == 0 && !m->dX) return VBNN_OK;
   vbnn_layer* L = m->layers[j];
-  const bool lrt = layer_lrt(L);
+  const bool lrt = layer_is_lrt(L);
   const int ldi = m->ld[j], ldo = m->ld[j + 1];
   const long long zs_out = (long long)N * ldo;
-  const bool w_batched = L->kind == VBNN_KIND_VB && !lrt;
-  cudaStream_t st = m->ctx->stream;
-
+  GemmArgs g;
+  memset(&g, 0, sizeof(g));
+  g.M = N; g.N = L->I; g.K = L->O; g.batch = Zrun;
+  g.A1 = {m->G[j], ldo, 1, zs_out};
+  if (lrt) g.A2 = {m->H[j], ldo, 1, zs_out};
+  weight_operands(g, L, 0, L->kind == VBNN_KIND_VB && !lrt, lrt);
+  EpiParams p;
+  memset(&p, 0, sizeof(p));
+  p.M = N; p.N = L->I;
   if (j > 0) {
-    vbnn_layer* Lp = m->layers[j - 1];
-    EpiParams p;
-    memset(&p, 0, sizeof(p));
-    p.M = N; p.N = L->I;
     p.out_act = m->G[j - 1]; p.ld_act = ldi; p.zs_act = (long long)N * ldi;
     p.xprev = m->act[j]; p.ld_x = ldi; p.zs_x = (long long)N * ldi;
     p.mask = 1;                                                    // nn.ReLU backward
-    if (layer_lrt(Lp)) { p.rprev = m->R[j - 1]; p.out_act2 = m->H[j - 1]; }
-    const int mode = lrt ? EPI_DX_LRT : EPI_DX;
-    if (m->bf16) {
-      TcGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = N; g.N = L->I; g.K = L->O; g.batch = Zrun;
-      g.A1 = {(const bf16*)m->G[j], ldo, 1, zs_out};
-      g.B1 = {lrt ? L->mu_bf16 : L->w_bf16, L->ldI, 0, w_batched ? (long long)L->O * L->ldI : 0};
-      if (lrt && lrt_split(m, 2)) {
-        // split LRT backward-data: T = H s2 first, then G mu with the 2 X .* T join in its epilogue
-        TcGemmArgs g1 = g;
-        g1.A1 = {(const bf16*)m->H[j], ldo, 1, zs_out};
-        g1.B1 = {L->s2_bf16, L->ldI, 0, 0};
-        EpiParams p0;
-        memset(&p0, 0, sizeof(p0));
-        p0.M = N; p0.N = L->I;
-        p0.out_f32 = m->aux; p0.ld_f32 = m->ld_aux; p0.zs_f32 = (long long)N * m->ld_aux;
-        VB_TRY(tc_gemm(m->ctx, EPI_STORE, g1, p0, EPI_DX_LRT));
-        p.aux = m->aux; p.ld_aux = m->ld_aux; p.zs_aux = (long long)N * m->ld_aux;
-        VB_TRY(tc_gemm(m->ctx, EPI_DX_LRT2, g, p, EPI_DX_LRT));
-      } else {
-      if (lrt) {
-        g.A2 = {(const bf16*)m->H[j], ldo, 1, zs_out};
-        g.B2 = {L->s2_bf16, L->ldI, 0, 0};
-      }
-      VB_TRY(tc_gemm(m->ctx, mode, g, p));
-      }
-    } else {
-      SimtGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = N; g.N = L->I; g.K = L->O;
-      g.A1 = (const float*)m->G[j]; g.sA1m = ldo; g.sA1k = 1; g.zsA1 = zs_out;
-      g.B1 = lrt ? L->means : L->weight; g.sB1k = L->I; g.sB1n = 1;
-      g.zsB1 = w_batched ? (long long)L->O * L->I : 0;
-      if (lrt) {
-        g.A2 = (const float*)m->H[j]; g.sA2m = ldo; g.sA2k = 1; g.zsA2 = zs_out;
-        g.B2 = L->s2_f32; g.sB2k = L->I; g.sB2n = 1; g.zsB2 = 0;
-      }
-      VB_TRY(gemm_simt_launch(mode, g, p, Zrun, st, &m->ctx->launches));
-    }
-  } else if (m->dX) {
+    if (layer_is_lrt(m->layers[j - 1])) { p.rprev = m->R[j - 1]; p.out_act2 = m->H[j - 1]; }
+  } else {
     // vbnn_mlp_step_grad_input: the first layer's gradInput summed over the Z samples, dX = sum_z dl_z/dX, written
-    // straight into the caller's [N x I0] buffer by ONE GEMM whose contraction runs over the samples too (K-concat:
-    // no atomics, no partials).  Nothing below the input: no ReLU mask.  The staged input act[0] is shared by every
-    // sample (zs_x = 0), so the LRT join is exact on the sums: sum_z (G_z mu + 2 X .* H_z s2) = (sum_z G_z) mu +
+    // straight into the caller's [N x I0] buffer by ONE GEMM whose contraction runs over the samples too (no atomics,
+    // no partials).  Nothing below the input: no ReLU mask.  The staged input act[0] is shared by every sample
+    // (zs_x = 0), so the LRT join is exact on the sums: sum_z (G_z mu + 2 X .* H_z s2) = (sum_z G_z) mu +
     // 2 X .* ((sum_z H_z) s2).
-    EpiParams p;
-    memset(&p, 0, sizeof(p));
-    p.M = N; p.N = L->I;
+    g.zsum = 1;
     p.out_f32 = m->dX; p.ld_f32 = L->I;
     if (lrt) { p.xprev = m->act[0]; p.ld_x = ldi; p.zs_x = 0; }
-    const int mode = lrt ? EPI_DX_LRT : EPI_DX;
-    if (m->bf16) {
-      TcGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = N; g.N = L->I; g.K = L->O; g.batch = Zrun; g.zsum = 1;
-      g.A1 = {(const bf16*)m->G[0], ldo, 1, zs_out};
-      g.B1 = {lrt ? L->mu_bf16 : L->w_bf16, L->ldI, 0, w_batched ? (long long)L->O * L->ldI : 0};
-      if (lrt && lrt_split(m, 2)) {
-        TcGemmArgs g1 = g;                  // sum_z H_z s2 into aux (z = 0 slice), then sum_z G_z mu joined with it
-        g1.A1 = {(const bf16*)m->H[0], ldo, 1, zs_out};
-        g1.B1 = {L->s2_bf16, L->ldI, 0, 0};
-        EpiParams p0;
-        memset(&p0, 0, sizeof(p0));
-        p0.M = N; p0.N = L->I;
-        p0.out_f32 = m->aux; p0.ld_f32 = m->ld_aux;
-        VB_TRY(tc_gemm(m->ctx, EPI_STORE, g1, p0, EPI_DX_LRT));
-        p.aux = m->aux; p.ld_aux = m->ld_aux;
-        VB_TRY(tc_gemm(m->ctx, EPI_DX_LRT2, g, p, EPI_DX_LRT));
-      } else {
-        if (lrt) {
-          g.A2 = {(const bf16*)m->H[0], ldo, 1, zs_out};
-          g.B2 = {L->s2_bf16, L->ldI, 0, 0};
-        }
-        VB_TRY(tc_gemm(m->ctx, mode, g, p));
-      }
-    } else {
-      SimtGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = N; g.N = L->I; g.K = L->O; g.zsum = Zrun;
-      g.A1 = (const float*)m->G[0]; g.sA1m = ldo; g.sA1k = 1; g.zsA1 = zs_out;
-      g.B1 = lrt ? L->means : L->weight; g.sB1k = L->I; g.sB1n = 1;
-      g.zsB1 = w_batched ? (long long)L->O * L->I : 0;
-      if (lrt) {
-        g.A2 = (const float*)m->H[0]; g.sA2m = ldo; g.sA2k = 1; g.zsA2 = zs_out;
-        g.B2 = L->s2_f32; g.sB2k = L->I; g.sB2n = 1; g.zsB2 = 0;
-      }
-      VB_TRY(gemm_simt_launch(mode, g, p, 1, st, &m->ctx->launches));
-    }
   }
-  return VBNN_OK;
+  const int mode = lrt ? EPI_DX_LRT : EPI_DX;
+  if (lrt && lrt_split(m, 2)) return gemm_lrt_split(m, mode, g, p);
+  return gemm(m->ctx, m->bf16, mode, g, p);
 }
 
 // accGradParameters of layer j (+ gradBias column sums)
 int backward_weight_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, int accumulate, bool scatter = false) {
   vbnn_layer* L = m->layers[j];
-  const bool lrt = layer_lrt(L);
+  const bool lrt = layer_is_lrt(L);
   const int ldi = m->ld[j], ldo = m->ld[j + 1];
   const long long zs_in = j == 0 ? 0 : (long long)N * ldi;
   const long long zs_out = (long long)N * ldo;
@@ -342,70 +243,50 @@ int backward_weight_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, int 
     // peer mode the epilogue's stores cross NVLink and the split form hides them (8 GPUs: 6.14 -> 5.97 ms).
     const int split_knob = knobs().dw_split;
     const bool split = split_knob >= 0 ? split_knob != 0 : (scatter && !peer_transport_ce(m, N));
+    GemmArgs g;
+    memset(&g, 0, sizeof(g));
+    g.M = L->O; g.N = L->I; g.K = N; g.batch = Zrun;
+    g.A1 = {m->G[j], ldo, 0, zs_out};
+    g.B1 = {m->act[j], ldi, 0, zs_in};
+    if (lrt) { g.A2 = {m->H[j], ldo, 0, zs_out}; g.B2 = {m->act2[j], ldi, 0, zs_in}; }
+    const int lin_tiles = ceil_div(L->O, 128) * ceil_div(L->I, 128);
     if (m->bf16 && lrt && split) {
       // The two LRT parameter gradients are independent (g_mu = G^T X, g_s = H^T X^2): as two
       // single-accumulator GEMMs each tile needs half the TMEM, so the accumulator is double-buffered
       // and the epilogue of tile i hides behind the MMAs of tile i+1 (the dual kernel cannot).
-      TcGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = L->O; g.N = L->I; g.K = N; g.batch = Zrun;
-      g.A1 = {(const bf16*)m->G[j], ldo, 0, zs_out};
-      g.B1 = {(const bf16*)m->act[j], ldi, 0, zs_in};
+      GemmArgs g1 = g;
+      g1.A2 = g1.B2 = GemmOperand{};
       EpiParams p1 = p;
       p1.gS = nullptr;
       p1.noise = nullptr;
-      VB_TRY(tc_gemm(m->ctx, EPI_DW, g, p1));
-      g.A1 = {(const bf16*)m->H[j], ldo, 0, zs_out};
-      g.B1 = {(const bf16*)m->act2[j], ldi, 0, zs_in};
+      VB_TRY(gemm(m->ctx, m->bf16, EPI_DW, g1, p1));
+      g1.A1 = g.A2; g1.B1 = g.B2;
       p1.gW = L->gS;                      // plain accumulate of H^T X^2 into gradSum
       if (p1.scatter_rows)                // ... or into the owners' gradSum receive slots
         for (int q = 0; q < 8; ++q) p1.gW_peer[q] = p.gS_peer[q];
       p1.scale = 1.f;
-      VB_TRY(tc_gemm(m->ctx, EPI_DW, g, p1));
-    } else if (m->bf16) {
-      TcGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = L->O; g.N = L->I; g.K = N; g.batch = Zrun;
-      g.A1 = {(const bf16*)m->G[j], ldo, 0, zs_out};
-      g.B1 = {(const bf16*)m->act[j], ldi, 0, zs_in};
-      if (lrt) {
-        g.A2 = {(const bf16*)m->H[j], ldo, 0, zs_out};
-        g.B2 = {(const bf16*)m->act2[j], ldi, 0, zs_in};
-      }
-      const int lin_tiles = ceil_div(L->O, 128) * ceil_div(L->I, 128);
-      if (L->kind == VBNN_KIND_LINEAR && Zrun > 1 && !scatter && m->dw_partials && lin_tiles * 2 <= kNumSMs &&
-          (L->I & 3) == 0) {
-        // plain nn.Linear with few output tiles (the 10 x 1200 output layer of C2: 10 tiles): one tile would walk
-        // all Z * N rows serially (50 us for 0.25 GFLOP).  Instead every (tile, sample) pair is its own work unit
-        // -- a batched plain-store GEMM into per-sample partial products -- and a fixed-order reduction adds them.
-        EpiParams p0;
-        memset(&p0, 0, sizeof(p0));
-        p0.M = L->O; p0.N = L->I;
-        p0.out_f32 = m->dw_partials; p0.ld_f32 = L->I; p0.zs_f32 = (long long)L->O * L->I;
-        VB_TRY(tc_gemm(m->ctx, EPI_STORE, g, p0, EPI_DW));
-        VB_TRY(launch_sum_partials(m->dw_partials, Zrun, (long long)L->O * L->I, (long long)L->O * L->I, p.scale, accumulate,
-                                   L->gW, st));
-        m->ctx->launches++;
-      } else {
-        if (L->kind == VBNN_KIND_LINEAR && Zrun > 1 && zs_in == (long long)N * ldi) {
-          // plain nn.Linear (no per-sample epsilon): sum_z G_z^T X_z is ONE GEMM over K = Z * N rows, the
-          // samples being contiguous in both operands -- no per-sample accumulator round trips
-          g.K = N * Zrun; g.batch = 1;
-          g.A1.zs = 0; g.B1.zs = 0;
-        }
-        VB_TRY(tc_gemm(m->ctx, mode, g, p));
-      }
+      VB_TRY(gemm(m->ctx, m->bf16, EPI_DW, g1, p1));
+    } else if (m->bf16 && L->kind == VBNN_KIND_LINEAR && Zrun > 1 && !scatter && m->dw_partials &&
+               lin_tiles * 2 <= kNumSMs && (L->I & 3) == 0) {
+      // plain nn.Linear with few output tiles (the 10 x 1200 output layer of C2: 10 tiles): one tile would walk
+      // all Z * N rows serially (50 us for 0.25 GFLOP).  Instead every (tile, sample) pair is its own work unit
+      // -- a batched plain-store GEMM into per-sample partial products -- and a fixed-order reduction adds them.
+      EpiParams p0;
+      memset(&p0, 0, sizeof(p0));
+      p0.M = L->O; p0.N = L->I;
+      p0.out_f32 = m->dw_partials; p0.ld_f32 = L->I; p0.zs_f32 = (long long)L->O * L->I;
+      VB_TRY(gemm(m->ctx, m->bf16, EPI_STORE, g, p0, EPI_DW));
+      VB_TRY(launch_sum_partials(m->dw_partials, Zrun, (long long)L->O * L->I, (long long)L->O * L->I, p.scale, accumulate,
+                                 L->gW, st));
+      m->ctx->launches++;
     } else {
-      SimtGemmArgs g;
-      memset(&g, 0, sizeof(g));
-      g.M = L->O; g.N = L->I; g.K = N;
-      g.A1 = (const float*)m->G[j]; g.sA1m = 1; g.sA1k = ldo; g.zsA1 = zs_out;
-      g.B1 = (const float*)m->act[j]; g.sB1k = ldi; g.sB1n = 1; g.zsB1 = zs_in;
-      if (lrt) {
-        g.A2 = (const float*)m->H[j]; g.sA2m = 1; g.sA2k = ldo; g.zsA2 = zs_out;
-        g.B2 = (const float*)m->act2[j]; g.sB2k = ldi; g.sB2n = 1; g.zsB2 = zs_in;
+      if (m->bf16 && L->kind == VBNN_KIND_LINEAR && Zrun > 1 && zs_in == (long long)N * ldi) {
+        // plain nn.Linear (no per-sample epsilon): sum_z G_z^T X_z is ONE GEMM over K = Z * N rows, the
+        // samples being contiguous in both operands -- no per-sample accumulator round trips
+        g.K = N * Zrun; g.batch = 1;
+        g.A1.zs = 0; g.B1.zs = 0;
       }
-      VB_TRY(gemm_simt_launch(mode, g, p, Zrun, st, &m->ctx->launches));
+      VB_TRY(gemm(m->ctx, m->bf16, mode, g, p));
     }
   }
   // gradBias += G^T 1 summed over all samples (quirk Q3: never divided by S)
@@ -562,7 +443,7 @@ int split_backward_body(vbnn_mlp* m, int N, const float* grad) {
   vbnn_layer* Lo = m->layers[Lc - 1];
   VB_TRY(prof_mark(m->ctx, 0));
   VB_TRY(launch_grad_logits(grad, (long long)m->Z * N, Lo->O, m->G[Lc - 1], m->ld[Lc],
-                            layer_lrt(Lo) ? m->R[Lc - 1] : nullptr, m->H[Lc - 1], m->bf16, m->ctx->stream));
+                            layer_is_lrt(Lo) ? m->R[Lc - 1] : nullptr, m->H[Lc - 1], m->bf16, m->ctx->stream));
   m->ctx->launches++;
   VB_TRY(prof_mark(m->ctx, 4));
   return step_backward(m, N, false);
@@ -654,24 +535,6 @@ int eval_forward(vbnn_mlp* m, const float* X, const float* T, int N, int n_sampl
   return VBNN_OK;
 }
 
-// launch() under a pair of CUDA events while profiling, accounted to class cls with `work` in its flops slot
-template <typename Launch>
-int prof_launch(vbnn_ctx* c, int cls, double work, Launch&& launch) {
-  if (!c->profiling) return launch();
-  vbnn_ctx::ProfRec r;
-  for (cudaEvent_t* e : {&r.a, &r.b}) {
-    if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); }
-    else VB_CUDA(cudaEventCreate(e));
-  }
-  r.cls = cls; r.flops = work;
-  VB_CUDA(cudaEventRecord(r.a, c->stream));
-  VB_TRY(launch());
-  VB_CUDA(cudaEventRecord(r.b, c->stream));
-  c->prof_recs.push_back(r);
-  if (c->prof_recs.size() + c->marks.size() >= 4096) VB_TRY(prof_collect(c));
-  return VBNN_OK;
-}
-
 // the first call of an evaluation entry point allocates its state: not while the stream is being captured
 int refuse_capture(cudaStream_t st, const char* who) {
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
@@ -684,7 +547,7 @@ int refuse_capture(cudaStream_t st, const char* who) {
 // per-block {sum, sum} partials of vbnn_mlp_predict and vbnn_mlp_predict_outputs [kMaxPartials x 2]
 int ensure_pred_partials(vbnn_mlp* m) {
   if (m->pred_partials) return VBNN_OK;
-  return dalloc(&m->pred_partials, (size_t)kMaxPartials * 2 * sizeof(double));
+  return dev_alloc(&m->pred_partials, (size_t)kMaxPartials * 2);
 }
 
 }  // namespace
@@ -729,7 +592,7 @@ extern "C" int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int
     m->grad_len.push_back(off - off_gW[j]);
   }
   m->grad_count = off;
-  r = dalloc(&m->grad_arena, off * 4);
+  r = dev_alloc(&m->grad_arena, off);
   if (r == VBNN_OK && cudaMemsetAsync(m->grad_arena, 0, off * 4, st) != cudaSuccess) r = VBNN_E_CUDA;
   for (int j = 0; j < Lc && r == VBNN_OK; ++j) {
     const bool vb = j < Lc - 1 || vb_output;
@@ -744,7 +607,7 @@ extern "C" int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int
   const size_t ZN = (size_t)m->Z * max_batch;
   m->act.assign(n_sizes, nullptr); m->act2.assign(n_sizes, nullptr);
   m->R.assign(Lc, nullptr); m->G.assign(Lc, nullptr); m->H.assign(Lc, nullptr);
-  auto A_ = [&](void** p, size_t bytes) { if (r == VBNN_OK) { char* q; r = dalloc(&q, bytes); *p = q; } };
+  auto A_ = [&](void** p, size_t bytes) { if (r == VBNN_OK) { char* q; r = dev_alloc(&q, bytes); *p = q; } };
   A_(&m->act[0], (size_t)max_batch * m->ld[0] * e);
   if (m->lrt) A_(&m->act2[0], (size_t)max_batch * m->ld[0] * e);
   for (int j = 0; j < Lc; ++j) {
@@ -775,7 +638,7 @@ extern "C" int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int
     std::vector<int*> ts;
     for (vbnn_layer* L : m->layers) ts.push_back(L->t_dev);
     m->n_t = (int)ts.size();
-    r = dalloc(&m->t_list_dev, ts.size() * sizeof(int*));
+    r = dev_alloc(&m->t_list_dev, ts.size());
     if (r == VBNN_OK &&
         cudaMemcpyAsync(m->t_list_dev, ts.data(), ts.size() * sizeof(int*), cudaMemcpyHostToDevice, st) != cudaSuccess)
       r = VBNN_E_CUDA;
@@ -1017,8 +880,8 @@ extern "C" int vbnn_mlp_backward_update(vbnn_mlp* m, const float* grad_dev, floa
 static int ensure_pipeline(vbnn_mlp* m) {
   if (m->pipeline_ready) return VBNN_OK;
   for (int s = 0; s < 2; ++s) {
-    VB_TRY(dalloc(&m->xstage[s], (size_t)m->max_batch * m->sizes[0] * 4));
-    VB_TRY(dalloc(&m->tstage[s], (size_t)m->max_batch * 4));
+    VB_TRY(dev_alloc(&m->xstage[s], (size_t)m->max_batch * m->sizes[0]));
+    VB_TRY(dev_alloc(&m->tstage[s], (size_t)m->max_batch));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].copied, cudaEventDisableTiming));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].consumed, cudaEventDisableTiming));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].done, cudaEventDisableTiming));
@@ -1040,7 +903,7 @@ static int submit_host_any(vbnn_mlp* m, const float* X_host, const uint8_t* X8_h
   vbnn_ctx* c = m->ctx;
   const int s = m->submit_idx & 1;
   vbnn_mlp::Slot& sl = m->slots[s];
-  if (X8_host && !m->xstage_u8[s]) VB_TRY(dalloc(&m->xstage_u8[s], (size_t)m->max_batch * m->sizes[0]));
+  if (X8_host && !m->xstage_u8[s]) VB_TRY(dev_alloc(&m->xstage_u8[s], (size_t)m->max_batch * m->sizes[0]));
   // copy engine: wait until the previous user of this staging buffer has been consumed
   if (m->submit_idx >= 2) VB_CUDA(cudaStreamWaitEvent(c->copy_stream, sl.consumed, 0));
   if (X8_host)
@@ -1142,9 +1005,9 @@ extern "C" int vbnn_mlp_predict(vbnn_mlp* m, const float* X, int N, int n_sample
     VB_TRY(ensure_pred_partials(m));
     for (float** q : {&m->pred_max, &m->pred_sum})
       if (*q) { cudaFree(*q); *q = nullptr; }
-    VB_TRY(dalloc(&m->pred_max, (size_t)m->max_batch * C * 4));
-    VB_TRY(dalloc(&m->pred_sum, (size_t)m->max_batch * C * 4));
-    VB_TRY(dalloc(&m->pred_ent, (size_t)m->max_batch * 4));
+    VB_TRY(dev_alloc(&m->pred_max, (size_t)m->max_batch * C));
+    VB_TRY(dev_alloc(&m->pred_sum, (size_t)m->max_batch * C));
+    VB_TRY(dev_alloc(&m->pred_ent, (size_t)m->max_batch));
   }
   const bool reduce = nll_host || acc_host;
   int grid = 0;
@@ -1200,7 +1063,7 @@ extern "C" int vbnn_mlp_predict_outputs(vbnn_mlp* m, const float* X, int N, int 
   if (!m->mom_state) {
     VB_TRY(refuse_capture(st, "vbnn_mlp_predict_outputs"));
     VB_TRY(ensure_pred_partials(m));
-    VB_TRY(dalloc(&m->mom_state, (size_t)m->max_batch * (3 * (size_t)C + 2) * 4));
+    VB_TRY(dev_alloc(&m->mom_state, (size_t)m->max_batch * (3 * (size_t)C + 2)));
   }
   const int K = gaussian ? C / 2 : C;
   const size_t NC = (size_t)N * C;
@@ -1253,7 +1116,7 @@ extern "C" int vbnn_mlp_get_outputs(vbnn_mlp* m, int sample_idx, float* logp_hos
            "vbnn_mlp_get_outputs: the last forward was vbnn_mlp_forward_train, whose outputs are in the caller's buffer");
   vbnn_ctx* c = m->ctx;
   const int N = m->last_N, C = m->sizes.back();
-  if (!m->logp) VB_TRY(dalloc(&m->logp, (size_t)m->max_batch * C * 4));
+  if (!m->logp) VB_TRY(dev_alloc(&m->logp, (size_t)m->max_batch * C));
   LossParams lp;
   memset(&lp, 0, sizeof(lp));
   lp.logits = m->logits + (size_t)sample_idx * N * m->ld_logits; lp.ld_logits = m->ld_logits;

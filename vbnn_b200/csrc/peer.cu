@@ -202,9 +202,6 @@ void local_bufs(const vbnn_layer* L, const void* (&ptr)[kBufsPerLayer], size_t (
   for (int k = 0; k < kBufsPerLayer; ++k) { ptr[k] = p[k]; bytes[k] = p[k] ? b[k] : 0; }
 }
 
-inline bool layer_lrt(const vbnn_layer* L) {
-  return L->kind == VBNN_KIND_VB && L->opts.reparam == VBNN_REPARAM_LOCAL;
-}
 inline uint32_t* flag_ptr(const vbnn_peer* P, int q, size_t off, int j, int r) {
   return reinterpret_cast<uint32_t*>(P->peer_block[q] + off) + (size_t)j * P->G + r;
 }
@@ -258,7 +255,7 @@ bool peer_transport_ce(const vbnn_mlp* m, int N) {
 
 bool peer_wire_bf16(const vbnn_mlp* m, int j, int N) {
   const vbnn_layer* L = m->layers[j];
-  return knobs().peer_wire_bf16 != 0 && peer_transport_ce(m, N) && m->bf16 && m->Z == 1 && layer_lrt(L) && (L->I & 7) == 0;
+  return knobs().peer_wire_bf16 != 0 && peer_transport_ce(m, N) && m->bf16 && m->Z == 1 && layer_is_lrt(L) && (L->I & 7) == 0;
 }
 
 void peer_scatter(const vbnn_mlp* m, int j, int N, EpiParams& p) {
@@ -405,7 +402,7 @@ int peer_after_dw(vbnn_mlp* m, int j) {
     u.B = L->opts.B; u.S = (float)L->opts.S;
     u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
     u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
-    u.lrt = layer_lrt(L);
+    u.lrt = layer_is_lrt(L);
     u.prior = layer_prior(L, roff);
     // knob peer_fused_push: the update kernel stores the refreshed operands to every rank itself instead of
     // 2 x (G-1) copy-engine copies.  It paid when layer 0's update was the tail of the minibatch (idle SMs); with
@@ -417,7 +414,7 @@ int peer_after_dw(vbnn_mlp* m, int j) {
       for (int q = 0; q < G; ++q) {
         if (q == me) continue;
         const int i = u.n_push++;
-        if (!layer_lrt(L)) {
+        if (!layer_is_lrt(L)) {
           u.push_mu[i] = (float*)pl.means.ptr[q] + roff; u.push_lv[i] = (float*)pl.lvars.ptr[q] + roff;
         } else if (L->mu_bf16) {
           u.push_mu16[i] = (bf16*)pl.mu_bf16.ptr[q] + roffb; u.push_s216[i] = (bf16*)pl.s2_bf16.ptr[q] + roffb;
@@ -430,7 +427,7 @@ int peer_after_dw(vbnn_mlp* m, int j) {
     c->launches++;
     L->prior_valid = true;
     if (pl.rows > 0 && !fused_push) {
-      if (!layer_lrt(L)) {                       // weight sampling reads mu / log sigma^2 (VBLinear.lua:59)
+      if (!layer_is_lrt(L)) {                    // weight sampling reads mu / log sigma^2 (VBLinear.lua:59)
         VB_TRY(push_shard(P, pl.means, roff * 4, (size_t)pl.rows * L->I * 4));
         VB_TRY(push_shard(P, pl.lvars, roff * 4, (size_t)pl.rows * L->I * 4));
       } else if (L->mu_bf16) {                   // tensor-core operands of the LRT GEMMs
@@ -662,7 +659,7 @@ extern "C" int vbnn_mlp_sync_replicas(vbnn_mlp* m) {
       if (L->w_bf16) VB_TRY(pull_shards(P, pl.weight, L->O, rb, pl.rpo, c->stream));
       continue;
     }
-    if (layer_lrt(L)) {
+    if (layer_is_lrt(L)) {
       if (L->mu_bf16) VB_TRY(pull_shards(P, pl.means, L->O, rb, pl.rpo, c->stream));
       VB_TRY(pull_shards(P, pl.lvars, L->O, rb, pl.rpo, c->stream));
     }

@@ -173,6 +173,22 @@ struct vbnn_mlp {
 };
 
 namespace vbnn {
+// cudaMalloc of count elements (none: nullptr) with the library's error reporting
+template <typename T>
+int dev_alloc(T** p, size_t count) {
+  *p = nullptr;
+  if (count == 0) return VBNN_OK;
+  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
+  if (e != cudaSuccess) {
+    set_error("cudaMalloc(%zu bytes) failed: %s", count * sizeof(T), cudaGetErrorString(e));
+    return e == cudaErrorMemoryAllocation ? VBNN_E_NOMEM : VBNN_E_CUDA;
+  }
+  return VBNN_OK;
+}
+// the layer runs the local reparameterisation: its forward reads mu and sigma^2 and draws the noise per output
+inline bool layer_is_lrt(const vbnn_layer* L) {
+  return L->kind == VBNN_KIND_VB && L->opts.reparam == VBNN_REPARAM_LOCAL;
+}
 int layer_create_internal(vbnn_ctx* ctx, int I, int O, int kind, const vbnn_opts* opts, int S_alloc,
                           float* gW, float* gS, float* gb, int id, vbnn_layer** out);
 int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t);
@@ -191,9 +207,30 @@ bool peer_wire_bf16(const vbnn_mlp* m, int j, int N);                     // lay
 int peer_wait_params(vbnn_mlp* m, int j, bool bump);                      // main stream, before layer j's forward (-1: all layers)
 int peer_after_dw(vbnn_mlp* m, int j);                                    // signal + owner update + push
 int peer_check(vbnn_mlp* m);                                              // host: a peer wait timed out?
-// tensor-core GEMM launch with optional event bracketing (ctx->profiling)
-// prof_cls: class the launch is accounted under (default: its mode)
-int tc_gemm(vbnn_ctx* ctx, int mode, const TcGemmArgs& g, const EpiParams& p, int prof_cls = -1);
+// The weight operands of the forward (kmajor = 1: B = W^T) and backward-data (kmajor = 0: B = W) GEMMs in the
+// layer's precision: B1 = mu for an LRT layer (MAP mode included), else W -- per sample when `batched`; with
+// `lrt` (the layer runs the LRT form) also B2 = sigma^2.
+void weight_operands(GemmArgs& g, const vbnn_layer* L, int kmajor, bool batched, bool lrt);
+// GEMM launch on the bf16 tcgen05 engine or the fp32 CUDA-core engine.  While ctx->profiling, a bf16 launch is
+// timed and accounted under prof_cls (default: its mode).
+int gemm(vbnn_ctx* ctx, bool bf16, int mode, const GemmArgs& g, const EpiParams& p, int prof_cls = -1);
 int prof_collect(vbnn_ctx* ctx);
 int prof_mark(vbnn_ctx* ctx, int id);     // id 0 starts a minibatch; no-op unless profiling
+// launch() under a pair of CUDA events while ctx->profiling, accounted to class cls with `work` in its flops slot
+template <typename Launch>
+int prof_launch(vbnn_ctx* c, int cls, double work, Launch&& launch) {
+  if (!c->profiling) return launch();
+  vbnn_ctx::ProfRec r;
+  for (cudaEvent_t* e : {&r.a, &r.b}) {
+    if (!c->prof_pool.empty()) { *e = c->prof_pool.back(); c->prof_pool.pop_back(); }
+    else VB_CUDA(cudaEventCreate(e));
+  }
+  r.cls = cls; r.flops = work;
+  VB_CUDA(cudaEventRecord(r.a, c->stream));
+  const int rc = launch();
+  VB_CUDA(cudaEventRecord(r.b, c->stream));
+  c->prof_recs.push_back(r);
+  if (c->prof_recs.size() + c->marks.size() >= 4096) VB_TRY(prof_collect(c));
+  return rc;
+}
 }  // namespace vbnn

@@ -18,6 +18,7 @@ const Entry kTable[] = {
     {"tc_dw64", &Knobs::tc_dw64},       {"dw_eps16", &Knobs::dw_eps16},       {"lrt_split", &Knobs::lrt_split}, {"dw_split", &Knobs::dw_split},
     {"dp_overlap", &Knobs::dp_overlap}, {"no_graph", &Knobs::no_graph},   {"upd_bps", &Knobs::upd_bps},   {"peer_fused_push", &Knobs::peer_fused_push}, {"peer_transport", &Knobs::peer_transport}, {"peer_one_stream", &Knobs::peer_one_stream},
     {"peer_push_ctas", &Knobs::peer_push_ctas}, {"peer_wire_bf16", &Knobs::peer_wire_bf16},
+    {"upd_coresident", &Knobs::upd_coresident},
 };
 
 // VBNN_<NAME>

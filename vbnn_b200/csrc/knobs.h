@@ -24,7 +24,10 @@ struct Knobs {
   int lrt_split = 1;    // bit 0: split LRT forward, bit 1: split LRT backward-data
   int dw_split = -1;    // LRT dW as two single-accumulator GEMMs: -1 = only in peer mode
   int dp_overlap = 1;   // NCCL mode: per-layer allreduce overlapped with backward
-  int upd_bps = 4;      // fused update: 256-thread blocks per SM in its grid
+  int upd_bps = 4;      // fused update: 256-thread blocks per SM in its grid; read when a layer is created, so it applies
+                        // to layers created after it is set (a layer's update grid and partial count stay fixed)
+  int upd_coresident = 0;  // one GPU: run the 128-thread co-resident update variant (peer mode's) where it applies
+                           // (I % 4 == 0, no diagnostics); for testing it without a second GPU
   int no_graph = 0;     // eager launches instead of CUDA graph replay
   int peer_transport = 0;  // gradient reduce-scatter: 0 = auto, 1 = NVLink stores from the dW epilogue, 2 = local staging + copy engines,
                            // 3 = local staging + one co-resident copy kernel per layer (transfer + signal fused)

@@ -249,6 +249,10 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
   u.lrt = layer_is_lrt(L);
   u.prior = layer_prior(L, 0);
+  // the grid that writes the next partials must be the one whose count (n_part, fixed at creation) the next update
+  // reads: update_grid() under a later upd_bps would write more or fewer of them
+  u.grid_override = L->n_part;
+  u.coresident = knobs().upd_coresident != 0;
   double* stat_dev = stats ? c->d_partials + kMaxPartials : nullptr;
   u.stat_partials = stat_dev;
   int grid = 0;

@@ -217,7 +217,8 @@ int vbnn_layer_calc_lc(vbnn_layer* layer, float* lc_dev, float* sum_host);
  *     buffers (vbnn_layer_get / _set / _device_ptr with VBNN_BUF_PRIOR_MEANS / _LVARS, which return VBNN_E_STATE
  *     under any other kind); an edit takes effect at the next update.  They are allocated by the first PER_WEIGHT
  *     call and kept until vbnn_layer_destroy, so a pointer from vbnn_layer_device_ptr stays valid across kind
- *     changes.  In peer mode each rank keeps its own copy: edit it on every rank.
+ *     changes.  In peer mode each rank keeps its own copy: edit it on every rank (the same rule holds for the
+ *     values of vbnn_layer_set_opts / vbnn_mlp_set_opts).
  *   - FIXED and PER_WEIGHT compute the KL terms from log var_hat (FIXED: log var0) without a division: they are
  *     finite wherever the exact value is representable in fp32 (for log var_hat >= -177), and the mean term is
  *     exactly 0 where mu == mu_hat.
@@ -237,6 +238,36 @@ int vbnn_layer_calc_lc(vbnn_layer* layer, float* lc_dev, float* sum_host);
 int vbnn_layer_set_prior(vbnn_layer* layer, int kind, float mu0, float var0);
 /* the current kind; mu0 / var0 (nullable) receive FIXED's scalars, NaN under the other kinds */
 int vbnn_layer_get_prior(const vbnn_layer* layer, int* kind, float* mu0, float* var0);
+
+/* Learning-rate schedules and KL annealing: the reference reads opt.B and its optimiser tables (learningRate, beta1,
+ * beta2, epsilon) at every update (VBLinear.lua:31-33,90-103,125-143), so a Torch7 user decays a rate or anneals the KL
+ * weight 1/B by writing them between minibatches.  The idiom here is get, modify, set.
+ *   - Live fields: B, lr_bias, lr_mu, lr_var, adam_beta1, adam_beta2, adam_eps.  B must be finite and > 0, each rate
+ *     finite and >= 0, each beta in [0, 1), adam_eps finite and > 0.  Every other field (var_init, msr_init, mu_init,
+ *     S, reparam, precision, strict_reference) must equal the layer's current value: they size buffers, choose
+ *     kernels or only matter at creation.  Otherwise VBNN_E_INVALID, naming the field.  A refused call changes
+ *     nothing; vbnn_mlp_set_opts checks every layer before it writes any.
+ *   - A new value applies to every update enqueued on the context's stream after the call -- vbnn_layer_update,
+ *     vbnn_mlp_update, vbnn_mlp_step, vbnn_mlp_step_grad_input, vbnn_mlp_backward_update, vbnn_mlp_submit_host*,
+ *     the peer-mode shard updates -- and to vbnn_layer_grads, vbnn_layer_calc_lc and vbnn_mlp_calc_lc.  lr_bias is
+ *     the SGD rate of the biases and of a plain nn.Linear output layer; Adam applies lr * sqrt(1 - beta2^t) /
+ *     (1 - beta1^t) with the current values and the layer's own t, as optim.adam does.
+ *   - The values live in a small device block per layer that the update kernels read, written by one launch on the
+ *     context's stream (counted by vbnn_mlp_launch_count).  No step graph is re-captured or dropped
+ *     (vbnn_mlp_graph_captures does not move), and the call does not synchronise.
+ *   - Accepted at any time outside stream capture, also while a vbnn_mlp_forward_train step is open: that step's
+ *     vbnn_mlp_backward_update then uses the new values.  While the context's stream is being captured:
+ *     VBNN_E_STATE (the host copy would disagree with the graph).
+ *   - vbnn_layer_get_opts returns the last values set, whether or not the device has reached the write yet.
+ *   - vbnn_layer_set_opts on a layer borrowed from a net gives that layer its own values (per-layer optimiser
+ *     tables in Torch7); vbnn_mlp_set_opts sets every layer of the net and replaces the net's own copy.
+ *   - Peer mode: the context's stream first waits for the library's side stream (as vbnn_mlp_join_streams does), so
+ *     the previous minibatch's shard update still reads the old values.  Each rank keeps its own copy: set the same
+ *     values on every rank.  NCCL mode needs nothing extra.
+ * NULL arguments: VBNN_E_INVALID. */
+int vbnn_layer_get_opts(const vbnn_layer* layer, vbnn_opts* out);
+int vbnn_layer_set_opts(vbnn_layer* layer, const vbnn_opts* opts);
+int vbnn_mlp_set_opts(vbnn_mlp* mlp, const vbnn_opts* opts);   /* every layer of the net */
 
 /* parameters() / field access (mlp.lua:37,48-49; main.lua:123; checkpointing utils.lua:73-80) */
 int vbnn_layer_get(vbnn_layer* layer, int which, float* dst_host);

@@ -144,6 +144,12 @@ function VBLinear:set_prior(kind, mean, var)
    V.check(C.vbnn_layer_set_prior(self.h, PRIOR[kind], mean or 0, var or 0))
 end
 
+-- Learning-rate schedules and KL annealing (vbnn_layer_set_opts): the reference reads opt.B and its optimiser tables at
+-- every update, so decay a rate or anneal opt.B, then call setOpt(opt) before the next minibatch
+function VBLinear:setOpt(opt)
+   V.check(C.vbnn_layer_set_opts(self.h, V.opts(opt)))
+end
+
 function VBLinear:clamp_to_map()                                     -- :105-107
    self:bind()
    V.check(C.vbnn_layer_clamp_to_map(self.h))

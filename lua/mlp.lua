@@ -53,6 +53,12 @@ function MLP:set_prior(kind, mean, var)
    end
 end
 
+-- VBLinear:setOpt on every layer of the net in one call (vbnn_mlp_set_opts); no step graph is re-captured
+function MLP:setOpt(opt)
+   V.check(C.vbnn_mlp_set_opts(self.h, V.opts(opt)))
+   self.opt = opt
+end
+
 function MLP:resetGradients()                                         -- mlp.lua:62-67
    self.s = 0
    V.check(C.vbnn_mlp_reset_gradients(self.h))

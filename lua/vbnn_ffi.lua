@@ -34,6 +34,8 @@ int vbnn_layer_update(vbnn_layer*, vbnn_stats*);
 int vbnn_layer_calc_lc(vbnn_layer*, float* lc_dev, float* sum_host);
 int vbnn_layer_set_prior(vbnn_layer*, int kind, float mu0, float var0);
 int vbnn_layer_get_prior(const vbnn_layer*, int* kind, float* mu0, float* var0);
+int vbnn_layer_get_opts(const vbnn_layer*, vbnn_opts* out);
+int vbnn_layer_set_opts(vbnn_layer*, const vbnn_opts*);
 int vbnn_layer_device_ptr(vbnn_layer*, int which, float** ptr_dev, size_t* count);
 int vbnn_layer_bind(vbnn_layer*, int which, float* ptr_dev);
 /* net level (lua/mlp.lua): the mlp.lua object and the main.lua:19-51 closure */
@@ -48,6 +50,7 @@ int vbnn_mlp_sample(vbnn_mlp*, int sample_idx);
 int vbnn_mlp_run(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, int sample_idx, float* err_host, float* acc_host);
 int vbnn_mlp_update(vbnn_mlp*);
 int vbnn_mlp_calc_lc(vbnn_mlp*, float* lc_host);
+int vbnn_mlp_set_opts(vbnn_mlp*, const vbnn_opts*);
 int vbnn_mlp_step(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev);
 int vbnn_mlp_step_grad_input(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N, float* result_dev, float* dX_dev);
 int vbnn_mlp_forward_train(vbnn_mlp*, const float* X_dev, int N, float* logits_dev);
@@ -114,12 +117,19 @@ function M.context(seed, net_level)
    return M.ctx
 end
 
+-- config.lua's table mapped as vbnn_b200/config.py maps it, at creation and by setOpt.  The fields the reference reads at
+-- every update: opt.B, opt.state / meanState / varState learningRate, and meanState's beta1 / beta2 / epsilon (optim.adam's
+-- 0.9, 0.999, 1e-8 where absent).  setOpt passes the whole table, so the library refuses a change of anything else (S,
+-- reparam, precision, ...) instead of ignoring it.
 function M.opts(opt)
    local o = ffi.new('vbnn_opts')
    C.vbnn_opts_default(o)
    o.var_init = opt.var_init; o.msr_init = opt.msr_init and 1 or 0; o.mu_init = opt.mu_init
    o.B = opt.B; o.S = opt.S
    o.lr_bias = opt.state.learningRate; o.lr_mu = opt.meanState.learningRate; o.lr_var = opt.varState.learningRate
+   o.adam_beta1 = opt.meanState.beta1 or 0.9
+   o.adam_beta2 = opt.meanState.beta2 or 0.999
+   o.adam_eps = opt.meanState.epsilon or 1e-8
    o.reparam = (opt.reparam == 'local') and 1 or 0
    o.precision = (opt.precision == 'bf16') and 1 or 0
    o.strict_reference = (opt.strict_reference == false) and 0 or 1

@@ -31,6 +31,11 @@ class VbnnOpts(C.Structure):
                 ("strict_reference", C.c_int)]
 
 
+# the fields vbnn_layer_set_opts may change (the reference reads them at every update), in the order
+# MLP.state_dict() stores them
+LIVE_OPTS = ("B", "lr_bias", "lr_mu", "lr_var", "adam_beta1", "adam_beta2", "adam_eps")
+
+
 class VbnnStats(C.Structure):
     _fields_ = [(n, C.c_float) for n in (
         "vlc_grad", "vle_grad", "mlc_grad", "mle_grad", "min_variance", "max_variance",
@@ -73,6 +78,9 @@ _PROTOS = {
     "vbnn_layer_calc_lc": (C.c_int, [_P, _P, _F]),
     "vbnn_layer_set_prior": (C.c_int, [_P, C.c_int, C.c_float, C.c_float]),
     "vbnn_layer_get_prior": (C.c_int, [_P, C.POINTER(C.c_int), _F, _F]),
+    "vbnn_layer_get_opts": (C.c_int, [_P, C.POINTER(VbnnOpts)]),
+    "vbnn_layer_set_opts": (C.c_int, [_P, C.POINTER(VbnnOpts)]),
+    "vbnn_mlp_set_opts": (C.c_int, [_P, C.POINTER(VbnnOpts)]),
     "vbnn_layer_get": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_layer_set": (C.c_int, [_P, C.c_int, _P]),
     "vbnn_layer_device_ptr": (C.c_int, [_P, C.c_int, C.POINTER(_P), C.POINTER(C.c_size_t)]),

@@ -30,20 +30,44 @@ def default_opt(**over):
 
 
 def opts_struct(opt) -> L.VbnnOpts:
+    """buildModel's mapping of the config dict to vbnn_opts; set_opt passes the same mapping to vbnn_*_set_opts,
+    which refuses a change of any field but the live ones (L.LIVE_OPTS)."""
     o = L.VbnnOpts()
     L.lib().vbnn_opts_default(o)
     o.var_init = float(opt["var_init"])
     o.msr_init = 1 if opt.get("msr_init") else 0
     o.mu_init = float(opt["mu_init"])
-    o.B = float(opt["B"])
     o.S = int(opt["S"])
+    _live_fields(o, opt)
+    o.reparam = L.REPARAM_LOCAL if opt.get("reparam", "weight") == "local" else L.REPARAM_WEIGHT
+    o.precision = L.PREC_BF16 if opt.get("precision", "fp32") == "bf16" else L.PREC_FP32
+    o.strict_reference = 1 if opt.get("strict_reference", True) else 0
+    return o
+
+
+def _live_fields(o, opt):
+    o.B = float(opt["B"])
     o.lr_bias = float(opt["state"]["learningRate"])
     o.lr_mu = float(opt["meanState"]["learningRate"])
     o.lr_var = float(opt["varState"]["learningRate"])
     o.adam_beta1 = float(opt["meanState"].get("beta1", 0.9))
     o.adam_beta2 = float(opt["meanState"].get("beta2", 0.999))
     o.adam_eps = float(opt["meanState"].get("epsilon", 1e-8))
-    o.reparam = L.REPARAM_LOCAL if opt.get("reparam", "weight") == "local" else L.REPARAM_WEIGHT
-    o.precision = L.PREC_BF16 if opt.get("precision", "fp32") == "bf16" else L.PREC_FP32
-    o.strict_reference = 1 if opt.get("strict_reference", True) else 0
-    return o
+
+
+def with_live(opt, src):
+    """A copy of the config dict opt whose live keys -- B and the optimiser tables state / meanState / varState, the
+    keys opts_struct reads the live fields from -- are src's.  src: a config dict, or {field: value} over L.LIVE_OPTS
+    (what a layer reports).  Every other key keeps opt's value."""
+    out = dict(opt)
+    if all(f in src for f in L.LIVE_OPTS):
+        out["B"] = src["B"]
+        out["state"] = dict(opt["state"], learningRate=src["lr_bias"])
+        out["meanState"] = dict(opt["meanState"], learningRate=src["lr_mu"], beta1=src["adam_beta1"],
+                                beta2=src["adam_beta2"], epsilon=src["adam_eps"])
+        out["varState"] = dict(opt["varState"], learningRate=src["lr_var"])
+        return out
+    out["B"] = src["B"]
+    for k in ("state", "meanState", "varState"):
+        out[k] = dict(src[k])
+    return out

@@ -197,8 +197,14 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
   __shared__ double sh[32];
   __shared__ float s_var_hat;
   __shared__ AdamCoef s_coef;
+  __shared__ LiveOpts s_hp;             // the layer's hyper-parameters, read once per block
+  // t for the epilogue's partials half: kept in shared memory, not in a register live across the main loop (the
+  // 128-thread variant is at its 80-register cap)
+  __shared__ int s_t;
   const int t_now = *p.t_dev;
   {
+    LiveOpts hp;
+    if (threadIdx.x == 0) hp = *p.hp;
     double r = 0.0;
     if (PK == VBNN_PRIOR_EMPIRICAL) {
       const double* part = p.partials + (p.partials_pingpong ? (size_t)(t_now & 1) * kMaxPartials : 0);
@@ -216,17 +222,20 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
         s_var_hat = 1.f;                                                // unused: kl_mu / kl_lvar
       }
       const int t = t_now + 1;                                          // state.t = state.t + 1
-      double bc1 = 1.0 - pow((double)p.beta1, (double)t);
-      double bc2 = 1.0 - pow((double)p.beta2, (double)t);
-      s_coef.step_mu = (float)((double)p.lr_mu * sqrt(bc2) / bc1);
-      s_coef.step_var = (float)((double)p.lr_var * sqrt(bc2) / bc1);
+      s_t = t;
+      double bc1 = 1.0 - pow((double)hp.beta1, (double)t);
+      double bc2 = 1.0 - pow((double)hp.beta2, (double)t);
+      s_coef.step_mu = (float)((double)hp.lr_mu * sqrt(bc2) / bc1);
+      s_coef.step_var = (float)((double)hp.lr_var * sqrt(bc2) / bc1);
+      s_hp = hp;
     }
     __syncthreads();
   }
   const float var_hat = s_var_hat;
-  const float inv_S = 1.f / p.S, inv_BV = 1.f / (p.B * var_hat), inv_2B = 1.f / (2.f * p.B);
+  const float B = s_hp.B, eps = s_hp.eps;
+  const float inv_S = 1.f / p.S, inv_BV = 1.f / (B * var_hat), inv_2B = 1.f / (2.f * B);
   const float inv_vh = 1.f / var_hat;
-  const float b1 = p.beta1, b2 = p.beta2, omb1 = 1.f - p.beta1, omb2 = 1.f - p.beta2;
+  const float b1 = s_hp.beta1, b2 = s_hp.beta2, omb1 = 1.f - s_hp.beta1, omb2 = 1.f - s_hp.beta2;
 
   float nxt = 0.f;                       // sigma_hat^2 numerator of the next minibatch
   double st[kStatSlots];
@@ -333,11 +342,11 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
       // optim.adam on means (:135-138)
       mm[j] = b1 * mm[j] + omb1 * gmu;
       vm[j] = b2 * vm[j] + omb2 * gmu * gmu;
-      const float dmu = -s_coef.step_mu * mm[j] / (sqrtf(vm[j]) + p.eps);
+      const float dmu = -s_coef.step_mu * mm[j] / (sqrtf(vm[j]) + eps);
       // optim.adam on lvars (:140-143)
       mv[j] = b1 * mv[j] + omb1 * gvar;
       vv[j] = b2 * vv[j] + omb2 * gvar * gvar;
-      const float dlv = -s_coef.step_var * mv[j] / (sqrtf(vv[j]) + p.eps);
+      const float dlv = -s_coef.step_var * mv[j] / (sqrtf(vv[j]) + eps);
       mu[j] += dmu;
       lv[j] += dlv;
       s2_new[j] = __expf(lv[j]);
@@ -387,7 +396,7 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
   if (p.next_partials) {
     double r = block_sum((double)nxt, sh);
     if (threadIdx.x == 0) {
-      const size_t idx = (p.partials_pingpong ? (size_t)((t_now + 1) & 1) * kMaxPartials : 0) + p.part_off + blockIdx.x;
+      const size_t idx = (p.partials_pingpong ? (size_t)(s_t & 1) * kMaxPartials : 0) + p.part_off + blockIdx.x;
       p.next_partials[idx] = r;
       for (int q = 0; q < p.n_peer; ++q) p.peer_partials[q][idx] = r;
       if (p.n_peer > 0) __threadfence_system();
@@ -421,9 +430,10 @@ __global__ void __launch_bounds__(TPB, TPB == 128 ? 6 : 1) k_update(UpdateParams
 // ------------------------------------------------------------------ grads (API parity) ---
 __global__ void __launch_bounds__(kThreads) k_grads(const float* mu, const float* lvar, float* gW,
                                                     float* gS, long long n, const float* var_hat_dev,
-                                                    PriorArgs pr, float B, float S, int lrt, float* mleg,
-                                                    float* mlcg, float* vleg, float* vlcg) {
+                                                    PriorArgs pr, const LiveOpts* hp, float S, int lrt,
+                                                    float* mleg, float* mlcg, float* vleg, float* vlcg) {
   const float var_hat = *var_hat_dev;                                   // EMPIRICAL
+  const float B = hp->B;
   const bool args = pr.kind != VBNN_PRIOR_EMPIRICAL;                    // mu_hat, l0 from pr: as k_update
   const bool do_mu = mleg || mlcg, do_var = vleg || vlcg;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
@@ -452,10 +462,11 @@ __global__ void __launch_bounds__(kThreads) k_grads(const float* mu, const float
 // ------------------------------------------------------------------ calc_lc -------------
 __global__ void __launch_bounds__(kThreads) k_calc_lc(const float* var_src, int var_kind,
                                                       const float* mu_src, int mu_is_sq, long long n,
-                                                      const float* var_hat_dev, PriorArgs pr, float B,
+                                                      const float* var_hat_dev, PriorArgs pr, const LiveOpts* hp,
                                                       float* lc_out, double* partials) {
   __shared__ double sh[32];
   const float var_hat = *var_hat_dev;                                   // EMPIRICAL
+  const float B = hp->B;
   const float log_sd_hat = 0.5f * logf(var_hat);
   const bool args = pr.kind != VBNN_PRIOR_EMPIRICAL;                    // mu_hat, l0 from pr
   double acc = 0.0;
@@ -490,8 +501,9 @@ __global__ void __launch_bounds__(kThreads) k_calc_lc(const float* var_src, int 
 }
 
 // ------------------------------------------------------------------ sgd -----------------
-__global__ void __launch_bounds__(kThreads) k_sgd(float* x, const float* g, long long n, float lr,
+__global__ void __launch_bounds__(kThreads) k_sgd(float* x, const float* g, long long n, const float* lr_dev,
                                                   bf16* xb, int I, int ld) {
+  const float lr = *lr_dev;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
        e += (long long)gridDim.x * blockDim.x) {
     float v = x[e] - lr * g[e];
@@ -506,7 +518,8 @@ __global__ void __launch_bounds__(kThreads) k_sgd(float* x, const float* g, long
 
 // peer mode: the gradient is the sum of the ranks' receive slots
 __global__ void __launch_bounds__(kThreads) k_sgd_slots(float* x, const float* g, int n_src, long long src_stride,
-                                                        long long n, float lr, bf16* xb, int I, int ld) {
+                                                        long long n, const float* lr_dev, bf16* xb, int I, int ld) {
+  const float lr = *lr_dev;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n;
        e += (long long)gridDim.x * blockDim.x) {
     float gs = 0.f;
@@ -979,6 +992,8 @@ __global__ void __launch_bounds__(kThreads) k_fill(float* dst, long long n, floa
     dst[e] = v;
 }
 
+__global__ void k_set_live_opts(LiveOpts* dst, LiveOpts v) { *dst = v; }
+
 __global__ void __launch_bounds__(kThreads) k_init_normal(float* dst, long long n, float mean,
                                                           float std, PhiloxStream ps) {
   const long long quads = (n + 3) >> 2;
@@ -1102,27 +1117,27 @@ int launch_update(const UpdateParams& p, int* grid_out, cudaStream_t st) {
 }
 
 int launch_grads(const float* mu, const float* lvar, float* gW, float* gS, long long n,
-                 const float* var_hat_dev, const PriorArgs& pr, float B, float S, int lrt, float* mleg, float* mlcg,
-                 float* vleg, float* vlcg, cudaStream_t st) {
-  k_grads<<<grid_for(n), kThreads, 0, st>>>(mu, lvar, gW, gS, n, var_hat_dev, pr, B, S, lrt, mleg, mlcg,
+                 const float* var_hat_dev, const PriorArgs& pr, const LiveOpts* hp, float S, int lrt, float* mleg,
+                 float* mlcg, float* vleg, float* vlcg, cudaStream_t st) {
+  k_grads<<<grid_for(n), kThreads, 0, st>>>(mu, lvar, gW, gS, n, var_hat_dev, pr, hp, S, lrt, mleg, mlcg,
                                             vleg, vlcg);
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }
 
 int launch_calc_lc(const float* var_src, int var_kind, const float* mu_src, int mu_is_sq, long long n,
-                   const float* var_hat_dev, const PriorArgs& pr, float B, float* lc_out, double* partials,
+                   const float* var_hat_dev, const PriorArgs& pr, const LiveOpts* hp, float* lc_out, double* partials,
                    int* n_partials_out, cudaStream_t st) {
   int grid = grid_for(n, 4);
   if (grid > kMaxPartials) grid = kMaxPartials;
-  k_calc_lc<<<grid, kThreads, 0, st>>>(var_src, var_kind, mu_src, mu_is_sq, n, var_hat_dev, pr, B, lc_out,
+  k_calc_lc<<<grid, kThreads, 0, st>>>(var_src, var_kind, mu_src, mu_is_sq, n, var_hat_dev, pr, hp, lc_out,
                                        partials);
   VB_CUDA(cudaGetLastError());
   *n_partials_out = grid;
   return VBNN_OK;
 }
 
-int launch_sgd(float* x, const float* g, long long n, float lr, bf16* x_bf16, int I, int ld_bf16,
+int launch_sgd(float* x, const float* g, long long n, const float* lr, bf16* x_bf16, int I, int ld_bf16,
                cudaStream_t st) {
   if (n <= 0) return VBNN_OK;
   k_sgd<<<grid_for(n), kThreads, 0, st>>>(x, g, n, lr, x_bf16, I, ld_bf16);
@@ -1130,7 +1145,7 @@ int launch_sgd(float* x, const float* g, long long n, float lr, bf16* x_bf16, in
   return VBNN_OK;
 }
 
-int launch_sgd_slots(float* x, const float* g, int n_src, long long src_stride, long long n, float lr,
+int launch_sgd_slots(float* x, const float* g, int n_src, long long src_stride, long long n, const float* lr,
                      bf16* x_bf16, int I, int ld_bf16, cudaStream_t st) {
   if (n <= 0) return VBNN_OK;
   k_sgd_slots<<<grid_for(n), kThreads, 0, st>>>(x, g, n_src, src_stride, n, lr, x_bf16, I, ld_bf16);
@@ -1291,6 +1306,12 @@ int launch_mul_act(const void* a, int lda, int a_is_bf16, const void* b, int ldb
 int launch_fill(float* dst, long long n, float v, cudaStream_t st) {
   if (n <= 0) return VBNN_OK;
   k_fill<<<grid_for(n), kThreads, 0, st>>>(dst, n, v);
+  VB_CUDA(cudaGetLastError());
+  return VBNN_OK;
+}
+
+int launch_set_live_opts(LiveOpts* dst, const LiveOpts& v, cudaStream_t st) {
+  k_set_live_opts<<<1, 1, 0, st>>>(dst, v);
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }

@@ -45,6 +45,12 @@ int launch_prior_finalize(const double* partials, int n_partials, long long W, f
                           const float* mu, const float* lvar, float* stdv, float* mu_sqe, const PriorArgs& pr,
                           cudaStream_t st);
 
+// The hyper-parameters the reference reads at every update (vbnn_layer_set_opts): one block per layer in device
+// memory.  The update kernels read it when they run, so a captured step graph follows a change without re-capture.
+struct LiveOpts { float B, lr_bias, lr_mu, lr_var, beta1, beta2, eps; };
+// *dst = v on the stream, by a one-thread kernel (the values travel as its arguments)
+int launch_set_live_opts(LiveOpts* dst, const LiveOpts& v, cudaStream_t st);
+
 // VBLinear:update (VBLinear.lua:124-166) minus the bias SGD: KL + likelihood gradients and both
 // Adam steps in one pass.
 struct UpdateParams {
@@ -59,8 +65,8 @@ struct UpdateParams {
   int partials_pingpong;                // partials / next_partials are 2 x kMaxPartials halves selected by (*t_dev & 1)
   float* var_hat_dev;                   // out: var_hat used by this update
   const int* t_dev;                     // Adam step counter (t BEFORE this update)
-  float B, S;
-  float lr_mu, lr_var, beta1, beta2, eps;
+  float S;
+  const LiveOpts* hp;                   // B, lr_mu, lr_var, beta1, beta2, eps of the layer
   int lrt;
   double* stat_partials;                // nullable [grid x kStatSlots]
   double* next_partials;                // nullable [grid]: sum(exp(lvar_new) + mu_new^2) per block, i.e.
@@ -88,22 +94,23 @@ struct UpdateParams {
 int launch_update(const UpdateParams& p, int* grid_out, cudaStream_t st);
 
 // compute_mugrads / compute_vargrads (VBLinear.lua:90-98) as standalone tensors (API parity).  EMPIRICAL reads var_hat
-// from var_hat_dev (mu_hat = 0); FIXED and PER_WEIGHT take mu_hat and log var_hat from pr, as k_update.
+// from var_hat_dev (mu_hat = 0); FIXED and PER_WEIGHT take mu_hat and log var_hat from pr, as k_update.  B from hp.
 int launch_grads(const float* mu, const float* lvar, float* gW, float* gS, long long n,
-                 const float* var_hat_dev, const PriorArgs& pr, float B, float S, int lrt, float* mleg, float* mlcg,
-                 float* vleg, float* vlcg, cudaStream_t st);
+                 const float* var_hat_dev, const PriorArgs& pr, const LiveOpts* hp, float S, int lrt, float* mleg,
+                 float* mlcg, float* vleg, float* vlcg, cudaStream_t st);
 
 // VBLinear:calc_lc (VBLinear.lua:99-103); mu_is_sq: mu_src is the mu_sqe cache (mu - mu_hat)^2.  Prior as in
-// launch_grads.
+// launch_grads, B from hp.
 int launch_calc_lc(const float* var_src, int var_kind /*0 lvar, 1 stdv*/, const float* mu_src,
-                   int mu_is_sq, long long n, const float* var_hat_dev, const PriorArgs& pr, float B, float* lc_out,
-                   double* partials, int* n_partials_out, cudaStream_t st);
+                   int mu_is_sq, long long n, const float* var_hat_dev, const PriorArgs& pr, const LiveOpts* hp,
+                   float* lc_out, double* partials, int* n_partials_out, cudaStream_t st);
 
-// x -= lr * g  (optim.sgd, VBLinear.lua:125-128, mlp.lua:120-123) + optional bf16 operand copy
-int launch_sgd(float* x, const float* g, long long n, float lr, bf16* x_bf16, int I, int ld_bf16,
+// x -= lr * g  (optim.sgd, VBLinear.lua:125-128, mlp.lua:120-123) + optional bf16 operand copy; *lr is read on the
+// device (LiveOpts::lr_bias)
+int launch_sgd(float* x, const float* g, long long n, const float* lr, bf16* x_bf16, int I, int ld_bf16,
                cudaStream_t st);
 // peer mode: g = sum of n_src receive slots src_stride floats apart
-int launch_sgd_slots(float* x, const float* g, int n_src, long long src_stride, long long n, float lr,
+int launch_sgd_slots(float* x, const float* g, int n_src, long long src_stride, long long n, const float* lr,
                      bf16* x_bf16, int I, int ld_bf16, cudaStream_t st);
 
 // LogSoftMax + ClassNLLCriterion forward/backward + accuracy (mlp.lua:30-32,78-82; utils.lua:11-27)

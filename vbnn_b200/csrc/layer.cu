@@ -115,6 +115,7 @@ int layer_create_internal(vbnn_ctx* ctx, int I, int O, int kind, const vbnn_opts
 #define A_(expr) do { if (r == VBNN_OK) r = (expr); } while (0)
   A_(dev_zalloc(&L->bias, O, st));
   A_(dev_zalloc(&L->t_dev, 1, st));
+  A_(dev_alloc(&L->hp, 1));
   if (gW) { L->gW = gW; L->gS = gS; L->gb = gb; L->grads_external = true; }
   else {
     A_(dev_zalloc(&L->gW, W, st));
@@ -144,6 +145,8 @@ int layer_create_internal(vbnn_ctx* ctx, int I, int O, int kind, const vbnn_opts
   }
 #undef A_
   if (r != VBNN_OK) { vbnn_layer_destroy(L); return r; }
+  // before any graph can capture a kernel that reads it
+  VB_TRY(launch_set_live_opts(L->hp, live_opts(*opts), st));
   // ---- initial values: VBLinear.lua:12-29 ----
   if (vb) {
     float var_init = opts->msr_init ? 2.0f / (float)I : opts->var_init;                 // :12-16
@@ -157,7 +160,7 @@ int layer_create_internal(vbnn_ctx* ctx, int I, int O, int kind, const vbnn_opts
     VB_TRY(launch_init_normal(L->weight, W, 0.f, sqrtf(2.0f / (float)I), layer_stream(L, kStreamInit, 0), st));
   }
   VB_TRY(layer_refresh_copies(L));
-  ctx->launches += 3;
+  ctx->launches += 4;
   *out = L;
   return VBNN_OK;
 }
@@ -225,13 +228,13 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   const long long W = (long long)L->O * L->I;
   if (L->kind == VBNN_KIND_LINEAR) {
     // optim.sgd over the whole output layer (mlp.lua:120-123; quirk Q4: intent, not the 110 slice)
-    VB_TRY(launch_sgd(L->weight, L->gW, W, L->opts.lr_bias, L->w_bf16, L->I, L->ldI, st));
-    VB_TRY(launch_sgd(L->bias, L->gb, L->O, L->opts.lr_bias, nullptr, 1, 1, st));
+    VB_TRY(launch_sgd(L->weight, L->gW, W, &L->hp->lr_bias, L->w_bf16, L->I, L->ldI, st));
+    VB_TRY(launch_sgd(L->bias, L->gb, L->O, &L->hp->lr_bias, nullptr, 1, 1, st));
     c->launches += 2;
     if (bump_t) VB_TRY(bump_layer_t(L));
     return VBNN_OK;
   }
-  VB_TRY(launch_sgd(L->bias, L->gb, L->O, L->opts.lr_bias, nullptr, 1, 1, st));          // VBLinear.lua:125-128
+  VB_TRY(launch_sgd(L->bias, L->gb, L->O, &L->hp->lr_bias, nullptr, 1, 1, st));         // VBLinear.lua:125-128
   // compute_prior (:130): the per-block sums of exp(lvar)+mu^2 were left behind by the previous
   // update of this layer (or by layer_refresh_prior_partials after set / init)
   UpdateParams u;
@@ -244,9 +247,8 @@ int layer_update_internal(vbnn_layer* L, vbnn_stats* stats, bool bump_t) {
   u.partials = L->prior_partials; u.n_partials = L->n_part;
   u.next_partials = L->prior_partials; u.partials_pingpong = 1;
   u.var_hat_dev = L->var_hat_dev; u.t_dev = L->t_dev;
-  u.B = L->opts.B; u.S = (float)L->opts.S;
-  u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
-  u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
+  u.S = (float)L->opts.S;
+  u.hp = L->hp;
   u.lrt = layer_is_lrt(L);
   u.prior = layer_prior(L, 0);
   // the grid that writes the next partials must be the one whose count (n_part, fixed at creation) the next update
@@ -496,7 +498,7 @@ extern "C" int vbnn_layer_destroy(vbnn_layer* L) {
   }
   DEV_FREE(L->m_mu); DEV_FREE(L->v_mu); DEV_FREE(L->m_var); DEV_FREE(L->v_var);
   DEV_FREE(L->eps); DEV_FREE(L->stdv); DEV_FREE(L->mu_sqe); DEV_FREE(L->s2_f32);
-  DEV_FREE(L->var_hat_dev); DEV_FREE(L->t_dev); DEV_FREE(L->prior_partials);
+  DEV_FREE(L->var_hat_dev); DEV_FREE(L->t_dev); DEV_FREE(L->hp); DEV_FREE(L->prior_partials);
   DEV_FREE(L->w_bf16); DEV_FREE(L->mu_bf16); DEV_FREE(L->s2_bf16); DEV_FREE(L->eps16);
   DEV_FREE(L->xs); DEV_FREE(L->xs2); DEV_FREE(L->gs_); DEV_FREE(L->hs); DEV_FREE(L->R);
   DEV_FREE(L->zeta_keep);
@@ -678,7 +680,7 @@ extern "C" int vbnn_layer_grads(vbnn_layer* L, float* mleg, float* mlcg, float* 
   VB_CHECK(L && L->kind == VBNN_KIND_VB, VBNN_E_INVALID, "vbnn_layer_grads: not a VB layer");
   VB_CHECK(L->prior_valid, VBNN_E_STATE, "vbnn_layer_grads before compute_prior");
   VB_TRY(launch_grads(L->means, L->lvars, L->gW, L->gS, (long long)L->O * L->I, L->var_hat_dev, layer_prior(L, 0),
-                      L->opts.B, (float)L->opts.S, layer_is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
+                      L->hp, (float)L->opts.S, layer_is_lrt(L), mleg, mlcg, vleg, vlcg, L->ctx->stream));
   L->ctx->launches++;
   return VBNN_OK;
 }
@@ -697,11 +699,11 @@ extern "C" int vbnn_layer_calc_lc(vbnn_layer* L, float* lc_dev, float* sum_host)
   int np = 0;
   if (L->opts.strict_reference && L->stdv && L->mu_sqe) {
     // quirk Q6: tensors cached by the last compute_prior (VBLinear.lua:100-101 read self.vars etc.)
-    VB_TRY(launch_calc_lc(L->stdv, 1, L->mu_sqe, 1, W, L->var_hat_dev, layer_prior(L, 0), L->opts.B, lc_dev,
+    VB_TRY(launch_calc_lc(L->stdv, 1, L->mu_sqe, 1, W, L->var_hat_dev, layer_prior(L, 0), L->hp, lc_dev,
                           c->d_partials, &np, st));
   } else {
     VB_TRY(layer_compute_prior_internal(L));
-    VB_TRY(launch_calc_lc(L->lvars, 0, L->means, 0, W, L->var_hat_dev, layer_prior(L, 0), L->opts.B, lc_dev,
+    VB_TRY(launch_calc_lc(L->lvars, 0, L->means, 0, W, L->var_hat_dev, layer_prior(L, 0), L->hp, lc_dev,
                           c->d_partials, &np, st));
   }
   c->launches++;
@@ -767,6 +769,73 @@ extern "C" int vbnn_layer_get_prior(const vbnn_layer* L, int* kind, float* mu0, 
   if (kind) *kind = L->prior_kind;
   if (mu0) *mu0 = fixed ? L->prior_mu0 : nanf("");
   if (var0) *var0 = fixed ? L->prior_var0 : nanf("");
+  return VBNN_OK;
+}
+
+LiveOpts vbnn::live_opts(const vbnn_opts& o) {
+  return LiveOpts{o.B, o.lr_bias, o.lr_mu, o.lr_var, o.adam_beta1, o.adam_beta2, o.adam_eps};
+}
+
+// vbnn_layer_set_opts / vbnn_mlp_set_opts: the fields that size buffers or choose kernels must be the layer's own, and
+// every live value must be one the update can use
+static int check_opts(const vbnn_layer* L, const vbnn_opts* o, const char* who) {
+  const vbnn_opts& c = L->opts;
+#define FIXED_(f) VB_CHECK(memcmp(&o->f, &c.f, sizeof(c.f)) == 0, VBNN_E_INVALID, "%s: %s cannot change on a live layer", \
+                           who, #f)
+  FIXED_(var_init); FIXED_(msr_init); FIXED_(mu_init); FIXED_(S); FIXED_(reparam); FIXED_(precision);
+  FIXED_(strict_reference);
+#undef FIXED_
+  VB_CHECK(isfinite(o->B) && o->B > 0.f, VBNN_E_INVALID, "%s: B must be finite and > 0 (got %g)", who, o->B);
+#define RATE_(f) VB_CHECK(isfinite(o->f) && o->f >= 0.f, VBNN_E_INVALID, "%s: %s must be finite and >= 0 (got %g)", \
+                          who, #f, o->f)
+  RATE_(lr_bias); RATE_(lr_mu); RATE_(lr_var);
+#undef RATE_
+#define BETA_(f) VB_CHECK(o->f >= 0.f && o->f < 1.f, VBNN_E_INVALID, "%s: %s must be in [0, 1) (got %g)", who, #f, o->f)
+  BETA_(adam_beta1); BETA_(adam_beta2);
+#undef BETA_
+  VB_CHECK(isfinite(o->adam_eps) && o->adam_eps > 0.f, VBNN_E_INVALID, "%s: adam_eps must be finite and > 0 (got %g)",
+           who, o->adam_eps);
+  return VBNN_OK;
+}
+
+// the host copy would disagree with a graph that captured the write
+static int refuse_set_in_capture(const vbnn_ctx* c, const char* who) {
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  VB_CUDA(cudaStreamIsCapturing(c->stream, &cs));
+  VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE, "%s: the context's stream is being captured", who);
+  return VBNN_OK;
+}
+
+static int write_opts(vbnn_layer* L, const vbnn_opts* o) {
+  VB_TRY(launch_set_live_opts(L->hp, live_opts(*o), L->ctx->stream));
+  L->ctx->launches++;
+  L->opts = *o;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_layer_get_opts(const vbnn_layer* L, vbnn_opts* out) {
+  VB_CHECK(L && out, VBNN_E_INVALID, "vbnn_layer_get_opts: null argument");
+  *out = L->opts;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_layer_set_opts(vbnn_layer* L, const vbnn_opts* opts) {
+  VB_CHECK(L && opts, VBNN_E_INVALID, "vbnn_layer_set_opts: null argument");
+  VB_TRY(refuse_set_in_capture(L->ctx, "vbnn_layer_set_opts"));
+  VB_TRY(check_opts(L, opts, "vbnn_layer_set_opts"));
+  VB_CUDA(cudaSetDevice(L->ctx->device));
+  if (L->owner) VB_TRY(mlp_wait_side(L->owner));
+  return write_opts(L, opts);
+}
+
+extern "C" int vbnn_mlp_set_opts(vbnn_mlp* m, const vbnn_opts* opts) {
+  VB_CHECK(m && opts, VBNN_E_INVALID, "vbnn_mlp_set_opts: null argument");
+  VB_TRY(refuse_set_in_capture(m->ctx, "vbnn_mlp_set_opts"));
+  for (const vbnn_layer* L : m->layers) VB_TRY(check_opts(L, opts, "vbnn_mlp_set_opts"));
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  VB_TRY(mlp_wait_side(m));
+  for (vbnn_layer* L : m->layers) VB_TRY(write_opts(L, opts));
+  m->opts = *opts;
   return VBNN_OK;
 }
 

@@ -936,13 +936,18 @@ extern "C" int vbnn_mlp_submit_host_u8(vbnn_mlp* m, const uint8_t* X_host, const
   return submit_host_any(m, nullptr, X_host, T_host, N, mean, inv_std);
 }
 
+int vbnn::mlp_wait_side(vbnn_mlp* m) {
+  if (m->peer && m->peer->active) {
+    VB_CUDA(cudaEventRecord(m->peer->ev_side, m->peer->side));     // the side stream already waits for the transfer stream
+    VB_CUDA(cudaStreamWaitEvent(m->ctx->stream, m->peer->ev_side, 0));
+  }
+  return VBNN_OK;
+}
+
 extern "C" int vbnn_mlp_join_streams(vbnn_mlp* m) {
   VB_CHECK(m, VBNN_E_INVALID, "null mlp");
   vbnn_ctx* c = m->ctx;
-  if (m->peer && m->peer->active) {
-    VB_CUDA(cudaEventRecord(m->peer->ev_side, m->peer->side));     // the side stream already waits for the transfer stream
-    VB_CUDA(cudaStreamWaitEvent(c->stream, m->peer->ev_side, 0));
-  }
+  VB_TRY(mlp_wait_side(m));
   if (c->comm_stream && !m->ev_red.empty()) {
     VB_CUDA(cudaEventRecord(m->ev_red[0], c->comm_stream));
     VB_CUDA(cudaStreamWaitEvent(c->stream, m->ev_red[0], 0));

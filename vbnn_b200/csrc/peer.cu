@@ -361,12 +361,12 @@ int peer_after_dw(vbnn_mlp* m, int j) {
   const size_t roff = (size_t)pl.row0 * L->I, roffb = (size_t)pl.row0 * L->ldI;
   // bias (and the plain nn.Linear output layer): optim.sgd, VBLinear.lua:125-128 / mlp.lua:120-123;
   // the bias is O floats: every rank applies the summed gradient itself
-  VB_TRY(launch_sgd_slots(L->bias, gb_slots, G, L->O, L->O, L->opts.lr_bias, nullptr, 1, 1, sd));
+  VB_TRY(launch_sgd_slots(L->bias, gb_slots, G, L->O, L->O, &L->hp->lr_bias, nullptr, 1, 1, sd));
   c->launches += 3;
   if (L->kind == VBNN_KIND_LINEAR) {
     if (pl.rows > 0) {
       VB_TRY(launch_sgd_slots(L->weight + roff, slot0, G, (long long)pl.slot_floats, (long long)pl.rows * L->I,
-                              L->opts.lr_bias, L->w_bf16 ? L->w_bf16 + roffb : nullptr, L->I, L->ldI, sd));
+                              &L->hp->lr_bias, L->w_bf16 ? L->w_bf16 + roffb : nullptr, L->I, L->ldI, sd));
       c->launches++;
       if (L->w_bf16) VB_TRY(push_shard(P, pl.w_bf16, roffb * 2, (size_t)pl.rows * L->ldI * 2));
       else VB_TRY(push_shard(P, pl.weight, roff * 4, (size_t)pl.rows * L->I * 4));
@@ -399,9 +399,8 @@ int peer_after_dw(vbnn_mlp* m, int j) {
     for (int q = 0; q < G; ++q)
       if (q != me) u.peer_partials[u.n_peer++] = (double*)pl.partials.ptr[q];
     u.var_hat_dev = L->var_hat_dev; u.t_dev = L->t_dev;
-    u.B = L->opts.B; u.S = (float)L->opts.S;
-    u.lr_mu = L->opts.lr_mu; u.lr_var = L->opts.lr_var;
-    u.beta1 = L->opts.adam_beta1; u.beta2 = L->opts.adam_beta2; u.eps = L->opts.adam_eps;
+    u.S = (float)L->opts.S;
+    u.hp = L->hp;
     u.lrt = layer_is_lrt(L);
     u.prior = layer_prior(L, roff);
     // knob peer_fused_push: the update kernel stores the refreshed operands to every rank itself instead of

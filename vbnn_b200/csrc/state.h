@@ -56,6 +56,7 @@ struct vbnn_layer {
                                      // an update reads one half while its blocks write the other)
   // half (t & 1) holds the sums of the CURRENT parameters, t = the layer's device step counter
   int* t_dev = nullptr;              // meanState.t == varState.t == biasState.evalCounter
+  vbnn::LiveOpts* hp = nullptr;      // B, rates, Adam constants the update kernels read (vbnn_layer_set_opts)
   // bf16 tensor-core operand copies [.. x ldI]
   bf16 *w_bf16 = nullptr, *mu_bf16 = nullptr, *s2_bf16 = nullptr;
   void* eps16 = nullptr;             // fp16 [S_alloc x O x ldI]: this minibatch's epsilon for the dW epilogue (mlp-owned layers)
@@ -197,6 +198,8 @@ int layer_compute_prior_internal(vbnn_layer* L);
 int layer_refresh_prior_partials(vbnn_layer* L);
 PriorArgs layer_prior(const vbnn_layer* L, size_t row_off);   // row_off: first element of a peer-mode row shard
 void mlp_drop_graphs(vbnn_mlp* m);                            // each step graph re-captures at its next use
+int mlp_wait_side(vbnn_mlp* m);                               // peer mode: the context's stream waits for the side stream
+LiveOpts live_opts(const vbnn_opts& o);                       // the fields of o the update reads at every call
 PhiloxStream layer_stream(const vbnn_layer* L, uint32_t kind, int sample);
 int comm_allreduce_internal(vbnn_ctx* ctx, float* buf, size_t count, cudaStream_t st);
 // peer mode (peer.cu)

@@ -8,7 +8,7 @@ import ctypes as C
 from typing import NamedTuple, Optional
 
 from . import _lib as L
-from .config import opts_struct
+from .config import opts_struct, with_live
 from .context import Context, as_dev_f32, default_context
 from .vblinear import Linear, VBLinear
 
@@ -76,6 +76,18 @@ class MLP:
         layer's current posterior its prior.  Each step graph of the net re-captures once at its next use."""
         for k in self.vb_indices:
             self.model[k].set_prior(kind, mean, var)
+
+    def set_opt(self, opt):
+        """VBLinear.set_opt on every layer in one call (vbnn_mlp_set_opts), for a learning-rate schedule or KL annealing:
+        decay opt's learning rates or change opt["B"], then set_opt(opt) before the next step.  No step graph is
+        re-captured.  A change of a key the net was built with (S, reparam, precision, ...) is refused
+        (VbnnError(E_INVALID), nothing changes).  self.opt (what checkpoint.save_net records) takes opt's live keys --
+        B, state, meanState, varState -- and keeps every other key.  In data-parallel training set the same values on
+        every rank."""
+        L.check(L.lib().vbnn_mlp_set_opts(self.handle, C.byref(opts_struct(opt))))
+        self.opt = with_live(self.opt, opt)
+        for m in self.model:
+            m.opt = self.opt
 
     def init_params(self, seed=4, he_means=False):
         """means per VBLinear.lua:22-29 (or He-scaled, SURVEY 8d), Linear weights N(0, 2/fan_in)
@@ -389,8 +401,10 @@ class MLP:
     # ---- checkpoint / resume (reference: u.safe_save(net) main.lua:181, utils.lua:73-80; resume
     # main.lua:146-148).  The reference torch.save()s the whole object graph; here the device state
     # is exported as a flat dict of CPU tensors (means, lvars, bias, Adam m/v/t per layer, the output
-    # layer, the Philox step counter) that torch.save / numpy can persist.
+    # layer, the Philox step counter, each layer's live hyper-parameters "{k}.opts" in L.LIVE_OPTS
+    # order) that torch.save / numpy can persist.
     def state_dict(self):
+        import torch
         sd = {"sizes": list(self.sizes), "step": self.ctx.get_step()}
         names = [("means", L.BUF_MEANS), ("lvars", L.BUF_LVARS), ("bias", L.BUF_BIAS), ("m_mu", L.BUF_ADAM_M_MU),
                  ("v_mu", L.BUF_ADAM_V_MU), ("m_var", L.BUF_ADAM_M_VAR), ("v_var", L.BUF_ADAM_V_VAR)]
@@ -412,6 +426,8 @@ class MLP:
                 sd[f"{k}.weight"] = m.get(L.BUF_WEIGHT)
                 sd[f"{k}.bias"] = m.get(L.BUF_BIAS)
             sd[f"{k}.t"] = m.t
+            live = m.opts
+            sd[f"{k}.opts"] = torch.tensor([live[f] for f in L.LIVE_OPTS], dtype=torch.float32)
         return sd
 
     def load_state_dict(self, sd):
@@ -423,6 +439,13 @@ class MLP:
         kinds = {c: n for n, c in L.PRIOR_KINDS.items()}
         for k, m in enumerate(self.model):
             L.check(L.lib().vbnn_layer_set_t(m.handle, int(sd[f"{k}.t"])))
+            if f"{k}.opts" in sd:                                        # older checkpoints keep the net's values
+                o = m._get_opts()
+                live = dict(zip(L.LIVE_OPTS, [float(v) for v in sd[f"{k}.opts"]]))
+                for f, v in live.items():
+                    setattr(o, f, v)
+                L.check(L.lib().vbnn_layer_set_opts(m.handle, C.byref(o)))
+                m.opt = with_live(self.opt, m.opts)
             if m.kind == L.KIND_VB:
                 # before the parameters: a per_weight prior snapshots them, then takes its own arrays below.  A
                 # checkpoint without prior keys (older files) is the empirical prior.
@@ -436,6 +459,9 @@ class MLP:
                     m.set(b, sd[f"{k}.{n}"])
             if m.kind == L.KIND_VB and f"{k}.stdv" not in sd:
                 m.compute_prior()
+        if "0.opts" in sd:
+            # the net's opt (what save_net records) follows the first layer, as MLP.set_opt sets every layer alike
+            self.opt = with_live(self.opt, self.model[0].opts)
         self.ctx.set_step(int(sd["step"]))
 
     # ---- data parallel over NVLink peer memory (new; include/vbnn.h "peer mode") ----

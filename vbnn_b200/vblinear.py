@@ -7,7 +7,7 @@ from __future__ import annotations
 import ctypes as C
 
 from . import _lib as L
-from .config import opts_struct
+from .config import opts_struct, with_live
 from .context import Context, DevView, as_dev_f32, default_context
 
 
@@ -193,6 +193,29 @@ class VBLinear:
         L.check(L.lib().vbnn_layer_get_prior(self.handle, C.byref(k), C.byref(m), C.byref(v)))
         name = {c: n for n, c in L.PRIOR_KINDS.items()}[k.value]
         return (name, m.value, v.value) if k.value == L.PRIOR_FIXED else (name, None, None)
+
+    # ---- hyper-parameters read at every update (vbnn_layer_set_opts) ----
+    def _get_opts(self):
+        o = L.VbnnOpts()
+        L.check(L.lib().vbnn_layer_get_opts(self.handle, C.byref(o)))
+        return o
+
+    def set_opt(self, opt):
+        """This layer's B, learning rates and Adam constants from a config dict, mapped as buildModel maps it: opt["B"],
+        state.learningRate (biases / nn.Linear), meanState.learningRate / beta1 / beta2 / epsilon (0.9, 0.999, 1e-8
+        where absent), varState.learningRate.  The Torch7 idiom of writing layer.meanState.learningRate or opt.B between
+        minibatches, made explicit: every later update, captured step graphs included, uses the new values.  The keys
+        that describe the layer as created (S, reparam, precision, strict_reference, var_init, msr_init, mu_init) must
+        be unchanged: otherwise VbnnError(E_INVALID) and nothing changes.  self.opt takes the live keys of opt only.  On
+        a layer of an MLP it gives this layer its own values."""
+        L.check(L.lib().vbnn_layer_set_opts(self.handle, C.byref(opts_struct(opt))))
+        self.opt = with_live(self.opt, opt)
+
+    @property
+    def opts(self):
+        """The live values {B, lr_bias, lr_mu, lr_var, adam_beta1, adam_beta2, adam_eps} the next update uses."""
+        o = self._get_opts()
+        return {f: getattr(o, f) for f in L.LIVE_OPTS}
 
     # ---- VBLinear.lua:77-103 ----
     def compute_prior(self):

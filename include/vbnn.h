@@ -296,7 +296,8 @@ int vbnn_layer_draw_noise(vbnn_layer* layer, uint32_t step, int sample_idx, int 
 /* ---------------------------------------------------------------- mlp.lua -------------
  * MLP:buildModel(opt)  mlp.lua:7-60.  sizes = {input_size, hidden..., #classes}; hidden layers
  * are VBLinear+ReLU, the last is nn.Linear (mlp.lua:29) or, with vb_output, a VBLinear
- * (convnet.lua:30).  Ends in LogSoftMax + ClassNLLCriterion (mlp.lua:30-32). */
+ * (convnet.lua:30).  Ends in LogSoftMax + ClassNLLCriterion (mlp.lua:30-32), or in the regression
+ * criterion chosen by vbnn_mlp_set_criterion. */
 int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int vb_output, int max_batch,
                     const vbnn_opts* opts, vbnn_mlp** out);
 int vbnn_mlp_destroy(vbnn_mlp* mlp);
@@ -379,6 +380,37 @@ int vbnn_mlp_step_grad_input(vbnn_mlp* mlp, const float* X_dev, const float* tar
  * vbnn_mlp_step_grad_input.  NULL X_dev / logits_dev / grad_dev and N outside 1..max_batch: VBNN_E_INVALID. */
 int vbnn_mlp_forward_train(vbnn_mlp* mlp, const float* X_dev, int N, float* logits_dev);
 int vbnn_mlp_backward_update(vbnn_mlp* mlp, const float* grad_dev, float* dX_dev);
+/* The net's criterion (mlp.lua:30-32 builds it as a separate, swappable object; a Torch7 regression net drops the
+ * LogSoftMax and uses nn.MSECriterion).  A new net is VBNN_CRIT_CLASS_NLL.  For sample s the output Y_s is [N x C];
+ * N_g = N * nranks is the global batch. */
+enum vbnn_criterion {
+  VBNN_CRIT_CLASS_NLL = 0,    /* LogSoftMax + ClassNLL, 1-based labels [N] (the reference, the default) */
+  VBNN_CRIT_MSE = 1,          /* nn.MSECriterion (size-averaged), targets dense fp32 [N x C]            */
+  VBNN_CRIT_GAUSSIAN_NLL = 2  /* C = 2K: columns [0,K) means m, [K,2K) log-variances s; targets [N x K] */
+};
+/* Choose the criterion of the fused minibatch: vbnn_mlp_step, _step_grad_input, _step_host, _submit_host, _submit_host_u8
+ * (targets_host [N x K]), vbnn_mlp_run and vbnn_mlp_test, on one GPU, in peer mode and in NCCL mode.  The split step
+ * (vbnn_mlp_forward_train / vbnn_mlp_backward_update) ignores it and stays the way to train under any other loss.
+ *   - MSE: l_s = 1/(N_g C) sum_{n,c} (Y_s - y)^2, as torch's mse_loss(Y_s, y) on one GPU.  K = C.
+ *   - GAUSSIAN_NLL: l_s = 1/(N_g K) sum_{n,k} 1/2 (s + (y - m)^2 e^{-s}), the parameterisation of VBNN_OUTPUT_GAUSSIAN, so
+ *     vbnn_mlp_predict_outputs(..., VBNN_OUTPUT_GAUSSIAN, ...) evaluates what this trains.  Formed from q = (y - m) e^{-s/2}:
+ *     every loss and gradient term is finite wherever its exact value is representable in fp32, and dl/dm is exactly 0
+ *     where y == m.
+ *   - The backward receives dl_s/dY_s; the samples are summed as for ClassNLL (quirk Q3 unchanged).
+ *   - A NaN target element adds 0 to the loss, the gradient and both scalars; the means still divide by N_g C or N_g K
+ *     (this is how a regression minibatch is padded, as a label outside 1..C pads a classification one).
+ *   - The {error, accuracy} scalars (result_dev, vbnn_mlp_collect, _step_host, _run, _test) become {mean over samples of
+ *     l_s, mean over samples of the MSE of the means 1/(N K) sum (y - m)^2}, both over this rank's rows and neither
+ *     scaled by 100; under MSE the two are equal.  vbnn_mlp_test averages them over its passes (mlp.lua:101).
+ *   - vbnn_mlp_get_outputs returns the raw outputs Y_s (a regression net has no LogSoftMax).  vbnn_mlp_predict is
+ *     unchanged; vbnn_mlp_predict_outputs is the evaluator of a regression net.
+ *   - The first set to MSE or GAUSSIAN_NLL grows the device targets buffer (and the host pipeline's staging buffers) to
+ *     max_batch x C floats, which covers both; it is the only call that allocates.  A set that changes the criterion
+ *     makes each step graph re-capture once at its next use; a set to the current value changes nothing.
+ * VBNN_E_INVALID: a NULL net, an unknown value, GAUSSIAN_NLL with an odd C.  VBNN_E_STATE: a split step is open,
+ * host-pipeline minibatches are not collected, or the context's stream is being captured. */
+int vbnn_mlp_set_criterion(vbnn_mlp* mlp, int criterion);
+int vbnn_mlp_get_criterion(const vbnn_mlp* mlp, int* criterion);
 /* same with HOST buffers: H2D of inputs + D2H of {error, accuracy} inside the call
  * (replaces inputs:cuda()/targets:cuda() main.lua:23-24 and the scalar reads mlp.lua:80-82). */
 int vbnn_mlp_step_host(vbnn_mlp* mlp, const float* X_host, const float* targets_host, int N,
@@ -463,7 +495,8 @@ enum vbnn_output_model {
 int vbnn_mlp_predict_outputs(vbnn_mlp* mlp, const float* X_dev, int N, int n_samples, int output_model,
                              const float* targets_dev, float* samples_dev, float* mean_dev,
                              float* epistemic_dev, float* aleatoric_dev, float* nll_host, float* rmse_host);
-/* last forward's LogSoftMax output [N x C] (self.model.output, visualize.lua:97) */
+/* last forward's LogSoftMax output [N x C] (self.model.output, visualize.lua:97); the raw outputs under
+ * VBNN_CRIT_MSE and VBNN_CRIT_GAUSSIAN_NLL */
 int vbnn_mlp_get_outputs(vbnn_mlp* mlp, int sample_idx, float* logp_host);
 /* kernels launched by this handle since creation (bench.py's gpu_launches) */
 int vbnn_mlp_launch_count(vbnn_mlp* mlp, long long* count);

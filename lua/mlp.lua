@@ -22,7 +22,9 @@ function MLP:buildModel(opt)                                          -- referen
    net.opt = opt
    local sizes = { opt.input_size }
    for _, h in ipairs(opt.hidden) do sizes[#sizes + 1] = h end
-   sizes[#sizes + 1] = #opt.classes
+   -- a regression net (opt.criterion 'mse' or 'gaussian_nll') may give its output width as opt.outputs
+   local crit = opt.criterion or 'class_nll'
+   sizes[#sizes + 1] = (crit ~= 'class_nll' and opt.outputs) or #opt.classes
    local csizes = ffi.new('int[?]', #sizes, sizes)
    local out = ffi.new('vbnn_mlp*[1]')
    -- hidden layers: VBLinear + ReLU; output: plain nn.Linear + LogSoftMax (mlp.lua:29-30), or a VBLinear with
@@ -36,7 +38,20 @@ function MLP:buildModel(opt)                                          -- referen
    assert(opt.prior == nil or opt.prior == 'empirical' or opt.prior == 'fixed',
           "opt.prior must be 'empirical' or 'fixed'")
    if opt.prior == 'fixed' then net:set_prior('fixed', opt.prior_mean, opt.prior_var) end
+   net.C = sizes[#sizes]
+   net:set_criterion(crit)
    return net
+end
+
+-- The criterion of the fused minibatch (vbnn_mlp_set_criterion), the swap of mlp.lua:30-32's criterion object:
+-- 'class_nll' (LogSoftMax + ClassNLL), 'mse' (nn.MSECriterion, targets [N x C]) or 'gaussian_nll' (C = 2K outputs:
+-- K means, K log-variances; targets [N x K]).  Under a regression criterion run / test / train_minibatch return
+-- (mean loss, MSE of the means) instead of (error, accuracy %).
+local CRITERION = { class_nll = 0, mse = 1, gaussian_nll = 2 }
+function MLP:set_criterion(name)
+   assert(CRITERION[name], "set_criterion: 'class_nll', 'mse' or 'gaussian_nll'")
+   V.check(C.vbnn_mlp_set_criterion(self.h, CRITERION[name]))
+   self.criterion = name
 end
 
 -- VBLinear:set_prior on every VB layer of the net (the hidden layers and a vb_output layer)
@@ -88,7 +103,7 @@ end
 function MLP:predict(input, nsamples, target)
    local n = input:size(1)
    if nsamples == nil then nsamples = self.opt.quicktest and 0 or self.opt.testSamples end
-   local logp = torch.CudaTensor(n, #self.opt.classes)
+   local logp = torch.CudaTensor(n, self.C)
    local unc = torch.CudaTensor(n, 4)
    if target then
       V.check(C.vbnn_mlp_predict(self.h, V.ptr(input), n, nsamples, V.ptr(target), V.ptr(logp), V.ptr(unc),
@@ -106,7 +121,7 @@ function MLP:predict_outputs(input, nsamples, model, target)
    local n = input:size(1)
    if nsamples == nil then nsamples = self.opt.quicktest and 0 or self.opt.testSamples end
    local gaussian = model == 'gaussian'
-   local k = gaussian and #self.opt.classes / 2 or #self.opt.classes
+   local k = gaussian and self.C / 2 or self.C
    local mean, epi = torch.CudaTensor(n, k), torch.CudaTensor(n, k)
    local ale = gaussian and torch.CudaTensor(n, k) or nil
    local nll = (gaussian and target) and ffi.new('float[1]') or nil
@@ -128,7 +143,8 @@ function MLP:update(opt)                                              -- mlp.lua
 end
 
 -- main.lua:28-40 in one enqueue: reset, S x (sample, run), update.  inputs / targets are HOST FloatTensors
--- (pinned memory makes the copy asynchronous); returns the mean error and accuracy of main.lua:38-39.
+-- (pinned memory makes the copy asynchronous); returns the mean error and accuracy of main.lua:38-39.  Under a
+-- regression criterion (set_criterion) targets are [N x K] and the pair is (mean loss, MSE of the means).
 function MLP:train_minibatch(inputs, targets)
    V.check(C.vbnn_mlp_submit_host(self.h, inputs:data(), targets:data(), inputs:size(1)))
    V.check(C.vbnn_mlp_collect(self.h, self.err, self.acc))
@@ -166,7 +182,7 @@ function MLP:forward_train(inputs)
    self.logits = self.logits or {}
    local Y = self.logits[n]
    if not Y then
-      Y = torch.CudaTensor(self.opt.S, n, #self.opt.classes)
+      Y = torch.CudaTensor(self.opt.S, n, self.C)
       self.logits[n] = Y
    end
    V.check(C.vbnn_mlp_forward_train(self.h, V.ptr(inputs), n, V.ptr(Y)))
@@ -177,7 +193,7 @@ end
 function MLP:backward_update(gradLogits, gradInput)
    local n = self.open_n
    assert(n, 'backward_update: call forward_train first')
-   assert(gradLogits:isContiguous() and gradLogits:nElement() == self.opt.S * n * #self.opt.classes,
+   assert(gradLogits:isContiguous() and gradLogits:nElement() == self.opt.S * n * self.C,
           'gradLogits must be a contiguous CudaTensor [S x N x C]')
    if gradInput then
       assert(gradInput:isContiguous() and gradInput:size(1) == n and gradInput:size(2) == self.opt.input_size,

@@ -21,6 +21,8 @@ PRIOR_EMPIRICAL, PRIOR_FIXED, PRIOR_PER_WEIGHT = 0, 1, 2
 PRIOR_KINDS = {"empirical": PRIOR_EMPIRICAL, "fixed": PRIOR_FIXED, "per_weight": PRIOR_PER_WEIGHT}
 OUTPUT_RAW, OUTPUT_GAUSSIAN = 0, 1
 OUTPUT_MODELS = {"raw": OUTPUT_RAW, "gaussian": OUTPUT_GAUSSIAN}
+CRIT_CLASS_NLL, CRIT_MSE, CRIT_GAUSSIAN_NLL = 0, 1, 2
+CRITERIA = {"class_nll": CRIT_CLASS_NLL, "mse": CRIT_MSE, "gaussian_nll": CRIT_GAUSSIAN_NLL}
 
 
 class VbnnOpts(C.Structure):
@@ -103,6 +105,8 @@ _PROTOS = {
     "vbnn_mlp_step_grad_input": (C.c_int, [_P, _P, _P, C.c_int, _P, _P]),
     "vbnn_mlp_forward_train": (C.c_int, [_P, _P, C.c_int, _P]),
     "vbnn_mlp_backward_update": (C.c_int, [_P, _P, _P]),
+    "vbnn_mlp_set_criterion": (C.c_int, [_P, C.c_int]),
+    "vbnn_mlp_get_criterion": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "vbnn_mlp_step_host": (C.c_int, [_P, _P, _P, C.c_int, _F, _F]),
     "vbnn_mlp_submit_host": (C.c_int, [_P, _P, _P, C.c_int]),
     "vbnn_mlp_collect": (C.c_int, [_P, _F, _F]),

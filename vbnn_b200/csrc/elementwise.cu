@@ -535,6 +535,40 @@ __global__ void __launch_bounds__(kThreads) k_sgd_slots(float* x, const float* g
 }
 
 // ------------------------------------------------------------------ loss ----------------
+// Adds each warp's {a, b} (lane 0's values) of one row iteration into result[2 (z_slot0 + z)], [.. + 1].  One atomic
+// pair per block instead of per row (8192 rows hammering two addresses serialised the whole kernel): the rows of one
+// block almost always share z; per-warp atomics otherwise.  Every thread of the block calls it (valid: r < rows).
+__device__ __forceinline__ void block_add_result(float* result, int z_slot0, int z, bool valid, float a_w, float b_w) {
+  const int warps_per_block = blockDim.x >> 5;
+  const int lane = threadIdx.x & 31;
+  __shared__ float sh_loss[kThreads / 32], sh_corr[kThreads / 32];
+  __shared__ int sh_z[kThreads / 32];
+  const int w = threadIdx.x >> 5;
+  if (lane == 0) { sh_loss[w] = a_w; sh_corr[w] = b_w; sh_z[w] = valid ? z : -1; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int z0 = -1; bool same = true;
+    for (int k = 0; k < warps_per_block; ++k) {
+      if (sh_z[k] < 0) continue;
+      if (z0 < 0) z0 = sh_z[k];
+      same &= sh_z[k] == z0;
+    }
+    if (same && z0 >= 0) {
+      float a = 0.f, c = 0.f;
+      for (int k = 0; k < warps_per_block; ++k) if (sh_z[k] >= 0) { a += sh_loss[k]; c += sh_corr[k]; }
+      atomicAdd(result + 2 * (z_slot0 + z0), a);
+      atomicAdd(result + 2 * (z_slot0 + z0) + 1, c);
+    } else {
+      for (int k = 0; k < warps_per_block; ++k)
+        if (sh_z[k] >= 0) {
+          atomicAdd(result + 2 * (z_slot0 + sh_z[k]), sh_loss[k]);
+          atomicAdd(result + 2 * (z_slot0 + sh_z[k]) + 1, sh_corr[k]);
+        }
+    }
+  }
+  __syncthreads();
+}
+
 // One warp per row: LogSoftMax + ClassNLL (size-averaged) forward and backward + argmax match.
 // Replaces cunn LogSoftMax/ClassNLLCriterion kernels plus the host accuracy loop of
 // utils.lua:11-27 (N device syncs per run()).
@@ -584,34 +618,67 @@ __global__ void __launch_bounds__(kThreads) k_loss(LossParams p) {
         my_corr = (arg == tgt) ? 1.f : 0.f;
       }
     }
-    // One atomic pair per block instead of per row (8192 rows hammering two addresses serialised the
-    // whole kernel): the rows of one block almost always share z; per-warp atomics otherwise.
-    __shared__ float sh_loss[kThreads / 32], sh_corr[kThreads / 32];
-    __shared__ int sh_z[kThreads / 32];
-    const int w = threadIdx.x >> 5;
-    if (lane == 0) { sh_loss[w] = my_loss; sh_corr[w] = my_corr; sh_z[w] = r < rows ? z : -1; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int z0 = -1; bool same = true;
-      for (int k = 0; k < warps_per_block; ++k) {
-        if (sh_z[k] < 0) continue;
-        if (z0 < 0) z0 = sh_z[k];
-        same &= sh_z[k] == z0;
+    block_add_result(p.result, p.z_slot0, z, r < rows, my_loss, my_corr);
+  }
+}
+
+// One warp per row: the MSE or heteroscedastic Gaussian NLL criterion (vbnn_mlp_set_criterion) forward and backward.
+// Per element q = (y - m) e^{-s/2} carries the scale: the loss term 1/2 (s + q^2), dm = -(q / D) e^{-s/2} and
+// ds = 1/2 (1 - q^2) / D (D = N_global K) are each finite wherever their exact value is representable in fp32 (s = +-100
+// included), and dm is exactly 0 where y == m, also where e^{-s/2} overflows.  expf, not __expf: e^{-s/2} must keep
+// its subnormal range.  T is the gradient operand's type (bf16 or fp32); H = T(T(G) .* R) as k_mul_act forms it.
+template <typename T, bool GAUSS>
+__global__ void __launch_bounds__(kThreads) k_loss_reg(LossParams p) {
+  const int warps_per_block = blockDim.x >> 5;
+  const int lane = threadIdx.x & 31;
+  const long long rows = (long long)p.Z * p.N;
+  const int K = GAUSS ? p.C >> 1 : p.C;
+  T* const g = reinterpret_cast<T*>(sizeof(T) == 2 ? (void*)p.g_bf16 : (void*)p.g_f32);
+  const float scale = p.grad_scale, half_scale = 0.5f * p.grad_scale, two_scale = 2.f * p.grad_scale;
+  for (long long r0 = (long long)blockIdx.x * warps_per_block; r0 < rows;
+       r0 += (long long)gridDim.x * warps_per_block) {
+    const long long r = r0 + (threadIdx.x >> 5);
+    float my_loss = 0.f, my_se = 0.f;
+    int z = 0;
+    if (r < rows) {
+      z = (int)(r / p.N);
+      const int n = (int)(r - (long long)z * p.N);
+      const float* x = p.logits + r * p.ld_logits;
+      const float* y = p.targets + (long long)n * K;
+      T* gr = g ? g + r * p.ld_g : nullptr;
+      T* hr = p.h ? static_cast<T*>(p.h) + r * p.ld_g : nullptr;
+      const T* rr = p.h ? static_cast<const T*>(p.r) + r * p.ld_g : nullptr;
+      auto put = [&](int c, float v) {
+        const T gt = from_f32<T>(v);
+        gr[c] = gt;
+        if (hr) hr[c] = from_f32<T>(to_f32(gt) * to_f32(rr[c]));
+      };
+      for (int k = lane; k < K; k += 32) {
+        const float t = y[k], m = x[k];
+        const bool miss = t != t;                                       // NaN target: a padding element
+        const float d = miss ? 0.f : t - m;
+        const float se = d * d;
+        if (GAUSS) {
+          const float s = x[K + k];
+          const float eh = expf(-0.5f * s);
+          const float q = d == 0.f ? 0.f : d * eh;
+          const float dm = d == 0.f ? 0.f : -(q * scale) * eh;
+          const float ds = miss ? 0.f : fmaf(-q, q * half_scale, half_scale);
+          if (!miss) my_loss += fmaf(0.5f * q, q, 0.5f * s);
+          my_se += se;
+          if (gr) { put(k, dm); put(K + k, ds); }
+        } else {
+          my_loss += se;
+          my_se += se;
+          if (gr) put(k, -two_scale * d);
+        }
       }
-      if (same && z0 >= 0) {
-        float a = 0.f, c = 0.f;
-        for (int k = 0; k < warps_per_block; ++k) if (sh_z[k] >= 0) { a += sh_loss[k]; c += sh_corr[k]; }
-        atomicAdd(p.result + 2 * (p.z_slot0 + z0), a);
-        atomicAdd(p.result + 2 * (p.z_slot0 + z0) + 1, c);
-      } else {
-        for (int k = 0; k < warps_per_block; ++k)
-          if (sh_z[k] >= 0) {
-            atomicAdd(p.result + 2 * (p.z_slot0 + sh_z[k]), sh_loss[k]);
-            atomicAdd(p.result + 2 * (p.z_slot0 + sh_z[k]) + 1, sh_corr[k]);
-          }
-      }
+      if (gr)                                    // zero the padding columns of G so the bf16 GEMMs read clean operands
+        for (int c = p.C + lane; c < p.ld_g; c += 32) gr[c] = from_f32<T>(0.f);
+      my_loss = warp_sum(my_loss);
+      my_se = warp_sum(my_se);
     }
-    __syncthreads();
+    block_add_result(p.result, p.z_slot0, z, r < rows, my_loss, my_se);
   }
 }
 
@@ -798,12 +865,12 @@ __global__ void __launch_bounds__(kThreads) k_predict_moments(MomentsParams p) {
   if (reduce && threadIdx.x == 0) { p.partials[2 * blockIdx.x] = blk_nll; p.partials[2 * blockIdx.x + 1] = blk_se; }
 }
 
-__global__ void k_finalize_result(const float* acc, int Z, int N, float* out2) {
+__global__ void k_finalize_result(const float* acc, int Z, float div, float scale1, float* out2) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
     float e = 0.f, a = 0.f;
     for (int z = 0; z < Z; ++z) {
-      e += acc[2 * z] / (float)N;                                       // ClassNLL size-average
-      a += acc[2 * z + 1] / (float)N * 100.f;                           // utils.lua:26
+      e += acc[2 * z] / div;                                            // ClassNLL size-average
+      a += acc[2 * z + 1] / div * scale1;                               // utils.lua:26
     }
     out2[0] = e / (float)Z;                                             // main.lua:39
     out2[1] = a / (float)Z;                                             // main.lua:38
@@ -1163,6 +1230,26 @@ int launch_loss(const LossParams& p, cudaStream_t st) {
   return VBNN_OK;
 }
 
+int launch_loss_reg(const LossParams& p, cudaStream_t st) {
+  VB_CHECK(p.criterion == VBNN_CRIT_MSE || p.criterion == VBNN_CRIT_GAUSSIAN_NLL, VBNN_E_INVALID,
+           "launch_loss_reg: criterion %d", p.criterion);
+  VB_CHECK(!p.h || p.r, VBNN_E_INVALID, "launch_loss_reg: h without r");
+  const long long rows = (long long)p.Z * p.N;
+  const int wpb = kThreads / 32;
+  long long blocks = (rows + wpb - 1) / wpb;
+  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
+  const bool gauss = p.criterion == VBNN_CRIT_GAUSSIAN_NLL;
+  if (p.g_bf16) {
+    if (gauss) k_loss_reg<bf16, true><<<(int)blocks, kThreads, 0, st>>>(p);
+    else k_loss_reg<bf16, false><<<(int)blocks, kThreads, 0, st>>>(p);
+  } else {
+    if (gauss) k_loss_reg<float, true><<<(int)blocks, kThreads, 0, st>>>(p);
+    else k_loss_reg<float, false><<<(int)blocks, kThreads, 0, st>>>(p);
+  }
+  VB_CUDA(cudaGetLastError());
+  return VBNN_OK;
+}
+
 int launch_predict(const PredictParams& p, int* grid_out, cudaStream_t st) {
   const int wpb = kThreads / 32;
   long long blocks = ((long long)p.N + wpb - 1) / wpb;
@@ -1194,8 +1281,8 @@ int launch_grad_logits(const float* grad, long long rows, int C, void* g, int ld
   return VBNN_OK;
 }
 
-int launch_finalize_result(const float* acc, int Z, int N, float* out2, cudaStream_t st) {
-  k_finalize_result<<<1, 32, 0, st>>>(acc, Z, N, out2);
+int launch_finalize_result(const float* acc, int Z, float div, float scale1, float* out2, cudaStream_t st) {
+  k_finalize_result<<<1, 32, 0, st>>>(acc, Z, div, scale1, out2);
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }

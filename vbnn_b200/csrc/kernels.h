@@ -123,8 +123,17 @@ struct LossParams {
   float* logp_out;                      // nullable [Z*N x C]
   float* result;                        // [2*Zslots]: result[2z] += sum nll, result[2z+1] += #correct
   int z_slot0;
+  // ---- regression criteria (launch_loss_reg) ----
+  int criterion;                        // enum vbnn_criterion: VBNN_CRIT_MSE or VBNN_CRIT_GAUSSIAN_NLL
+  const void* r; void* h;               // nullable, typed as the gradient: LRT output layer, h = g .* r [Z*N x ld_g]
 };
 int launch_loss(const LossParams& p, cudaStream_t st);
+// The regression criteria of vbnn_mlp_set_criterion, one warp per row like launch_loss.  targets are dense [N x K]
+// (MSE: K = C; GAUSSIAN_NLL: K = C / 2, columns [0, K) of a row are means m, [K, 2K) log-variances s); a NaN target
+// adds nothing.  grad_scale = 1 / (N_global K).  Per (z, n) it writes dl/dY into g (padding columns zeroed as
+// launch_loss leaves them) and h, and adds {sum of loss terms, sum (y - m)^2} into result[2z], result[2z+1]: MSE's loss
+// term is (y - m)^2 itself, GAUSSIAN_NLL's 1/2 (s + q^2) with q = (y - m) e^{-s/2}.
+int launch_loss_reg(const LossParams& p, cudaStream_t st);
 // A caller-supplied dLoss/dlogits (vbnn_mlp_backward_update), dense fp32 [rows x C], into the output layer's
 // gradient operand g [rows x ld_g] (bf16 or fp32, padding columns zeroed as launch_loss leaves them) and, when r is
 // set (LRT output layer), h = g .* r [rows x ld_g] in the same pass (launch_mul_act's H).
@@ -202,7 +211,8 @@ int launch_philox_matrix(float* dst, int rows, int cols, int row0, PhiloxStream 
 int launch_bump(uint32_t* step, int** t_ptrs_dev, int n_t, cudaStream_t st);
 int launch_snr(const float* mu, const float* lvar, long long n, float thresh, uint8_t* mask,
                unsigned long long* count_dev, cudaStream_t st);
-// result[0] = mean over Z of loss sums / N, result[1] = mean accuracy % (main.lua:38-39)
-int launch_finalize_result(const float* acc, int Z, int N, float* out2, cudaStream_t st);
+// result[0] = mean over Z of loss sums / div, result[1] = mean over Z of acc[2z+1] / div * scale1: ClassNLL passes
+// div = N, scale1 = 100 (mean accuracy %, main.lua:38-39); the regression criteria div = N K, scale1 = 1
+int launch_finalize_result(const float* acc, int Z, float div, float scale1, float* out2, cudaStream_t st);
 
 }  // namespace vbnn

@@ -20,6 +20,25 @@ inline int nlayers(const vbnn_mlp* m) { return (int)m->layers.size(); }
 inline bool lrt_split(const vbnn_mlp* m, int which) {
   return (knobs().lrt_split & which) != 0 && m->aux != nullptr;
 }
+inline bool regression(const vbnn_mlp* m) { return m->criterion != VBNN_CRIT_CLASS_NLL; }
+// K: target floats per row under the net's criterion (ClassNLL: one label)
+inline int target_cols(const vbnn_mlp* m) {
+  const int C = m->sizes.back();
+  return m->criterion == VBNN_CRIT_MSE ? C : m->criterion == VBNN_CRIT_GAUSSIAN_NLL ? C / 2 : 1;
+}
+// the divisor of the finalised scalars: N rows, or the N K target elements of a regression criterion
+inline float result_div(const vbnn_mlp* m, int N) {
+  return regression(m) ? (float)((double)N * target_cols(m)) : (float)N;
+}
+// the finalised {error, accuracy} pair; under MSE both are the mean squared error, and the second is copied from the
+// first so that they stay equal bit for bit (the two sums are accumulated by separate atomics, in different orders)
+int finalize_result(vbnn_mlp* m, int N, cudaStream_t st) {
+  VB_TRY(launch_finalize_result(m->result_acc, m->Z, result_div(m, N), regression(m) ? 1.f : 100.f, m->result, st));
+  m->ctx->launches++;
+  if (m->criterion == VBNN_CRIT_MSE)
+    VB_CUDA(cudaMemcpyAsync(m->result + 1, m->result, 4, cudaMemcpyDeviceToDevice, st));
+  return VBNN_OK;
+}
 
 // ---- stage the caller's minibatch into operand form (outside the graph: pointers vary) ----
 int stage_input(vbnn_mlp* m, const float* X, const float* T, int N) {
@@ -37,7 +56,7 @@ int stage_input(vbnn_mlp* m, const float* X, const float* T, int N) {
       m->ctx->launches++;
     }
   }
-  if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * 4, cudaMemcpyDeviceToDevice, st));
+  if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * target_cols(m) * 4, cudaMemcpyDeviceToDevice, st));
   m->last_N = N;
   m->outputs_external = false;
   return VBNN_OK;
@@ -54,7 +73,7 @@ int stage_input_u8(vbnn_mlp* m, const uint8_t* X, const float* T, int N, float m
     VB_TRY(launch_cast_u8(X, N, I0, mean, inv_std, nullptr, nullptr, 0, (float*)m->act[0],
                           m->lrt ? (float*)m->act2[0] : nullptr, ld0, st));
   m->ctx->launches++;
-  if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * 4, cudaMemcpyDeviceToDevice, st));
+  if (T) VB_CUDA(cudaMemcpyAsync(m->targets, T, (size_t)N * target_cols(m) * 4, cudaMemcpyDeviceToDevice, st));
   m->last_N = N;
   m->outputs_external = false;
   return VBNN_OK;
@@ -170,6 +189,15 @@ int loss_all(vbnn_mlp* m, int N, int Zrun, bool backward, float* logp_out, float
   lp.logp_out = logp_out;
   lp.result = result;
   lp.z_slot0 = 0;
+  if (regression(m)) {
+    // the mean over the global batch's N_g K target elements; an LRT output layer's H = G .* R in the same pass
+    lp.criterion = m->criterion;
+    lp.grad_scale = (float)(1.0 / ((double)N * m->ctx->nranks * target_cols(m)));
+    if (backward && layer_is_lrt(Lo)) { lp.r = m->R[Lc - 1]; lp.h = m->H[Lc - 1]; }
+    VB_TRY(launch_loss_reg(lp, m->ctx->stream));
+    m->ctx->launches++;
+    return VBNN_OK;
+  }
   VB_TRY(launch_loss(lp, m->ctx->stream));
   m->ctx->launches++;
   if (backward && layer_is_lrt(Lo)) {
@@ -404,7 +432,7 @@ int step_backward(vbnn_mlp* m, int N, bool finalize) {
   cudaStream_t st = m->ctx->stream;
   if (m->peer && m->peer->active) {
     VB_TRY(backward_samples(m, N, m->Z, 0, 0, false, true));
-    if (finalize) { VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st)); m->ctx->launches++; }
+    if (finalize) VB_TRY(finalize_result(m, N, st));
     VB_TRY(launch_bump(m->ctx->d_step, m->t_list_dev, 0, st));    // the layers' t counters advance on the side stream
     m->ctx->launches++;
     VB_TRY(prof_mark(m->ctx, 7));
@@ -416,10 +444,7 @@ int step_backward(vbnn_mlp* m, int N, bool finalize) {
   if (dp && !overlap) VB_TRY(comm_allreduce_internal(m->ctx, m->grad_arena, m->grad_count, st));
   VB_TRY(update_all(m, overlap));                                                              // :40
   VB_TRY(prof_mark(m->ctx, 6));
-  if (finalize) {                                                                              // :38-39
-    VB_TRY(launch_finalize_result(m->result_acc, m->Z, N, m->result, st));
-    m->ctx->launches++;
-  }
+  if (finalize) VB_TRY(finalize_result(m, N, st));                                             // :38-39
   VB_TRY(launch_bump(m->ctx->d_step, m->t_list_dev, m->n_t, st));
   m->ctx->launches++;
   VB_TRY(prof_mark(m->ctx, 7));
@@ -775,8 +800,9 @@ extern "C" int vbnn_mlp_run(vbnn_mlp* m, const float* X, const float* T, int N, 
   if (err_host || acc_host) {
     VB_CUDA(cudaMemcpyAsync(c->h_scalars, racc, 8, cudaMemcpyDeviceToHost, st));
     VB_CUDA(cudaStreamSynchronize(st));
-    if (err_host) *err_host = c->h_scalars[0] / (float)N;                    // mlp.lua:80
-    if (acc_host) *acc_host = c->h_scalars[1] / (float)N * 100.f;            // mlp.lua:82
+    if (err_host) *err_host = c->h_scalars[0] / result_div(m, N);            // mlp.lua:80
+    const float second = c->h_scalars[m->criterion == VBNN_CRIT_MSE ? 0 : 1];   // MSE: the same sum for both
+    if (acc_host) *acc_host = second / result_div(m, N) * (regression(m) ? 1.f : 100.f);            // mlp.lua:82
   }
   return VBNN_OK;
 }
@@ -881,7 +907,7 @@ static int ensure_pipeline(vbnn_mlp* m) {
   if (m->pipeline_ready) return VBNN_OK;
   for (int s = 0; s < 2; ++s) {
     VB_TRY(dev_alloc(&m->xstage[s], (size_t)m->max_batch * m->sizes[0]));
-    VB_TRY(dev_alloc(&m->tstage[s], (size_t)m->max_batch));
+    VB_TRY(dev_alloc(&m->tstage[s], (size_t)m->max_batch * m->tgt_cols));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].copied, cudaEventDisableTiming));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].consumed, cudaEventDisableTiming));
     VB_CUDA(cudaEventCreateWithFlags(&m->slots[s].done, cudaEventDisableTiming));
@@ -910,7 +936,7 @@ static int submit_host_any(vbnn_mlp* m, const float* X_host, const uint8_t* X8_h
     VB_CUDA(cudaMemcpyAsync(m->xstage_u8[s], X8_host, (size_t)N * m->sizes[0], cudaMemcpyHostToDevice, c->copy_stream));
   else
     VB_CUDA(cudaMemcpyAsync(m->xstage[s], X_host, (size_t)N * m->sizes[0] * 4, cudaMemcpyHostToDevice, c->copy_stream));
-  VB_CUDA(cudaMemcpyAsync(m->tstage[s], T_host, (size_t)N * 4, cudaMemcpyHostToDevice, c->copy_stream));
+  VB_CUDA(cudaMemcpyAsync(m->tstage[s], T_host, (size_t)N * target_cols(m) * 4, cudaMemcpyHostToDevice, c->copy_stream));
   VB_CUDA(cudaEventRecord(sl.copied, c->copy_stream));
   // compute stream
   VB_CUDA(cudaStreamWaitEvent(c->stream, sl.copied, 0));
@@ -968,6 +994,49 @@ extern "C" int vbnn_mlp_collect(vbnn_mlp* m, float* err_host, float* acc_host) {
   return VBNN_OK;
 }
 
+extern "C" int vbnn_mlp_set_criterion(vbnn_mlp* m, int criterion) {
+  VB_CHECK(m, VBNN_E_INVALID, "vbnn_mlp_set_criterion: null mlp");
+  const int C = m->sizes.back();
+  VB_CHECK(criterion == VBNN_CRIT_CLASS_NLL || criterion == VBNN_CRIT_MSE || criterion == VBNN_CRIT_GAUSSIAN_NLL,
+           VBNN_E_INVALID, "vbnn_mlp_set_criterion: unknown criterion %d", criterion);
+  VB_CHECK(criterion != VBNN_CRIT_GAUSSIAN_NLL || C % 2 == 0, VBNN_E_INVALID,
+           "vbnn_mlp_set_criterion: VBNN_CRIT_GAUSSIAN_NLL needs an even number of outputs, the net has %d", C);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_set_criterion"));
+  VB_CHECK(m->inflight == 0, VBNN_E_STATE, "vbnn_mlp_set_criterion: %d host-pipeline minibatch(es) not collected",
+           m->inflight);
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  VB_CUDA(cudaStreamIsCapturing(m->ctx->stream, &cs));
+  VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE,
+           "vbnn_mlp_set_criterion: the context's stream is being captured (the step graphs bake the criterion in)");
+  if (criterion == m->criterion) return VBNN_OK;
+  if (criterion != VBNN_CRIT_CLASS_NLL && m->tgt_cols == 1) {
+    // grow the staged targets (and the pipeline's staging) once to max_batch x C, enough for either regression
+    // criterion; the buffers being replaced may still be read by enqueued work
+    float* nt[3] = {nullptr, nullptr, nullptr};
+    const int n_new = m->pipeline_ready ? 3 : 1;
+    int r = VBNN_OK;
+    for (int k = 0; k < n_new && r == VBNN_OK; ++k) r = dev_alloc(&nt[k], (size_t)m->max_batch * C);
+    if (r != VBNN_OK) { for (float* q : nt) if (q) cudaFree(q); return r; }
+    VB_CUDA(cudaStreamSynchronize(m->ctx->stream));
+    VB_CUDA(cudaStreamSynchronize(m->ctx->copy_stream));
+    cudaFree(m->targets);
+    m->targets = nt[0];
+    if (m->pipeline_ready)
+      for (int s = 0; s < 2; ++s) { cudaFree(m->tstage[s]); m->tstage[s] = nt[1 + s]; }
+    m->tgt_cols = C;
+  }
+  mlp_drop_graphs(m);                     // the loss kernel, its divisors and the staging size are baked into them
+  m->criterion = criterion;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_get_criterion(const vbnn_mlp* m, int* criterion) {
+  VB_CHECK(m && criterion, VBNN_E_INVALID, "vbnn_mlp_get_criterion: null argument");
+  *criterion = m->criterion;
+  return VBNN_OK;
+}
+
 extern "C" int vbnn_mlp_step_host(vbnn_mlp* m, const float* X_host, const float* T_host, int N,
                                   float* err_host, float* acc_host) {
   VB_TRY(vbnn_mlp_submit_host(m, X_host, T_host, N));
@@ -989,8 +1058,10 @@ extern "C" int vbnn_mlp_test(vbnn_mlp* m, const float* X, const float* T, int N,
   VB_CUDA(cudaStreamSynchronize(st));
   double e = 0, a = 0;
   for (int z = 0; z < m->Z; ++z) { e += c->h_scalars[2 * z]; a += c->h_scalars[2 * z + 1]; }
-  if (err_host) *err_host = (float)(e / ((double)total * N));               // mlp.lua:101
-  if (acc_host) *acc_host = (float)(a / ((double)total * N) * 100.0);
+  if (m->criterion == VBNN_CRIT_MSE) a = e;                                 // the same sum: equal bit for bit
+  const double div = (double)total * N * (regression(m) ? target_cols(m) : 1);
+  if (err_host) *err_host = (float)(e / div);                               // mlp.lua:101
+  if (acc_host) *acc_host = (float)(a / div * (regression(m) ? 1.0 : 100.0));
   return VBNN_OK;
 }
 
@@ -1121,6 +1192,12 @@ extern "C" int vbnn_mlp_get_outputs(vbnn_mlp* m, int sample_idx, float* logp_hos
            "vbnn_mlp_get_outputs: the last forward was vbnn_mlp_forward_train, whose outputs are in the caller's buffer");
   vbnn_ctx* c = m->ctx;
   const int N = m->last_N, C = m->sizes.back();
+  if (regression(m)) {                    // no LogSoftMax: the raw outputs of sample sample_idx
+    VB_CUDA(cudaMemcpy2DAsync(logp_host, (size_t)C * 4, m->logits + (size_t)sample_idx * N * m->ld_logits,
+                              (size_t)m->ld_logits * 4, (size_t)C * 4, N, cudaMemcpyDeviceToHost, c->stream));
+    VB_CUDA(cudaStreamSynchronize(c->stream));
+    return VBNN_OK;
+  }
   if (!m->logp) VB_TRY(dev_alloc(&m->logp, (size_t)m->max_batch * C));
   LossParams lp;
   memset(&lp, 0, sizeof(lp));

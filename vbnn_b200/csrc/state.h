@@ -134,7 +134,9 @@ struct vbnn_mlp {
   // vbnn_mlp_predict_outputs state, allocated by its first call: {f0, sum d, sum d^2} [3 x max_batch x C], then the
   // per-row log-sum-exp max / sum [2 x max_batch]
   float* mom_state = nullptr;
-  float* targets = nullptr;          // staged targets [N]
+  int criterion = VBNN_CRIT_CLASS_NLL;    // vbnn_mlp_set_criterion
+  int tgt_cols = 1;                  // floats per row that targets / tstage hold: 1, or C once a regression criterion was set
+  float* targets = nullptr;          // staged targets [N x target columns of the criterion]
   float* xstage[2] = {nullptr, nullptr};   // fp32 H2D staging for the host-buffer API
   float* tstage[2] = {nullptr, nullptr};
   uint8_t* xstage_u8[2] = {nullptr, nullptr};   // uint8 H2D staging (vbnn_mlp_submit_host_u8)

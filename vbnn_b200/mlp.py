@@ -44,7 +44,12 @@ class MLP:
     def buildModel(self, opt, ctx: Context = None, max_batch=None):
         self.opt = opt
         self.ctx = ctx or default_context(seed=opt.get("seed", 3))
-        sizes = [int(opt["input_size"])] + [int(h) for h in opt["hidden"]] + [len(opt["classes"])]
+        criterion = opt.get("criterion", "class_nll")
+        if criterion not in L.CRITERIA:
+            raise L.VbnnError(L.E_INVALID, f"opt.criterion must be one of {sorted(L.CRITERIA)}, got {criterion!r}")
+        # a regression net may give its output width as opt.outputs instead of a list of classes
+        n_out = int(opt["outputs"]) if criterion != "class_nll" and "outputs" in opt else len(opt["classes"])
+        sizes = [int(opt["input_size"])] + [int(h) for h in opt["hidden"]] + [n_out]
         self.sizes = sizes
         self.max_batch = int(max_batch or max(opt["batchSize"], opt.get("testBatchSize", 1)))
         arr = (C.c_int * len(sizes))(*sizes)
@@ -69,7 +74,33 @@ class MLP:
             raise L.VbnnError(L.E_INVALID, f"opt.prior must be 'empirical' or 'fixed', got {prior!r}")
         if prior == "fixed":
             self.set_prior("fixed", opt.get("prior_mean", 0.0), opt.get("prior_var"))
+        self.criterion = "class_nll"
+        if criterion != "class_nll":
+            self.set_criterion(criterion)
         return self
+
+    def set_criterion(self, criterion):
+        """The criterion of the fused minibatch (vbnn_mlp_set_criterion), the swap of mlp.lua:30-32's criterion object:
+        "class_nll" (LogSoftMax + ClassNLL, the default), "mse" (nn.MSECriterion, targets [N x C]) or "gaussian_nll"
+        (C = 2K outputs read as K means and K log-variances, targets [N x K], the loss 1/2 (s + (y - m)^2 e^{-s})
+        averaged over N K).  train_step, train_step_host, submit_host*, run and test follow it; their (error, accuracy)
+        pair becomes (mean loss, MSE of the means) under a regression criterion.  NaN targets are padding: they add
+        nothing.  Refused while a forward_train step is open or host minibatches are uncollected."""
+        if criterion not in L.CRITERIA:
+            raise L.VbnnError(L.E_INVALID, f"criterion must be one of {sorted(L.CRITERIA)}, got {criterion!r}")
+        L.check(L.lib().vbnn_mlp_set_criterion(self.handle, L.CRITERIA[criterion]))
+        self.criterion = criterion
+
+    def _target_cols(self):
+        """targets per input row: 1 label (class_nll), C (mse) or C / 2 (gaussian_nll)"""
+        return {"class_nll": 1, "mse": self.sizes[-1], "gaussian_nll": self.sizes[-1] // 2}[self.criterion]
+
+    def _check_targets(self, t, n):
+        """t flattened; one label or one [K] row of regression targets per input row"""
+        k = self._target_cols()
+        if t.shape[0] != n * k:
+            want = "N targets" if k == 1 else f"[N x {k}] targets"
+            raise L.VbnnError(L.E_INVALID, f"inputs must be [N x {self.sizes[0]}] with {want}")
 
     def set_prior(self, kind, mean=0.0, var=None):
         """VBLinear.set_prior on every VB layer (the hidden layers and a vb_output layer); "per_weight" makes each
@@ -108,8 +139,9 @@ class MLP:
         x = as_dev_f32(inputs, self.ctx.device)
         x = x.reshape(x.shape[0], -1)                                   # nn.Reshape (mlp.lua:12)
         t = as_dev_f32(targets, self.ctx.device).reshape(-1)
-        if x.shape[1] != self.sizes[0] or t.shape[0] != x.shape[0]:
+        if x.shape[1] != self.sizes[0]:
             raise L.VbnnError(L.E_INVALID, f"inputs must be [N x {self.sizes[0]}] with N targets")
+        self._check_targets(t, x.shape[0])
         return x, t
 
     # ---- mlp.lua:62-84 ----
@@ -354,7 +386,9 @@ class MLP:
         if x.is_cuda or t.is_cuda:
             raise L.VbnnError(L.E_INVALID, "train_step_host expects host tensors")
         x = x.reshape(x.shape[0], -1).contiguous()
-        return x, t.reshape(-1).contiguous()
+        t = t.reshape(-1).contiguous()
+        self._check_targets(t, x.shape[0])
+        return x, t
 
     def submit_host(self, inputs_host, targets_host):
         x, t = self._host_io(inputs_host, targets_host)
@@ -373,6 +407,7 @@ class MLP:
             raise L.VbnnError(L.E_INVALID, "submit_host_u8 expects a uint8 host tensor")
         x = x.reshape(x.shape[0], -1).contiguous()
         t = torch.as_tensor(targets_host, dtype=torch.float32).reshape(-1).contiguous()
+        self._check_targets(t, x.shape[0])
         self._keep = getattr(self, "_keep", [])
         self._keep.append((x, t))
         self._keep = self._keep[-4:]
@@ -388,7 +423,8 @@ class MLP:
         return err.value, acc.value
 
     def outputs(self, sample_idx=0, n=None):
-        """LogSoftMax output of the last forward (self.model.output in the reference)."""
+        """Output of the last forward (self.model.output in the reference), [n x C] on the host: the LogSoftMax under
+        "class_nll", the raw outputs under a regression criterion (the net has no LogSoftMax then)."""
         import torch
         n = n or self._last_n()
         out = torch.empty(n, self.sizes[-1], dtype=torch.float32)

@@ -543,6 +543,10 @@ int vbnn_gemm_bf16(vbnn_ctx* ctx, const uint16_t* A_dev, int lda, int a_kmajor,
                    const uint16_t* B_dev, int ldb, int b_kmajor, float* D_dev, int ldd,
                    int M, int N, int K, int batch, long long strideA, long long strideB,
                    long long strideD);
+/* The N(0,1) matrix out_dev[rows x cols] the fused kernels draw (csrc/philox.cuh): row r, columns 4c .. 4c+3 are
+ * the 4 normals of Philox counter (idx4, stream, sample, step) with key seed, idx4 = (row0 + r) * ceil(cols/4) + c
+ * computed in uint32.  Counters past 2^32 - 1 therefore wrap to 0 and repeat the first values of the stream; the
+ * layers refuse shapes whose own counters would wrap (VBNN_E_UNSUPPORTED), this entry point does not. */
 int vbnn_philox_normal(vbnn_ctx* ctx, uint64_t seed, uint32_t step, uint32_t stream,
                        uint32_t sample, int rows, int cols, int row0, float* out_dev);
 /* Experiment switches (csrc/knobs.h: "tc_bn", "tc_cg", "lrt_split", "dw_split", "no_graph", ...; the same

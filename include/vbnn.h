@@ -51,7 +51,7 @@ enum vbnn_reparam {
   VBNN_REPARAM_LOCAL = 1   /* local reparameterisation: Y = X mu^T + sqrt(X^2 s2^T)*zeta (new)    */
 };
 /* Local reparameterisation keeps R = zeta / (2 sqrt(V)), V = X^2 s2^T, for the backward.  Where V == 0 (an all-zero
- * input row: zero-padded minibatch rows, or a hidden row whose units are all dead after ReLU) R := 0, so the variance
+ * input row: zero-padded minibatch rows, or a hidden row whose units are all dead after ReLU or all 0 after tanh) R := 0, so the variance
  * term adds nothing to gradInput or gradSum for that row; the row's output is X mu^T + b.  Any V > 0, subnormal ones
  * included, gets the finite zeta / (2 sqrt(V)). */
 
@@ -295,7 +295,7 @@ int vbnn_layer_draw_noise(vbnn_layer* layer, uint32_t step, int sample_idx, int 
 
 /* ---------------------------------------------------------------- mlp.lua -------------
  * MLP:buildModel(opt)  mlp.lua:7-60.  sizes = {input_size, hidden..., #classes}; hidden layers
- * are VBLinear+ReLU, the last is nn.Linear (mlp.lua:29) or, with vb_output, a VBLinear
+ * are VBLinear+ReLU (or the activation of vbnn_mlp_set_activation), the last is nn.Linear (mlp.lua:29) or, with vb_output, a VBLinear
  * (convnet.lua:30).  Ends in LogSoftMax + ClassNLLCriterion (mlp.lua:30-32), or in the regression
  * criterion chosen by vbnn_mlp_set_criterion. */
 int vbnn_mlp_create(vbnn_ctx* ctx, const int* sizes, int n_sizes, int vb_output, int max_batch,
@@ -411,6 +411,40 @@ enum vbnn_criterion {
  * host-pipeline minibatches are not collected, or the context's stream is being captured. */
 int vbnn_mlp_set_criterion(vbnn_mlp* mlp, int criterion);
 int vbnn_mlp_get_criterion(const vbnn_mlp* mlp, int* criterion);
+/* The nonlinearity of every hidden layer (mlp.lua:19,27: nn.ReLU, which a Torch7 user swaps for nn.Tanh, nn.Sigmoid or
+ * nn.ELU).  A new net is VBNN_ACT_RELU.  The output layer stays linear and the criteria are unchanged.  With y the
+ * pre-activation (bias and local-reparameterisation noise included) and a = f(y) the stored output, the backward
+ * multiplies by f' formed FROM a, as Torch7's updateGradInput of these modules does: */
+enum vbnn_activation {
+  VBNN_ACT_RELU = 0,          /* max(y, 0);                     f' = a > 0 ? 1 : 0           */
+  VBNN_ACT_TANH = 1,          /* tanh(y);                       f' = 1 - a^2                 */
+  VBNN_ACT_SIGMOID = 2,       /* 1 / (1 + e^{-y});              f' = a (1 - a)               */
+  VBNN_ACT_ELU = 3            /* y > 0 ? y : e^y - 1 (alpha 1); f' = a > 0 ? 1 : a + 1       */
+};
+/* Choose it for every net-level entry point: vbnn_mlp_step, _step_grad_input, _step_host, _submit_host, _submit_host_u8,
+ * the split step, vbnn_mlp_run, vbnn_mlp_test (MC and MAP), vbnn_mlp_predict and vbnn_mlp_predict_outputs, on one GPU,
+ * in peer mode and in NCCL mode (where every rank must set the same value, as with vbnn_mlp_set_opts).  The layer-level
+ * ABI is unchanged: vbnn_layer_forward is nn.Linear, and its caller runs the activation.
+ *   - The activation and its derivative are fused into the forward and backward-data GEMM epilogues: no launch is
+ *     added, and the ReLU kernels are the ones ReLU always ran.  vbnn_mlp_step_grad_input's dX has no f' term (nothing
+ *     is below the input).  Local reparameterisation: the backward-data join is g = (G mu + 2 a .* (H s2)) .* f'(a),
+ *     and a^2 is the square of a after its rounding to the operand type.
+ *   - Accuracy.  VBNN_PREC_FP32 uses tanhf, expf and expm1f (a few ulp).  VBNN_PREC_BF16 uses fast forms, each far below
+ *     the 2^-9 of the bf16 operand it is rounded to: tanh.approx.f32 (2^-11 relative, PTX ISA); sigmoid from
+ *     e = __expf(-|y|) and a fast divide, as 1 / (1 + e) or e / (1 + e) (never 1/2 tanh(y/2) + 1/2, whose relative error
+ *     blows up as sigmoid(y) -> 0); ELU's e^y - 1 as a cubic above y = -1/16 and __expf(y) - 1 below (2^-16 relative).
+ *     In bf16 f' is formed from the bf16 operand a, so it carries that rounding: 1 - a^2 is off by up to about 2 * 2^-9
+ *     near |a| = 1 (Torch7's rule applied to the stored operand).
+ *   - Saturation: every finite y gives a finite a and f'.  At y = +-100: tanh -> +-1 with f' exactly 0; sigmoid -> 1
+ *     with f' = 0, and -> e^-100 (fp32, a subnormal) or 0 (bf16) with f' as small; ELU -> -1 with f' exactly 0.  The
+ *     local-reparameterisation rule "V = 0 => R = 0" is unchanged: tanh(0) = 0 keeps an all-zero row all-zero, and
+ *     sigmoid and ELU rows are never zero.
+ *   - A set that changes the activation makes each step graph re-capture once at its next use; a set to the current
+ *     value changes nothing.  A net without hidden layers accepts the value, and nothing it computes changes.
+ * VBNN_E_INVALID: a NULL net or an unknown value.  VBNN_E_STATE: a split step is open, host-pipeline minibatches are not
+ * collected, or the context's stream is being captured. */
+int vbnn_mlp_set_activation(vbnn_mlp* mlp, int activation);
+int vbnn_mlp_get_activation(const vbnn_mlp* mlp, int* activation);
 /* same with HOST buffers: H2D of inputs + D2H of {error, accuracy} inside the call
  * (replaces inputs:cuda()/targets:cuda() main.lua:23-24 and the scalar reads mlp.lua:80-82). */
 int vbnn_mlp_step_host(vbnn_mlp* mlp, const float* X_host, const float* targets_host, int N,

@@ -27,7 +27,7 @@ function MLP:buildModel(opt)                                          -- referen
    sizes[#sizes + 1] = (crit ~= 'class_nll' and opt.outputs) or #opt.classes
    local csizes = ffi.new('int[?]', #sizes, sizes)
    local out = ffi.new('vbnn_mlp*[1]')
-   -- hidden layers: VBLinear + ReLU; output: plain nn.Linear + LogSoftMax (mlp.lua:29-30), or a VBLinear with
+   -- hidden layers: VBLinear + ReLU (or opt.activation); output: plain nn.Linear + LogSoftMax (mlp.lua:29-30), or a VBLinear with
    -- opt.vb_output (the convnet.lua:30 head)
    V.check(C.vbnn_mlp_create(V.context(opt.seed, true), csizes, #sizes, opt.vb_output and 1 or 0, opt.batchSize,
                              V.opts(opt), out))
@@ -40,7 +40,18 @@ function MLP:buildModel(opt)                                          -- referen
    if opt.prior == 'fixed' then net:set_prior('fixed', opt.prior_mean, opt.prior_var) end
    net.C = sizes[#sizes]
    net:set_criterion(crit)
+   net:set_activation(opt.activation or 'relu')
    return net
+end
+
+-- The nonlinearity of every hidden layer (vbnn_mlp_set_activation), the one-word edit of mlp.lua:19,27: 'relu'
+-- (nn.ReLU, the default), 'tanh' (nn.Tanh), 'sigmoid' (nn.Sigmoid) or 'elu' (nn.ELU, alpha 1).  The output layer
+-- stays linear.
+local ACTIVATION = { relu = 0, tanh = 1, sigmoid = 2, elu = 3 }
+function MLP:set_activation(name)
+   assert(ACTIVATION[name], "set_activation: 'relu', 'tanh', 'sigmoid' or 'elu'")
+   V.check(C.vbnn_mlp_set_activation(self.h, ACTIVATION[name]))
+   self.activation = name
 end
 
 -- The criterion of the fused minibatch (vbnn_mlp_set_criterion), the swap of mlp.lua:30-32's criterion object:

@@ -61,6 +61,8 @@ int vbnn_mlp_test(vbnn_mlp*, const float* X_dev, const float* targets_dev, int N
 int vbnn_mlp_predict(vbnn_mlp*, const float* X_dev, int N, int n_samples, const float* targets_dev, float* logp_dev, float* unc_dev, float* nll_host, float* acc_host);
 int vbnn_mlp_set_criterion(vbnn_mlp*, int criterion);
 int vbnn_mlp_get_criterion(const vbnn_mlp*, int* criterion);
+int vbnn_mlp_set_activation(vbnn_mlp*, int activation);
+int vbnn_mlp_get_activation(const vbnn_mlp*, int* activation);
 int vbnn_mlp_predict_outputs(vbnn_mlp*, const float* X_dev, int N, int n_samples, int output_model, const float* targets_dev, float* samples_dev, float* mean_dev, float* epistemic_dev, float* aleatoric_dev, float* nll_host, float* rmse_host);
 /* data parallel: NCCL id, then (optionally) the peer-memory exchange */
 int vbnn_comm_unique_id(void* id128);

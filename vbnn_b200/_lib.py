@@ -23,6 +23,8 @@ OUTPUT_RAW, OUTPUT_GAUSSIAN = 0, 1
 OUTPUT_MODELS = {"raw": OUTPUT_RAW, "gaussian": OUTPUT_GAUSSIAN}
 CRIT_CLASS_NLL, CRIT_MSE, CRIT_GAUSSIAN_NLL = 0, 1, 2
 CRITERIA = {"class_nll": CRIT_CLASS_NLL, "mse": CRIT_MSE, "gaussian_nll": CRIT_GAUSSIAN_NLL}
+ACT_RELU, ACT_TANH, ACT_SIGMOID, ACT_ELU = 0, 1, 2, 3
+ACTIVATIONS = {"relu": ACT_RELU, "tanh": ACT_TANH, "sigmoid": ACT_SIGMOID, "elu": ACT_ELU}
 
 
 class VbnnOpts(C.Structure):
@@ -107,6 +109,8 @@ _PROTOS = {
     "vbnn_mlp_backward_update": (C.c_int, [_P, _P, _P]),
     "vbnn_mlp_set_criterion": (C.c_int, [_P, C.c_int]),
     "vbnn_mlp_get_criterion": (C.c_int, [_P, C.POINTER(C.c_int)]),
+    "vbnn_mlp_set_activation": (C.c_int, [_P, C.c_int]),
+    "vbnn_mlp_get_activation": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "vbnn_mlp_step_host": (C.c_int, [_P, _P, _P, C.c_int, _F, _F]),
     "vbnn_mlp_submit_host": (C.c_int, [_P, _P, _P, C.c_int]),
     "vbnn_mlp_collect": (C.c_int, [_P, _F, _F]),

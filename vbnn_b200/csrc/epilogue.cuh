@@ -3,9 +3,9 @@
 //
 // One "quad" = 4 consecutive output columns of one output row; col % 4 == 0 so that a quad is
 // exactly one Philox counter (philox.cuh).  What each mode replaces in the reference:
-//   EPI_FWD      nn.Linear:updateOutput bias add (addr) + nn.ReLU           (mlp.lua:19,27,77)
+//   EPI_FWD      nn.Linear:updateOutput bias add (addr) + the activation     (mlp.lua:19,27,77)
 //   EPI_FWD_LRT  local reparameterisation forward (SURVEY.md 8a A12; not in the reference)
-//   EPI_DX       nn.Linear:updateGradInput + nn.ReLU backward               (mlp.lua:79)
+//   EPI_DX       nn.Linear:updateGradInput + the activation's backward       (mlp.lua:79)
 //   EPI_DX_LRT   A12 backward-data
 //   EPI_DW       VBLinear:accGradParameters: gradWeight += s*G^T X and
 //                gradSum += (G^T X) .* eps from ONE GEMM                    (VBLinear.lua:113-115)
@@ -14,6 +14,8 @@
 //                read back from global memory instead of a second TMEM accumulator
 #pragma once
 #include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 #include "philox.cuh"
@@ -35,6 +37,22 @@ enum EpiMode : int {
   EPI_DX_LRT2 = 8,           // acc = G mu, aux = H s2
 };
 
+// The hidden-layer activation of the FWD family (applied to the pre-activation) and of the DX family (its derivative,
+// formed from the stored output of the layer below, multiplied in): EpiParams::act.  EPI_ACT_NONE (0, what a zeroed
+// EpiParams holds) is nn.Linear alone.  The GEMM kernels are instantiated per kind (template ACT, the kind EPI_ACT_RELU
+// or one of the smooth kinds): the EPI_ACT_RELU kernels keep the runtime test p.act == EPI_ACT_RELU, which also serves
+// EPI_ACT_NONE, so that ReLU compiles to the code it always did; a smooth-kind kernel always applies its kind and
+// runs only where p.act holds it (epi_act_kernel).
+enum EpiAct : int {
+  EPI_ACT_NONE = 0,
+  EPI_ACT_RELU = 1 + VBNN_ACT_RELU,
+  EPI_ACT_TANH = 1 + VBNN_ACT_TANH,
+  EPI_ACT_SIGMOID = 1 + VBNN_ACT_SIGMOID,
+  EPI_ACT_ELU = 1 + VBNN_ACT_ELU,
+};
+// the kernel instantiation that serves EpiParams::act
+__host__ __device__ constexpr int epi_act_kernel(int act) { return act >= EPI_ACT_TANH && act <= EPI_ACT_ELU ? act : EPI_ACT_RELU; }
+
 __host__ __device__ constexpr bool epi_is_dual(int mode) {
   return mode == EPI_FWD_LRT || mode == EPI_DX_LRT || mode == EPI_DW_LRT;
 }
@@ -50,11 +68,10 @@ struct EpiParams {
   void* out_act; void* out_act2; void* r_out; int ld_act; long long zs_act;
   // inputs read by the epilogue
   const float* bias;         // [N]               (FWD, FWD_LRT)
-  int relu;                  // apply ReLU        (FWD, FWD_LRT)
-  const void* xprev;         // AT [M x ld_x]     (DX: mask source; DX_LRT: X and mask source)
+  int act;                   // enum EpiAct: FWD / FWD_LRT apply it, DX / DX_LRT multiply by its derivative at xprev
+  const void* xprev;         // AT [M x ld_x]     (DX: the activation's output a; DX_LRT: X and a)
   const void* rprev;         // AT [M x ld_x]     (DX_LRT: R of the previous layer, nullable)
   int ld_x; long long zs_x;
-  int mask;                  // DX/DX_LRT: multiply by (xprev > 0)
   const float* noise;        // injected eps [M x N] (DW) / zeta [M x N] (FWD_LRT); NULL -> Philox
   long long zs_noise;
   // DW, weight sampling on the tensor-core path: the epsilon k_sample_w drew for this minibatch, kept as fp16
@@ -164,26 +181,66 @@ __device__ __forceinline__ float lrt_rsqrt(float v) {
   return v > 0.f ? rsqrt_fast(v * 18446744073709551616.f) * 4294967296.f : 0.f;
 }
 
+// e^y - 1 for y <= 0 on the bf16 engine: __expf(y) - 1 loses its digits to cancellation as y -> 0 (at y = -2^-10 only
+// ~2^-13 of relative accuracy is left), so -1/16 < y uses the cubic y + y^2/2 + y^3/6 (truncation below |y|^3/24 <=
+// 2^-16.5 relative).  Below -1/16, __expf's few ulp on e^y >= 0 over |e^y - 1| >= 0.06 stay below 2^-18 relative.
+__device__ __forceinline__ float expm1_neg_fast(float y) {
+  return y > -0.0625f ? y * fmaf(y, fmaf(y, 0.16666667f, 0.5f), 1.f) : __expf(y) - 1.f;
+}
+__device__ __forceinline__ float tanh_fast(float y) {
+  float a;
+  asm("tanh.approx.f32 %0, %1;" : "=f"(a) : "f"(y));
+  return a;
+}
+
+// The activation a = f(y) of a smooth kind (ReLU stays inline in the epilogues).  FAST (the bf16 tensor-core engine):
+// tanh.approx.f32 (2^-11 relative, PTX ISA), sigmoid from __expf(-|y|) and a fast divide, ELU from expm1_neg_fast; the
+// fp32 engine uses tanhf, expf and expm1f.  Sigmoid is e / (1 + e) below 0 with e = e^{-|y|}, never 1/2 tanh(y/2) + 1/2,
+// whose relative error blows up as sigmoid(y) -> 0.  Every finite y gives a finite a: +-1 (tanh), 0 / 1 (sigmoid) and
+// -1 (ELU) where the kinds saturate.
+template <int ACT, bool FAST>
+__device__ __forceinline__ float act_fwd(float y) {
+  if constexpr (ACT == EPI_ACT_TANH) {
+    return FAST ? tanh_fast(y) : tanhf(y);
+  } else if constexpr (ACT == EPI_ACT_SIGMOID) {
+    const float e = FAST ? __expf(-fabsf(y)) : expf(-fabsf(y));
+    const float r = FAST ? __fdividef(1.f, 1.f + e) : 1.f / (1.f + e);
+    return y >= 0.f ? r : e * r;
+  } else {
+    static_assert(ACT == EPI_ACT_ELU, "act_fwd: smooth kinds only");
+    return y > 0.f ? y : (FAST ? expm1_neg_fast(y) : expm1f(y));
+  }
+}
+// f'(y) from the stored output a = f(y), as Torch7's updateGradInput forms it: 1 - a^2 (one rounding), a (1 - a),
+// a > 0 ? 1 : a + 1.  Exactly 0 where a saturates at +-1 / 0 / 1 / -1.
+template <int ACT>
+__device__ __forceinline__ float act_grad(float a) {
+  if constexpr (ACT == EPI_ACT_TANH) return fmaf(-a, a, 1.f);
+  else if constexpr (ACT == EPI_ACT_SIGMOID) return a * (1.f - a);
+  else { static_assert(ACT == EPI_ACT_ELU, "act_grad: smooth kinds only"); return a > 0.f ? 1.f : a + 1.f; }
+}
+
 // Process one quad.  a1/a2: accumulator values (a2 only for dual modes).
-template <int MODE, typename AT>
+template <int MODE, int ACT, typename AT>
 __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream& ps0, int z, int row, int col,
                                          const float (&a1)[4], const float (&a2)[4]);
 
 // split modes: fetch the other product, then run the dual-mode code
-template <int MODE, typename AT>
+template <int MODE, int ACT, typename AT>
 __device__ __forceinline__ void epi_quad_split(const EpiParams& p, const PhiloxStream& ps0, int z, int row, int col,
                                                const float (&acc)[4]) {
   if (row >= p.M || col >= p.N) return;
   float o[4];
   load4<float>(p.aux + z * p.zs_aux + (long long)row * p.ld_aux + col, o, min(4, p.N - col), (p.ld_aux & 3) == 0);
-  if constexpr (MODE == EPI_FWD_LRT2) epi_quad<EPI_FWD_LRT, AT>(p, ps0, z, row, col, o, acc);     // (mean, variance)
-  else epi_quad<EPI_DX_LRT, AT>(p, ps0, z, row, col, acc, o);                                    // (G mu, H s2)
+  if constexpr (MODE == EPI_FWD_LRT2) epi_quad<EPI_FWD_LRT, ACT, AT>(p, ps0, z, row, col, o, acc);     // (mean, variance)
+  else epi_quad<EPI_DX_LRT, ACT, AT>(p, ps0, z, row, col, acc, o);                                    // (G mu, H s2)
 }
 
-template <int MODE, typename AT>
+template <int MODE, int ACT, typename AT>
 __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream& ps0, int z, int row, int col,
                                          const float (&a1)[4], const float (&a2)[4]) {
-  if constexpr (MODE == EPI_FWD_LRT2 || MODE == EPI_DX_LRT2) { epi_quad_split<MODE, AT>(p, ps0, z, row, col, a1); return; }
+  if constexpr (MODE == EPI_FWD_LRT2 || MODE == EPI_DX_LRT2) { epi_quad_split<MODE, ACT, AT>(p, ps0, z, row, col, a1); return; }
+  constexpr bool FAST = !std::is_same<AT, float>::value;
   if (row >= p.M || col >= p.N) return;
   const int nvalid = min(4, p.N - col);
   const bool vec_act = (p.ld_act & 3) == 0;
@@ -197,7 +254,8 @@ __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream&
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       y[j] = a1[j] + b[j];
-      if (p.relu) y[j] = fmaxf(y[j], 0.f);
+      if constexpr (ACT == EPI_ACT_RELU) { if (p.act == EPI_ACT_RELU) y[j] = fmaxf(y[j], 0.f); }
+      else y[j] = act_fwd<ACT, FAST>(y[j]);
     }
     if (p.out_f32)
       store4<float>(p.out_f32 + z * p.zs_f32 + (long long)row * p.ld_f32 + col, y, nvalid, vec_f32);
@@ -228,7 +286,8 @@ __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream&
       store4<float>(p.out_f32 + z * p.zs_f32 + (long long)row * p.ld_f32 + col, y, nvalid, vec_f32);
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      if (p.relu) y[j] = fmaxf(y[j], 0.f);
+      if constexpr (ACT == EPI_ACT_RELU) { if (p.act == EPI_ACT_RELU) y[j] = fmaxf(y[j], 0.f); }
+      else y[j] = act_fwd<ACT, FAST>(y[j]);
       // square the value the next layer will actually read (after rounding to AT)
       float yr = to_f32(from_f32<AT>(y[j]));
       y2[j] = yr * yr;
@@ -247,7 +306,8 @@ __device__ __forceinline__ void epi_quad(const EpiParams& p, const PhiloxStream&
     for (int j = 0; j < 4; ++j) {
       g[j] = a1[j];
       if constexpr (MODE == EPI_DX_LRT) g[j] += 2.f * x[j] * a2[j];
-      if (p.mask) g[j] = x[j] > 0.f ? g[j] : 0.f;
+      if constexpr (ACT == EPI_ACT_RELU) { if (p.act == EPI_ACT_RELU) g[j] = x[j] > 0.f ? g[j] : 0.f; }
+      else g[j] *= act_grad<ACT>(x[j]);
     }
     if (p.out_f32)
       store4<float>(p.out_f32 + z * p.zs_f32 + (long long)row * p.ld_f32 + col, g, nvalid, vec_f32);

@@ -150,8 +150,8 @@ inline bool epi_can_stage(int mode, const EpiParams& p) {
 }
 
 // One full 32-column chunk of one warp (rows row0 .. row0+31, columns col0 .. col0+31 all < N).
-// v1 / v2: this thread's accumulator row (lane = row).  AT = bf16.
-template <int MODE>
+// v1 / v2: this thread's accumulator row (lane = row).  AT = bf16, so a smooth activation takes its fast forms.
+template <int MODE, int ACT>
 __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const PhiloxStream& ps0, int z, int row0, int lane,
                                                  int col0, const float (&v1)[32], const float (&v2)[32], uint32_t stage) {
   const int rows_valid = min(32, p.M - row0);        // <= 0 never happens: the caller skips such warps
@@ -160,8 +160,8 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
     // split LRT: the other product comes from global memory (coalesced through the staging tile)
     float o[32];
     get_tile_f32(stage, lane, p.aux + z * p.zs_aux + (long long)row0 * p.ld_aux + col0, p.ld_aux, rows_valid, o);
-    if constexpr (MODE == EPI_FWD_LRT2) epi_chunk_staged<EPI_FWD_LRT>(p, ps0, z, row0, lane, col0, o, v1, stage);
-    else epi_chunk_staged<EPI_DX_LRT>(p, ps0, z, row0, lane, col0, v1, o, stage);
+    if constexpr (MODE == EPI_FWD_LRT2) epi_chunk_staged<EPI_FWD_LRT, ACT>(p, ps0, z, row0, lane, col0, o, v1, stage);
+    else epi_chunk_staged<EPI_DX_LRT, ACT>(p, ps0, z, row0, lane, col0, v1, o, stage);
     return;
   }
   if constexpr (MODE == EPI_STORE) {
@@ -175,7 +175,8 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         float t = v1[4 * j + e] + b[e];
-        y[4 * j + e] = p.relu ? fmaxf(t, 0.f) : t;
+        if constexpr (ACT == EPI_ACT_RELU) y[4 * j + e] = p.act == EPI_ACT_RELU ? fmaxf(t, 0.f) : t;
+        else y[4 * j + e] = act_fwd<ACT, true>(t);
       }
     }
     if (p.out_f32)
@@ -204,7 +205,8 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
         const float rs = lrt_rsqrt(v);
         const float y = v1[4 * j + e] + b[e] + (v * rs) * zt[e];
         yf[4 * j + e] = y;
-        ya[e] = p.relu ? fmaxf(y, 0.f) : y;
+        if constexpr (ACT == EPI_ACT_RELU) ya[e] = p.act == EPI_ACT_RELU ? fmaxf(y, 0.f) : y;
+        else ya[e] = act_fwd<ACT, true>(y);
         rr[e] = 0.5f * zt[e] * rs;
       }
       wa[2 * j] = pack_bf16(ya[0], ya[1]); wa[2 * j + 1] = pack_bf16(ya[2], ya[3]);
@@ -223,7 +225,7 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
   } else if constexpr (MODE == EPI_DX || MODE == EPI_DX_LRT) {
     const long long xoff = z * p.zs_x + (long long)row0 * p.ld_x + col0;
     uint32_t wx[16];
-    const bool need_x = p.xprev != nullptr && (p.mask || MODE == EPI_DX_LRT);
+    const bool need_x = p.xprev != nullptr && (ACT != EPI_ACT_RELU || p.act == EPI_ACT_RELU || MODE == EPI_DX_LRT);
     if (need_x) get_tile_bf16(stage, lane, (const bf16*)p.xprev + xoff, p.ld_x, rows_valid, wx);
     float g[32];
 #pragma unroll
@@ -231,7 +233,11 @@ __device__ __forceinline__ void epi_chunk_staged(const EpiParams& p, const Philo
       const float x0 = need_x ? bf16_lo(wx[j]) : 0.f, x1 = need_x ? bf16_hi(wx[j]) : 0.f;
       float g0 = v1[2 * j], g1 = v1[2 * j + 1];
       if constexpr (MODE == EPI_DX_LRT) { g0 += 2.f * x0 * v2[2 * j]; g1 += 2.f * x1 * v2[2 * j + 1]; }
-      if (p.mask) { g0 = x0 > 0.f ? g0 : 0.f; g1 = x1 > 0.f ? g1 : 0.f; }
+      if constexpr (ACT == EPI_ACT_RELU) {
+        if (p.act == EPI_ACT_RELU) { g0 = x0 > 0.f ? g0 : 0.f; g1 = x1 > 0.f ? g1 : 0.f; }
+      } else {
+        g0 *= act_grad<ACT>(x0); g1 *= act_grad<ACT>(x1);
+      }
       g[2 * j] = g0; g[2 * j + 1] = g1;
     }
     if (p.out_f32)

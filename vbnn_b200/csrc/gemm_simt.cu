@@ -65,7 +65,7 @@ __device__ __forceinline__ void load_tile(float (*dst)[TM + 4], const float* __r
 // `scratch` [(z * ksplit + ks) * NACC + a][M x N]; k_simt_finish then adds the slices in a fixed order and runs the fused
 // epilogue.  For the tiny launch-bound configs (C1: 100 x 100 outputs, K = 784 -- 4 CTAs walking 49 k-steps serially)
 // this turns one long dependent chain into ksplit short ones.
-template <int MODE, bool DUAL>
+template <int MODE, int ACT, bool DUAL>
 __global__ void __launch_bounds__(256) gemm_simt_kernel(SimtGemmArgs g, EpiParams p, int ksplit, float* scratch) {
   __shared__ SimtSmem<DUAL> sm;
   const int z = blockIdx.z / ksplit, ks = blockIdx.z - z * ksplit;
@@ -132,11 +132,11 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(SimtGemmArgs g, EpiParam
   }
   const PhiloxStream ps = epi_stream(p);
 #pragma unroll
-  for (int i = 0; i < 4; ++i) epi_quad<MODE, float>(p, ps, z, m0 + ty * 4 + i, n0 + tx * 4, acc1[i], acc2[i]);
+  for (int i = 0; i < 4; ++i) epi_quad<MODE, ACT, float>(p, ps, z, m0 + ty * 4 + i, n0 + tx * 4, acc1[i], acc2[i]);
 }
 
 // one thread per quad: add the K slices in slice order, then the same fused epilogue
-template <int MODE, bool DUAL>
+template <int MODE, int ACT, bool DUAL>
 __global__ void __launch_bounds__(256) k_simt_finish(int M, int N, int batch, int ksplit, const float* scratch, EpiParams p) {
   constexpr int NACC = DUAL ? 2 : 1;
   const int Q = (N + 3) >> 2;
@@ -153,7 +153,7 @@ __global__ void __launch_bounds__(256) k_simt_finish(int M, int N, int batch, in
       for (int j = 0; j < 4; ++j)
         if (col + j < N) { a1[j] += s1[j]; if (DUAL) a2[j] += s1[MN + j]; }
     }
-    epi_quad<MODE, float>(p, ps, z, row, col, a1, a2);
+    epi_quad<MODE, ACT, float>(p, ps, z, row, col, a1, a2);
   }
 }
 
@@ -183,7 +183,7 @@ static int choose_ksplit(const SimtGemmArgs& g, int batch) {
   return ks < 1 ? 1 : (ks > 8 ? 8 : ks);
 }
 
-template <int MODE>
+template <int MODE, int ACT>
 static int launch_one(const SimtGemmArgs& g, const EpiParams& p, int batch, cudaStream_t st) {
   constexpr bool DUAL = epi_is_dual(MODE);
   int ksplit = choose_ksplit(g, batch);
@@ -196,18 +196,18 @@ static int launch_one(const SimtGemmArgs& g, const EpiParams& p, int batch, cuda
     if (!scratch || need > kScratchFloats) ksplit = 1;
   }
   dim3 grid(ceil_div(g.N, TN), ceil_div(g.M, TM), batch * ksplit);
-  gemm_simt_kernel<MODE, DUAL><<<grid, 256, 0, st>>>(g, p, ksplit, scratch);
+  gemm_simt_kernel<MODE, ACT, DUAL><<<grid, 256, 0, st>>>(g, p, ksplit, scratch);
   if (ksplit > 1) {
     const long long quads = (long long)batch * g.M * ((g.N + 3) / 4);
     int blocks = (int)((quads + 255) / 256);
     if (blocks > kNumSMs * 4) blocks = kNumSMs * 4;
-    k_simt_finish<MODE, DUAL><<<blocks, 256, 0, st>>>(g.M, g.N, batch, ksplit, scratch, p);
+    k_simt_finish<MODE, ACT, DUAL><<<blocks, 256, 0, st>>>(g.M, g.N, batch, ksplit, scratch, p);
   }
   VB_CUDA(cudaGetLastError());
   return VBNN_OK;
 }
 
-template <int MODE>
+template <int MODE, int ACT = EPI_ACT_RELU>
 static int launch_mode(const SimtGemmArgs& g, const EpiParams& p, int batch, cudaStream_t st) {
   constexpr bool DUAL = epi_is_dual(MODE);
   if (g.M <= 0 || g.N <= 0) return VBNN_OK;
@@ -222,11 +222,22 @@ static int launch_mode(const SimtGemmArgs& g, const EpiParams& p, int batch, cud
       if (pz.noise) pz.noise += z * p.zs_noise;
       if (pz.eps16) pz.eps16 = reinterpret_cast<const char*>(pz.eps16) + (long long)z * p.zs_e16 * 2;
       pz.accumulate = p.accumulate || z > 0;
-      VB_TRY(launch_one<MODE>(gz, pz, 1, st));
+      VB_TRY((launch_one<MODE, ACT>(gz, pz, 1, st)));
     }
     return VBNN_OK;
   }
-  return launch_one<MODE>(g, p, batch, st);
+  return launch_one<MODE, ACT>(g, p, batch, st);
+}
+
+// the FWD / DX modes: the kernel instantiation of the activation kind p.act
+template <int MODE>
+static int launch_act(const SimtGemmArgs& g, const EpiParams& p, int batch, cudaStream_t st) {
+  switch (epi_act_kernel(p.act)) {
+    case EPI_ACT_TANH: return launch_mode<MODE, EPI_ACT_TANH>(g, p, batch, st);
+    case EPI_ACT_SIGMOID: return launch_mode<MODE, EPI_ACT_SIGMOID>(g, p, batch, st);
+    case EPI_ACT_ELU: return launch_mode<MODE, EPI_ACT_ELU>(g, p, batch, st);
+  }
+  return launch_mode<MODE, EPI_ACT_RELU>(g, p, batch, st);
 }
 
 // A (m,k) / B (k,n) of a GemmOperand as a stride pair
@@ -257,10 +268,10 @@ int gemm_simt_launch(int mode, const GemmArgs& a, const EpiParams& p, cudaStream
   }
   switch (mode) {
     case EPI_STORE: return launch_mode<EPI_STORE>(g, p, batch, st);
-    case EPI_FWD: return launch_mode<EPI_FWD>(g, p, batch, st);
-    case EPI_FWD_LRT: return launch_mode<EPI_FWD_LRT>(g, p, batch, st);
-    case EPI_DX: return launch_mode<EPI_DX>(g, p, batch, st);
-    case EPI_DX_LRT: return launch_mode<EPI_DX_LRT>(g, p, batch, st);
+    case EPI_FWD: return launch_act<EPI_FWD>(g, p, batch, st);
+    case EPI_FWD_LRT: return launch_act<EPI_FWD_LRT>(g, p, batch, st);
+    case EPI_DX: return launch_act<EPI_DX>(g, p, batch, st);
+    case EPI_DX_LRT: return launch_act<EPI_DX_LRT>(g, p, batch, st);
     case EPI_DW: return launch_mode<EPI_DW>(g, p, batch, st);
     case EPI_DW_LRT: return launch_mode<EPI_DW_LRT>(g, p, batch, st);
   }

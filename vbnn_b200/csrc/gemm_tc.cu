@@ -344,7 +344,7 @@ __device__ __forceinline__ void load_operand(const CUtensorMap* tm, uint32_t dst
   }
 }
 
-template <int MODE, int BN, int CG, bool AK, bool BKM>
+template <int MODE, int ACT, int BN, int CG, bool AK, bool BKM>
 __global__ void __launch_bounds__(NTHREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__ CUtensorMap tmB1,
                const __grid_constant__ CUtensorMap tmA2, const __grid_constant__ CUtensorMap tmB2,
@@ -726,11 +726,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
           if (DUAL) tmem_ld32(t0 + BN + c * 32, v2);
           tmem_ld_wait();
           if (sh.staged && n0 + c * 32 + 32 <= sh.N) {
-            epi_chunk_staged<MODE>(p, ps, z, m0 + q * 32, lane, n0 + c * 32, v1, v2, my_stage);
+            epi_chunk_staged<MODE, ACT>(p, ps, z, m0 + q * 32, lane, n0 + c * 32, v1, v2, my_stage);
           } else {
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
-              epi_quad<MODE, bf16>(p, ps, z, row, n0 + c * 32 + j * 4,
+              epi_quad<MODE, ACT, bf16>(p, ps, z, row, n0 + c * 32 + j * 4,
                                    *reinterpret_cast<const float(*)[4]>(&v1[j * 4]),
                                    *reinterpret_cast<const float(*)[4]>(&v2[DUAL ? j * 4 : 0]));
             }
@@ -811,7 +811,7 @@ int make_tmap(CUtensorMap* tm, const GemmOperand& op, int rows_mn, int K, int ba
 
 struct TcChoice { int bn, cg; };   // bn == 64: multi-sample dW with register accumulation
 
-template <int MODE, int BN, int CG, bool AK, bool BKM>
+template <int MODE, int ACT, int BN, int CG, bool AK, bool BKM>
 int launch_cfg(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
   using C = TcCfg<MODE, BN, CG>;
   TcShape sh;
@@ -849,7 +849,7 @@ int launch_cfg(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
   } else {
     tA2 = tA1; tB2 = tB1;
   }
-  auto kern = gemm_tc_kernel<MODE, BN, CG, AK, BKM>;
+  auto kern = gemm_tc_kernel<MODE, ACT, BN, CG, AK, BKM>;
   static bool attr_set = false;
   if (!attr_set) {
     VB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
@@ -906,22 +906,33 @@ TcChoice choose_cfg(const GemmArgs& g) {
   return c2 <= c1 ? TcChoice{256, 2} : TcChoice{128, 1};
 }
 
-template <int MODE, bool AK, bool BKM>
+template <int MODE, bool AK, bool BKM, int ACT = EPI_ACT_RELU>
 int launch_any(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
   const TcChoice c = choose_cfg<MODE>(g);
   if constexpr (epi_z_accumulates(MODE)) {
-    if (c.bn == 64) return launch_cfg<MODE, 64, 1, AK, BKM>(g, p, st);
+    if (c.bn == 64) return launch_cfg<MODE, ACT, 64, 1, AK, BKM>(g, p, st);
     if constexpr (!epi_is_dual(MODE)) {
-      if (c.bn == 128 && c.cg == 2) return launch_cfg<MODE, 128, 2, AK, BKM>(g, p, st);
+      if (c.bn == 128 && c.cg == 2) return launch_cfg<MODE, ACT, 128, 2, AK, BKM>(g, p, st);
     }
   }
   if constexpr (epi_is_dual(MODE)) {
     // 256 x 128 pair tile: two accumulators use 256 TMEM columns, so the accumulator is double-buffered
-    if (c.cg == 2 && c.bn == 128) return launch_cfg<MODE, 128, 2, AK, BKM>(g, p, st);
+    if (c.cg == 2 && c.bn == 128) return launch_cfg<MODE, ACT, 128, 2, AK, BKM>(g, p, st);
   }
-  if (c.cg == 2) return launch_cfg<MODE, 256, 2, AK, BKM>(g, p, st);
-  if (c.bn == 256 && !epi_is_dual(MODE)) return launch_cfg<MODE, epi_is_dual(MODE) ? 128 : 256, 1, AK, BKM>(g, p, st);
-  return launch_cfg<MODE, 128, 1, AK, BKM>(g, p, st);
+  if (c.cg == 2) return launch_cfg<MODE, ACT, 256, 2, AK, BKM>(g, p, st);
+  if (c.bn == 256 && !epi_is_dual(MODE)) return launch_cfg<MODE, ACT, epi_is_dual(MODE) ? 128 : 256, 1, AK, BKM>(g, p, st);
+  return launch_cfg<MODE, ACT, 128, 1, AK, BKM>(g, p, st);
+}
+
+// the FWD / DX modes: the kernel instantiation of the activation kind p.act
+template <int MODE, bool AK, bool BKM>
+int launch_act(const GemmArgs& g, const EpiParams& p, cudaStream_t st) {
+  switch (epi_act_kernel(p.act)) {
+    case EPI_ACT_TANH: return launch_any<MODE, AK, BKM, EPI_ACT_TANH>(g, p, st);
+    case EPI_ACT_SIGMOID: return launch_any<MODE, AK, BKM, EPI_ACT_SIGMOID>(g, p, st);
+    case EPI_ACT_ELU: return launch_any<MODE, AK, BKM, EPI_ACT_ELU>(g, p, st);
+  }
+  return launch_any<MODE, AK, BKM, EPI_ACT_RELU>(g, p, st);
 }
 
 }  // namespace
@@ -940,22 +951,22 @@ int gemm_tc_launch(int mode, const GemmArgs& g, const EpiParams& p, cudaStream_t
       return launch_any<EPI_STORE, false, false>(g, p, st);
     case EPI_FWD:
       VB_CHECK(ak && bk, VBNN_E_INVALID, "EPI_FWD expects K-major operands");
-      return launch_any<EPI_FWD, true, true>(g, p, st);
+      return launch_act<EPI_FWD, true, true>(g, p, st);
     case EPI_FWD_LRT:
       VB_CHECK(ak && bk, VBNN_E_INVALID, "EPI_FWD_LRT expects K-major operands");
-      return launch_any<EPI_FWD_LRT, true, true>(g, p, st);
+      return launch_act<EPI_FWD_LRT, true, true>(g, p, st);
     case EPI_DX:
       VB_CHECK(ak && !bk, VBNN_E_INVALID, "EPI_DX expects K-major A, MN-major B");
-      return launch_any<EPI_DX, true, false>(g, p, st);
+      return launch_act<EPI_DX, true, false>(g, p, st);
     case EPI_DX_LRT:
       VB_CHECK(ak && !bk, VBNN_E_INVALID, "EPI_DX_LRT expects K-major A, MN-major B");
-      return launch_any<EPI_DX_LRT, true, false>(g, p, st);
+      return launch_act<EPI_DX_LRT, true, false>(g, p, st);
     case EPI_FWD_LRT2:
       VB_CHECK(ak && bk && p.aux, VBNN_E_INVALID, "EPI_FWD_LRT2 expects K-major operands and the mean product");
-      return launch_any<EPI_FWD_LRT2, true, true>(g, p, st);
+      return launch_act<EPI_FWD_LRT2, true, true>(g, p, st);
     case EPI_DX_LRT2:
       VB_CHECK(ak && !bk && p.aux, VBNN_E_INVALID, "EPI_DX_LRT2 expects K-major A, MN-major B and the H s2 product");
-      return launch_any<EPI_DX_LRT2, true, false>(g, p, st);
+      return launch_act<EPI_DX_LRT2, true, false>(g, p, st);
     case EPI_DW:
       VB_CHECK(!ak && !bk, VBNN_E_INVALID, "EPI_DW expects MN-major operands");
       return launch_any<EPI_DW, false, false>(g, p, st);

@@ -566,7 +566,7 @@ extern "C" int vbnn_layer_forward(vbnn_layer* L, const float* X, int N, float* Y
   memset(&p, 0, sizeof(p));
   p.M = N; p.N = L->O;
   p.out_f32 = Y; p.ld_f32 = L->O;
-  p.bias = L->bias; p.relu = 0;
+  p.bias = L->bias; p.act = EPI_ACT_NONE;         // nn.Linear: the caller runs the activation
   p.ld_act = L->ldO;
   int mode = EPI_FWD;
   if (lrt) {
@@ -610,7 +610,7 @@ extern "C" int vbnn_layer_backward_data(vbnn_layer* L, const float* X, const flo
   p.M = N; p.N = L->I;
   p.out_f32 = dX; p.ld_f32 = L->I;
   p.ld_act = L->ldI;
-  p.mask = 0;
+  p.act = EPI_ACT_NONE;
   const int mode = lrt ? EPI_DX_LRT : EPI_DX;
   GemmArgs g;
   memset(&g, 0, sizeof(g));

@@ -142,7 +142,7 @@ int forward_layer(vbnn_mlp* m, int j, int N, int Zrun, int sample0, bool map_mod
   memset(&p, 0, sizeof(p));
   p.M = N; p.N = L->O;
   p.bias = L->bias;
-  p.relu = last ? 0 : 1;
+  p.act = last ? EPI_ACT_NONE : 1 + m->activation;            // enum EpiAct from enum vbnn_activation
   p.ld_act = ldo; p.zs_act = (long long)N * ldo;
   if (last && m->ext_logits) {            // vbnn_mlp_forward_train: straight into the caller's dense [Z x N x C]
     p.out_f32 = m->ext_logits; p.ld_f32 = L->O; p.zs_f32 = (long long)N * L->O;
@@ -208,7 +208,7 @@ int loss_all(vbnn_mlp* m, int N, int Zrun, bool backward, float* logp_out, float
   return VBNN_OK;
 }
 
-// updateGradInput of layer j (its gradInput is layer j-1's gradOutput, ReLU backward fused)
+// updateGradInput of layer j (its gradInput is layer j-1's gradOutput, the activation's backward fused)
 int backward_data_layer(vbnn_mlp* m, int j, int N, int Zrun) {
   if (j == 0 && !m->dX) return VBNN_OK;
   vbnn_layer* L = m->layers[j];
@@ -227,12 +227,12 @@ int backward_data_layer(vbnn_mlp* m, int j, int N, int Zrun) {
   if (j > 0) {
     p.out_act = m->G[j - 1]; p.ld_act = ldi; p.zs_act = (long long)N * ldi;
     p.xprev = m->act[j]; p.ld_x = ldi; p.zs_x = (long long)N * ldi;
-    p.mask = 1;                                                    // nn.ReLU backward
+    p.act = 1 + m->activation;                                     // the activation's backward, from act[j]
     if (layer_is_lrt(m->layers[j - 1])) { p.rprev = m->R[j - 1]; p.out_act2 = m->H[j - 1]; }
   } else {
     // vbnn_mlp_step_grad_input: the first layer's gradInput summed over the Z samples, dX = sum_z dl_z/dX, written
     // straight into the caller's [N x I0] buffer by ONE GEMM whose contraction runs over the samples too (no atomics,
-    // no partials).  Nothing below the input: no ReLU mask.  The staged input act[0] is shared by every sample
+    // no partials).  Nothing below the input: no activation's derivative.  The staged input act[0] is shared by every sample
     // (zs_x = 0), so the LRT join is exact on the sums: sum_z (G_z mu + 2 X .* H_z s2) = (sum_z G_z) mu +
     // 2 X .* ((sum_z H_z) s2).
     g.zsum = 1;
@@ -1034,6 +1034,30 @@ extern "C" int vbnn_mlp_set_criterion(vbnn_mlp* m, int criterion) {
 extern "C" int vbnn_mlp_get_criterion(const vbnn_mlp* m, int* criterion) {
   VB_CHECK(m && criterion, VBNN_E_INVALID, "vbnn_mlp_get_criterion: null argument");
   *criterion = m->criterion;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_set_activation(vbnn_mlp* m, int activation) {
+  VB_CHECK(m, VBNN_E_INVALID, "vbnn_mlp_set_activation: null mlp");
+  VB_CHECK(activation >= VBNN_ACT_RELU && activation <= VBNN_ACT_ELU, VBNN_E_INVALID,
+           "vbnn_mlp_set_activation: unknown activation %d", activation);
+  VB_TRY(refuse_open_step(m, "vbnn_mlp_set_activation"));
+  VB_CHECK(m->inflight == 0, VBNN_E_STATE, "vbnn_mlp_set_activation: %d host-pipeline minibatch(es) not collected",
+           m->inflight);
+  VB_CUDA(cudaSetDevice(m->ctx->device));
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  VB_CUDA(cudaStreamIsCapturing(m->ctx->stream, &cs));
+  VB_CHECK(cs == cudaStreamCaptureStatusNone, VBNN_E_STATE,
+           "vbnn_mlp_set_activation: the context's stream is being captured (the step graphs bake the activation in)");
+  if (activation == m->activation) return VBNN_OK;
+  if (nlayers(m) > 1) mlp_drop_graphs(m);  // the hidden layers' FWD / DX GEMM kernels are baked into them
+  m->activation = activation;
+  return VBNN_OK;
+}
+
+extern "C" int vbnn_mlp_get_activation(const vbnn_mlp* m, int* activation) {
+  VB_CHECK(m && activation, VBNN_E_INVALID, "vbnn_mlp_get_activation: null argument");
+  *activation = m->activation;
   return VBNN_OK;
 }
 

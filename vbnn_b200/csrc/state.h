@@ -135,6 +135,7 @@ struct vbnn_mlp {
   // per-row log-sum-exp max / sum [2 x max_batch]
   float* mom_state = nullptr;
   int criterion = VBNN_CRIT_CLASS_NLL;    // vbnn_mlp_set_criterion
+  int activation = VBNN_ACT_RELU;         // vbnn_mlp_set_activation: every hidden layer's
   int tgt_cols = 1;                  // floats per row that targets / tstage hold: 1, or C once a regression criterion was set
   float* targets = nullptr;          // staged targets [N x target columns of the criterion]
   float* xstage[2] = {nullptr, nullptr};   // fp32 H2D staging for the host-buffer API

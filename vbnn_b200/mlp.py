@@ -47,6 +47,9 @@ class MLP:
         criterion = opt.get("criterion", "class_nll")
         if criterion not in L.CRITERIA:
             raise L.VbnnError(L.E_INVALID, f"opt.criterion must be one of {sorted(L.CRITERIA)}, got {criterion!r}")
+        activation = opt.get("activation", "relu")
+        if activation not in L.ACTIVATIONS:
+            raise L.VbnnError(L.E_INVALID, f"opt.activation must be one of {sorted(L.ACTIVATIONS)}, got {activation!r}")
         # a regression net may give its output width as opt.outputs instead of a list of classes
         n_out = int(opt["outputs"]) if criterion != "class_nll" and "outputs" in opt else len(opt["classes"])
         sizes = [int(opt["input_size"])] + [int(h) for h in opt["hidden"]] + [n_out]
@@ -77,6 +80,9 @@ class MLP:
         self.criterion = "class_nll"
         if criterion != "class_nll":
             self.set_criterion(criterion)
+        self.activation = "relu"
+        if activation != "relu":
+            self.set_activation(activation)
         return self
 
     def set_criterion(self, criterion):
@@ -90,6 +96,16 @@ class MLP:
             raise L.VbnnError(L.E_INVALID, f"criterion must be one of {sorted(L.CRITERIA)}, got {criterion!r}")
         L.check(L.lib().vbnn_mlp_set_criterion(self.handle, L.CRITERIA[criterion]))
         self.criterion = criterion
+
+    def set_activation(self, activation):
+        """The nonlinearity of every hidden layer (vbnn_mlp_set_activation), the one-word edit of mlp.lua:19,27: "relu"
+        (nn.ReLU, the default), "tanh" (nn.Tanh), "sigmoid" (nn.Sigmoid) or "elu" (nn.ELU, alpha 1).  The output layer
+        stays linear.  Every net-level entry point follows it; each step graph re-captures once at its next use.  Refused
+        while a forward_train step is open or host minibatches are uncollected.  Data parallel: set it on every rank."""
+        if activation not in L.ACTIVATIONS:
+            raise L.VbnnError(L.E_INVALID, f"activation must be one of {sorted(L.ACTIVATIONS)}, got {activation!r}")
+        L.check(L.lib().vbnn_mlp_set_activation(self.handle, L.ACTIVATIONS[activation]))
+        self.activation = activation
 
     def _target_cols(self):
         """targets per input row: 1 label (class_nll), C (mse) or C / 2 (gaussian_nll)"""
@@ -438,10 +454,10 @@ class MLP:
     # main.lua:146-148).  The reference torch.save()s the whole object graph; here the device state
     # is exported as a flat dict of CPU tensors (means, lvars, bias, Adam m/v/t per layer, the output
     # layer, the Philox step counter, each layer's live hyper-parameters "{k}.opts" in L.LIVE_OPTS
-    # order) that torch.save / numpy can persist.
+    # order, the hidden-layer "activation") that torch.save / numpy can persist.
     def state_dict(self):
         import torch
-        sd = {"sizes": list(self.sizes), "step": self.ctx.get_step()}
+        sd = {"sizes": list(self.sizes), "step": self.ctx.get_step(), "activation": self.activation}
         names = [("means", L.BUF_MEANS), ("lvars", L.BUF_LVARS), ("bias", L.BUF_BIAS), ("m_mu", L.BUF_ADAM_M_MU),
                  ("v_mu", L.BUF_ADAM_V_MU), ("m_var", L.BUF_ADAM_M_VAR), ("v_var", L.BUF_ADAM_V_VAR)]
         for k, m in enumerate(self.model):
@@ -469,6 +485,8 @@ class MLP:
     def load_state_dict(self, sd):
         if list(sd["sizes"]) != list(self.sizes):
             raise L.VbnnError(L.E_INVALID, f"checkpoint is for sizes {sd['sizes']}, net has {self.sizes}")
+        # the parameters were trained under this activation: the net takes it (a checkpoint without the key is ReLU)
+        self.set_activation(sd.get("activation", "relu"))
         codes = dict(means=L.BUF_MEANS, lvars=L.BUF_LVARS, bias=L.BUF_BIAS, m_mu=L.BUF_ADAM_M_MU, v_mu=L.BUF_ADAM_V_MU,
                      m_var=L.BUF_ADAM_M_VAR, v_var=L.BUF_ADAM_V_VAR, weight=L.BUF_WEIGHT, stdv=L.BUF_STDV,
                      mu_sqe=L.BUF_MU_SQE)
